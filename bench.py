@@ -2,11 +2,17 @@
 """Benchmark of the NeuMF train step (BASELINE.json metric: NCF train samples/sec) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ml-20m|ml-1m|large-sharded] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = the device negative sampler over the step's positives + one optimisation step (forward + BCE +
 backward + deterministic embedding-gradient reduction + legacy-Keras dense Adam + train-batch HR/DCG).  `value`
 includes the sampler, `value_excl_sampler` does not (SURVEY 8d).  N > 1 runs under torchrun, one rank per GPU, weak
 scaling (every rank has its own batch of the same size), gradients summed over NCCL.  Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` (ml-20m / ml-1m) writes what the last headline step computed as DIR/<name>.npy, so that two builds
+run with the same arguments (hence the same seeded inputs) can be compared output for output: the step outputs, the
+batch the device sampler drew, and the weights after the step (tables larger than DUMP_TABLE_ROWS rows as a fixed,
+seeded sample of rows, with the row ids beside them).
 
 `--impl reference` times the CPU restatement of the reference's Keras path (oracle/, NumPy fp32, all host threads
 BLAS will use) on a bounded sample of the same workload; TensorFlow is not installable here, so this is the "port"
@@ -370,6 +376,33 @@ def config_dict(args, wl, rows_override=None):
 # GPU arm
 # ---------------------------------------------------------------------------------------------------
 
+DUMP_TABLE_ROWS = 16384
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, step_out, batch, weights):
+    """--dump-outputs: the step outputs [loss_sum, hit_sum, dcg_sum, l2_penalty, bad_ids, ...] of the last headline
+    step, the (users, items, labels) batch the sampler drew for it, and the weights after it.  Ids are written as
+    float64 (exact).  Rows of a table taller than DUMP_TABLE_ROWS are a sample drawn with a generator seeded by the
+    table's height, so the user-side (and item-side) tables share one set of rows, stored as <table>.rows."""
+    arrays = {"step_out": np.asarray(step_out, np.float64)}
+    for name, t in zip(("batch_users", "batch_items", "batch_labels"), batch):
+        a = t.cpu().numpy()
+        arrays[name] = a.astype(np.float64 if a.dtype.kind in "iu" else np.float32)
+    for name, w in weights.items():
+        key = "weights." + name.replace("/", ".")
+        if w.ndim == 2 and w.shape[0] > DUMP_TABLE_ROWS:
+            rows = np.sort(np.random.default_rng(w.shape[0]).choice(w.shape[0], DUMP_TABLE_ROWS, replace=False))
+            arrays[key + ".rows"] = rows.astype(np.float64)
+            w = w[rows]
+        arrays[key] = np.ascontiguousarray(w, np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: {} bytes exceed the {}-byte limit".format(total, DUMP_MAX_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
 def refuse_diagnostics(args):
     """A bench value must come from the product build with no diagnostic switch: any MR_* environment variable
     (variant libraries via MR_LIB_PATH, MR_DP_OVERLAP, ...) makes the run a profiling run, allowed only with --lean."""
@@ -495,14 +528,22 @@ def run_gpu(args, wl):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()), last, prof
 
+    last_batch = [None]
+
+    def headline_step(i):
+        last_batch[0] = sample(args.warmup + i)
+        return train(*last_batch[0])
+
     for i in range(args.warmup):
         train(*sample(i))
     # ---- timed region 1 (the headline): sampler + train step, positives resident in HBM ---------------------------
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    ms_total, last, (phases, launches) = timed(lambda i: train(*sample(args.warmup + i)), args.steps, profile=True)
+    ms_total, last, (phases, launches) = timed(headline_step, args.steps, profile=True)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before region 2 trains the weights further
+        dump_outputs(args.dump_outputs, last.cpu().numpy(), last_batch[0], eng.get_weights())
     # ---- timed region 2: the train step alone on pre-sampled batches -----------------------------------------------
     ms_nosampler, _, _ = timed(lambda i: train(*resident[i % n_batches]), args.steps)
     value = global_rows * args.steps / (ms_total / 1e3)
@@ -858,7 +899,13 @@ def main():
     ap.add_argument("--workload", default="ml-20m", choices=sorted(WORKLOADS))
     ap.add_argument("--lean", action="store_true",
                     help="profiling runs (ncu): skip the e2e, eval and CPU-baseline legs; not a bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the step outputs, sampled batch and weights of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or WORKLOADS[args.workload].get("sharded")):
+        ap.error("--dump-outputs covers the replicated-table GPU workloads (ml-20m, ml-1m)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
     wl = WORKLOADS[args.workload]

@@ -1,9 +1,9 @@
 """Generate golden vectors by executing the REFERENCE's own Python source for the rank layer,
 ranking metrics and batch generator.
 
-Run in the build container only (needs /root/reference; the GPU box does not have it):
+Needs a checkout of the reference (carlamb/MovieRecommender-TF-TRT) and pandas; no GPU:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 TensorFlow is not installed, so the reference's `movierec/model.py` and `data_pipeline.py` are
 imported with a NumPy stand-in for the dozen `tf.python.keras.backend` calls they make
@@ -25,7 +25,6 @@ import types
 import numpy as np
 import pandas as pd
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -107,13 +106,14 @@ def _load(name, path):
     return m
 
 
-def main():
+def main(ref_root):
     _install_fake_tf()
-    sys.path.insert(0, os.path.join(REF, "movierec"))  # the reference imports `util.*` top-level
-    ref_model = _load("ref_model", os.path.join(REF, "movierec", "model.py"))
+    ref = os.path.abspath(ref_root)
+    sys.path.insert(0, os.path.join(ref, "movierec"))  # the reference imports `util.*` top-level
+    ref_model = _load("ref_model", os.path.join(ref, "movierec", "model.py"))
     if not hasattr(pd.Series, "append"):
         pd.Series.append = lambda self, other: pd.concat([self, other])
-    ref_dp = _load("ref_data_pipeline", os.path.join(REF, "movierec", "data_pipeline.py"))
+    ref_dp = _load("ref_data_pipeline", os.path.join(ref, "movierec", "data_pipeline.py"))
     K = _NumpyBackend
 
     # -- the stand-in must itself pass the reference's rank-layer test (test_model.py:168-190)
@@ -183,4 +183,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: python tests/golden/make_golden.py <reference checkout>")
+    main(sys.argv[1])

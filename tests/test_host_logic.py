@@ -73,12 +73,12 @@ def test_workspace_queries_are_host_only():
     assert nat.lib.mr_rank_eval_workspace_bytes(ctypes.byref(m), 1000, 100) >= 1000 * 100 * 4
 
 
-def test_compute_without_cuda_fails_loudly():
+def test_compute_without_cuda_fails_loudly(tmp_path):
     import torch
     if torch.cuda.is_available():
         pytest.skip("a GPU is present")
     with pytest.raises(RuntimeError, match="no CPU fallback"):
-        model.MovierecModel(copy.deepcopy(TEST_PARAMS), output_dir="/tmp/mr_test_models")
+        model.MovierecModel(copy.deepcopy(TEST_PARAMS), output_dir=str(tmp_path))
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         model.RankLayer(2, 3, "rank").call(np.array([0.9, 0.8, 0.7, 0.6]))
 
@@ -299,3 +299,36 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["e2e"] == {"value": line["value"], "unit": line["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["cpu_baseline"]["kind"] in ("port", "reference") and line["cpu_baseline"]["cores"] >= 1
     assert "ml-20m" in line["config"]["workload"] and line["config"]["baseline_config"] == "BASELINE.json configs[2]"
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float arrays only, ids exact, tall tables sampled on rows shared by the tables of one
+    side and the same in every run, the size limit enforced."""
+    import torch
+    import bench
+    rng = np.random.default_rng(0)
+    n = bench.DUMP_TABLE_ROWS + 5
+    w = {"user_embedding/embeddings": rng.random((n, 4), dtype=np.float32),
+         "gmf_user_embedding/embeddings": rng.random((n, 2), dtype=np.float32),
+         "hidden_1/kernel": rng.random((8, 4), dtype=np.float32)}
+    batch = (torch.tensor([3, 3, 7], dtype=torch.int32), torch.tensor([1, 2, 2 ** 24 + 1], dtype=torch.int32),
+             torch.tensor([0.0, 0.0, 1.0]))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), np.arange(8, dtype=np.float32), batch, w)
+    names = sorted(os.listdir(str(tmp_path / "a")))
+    assert names == sorted(os.listdir(str(tmp_path / "b")))
+    got = {f[:-4]: np.load(str(tmp_path / "a" / f)) for f in names}
+    for f in names:
+        assert got[f[:-4]].dtype in (np.float32, np.float64), f
+        np.testing.assert_array_equal(got[f[:-4]], np.load(str(tmp_path / "b" / f)))
+    assert got["batch_items"].tolist() == [1, 2, 2 ** 24 + 1] and got["step_out"].tolist() == list(range(8))
+    rows = got["weights.user_embedding.embeddings.rows"]
+    np.testing.assert_array_equal(rows, got["weights.gmf_user_embedding.embeddings.rows"])
+    assert len(np.unique(rows)) == bench.DUMP_TABLE_ROWS
+    np.testing.assert_array_equal(got["weights.user_embedding.embeddings"], w["user_embedding/embeddings"][rows.astype(int)])
+    np.testing.assert_array_equal(got["weights.hidden_1.kernel"], w["hidden_1/kernel"])
+    assert "weights.hidden_1.kernel.rows" not in got
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 1000)
+    with pytest.raises(SystemExit, match="limit"):
+        bench.dump_outputs(str(tmp_path / "c"), np.zeros(8), batch, w)
+    assert not (tmp_path / "c").exists()
