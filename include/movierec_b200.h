@@ -29,10 +29,11 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 100     /* major*100 + minor */
+#define MR_VERSION 101     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
+#define MR_MAX_TOPK 256    /* k of the catalogue top-k calls */
 
 typedef enum MrStatus {
   MR_OK = 0,
@@ -206,6 +207,34 @@ size_t mr_rank_scores_workspace_bytes(int64_t G);
 int mr_rank_scores(const float* scores, int64_t G, int32_t group, int32_t k, const int32_t* label_col,
                    const float* labels, int32_t* rank, int32_t* pos, float* sums, void* ws, size_t ws_bytes,
                    void* stream);
+
+/* Top-k selection on caller-supplied scores (the counterpart of mr_rank_scores for whole rows): scores is U x N
+ * row-major.  For row u the candidates are the items 0..N-1 minus the exclusion list of row r = excl_ids ? excl_ids[u]
+ * : u, i.e. excl_items[excl_rowptr[r] .. excl_rowptr[r+1]), sorted ascending as mr_build_user_csr writes it.  Rows
+ * r outside [0, excl_rows), ids outside [0, N) and excl_rowptr == NULL mean "nothing excluded".  Order: the RankLayer
+ * order (descending score, NaN as -inf, -0 == +0, the lower item id first among ties).
+ * targets (U, may be NULL): the target is never excluded; pos[u] = its 0-based place among the row's candidates (N
+ * for a target outside [0, N)); sums = {hit_sum, dcg_sum} over the U targets (hit = pos < k, dcg = ln2/ln(pos+2)*hit).
+ * pos and sums need targets.  top_items / top_scores (U x k, each may be NULL): the k best candidates in order;
+ * slots beyond the number of candidates hold item -1 and score NaN.  1 <= k <= MR_MAX_TOPK.  Deterministic (the
+ * selection compares distinct integer keys).  The workspace does not grow with U beyond one chunk of users. */
+size_t mr_topk_scores_workspace_bytes(int64_t U, int32_t N, int32_t k);
+int mr_topk_scores(const float* scores, int64_t U, int32_t N, int32_t k, const int32_t* excl_ids, int32_t excl_rows,
+                   const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
+                   float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream);
+
+/* The same for the model's probabilities of every (users[u], item) pair, item = 0..num_items-1: the K best unseen items
+ * of the whole catalogue per user, and leave-one-out HR / NDCG against every non-excluded item (no reference
+ * counterpart; the reference client scores one user x N candidates, trt_client.py:47-57).  Exclusion lists are indexed
+ * by user id.  scores (U x num_items, may be NULL) receives the probabilities.  Users are scored in chunks of about
+ * 2^22 rows with the launch sequence mr_rank_eval takes for the model, so a pair's probability is the one
+ * mr_rank_eval gives it when both take the same item projection.  An out-of-range user gets -1 / NaN rows and
+ * pos = num_items; an out-of-range target gets pos = num_items. */
+size_t mr_catalogue_topk_workspace_bytes(const MrModel* model, int64_t U, int32_t k);
+int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int32_t k, int32_t excl_rows,
+                      const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
+                      float* top_scores, int32_t* pos, float* sums, float* scores, void* ws, size_t ws_bytes,
+                      void* stream);
 
 /* On-device negative sampler -- replaces _get_random_negatives_and_positive
  * (data_pipeline.py:99-113): for positive p (global index first_index + p, user pos_users[p]) draw

@@ -574,11 +574,12 @@ static bool eval_fused_ok(const MrModel& m, int group) {
          group <= 256 && eval_sub_batch(group) > 0;
 }
 
-static TcWs carve_eval(const MrModel& m, int group, int64_t rows, void* ws) {
+// sb_rows > 0: rows per launch chosen by the caller (the catalogue sweep: whole users, no alignment rule)
+static TcWs carve_eval(const MrModel& m, int group, int64_t rows, void* ws, int64_t sb_rows = 0) {
   TcWs t{};
   Carver cv(ws);
-  int64_t sb = eval_sub_batch(group);
-  if (rows < sb) sb = (rows + 127) / 128 * 128;
+  int64_t sb = sb_rows > 0 ? sb_rows : eval_sub_batch(group);
+  if (sb_rows <= 0 && rows < sb) sb = (rows + 127) / 128 * 128;
   const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
   t.pack_fu = cv.take<float>((size_t)2 * d_u * m.L[1]);
   t.pack_fi = cv.take<float>((size_t)2 * d_i * m.L[1]);
@@ -592,16 +593,10 @@ static TcWs carve_eval(const MrModel& m, int group, int64_t rows, void* ws) {
   return t;
 }
 
-// users: one id per group; items: G * group, the positive last.  Forward with the user half of the first layer
-// once per user, then the fused score + position kernel.
-static int rank_eval_fused(const MrModel& m, const int32_t* users, const int32_t* items, int64_t G, int group, int k,
-                           int32_t* pos, float* probs, float* sums, int32_t* flags, float* partials, void* tc_ws,
-                           cudaStream_t st) {
-  const int64_t rows = G * group;
-  TcWs t = carve_eval(m, group, rows, tc_ws);
+// Once per eval call: the first layer's two halves and the later layers packed as MMA operands, and Pi when the
+// item projection is on.
+static int eval_prepare(const MrModel& m, const TcWs& t, cudaStream_t st) {
   const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
-  prof_mark(MR_PHASE_MISC, st);
-  MR_CUDA(cudaMemsetAsync(flags, 0, 256, st));
   int rc = launch_pack_weights(m.W[1], d_u, m.L[1], 0, t.pack_fu, st);
   if (rc == MR_OK) rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], d_i, m.L[1], 0, t.pack_fi, st);
   for (int l = 2; rc == MR_OK && l < m.n_layers; ++l) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, t.pack_f[l], st);
@@ -609,8 +604,21 @@ static int rank_eval_fused(const MrModel& m, const int32_t* users, const int32_t
   if (t.Pi != nullptr) {
     prof_mark(MR_PHASE_TC_DENSE_FWD, st);
     rc = tc_project_items(m, t, st);
-    if (rc != MR_OK) return rc;
   }
+  return rc;
+}
+
+// users: one id per group; items: G * group, the positive last.  Forward with the user half of the first layer
+// once per user, then the fused score + position kernel.
+static int rank_eval_fused(const MrModel& m, const int32_t* users, const int32_t* items, int64_t G, int group, int k,
+                           int32_t* pos, float* probs, float* sums, int32_t* flags, float* partials, void* tc_ws,
+                           cudaStream_t st) {
+  const int64_t rows = G * group;
+  TcWs t = carve_eval(m, group, rows, tc_ws);
+  prof_mark(MR_PHASE_MISC, st);
+  MR_CUDA(cudaMemsetAsync(flags, 0, 256, st));
+  int rc = eval_prepare(m, t, st);
+  if (rc != MR_OK) return rc;
   const int64_t sb = eval_sub_batch(group);
   for (int64_t r0 = 0; r0 < rows; r0 += sb) {
     const int64_t r1 = r0 + sb < rows ? r0 + sb : rows;
@@ -637,6 +645,51 @@ static int rank_eval_fused(const MrModel& m, const int32_t* users, const int32_t
   rc = launch_rank_metrics(pos, G, k, sums, partials, st);
   prof_mark(-1, st);
   return rc;
+}
+
+// ---- catalogue top-k: every user against every item, in chunks of whole users --------------------------------
+// Users per chunk: about kEvalSubBatchCap rows (the ranking eval's launch size), at least one user, and at most
+// kCatalogueMaxChunkUsers so that the selection's per-slice lists stay bounded when the catalogue is tiny.
+constexpr int64_t kCatalogueMaxChunkUsers = 16384;
+
+static int64_t catalogue_chunk_users(int32_t N) {
+  int64_t c = kEvalSubBatchCap / (N < 1 ? 1 : N);
+  if (c > kCatalogueMaxChunkUsers) c = kCatalogueMaxChunkUsers;
+  return c < 1 ? 1 : c;
+}
+
+// The scoring sequence of a chunk, the one mr_rank_eval takes for the model with each user as one group of width
+// num_items: the tensor-core tower with the projected first layer in the second layer's producers and the partial-
+// logit head (>= 3 layers), the default tower's projected tables, or the plain forward.  Decided on the full chunk
+// size so that the choice does not depend on how many users a call has.
+enum { CAT_TC = 0, CAT_SMALL = 1, CAT_FORWARD = 2 };
+static int catalogue_path(const MrModel& m) {
+  const int64_t rows = catalogue_chunk_users(m.num_items) * m.num_items;
+  if (use_tc(m) && m.n_layers >= 3 && catalogue_head_supported(m)) return CAT_TC;
+  if (small_eval_ok(m, rows)) return CAT_SMALL;
+  return CAT_FORWARD;
+}
+
+static size_t catalogue_scoring_bytes(const MrModel& m, int64_t C) {
+  const int64_t rows = C * m.num_items;
+  switch (catalogue_path(m)) {
+    case CAT_TC: return carve_eval(m, m.num_items, catalogue_chunk_users(m.num_items) * m.num_items, nullptr, rows).total;
+    case CAT_SMALL:
+      return align_up((size_t)m.num_items * m.L[1] * sizeof(float), 256) +
+             align_up((size_t)m.num_users * m.L[1] * sizeof(float), 256);
+    default: return mr_forward_workspace_bytes(&m, rows);
+  }
+}
+
+static int64_t clamp_users(int64_t U, int64_t C) { return U < 1 ? 1 : (U < C ? U : C); }
+
+static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const int64_t* excl_rowptr,
+                      const int32_t* excl_items, const int32_t* targets, const int32_t* pos, const float* sums) {
+  MR_REQUIRE(U >= 0 && N >= 1, "topk: bad U=%lld N=%d", (long long)U, N);
+  MR_REQUIRE(k >= 1 && k <= MR_MAX_TOPK, "topk: k=%d out of [1,%d]", k, MR_MAX_TOPK);
+  MR_REQUIRE(excl_rows >= 0 && (excl_rowptr == nullptr || excl_items != nullptr), "topk: bad exclusion lists");
+  MR_REQUIRE(targets != nullptr || (pos == nullptr && sums == nullptr), "topk: pos / sums need targets");
+  return MR_OK;
 }
 
 }  // namespace mr
@@ -1538,6 +1591,156 @@ int mr_rank_scores(const float* scores, int64_t G, int32_t group, int32_t k, con
   }
   return launch_rank_scores(scores, G, group, k, label_col, rank, pos, sums, static_cast<float*>(ws), (cudaStream_t)stream,
                             labels);
+}
+
+size_t mr_topk_scores_workspace_bytes(int64_t U, int32_t N, int32_t k) {
+  if (U < 0 || N < 1 || k < 1 || k > MR_MAX_TOPK) return 0;
+  return topk_workspace_bytes(clamp_users(U, catalogue_chunk_users(N)), N, k) + 256;
+}
+
+int mr_topk_scores(const float* scores, int64_t U, int32_t N, int32_t k, const int32_t* excl_ids, int32_t excl_rows,
+                   const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
+                   float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream) {
+  int rc = topk_check(U, N, k, excl_rows, excl_rowptr, excl_items, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (U == 0) {
+    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+    return MR_OK;
+  }
+  MR_REQUIRE(scores != nullptr && ws != nullptr, "topk_scores: scores / ws is NULL");
+  if (ws_bytes < mr_topk_scores_workspace_bytes(U, N, k)) {
+    set_error("topk_scores workspace too small: %zu < %zu", ws_bytes, mr_topk_scores_workspace_bytes(U, N, k));
+    return MR_ERR_WORKSPACE;
+  }
+  const int64_t C = catalogue_chunk_users(N);
+  TopkArgs a{};
+  a.N = N;
+  a.k = k;
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_items;
+  a.targets = targets;
+  a.top_items = top_items;
+  a.top_scores = top_scores;
+  a.pos = pos;
+  prof_mark(MR_PHASE_RANK, st);
+  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
+    a.u0 = u0;
+    a.U = U - u0 < C ? U - u0 : C;
+    a.scores = scores + u0 * N;
+    rc = launch_topk(a, ws, st);
+  }
+  if (rc == MR_OK) rc = launch_topk_metrics(pos, U, k, sums, st);
+  prof_mark(-1, st);
+  return rc;
+}
+
+size_t mr_catalogue_topk_workspace_bytes(const MrModel* model, int64_t U, int32_t k) {
+  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
+      model->num_users < 1 || U < 0 || k < 1 || k > MR_MAX_TOPK)
+    return 0;
+  const MrModel& m = *model;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(m.num_items));
+  const size_t rows = (size_t)C * m.num_items;
+  return align_up(rows * sizeof(int32_t), 256) + align_up(rows * sizeof(float), 256) +
+         align_up(topk_workspace_bytes(C, m.num_items, k), 256) + catalogue_scoring_bytes(m, C) + 512;
+}
+
+int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int32_t k, int32_t excl_rows,
+                      const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
+                      float* top_scores, int32_t* pos, float* sums, float* scores, void* ws, size_t ws_bytes,
+                      void* stream) {
+  int rc = check_model(model);
+  if (rc != MR_OK) return rc;
+  const MrModel& m = *model;
+  const int32_t N = m.num_items;
+  rc = topk_check(U, N, k, excl_rows, excl_rowptr, excl_items, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (U == 0) {
+    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+    return MR_OK;
+  }
+  MR_REQUIRE(users != nullptr && ws != nullptr, "catalogue_topk: users / ws is NULL");
+  if (ws_bytes < mr_catalogue_topk_workspace_bytes(model, U, k)) {
+    set_error("catalogue_topk workspace too small: %zu < %zu", ws_bytes, mr_catalogue_topk_workspace_bytes(model, U, k));
+    return MR_ERR_WORKSPACE;
+  }
+  const int64_t Cmax = catalogue_chunk_users(N);
+  const int64_t C = clamp_users(U, Cmax);
+  Carver cv(ws);
+  int32_t* iota = cv.take<int32_t>((size_t)C * N);
+  float* probs_buf = cv.take<float>((size_t)C * N);
+  const size_t topk_bytes = topk_workspace_bytes(C, N, k);
+  void* topk_ws = cv.take<char>(topk_bytes);
+  void* score_ws = static_cast<char*>(ws) + cv.off;
+  const int path = catalogue_path(m);
+  TcWs t{};
+  float *Pi = nullptr, *Pu = nullptr;
+  size_t fwd_bytes = 0;
+  prof_mark(MR_PHASE_MISC, st);
+  rc = launch_tile_iota(iota, C * N, N, st);
+  if (rc != MR_OK) return rc;
+  if (path == CAT_TC) {
+    t = carve_eval(m, N, Cmax * N, score_ws, C * N);
+    rc = eval_prepare(m, t, st);
+  } else if (path == CAT_SMALL) {  // Pi, Pu over the tables, as mr_rank_eval's default-tower path
+    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
+    Carver cs(score_ws);
+    Pi = cs.take<float>((size_t)m.num_items * L1);
+    Pu = cs.take<float>((size_t)m.num_users * L1);
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, Pi, st);
+    if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, m.W[1], L1, L1, false, m.b[1], Pu, st);
+  } else {
+    fwd_bytes = mr_forward_workspace_bytes(model, C * N);
+  }
+  TopkArgs a{};
+  a.N = N;
+  a.k = k;
+  a.excl_ids = users;  // exclusion lists are indexed by user id
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_items;
+  a.targets = targets;
+  a.users = users;
+  a.num_users = m.num_users;
+  a.top_items = top_items;
+  a.top_scores = top_scores;
+  a.pos = pos;
+  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
+    const int64_t c = U - u0 < C ? U - u0 : C;
+    const int64_t rows = c * N;
+    float* out = scores != nullptr ? scores + u0 * N : probs_buf;
+    if (path == CAT_TC) {
+      // each chunk starts at row 0 of its own users: one group = one user, Zu once per user
+      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+      rc = tc_forward_rows(m, t, users + u0, iota, 1, 0, rows, st, N, true, true);
+      if (rc == MR_OK) {
+        prof_mark(MR_PHASE_HEAD, st);
+        rc = launch_catalogue_head(m, t.H[m.n_layers - 1], users + u0, rows, N, out, st);
+      }
+    } else if (path == CAT_SMALL) {
+      prof_mark(MR_PHASE_FUSED_TILE, st);
+      rc = launch_small_tower_forward(m, Pi, Pu, users + u0, iota, rows, N, out, st);
+    } else {
+      rc = mr_neumf_forward(model, users + u0, iota, rows, N, nullptr, out, nullptr, nullptr, score_ws, fwd_bytes, stream);
+    }
+    if (rc != MR_OK) break;
+    prof_mark(MR_PHASE_RANK, st);
+    a.u0 = u0;
+    a.U = c;
+    a.scores = out;
+    rc = launch_topk(a, topk_ws, st);
+  }
+  if (rc == MR_OK) {
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_topk_metrics(pos, U, k, sums, st);
+  }
+  prof_mark(-1, st);
+  return rc;
 }
 
 int mr_sample_negatives(const int64_t* csr_rowptr, const int32_t* csr_items, int32_t num_items, const int32_t* pos_users,

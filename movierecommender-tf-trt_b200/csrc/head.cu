@@ -578,6 +578,28 @@ __global__ void __launch_bounds__(kHeadThreads, 2) head_rank_kernel(const HeadPa
   }
 }
 
+// Probability of one row of the partial-logit form, eight lanes per row: lane `sub` of the row's eight holds columns
+// 32 v + 4 sub .. + 3 of wu = w_out[:f] * (user GMF row) and of the item GMF row; z = the last hidden layer already
+// dotted with its output weights.  All 32 lanes must call it (the shuffles).  head_rank_warp_kernel and
+// catalogue_head_kernel both score through it, so a (user, item) pair gets bit-identical probabilities from the
+// sampled ranking eval and from the catalogue sweep.
+template <int NV>
+__device__ __forceinline__ float gmf_head_prob(const float4 (&wu)[NV], const float4 (&gi)[NV], float z, float b_out,
+                                               bool bad) {
+  float s = 0.f;
+#pragma unroll
+  for (int v = 0; v < NV; ++v) {
+    s = fmaf(wu[v].x, gi[v].x, s);
+    s = fmaf(wu[v].y, gi[v].y, s);
+    s = fmaf(wu[v].z, gi[v].z, s);
+    s = fmaf(wu[v].w, gi[v].w, s);
+  }
+  s += __shfl_xor_sync(0xffffffffu, s, 1);
+  s += __shfl_xor_sync(0xffffffffu, s, 2);
+  s += __shfl_xor_sync(0xffffffffu, s, 4);
+  return bad ? nanf("") : sigmoidf_stable(s + z + b_out);
+}
+
 // Score + position with ONE WARP PER GROUP, for the partial-logit form (p.h_last = one float per row: the last
 // hidden layer already dotted with its output-unit weights by tc_dense EPI_HEAD_DOT).  What is left per candidate
 // is the GMF term, a dot product of f = 32 * NV floats: eight lanes take one row (NV 128-bit loads each, 128
@@ -635,19 +657,8 @@ __global__ void __launch_bounds__(kHeadThreads) head_rank_warp_kernel(const Head
 #pragma unroll
       for (int k = 0; k < KS; ++k) {
         const int row = (s0 + k) * 4 + quad;
-        float s = 0.f;
-#pragma unroll
-        for (int v = 0; v < NV; ++v) {
-          s = fmaf(gu[v].x, gi[k][v].x, s);
-          s = fmaf(gu[v].y, gi[k][v].y, s);
-          s = fmaf(gu[v].z, gi[k][v].z, s);
-          s = fmaf(gu[v].w, gi[k][v].w, s);
-        }
-        s += __shfl_xor_sync(0xffffffffu, s, 1);
-        s += __shfl_xor_sync(0xffffffffu, s, 2);
-        s += __shfl_xor_sync(0xffffffffu, s, 4);
         const bool bad = bad_u || (unsigned)it[k] >= (unsigned)m.num_items;
-        const float pr = bad ? nanf("") : sigmoidf_stable(s + z[k] + b_out);
+        const float pr = gmf_head_prob<NV>(gu, gi[k], z[k], b_out, bad);
         if (sub == 0 && row < group) {
           my_sc[row] = pr;
           if (probs != nullptr) probs[p.row0 + lr0 + row] = pr;
@@ -662,6 +673,53 @@ __global__ void __launch_bounds__(kHeadThreads) head_rank_warp_kernel(const Head
     cnt = warp_sum_int(cnt);
     if (lane == 0) pos[gg] = cnt;
     __syncwarp();
+  }
+}
+
+// Catalogue sweep: the partial-logit form for `rows` rows where row r pairs users[r / group] with item r % group (one
+// user against the whole catalogue per `group` rows).  Row-parallel -- a group here is tens of thousands of rows, far
+// beyond the warp-per-group kernel's shared-memory slice -- with the per-row arithmetic of head_rank_warp_kernel
+// (gmf_head_prob).  Four rows per warp step, KS steps in flight.
+template <int NV>
+__global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrModel m, const float* __restrict__ h_dot,
+                                                                      const int32_t* __restrict__ users, int64_t rows,
+                                                                      int group, float* __restrict__ probs) {
+  constexpr int f = 32 * NV, KS = NV >= 4 ? 1 : 2;  // (KS = 4 spills at NV = 1 and needs 170 registers at NV = 4)
+  const int lane = threadIdx.x & 31;
+  const int sub = lane & 7, quad = lane >> 3;
+  float4 wg[NV];
+#pragma unroll
+  for (int v = 0; v < NV; ++v) wg[v] = ldg4(m.w_out + 32 * v + 4 * sub);
+  const float b_out = __ldg(m.b_out);
+  const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t r0 = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * (4 * KS); r0 < rows;
+       r0 += nwarps * (4 * KS)) {
+    float4 wu[KS][NV], gi[KS][NV];
+    float z[KS];
+    bool bad[KS];
+#pragma unroll
+    for (int k = 0; k < KS; ++k) {
+      int64_t row = r0 + 4 * k + quad;
+      if (row >= rows) row = rows - 1;  // dead slots re-read the last row
+      const int64_t slot = row / group;
+      const int it = (int)(row - slot * group);
+      int u = __ldg(users + slot);
+      bad[k] = (unsigned)u >= (unsigned)m.num_users;
+      if (bad[k]) u = 0;
+      z[k] = __ldg(h_dot + row);
+#pragma unroll
+      for (int v = 0; v < NV; ++v) {
+        const float4 x = ldg4(m.user_gmf + (size_t)u * f + 32 * v + 4 * sub);
+        wu[k][v] = make_float4(x.x * wg[v].x, x.y * wg[v].y, x.z * wg[v].z, x.w * wg[v].w);
+        gi[k][v] = ldg4(m.item_gmf + (size_t)it * f + 32 * v + 4 * sub);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < KS; ++k) {
+      const int64_t row = r0 + 4 * k + quad;
+      const float pr = gmf_head_prob<NV>(wu[k], gi[k], z[k], b_out, bad[k]);
+      if (sub == 0 && row < rows) probs[row] = pr;
+    }
   }
 }
 
@@ -785,11 +843,34 @@ int launch_head(const HeadArgs& a, cudaStream_t st) {
 
 bool head_rank_supported(const MrModel& m) { return m.mf_dim + m.L[m.n_layers - 1] <= 128; }
 
+bool catalogue_head_supported(const MrModel& m) {
+  const bool widths = m.mf_dim == 32 || m.mf_dim == 64 || m.mf_dim == 128;  // gmf_head_prob<1 | 2 | 4>
+  return widths && (reinterpret_cast<uintptr_t>(m.user_gmf) | reinterpret_cast<uintptr_t>(m.item_gmf) |
+                    reinterpret_cast<uintptr_t>(m.w_out)) % 16 == 0;
+}
+
 bool head_rank_takes_dot(const MrModel& m, int group) {
-  const bool widths = m.mf_dim == 32 || m.mf_dim == 64 || m.mf_dim == 128;  // head_rank_warp_kernel<1 | 2 | 4>
-  return widths && group >= 2 && group <= 256 &&
-         (reinterpret_cast<uintptr_t>(m.user_gmf) | reinterpret_cast<uintptr_t>(m.item_gmf) |
-          reinterpret_cast<uintptr_t>(m.w_out)) % 16 == 0;
+  return catalogue_head_supported(m) && group >= 2 && group <= 256;
+}
+
+int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t rows, int group,
+                          float* probs, cudaStream_t st) {
+  if (!catalogue_head_supported(m) || group < 1) {
+    set_error("catalogue head: needs mf_dim 32, 64 or 128 and 16-byte aligned GMF tables / output weights");
+    return MR_ERR_INVALID;
+  }
+  if (rows == 0) return MR_OK;
+  const int64_t want = (rows + 4 * (kHeadThreads / 32) - 1) / (4 * (kHeadThreads / 32));
+  const int64_t cap = (int64_t)sm_count() * 8;
+  const unsigned grid = (unsigned)(want < cap ? want : cap);
+  if (m.mf_dim == 32)
+    catalogue_head_kernel<1><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs);
+  else if (m.mf_dim == 64)
+    catalogue_head_kernel<2><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs);
+  else
+    catalogue_head_kernel<4><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs);
+  MR_LAUNCH_CHECK("catalogue_head_kernel");
+  return MR_OK;
 }
 
 // Fused score + rank of whole groups (forward only): a.users holds ONE id per group (global group index),

@@ -82,6 +82,30 @@ size_t rank_partials_count(int64_t G);
 int launch_rank_scores(const float* scores, int64_t G, int group, int k, const int32_t* label_col, int32_t* rank,
                        int32_t* pos, float* sums, float* partials, cudaStream_t st, const float* labels = nullptr);
 
+// ---- topk.cu: top-k selection over rows of scores with per-row exclusion lists ------------------------------
+struct TopkArgs {
+  const float* scores;  // the chunk's rows: U x N, row 0 = global row u0
+  int64_t U, u0;
+  int32_t N, k;
+  // every array below is indexed by the GLOBAL row u0 + u
+  const int32_t* excl_ids;  // exclusion list of row u = excl_ids[u] (NULL: u); lists outside [0, excl_rows) are empty
+  int32_t excl_rows;
+  const int64_t* excl_rowptr;
+  const int32_t* excl_items;
+  const int32_t* targets;   // NULL = no positions
+  const int32_t* users;     // optional: a row whose users[u] lies outside [0, num_users) gets -1 / NaN and pos = N
+  int32_t num_users;
+  int32_t* top_items;
+  float* top_scores;
+  int32_t* pos;
+};
+size_t topk_workspace_bytes(int64_t U, int32_t N, int32_t k);  // per chunk of U rows
+int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st);
+// sums = {hit_sum, dcg_sum} of pos[0, U) in a fixed order, no workspace
+int launch_topk_metrics(const int32_t* pos, int64_t U, int k, float* sums, cudaStream_t st);
+// out[r] = r % N for r < rows
+int launch_tile_iota(int32_t* out, int64_t rows, int32_t N, cudaStream_t st);
+
 // ---- sampler.cu ------------------------------------------------------------------------------
 int launch_sample_negatives(const int64_t* rowptr, const int32_t* csr_items, int32_t num_items,
                             const int32_t* pos_users, const int32_t* pos_items, int64_t P, int64_t first_index,
@@ -175,6 +199,11 @@ int launch_head(const HeadArgs& a, cudaStream_t st);
 bool head_rank_supported(const MrModel& m);
 bool head_rank_takes_dot(const MrModel& m, int group);  // launch_head_rank accepts h_is_dot for this model
 int launch_head_rank(const HeadArgs& a, int group, int32_t* pos, float* probs, cudaStream_t st);
+// catalogue sweep head: probs[r] from the partial logit h_dot[r] (tc_dense TC_EPI_HEAD_DOT) and the GMF term of
+// (users[r / group], item r % group), with the per-row arithmetic of launch_head_rank's partial-logit kernel
+bool catalogue_head_supported(const MrModel& m);
+int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t rows, int group,
+                          float* probs, cudaStream_t st);
 // metric sums from positions (rank.cu): sums = {hit_sum, dcg_sum}
 int launch_rank_metrics(const int32_t* pos, int64_t G, int k, float* sums, float* partials, cudaStream_t st);
 

@@ -517,6 +517,48 @@ class NeuMFEngine(object):
             self.last_eval_bad = self._ids_out_of_range(users, items)
         return pos, sums, rank, probs
 
+    def catalogue_topk(self, users, k, exclude=None, targets=None, want_scores=False):
+        """The k best items of the whole catalogue for each user (RankLayer order over the probabilities), minus the
+        user's exclusion list, and the place of a target item among the same candidates (mr_catalogue_topk).
+        exclude: None or (rowptr int64, items int32) -- per user id, an ascending item list (host or device).
+        Returns device tensors (items (U, k) int32, scores (U, k) float32, pos (U,) int32 or None, sums (2,) float32
+        [hit_sum, dcg_sum] or None, scores_full (U, num_items) float32 or None); pos / sums need targets.  Slots beyond
+        the number of candidates hold item -1 / score NaN.  Leaves in `self.last_catalogue_bad` a one-element device
+        tensor, non-zero when a user or target id was out of range (such a user's rows are -1 / NaN)."""
+        dev = self.device
+        users = as_device_i32(users, dev)
+        U = users.numel()
+        k = int(k)
+        t = as_device_i32(targets, dev) if targets is not None else None
+        if t is not None and t.numel() != U:
+            raise ValueError("targets ({}) and users ({}) differ in length".format(t.numel(), U))
+        rowptr = items = None
+        excl_rows = 0
+        if exclude is not None:
+            rp, it = exclude
+            rowptr = (rp if isinstance(rp, torch.Tensor) else torch.from_numpy(np.asarray(rp, dtype=np.int64)))
+            rowptr = rowptr.reshape(-1).to(dev, torch.int64).contiguous()
+            items = as_device_i32(it, dev)
+            if items.numel() == 0:  # every list empty: the library still wants a pointer
+                items = torch.zeros(1, dtype=torch.int32, device=dev)
+            excl_rows = max(rowptr.numel() - 1, 0)
+        top_items = torch.empty((U, k), dtype=torch.int32, device=dev)
+        top_scores = torch.empty((U, k), dtype=torch.float32, device=dev)
+        pos = torch.empty(U, dtype=torch.int32, device=dev) if t is not None else None
+        sums = torch.zeros(2, dtype=torch.float32, device=dev) if t is not None else None
+        full = torch.empty((U, self.num_items), dtype=torch.float32, device=dev) if want_scores else None
+        ws = self._workspace(max(int(nat.lib.mr_catalogue_topk_workspace_bytes(C.byref(self._model), U, k)), 256))
+        nat.check(nat.lib.mr_catalogue_topk(C.byref(self._model), _ptr(users), U, k, excl_rows, _ptr(rowptr), _ptr(items),
+                                            _ptr(t), _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(full),
+                                            _ptr(ws), ws.numel(), self._stream()), "mr_catalogue_topk")
+        bad = torch.zeros(1, dtype=torch.float32, device=dev)
+        if U:
+            bad = ((users.min() < 0) | (users.max() >= self.num_users)).to(torch.float32).reshape(1)
+            if t is not None:
+                bad = bad + ((t.min() < 0) | (t.max() >= self.num_items)).to(torch.float32).reshape(1)
+        self.last_catalogue_bad = bad
+        return top_items, top_scores, pos, sums, full
+
     def _ids_out_of_range(self, users, items):
         if users.numel() == 0:
             return torch.zeros(1, dtype=torch.float32, device=self.device)
@@ -625,6 +667,43 @@ def rank_scores(scores, group, k, label_col=None, want_rank=True, device=None, l
     nat.check(nat.lib.mr_rank_scores(_ptr(s), G, int(group), int(k), _ptr(lc), _ptr(lab), _ptr(rank), _ptr(pos), _ptr(sums),
                                      _ptr(ws), nbytes, st), "mr_rank_scores")
     return rank, pos, sums
+
+
+def topk_scores(scores, k, exclude=None, excl_ids=None, targets=None, device=None):
+    """Top-k of each row of a (U, N) score matrix in the RankLayer order, minus the row's exclusion list
+    (mr_topk_scores).  exclude: None or (rowptr int64, items int32); row u uses list excl_ids[u] (default u).
+    Returns device tensors (items (U, k) int32, scores (U, k) float32, pos (U,) int32 or None, sums (2,) or None)."""
+    require_cuda()
+    device = torch.device(device if device is not None else "cuda:{}".format(torch.cuda.current_device()))
+    s = scores if isinstance(scores, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(scores)))
+    if s.dim() != 2:
+        raise ValueError("scores must be (U, N), got shape {}".format(tuple(s.shape)))
+    U, N = int(s.shape[0]), int(s.shape[1])
+    s = s.to(device, torch.float32).contiguous()
+    k = int(k)
+    ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
+    t = as_device_i32(targets, device) if targets is not None else None
+    rowptr = items = None
+    excl_rows = 0
+    if exclude is not None:
+        rp, it = exclude
+        rowptr = (rp if isinstance(rp, torch.Tensor) else torch.from_numpy(np.asarray(rp, dtype=np.int64)))
+        rowptr = rowptr.reshape(-1).to(device, torch.int64).contiguous()
+        items = as_device_i32(it, device)
+        if items.numel() == 0:
+            items = torch.zeros(1, dtype=torch.int32, device=device)
+        excl_rows = max(rowptr.numel() - 1, 0)
+    top_items = torch.empty((U, k), dtype=torch.int32, device=device)
+    top_scores = torch.empty((U, k), dtype=torch.float32, device=device)
+    pos = torch.empty(U, dtype=torch.int32, device=device) if t is not None else None
+    sums = torch.zeros(2, dtype=torch.float32, device=device) if t is not None else None
+    nbytes = max(int(nat.lib.mr_topk_scores_workspace_bytes(U, N, k)), 256)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+    nat.check(nat.lib.mr_topk_scores(_ptr(s), U, N, k, _ptr(ids), excl_rows, _ptr(rowptr), _ptr(items), _ptr(t),
+                                     _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(ws), nbytes, st),
+              "mr_topk_scores")
+    return top_items, top_scores, pos, sums
 
 
 def gather_rows(table, idx):

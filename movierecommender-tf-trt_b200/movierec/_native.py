@@ -12,6 +12,7 @@ import os
 MR_MAX_LAYERS = 8
 MR_MAX_WIDTH = 1024
 MR_MAX_NEGS = 1023
+MR_MAX_TOPK = 256
 MR_STEP_OUT_FLOATS = 8
 OUT_LOSS_SUM, OUT_HIT_SUM, OUT_DCG_SUM, OUT_L2_PENALTY, OUT_BAD_IDS = 0, 1, 2, 3, 4
 TRAIN_USERS_GROUPED = 1  # MR_TRAIN_USERS_GROUPED
@@ -85,6 +86,10 @@ SIGNATURES = {
     "mr_rank_eval": (C.c_int, [_PM, _vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_rank_scores_workspace_bytes": (_sz, [_i64]),
     "mr_rank_scores": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mr_topk_scores_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "mr_topk_scores": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mr_catalogue_topk_workspace_bytes": (_sz, [_PM, _i64, _i32]),
+    "mr_catalogue_topk": (C.c_int, [_PM, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_sample_negatives": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i64, _i32, _u64, _u64, _vp, _vp, _vp, _vp]),
     "mr_sort_workspace_bytes": (_sz, [_i64]),
     "mr_sort_pairs": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _sz, _vp]),

@@ -124,6 +124,13 @@ class MovieLensDataGenerator(object):
             d[key] = int((below[rp[1:]] - below[rp[:-1]]).max().item()) if rp.numel() > 1 else 0
         return d[key]
 
+    def user_item_lists(self):
+        """(rowptr int64, items int32) device tensors: per user, the ascending distinct items of data ∪ extra_data --
+        the items the sampler never draws as negatives, and the exclusion lists of a full-catalogue evaluation."""
+        if self._device is None:
+            self._upload()
+        return self._device["rowptr"], self._device["csr"]
+
     def device_batch(self, idx):
         """Batch `idx` as device tensors ([x_user int32, x_item int32], y float32), layout of the
         reference's __getitem__ (:136-150): users repeated, negatives first, positive last."""

@@ -167,6 +167,17 @@ class NeuMFModel(object):
         p = probs.cpu().numpy()
         return items[order], p[order]
 
+    def recommend_for_users(self, users, top_k=10, exclude=None):
+        """The top_k best items of the WHOLE catalogue for each of `users` (RankLayer order: descending score, the
+        lower item id first among ties), leaving out each user's exclusion list.  exclude: None, a
+        MovieLensDataGenerator (the items its sampler never draws for the user: data ∪ extra_data) or a
+        (rowptr, items) pair of ascending per-user lists.  Returns NumPy (items (U, top_k) int32, scores (U, top_k)
+        float32); slots beyond the number of candidates hold -1 / NaN.  One device call for all users."""
+        eng = self.engine
+        items, scores, _, _, _ = eng.catalogue_topk(users, top_k, exclude=_exclusion_lists(exclude))
+        self._raise_on_bad_ids(float(eng.last_catalogue_bad.item()))
+        return items.cpu().numpy(), scores.cpu().numpy()
+
     def _step_logs(self, out, rows, group):
         loss = out[0] / rows + out[3]
         return {"loss": loss, OUTPUT_PRED + "_loss": out[0] / rows,
@@ -571,6 +582,30 @@ class MovierecModel(object):
         self.model._raise_on_bad_ids(s[2])
         G = max(int(pos.numel()), 1)
         return s[0] / G, s[1] / G
+
+    def evaluate_full_catalogue(self, users, items, exclude=None, k=None):
+        """Leave-one-out ranking evaluation against ALL items (no sampled negatives): for user users[g], the held-out
+        item items[g] is ranked among every item not in the user's exclusion list (the held-out item itself always
+        counts).  exclude: as NeuMFModel.recommend_for_users -- typically the training generator, whose lists hold
+        every item the user has already rated.  Returns (hr, ndcg) at k (default: the model's k), like evaluate()."""
+        k = self._k if k is None else k
+        import torch
+        eng = self.model.engine
+        _, _, pos, sums, _ = eng.catalogue_topk(users, k, exclude=_exclusion_lists(exclude), targets=items)
+        s = torch.cat([sums.reshape(-1), eng.last_catalogue_bad.to(sums.dtype)]).cpu().numpy().astype(np.float64)
+        self.model._raise_on_bad_ids(s[2])
+        G = max(int(pos.numel()), 1)
+        return s[0] / G, s[1] / G
+
+
+def _exclusion_lists(exclude):
+    """None | MovieLensDataGenerator | (rowptr, items) -> None | (rowptr, items)."""
+    if exclude is None:
+        return None
+    if hasattr(exclude, "user_item_lists"):
+        return exclude.user_item_lists()
+    rowptr, items = exclude
+    return rowptr, items
 
 
 class RankLayer(object):
