@@ -142,7 +142,8 @@ enum { MR_OUT_LOSS_SUM = 0, /* sum over rows of BCE (model.py:213-215), unscaled
        MR_OUT_HIT_SUM = 1,  /* sum over groups of hit@k  (model.py:454) */
        MR_OUT_DCG_SUM = 2,  /* sum over groups of ln2/ln(pos+2)*hit (model.py:414-415) */
        MR_OUT_L2_PENALTY = 3, /* sum of l2 regulariser terms (0 when all l2 == 0) */
-       MR_OUT_BAD_IDS = 4,  /* bit 0: a user/item id was out of range (row skipped); bit 1: MR_TRAIN_USERS_GROUPED
+       MR_OUT_BAD_IDS = 4,  /* bit 0: a user/item id was out of range (row skipped: the step is what it would be
+                               with any other out-of-range id there); bit 1: MR_TRAIN_USERS_GROUPED
                                was passed but some row's user differs from its group's first row (step invalid) */
        MR_STEP_OUT_FLOATS = 8 };
 
@@ -253,14 +254,18 @@ int mr_sample_negatives(const int64_t* csr_rowptr, const int32_t* csr_items, int
  * shards is a DEVICE array of `world` pointers to the ranks' slices (each (ceil(total_rows/world), dim) fp32 in the
  * owning GPU's memory, mapped into this process through NVLink peer access -- e.g. torch symmetric memory).
  * out[i,:] = row ids[i] (NaN for an out-of-range id).  This one kernel is the gather AND the exchange of the
- * gathered rows of a row-sharded step.  The caller orders it against the owners' updates (a cross-rank barrier). */
+ * gathered rows of a row-sharded step.  The caller orders it against the owners' updates (a cross-rank barrier).
+ * Precondition (not checked): every shard base is 16-byte aligned -- allocation starts are; when dim % 4 == 0 and out
+ * is 16-byte aligned the rows are read as float4. */
 int mr_gather_rows_sharded(const float* const* shards, int32_t world, int64_t total_rows, int32_t dim,
                            const int32_t* ids, int64_t n, float* out, void* stream);
 
 /* Owner-side update of ROW-SHARDED tables (data-parallel runs whose tables do not fit one GPU): n pairs
  * (local row id, gradient row [g0 | g1]) received from all ranks, duplicates allowed.  The pairs are
- * stably sorted by row id, summed per id in arrival order (deterministic, no atomics) and the sparse-row
- * Adam / SGD update is applied to table0 (num_rows x d0) and table1 (num_rows x d1; d1 may be 0).
+ * stably sorted by row id and summed per id by a tree over 32-entry chunks of the sorted list, whose order depends
+ * only on the positions of the pairs (deterministic, no atomics); then the sparse-row Adam / SGD update is applied
+ * once per id to table0 (num_rows x d0) and table1 (num_rows x d1; d1 may be 0).  Ids outside [0, num_rows) are
+ * ignored: no row changes for them, and the other ids' rows are updated exactly as without them.
  * lr_t is Adam's bias-corrected step size lr*sqrt(1-b2^t)/(1-b1^t) for the current step. */
 size_t mr_sparse_rows_workspace_bytes(int64_t n, int32_t d0, int32_t d1);
 int mr_sparse_rows_update(float* table0, float* m0, float* v0, int32_t d0, float* table1, float* m1, float* v1,
@@ -337,6 +342,7 @@ int mr_sort_pairs(const int32_t* keys, int64_t n, int32_t key_bits, int32_t* sor
  * new weights as one kernel over NVLink peer memory.  grad_peers / param_peers are HOST arrays of `world` device
  * pointers: rank r's flat gradient buffer and flat parameter buffer (same layout on every rank, 16-byte aligned,
  * mapped into this process by peer access -- e.g. torch symmetric memory; entry `rank` is this rank's own buffer).
+ * world is 1..8 or 16; m and v (Adam) are 16-byte aligned too.  Violations return MR_ERR_INVALID before any launch.
  * For the elements [lo, hi) this rank owns (multiples of 4):
  *     g = grad_peers[0][i] + grad_peers[1][i] + ... (rank order, the same on every rank) + 2*l2*p[i]
  *     Adam / SGD step of mr_optimizer_flat with THIS rank's m[i], v[i] (optimizer state is sharded by owner)

@@ -121,10 +121,19 @@ __global__ void flag_to_float_kernel(const int32_t* flags, float* out) {
   *out = (float)((flags[0] ? 1 : 0) | (flags[1] ? 2 : 0));
 }
 
-static int bits_for(int32_t n) {
+static int bits_for(int64_t n) {
   int b = 1;
   while (b < 31 && ((int64_t)1 << b) < n) ++b;
   return b;
+}
+
+// Sort of the row ids that key a segmented reduction over a table of num_rows rows: ids outside [0, num_rows) sort as
+// the sentinel num_rows (one value more than the valid ids, hence bits_for(num_rows + 1)), after every valid id, so
+// they can never split a valid id's run; the reduction skips the sentinel's run.
+static int sort_row_ids(const int32_t* ids, int64_t n, int32_t num_rows, int32_t* sorted_keys, int32_t* sorted_index,
+                        void* ws, size_t ws_bytes, cudaStream_t st) {
+  return launch_sort_pairs(ids, n, bits_for((int64_t)num_rows + 1), sorted_keys, sorted_index, ws, ws_bytes, st,
+                           num_rows);
 }
 
 static int check_model(const MrModel* m) {
@@ -901,11 +910,10 @@ int mr_neumf_train_grads(MrModel* model, MrOptState* opt, MrGrads* grads, const 
       if (rc == MR_OK) rc = launch_group_heads(users, B / group, group, t.group_users, ss);
       if (rc != MR_OK) return rc;
     }
-    rc = launch_sort_pairs(by_group ? t.group_users : users, n_user_rows, bits_for(m.num_users), t.sorted_keys,
-                           t.sorted_index, t.sort_ws, t.sort_ws_bytes, ss);
+    rc = sort_row_ids(by_group ? t.group_users : users, n_user_rows, m.num_users, t.sorted_keys, t.sorted_index,
+                      t.sort_ws, t.sort_ws_bytes, ss);
     if (rc == MR_OK)
-      rc = launch_sort_pairs(items, B, bits_for(m.num_items), t.sorted_keys_i, t.sorted_index_i, t.sort_ws,
-                             t.sort_ws_bytes, ss);
+      rc = sort_row_ids(items, B, m.num_items, t.sorted_keys_i, t.sorted_index_i, t.sort_ws, t.sort_ws_bytes, ss);
     if (rc != MR_OK) return rc;
     if (side != nullptr) MR_CUDA(cudaEventRecord(side->join, ss));
     prof_mark(MR_PHASE_MISC, st);
@@ -1789,7 +1797,7 @@ int mr_sparse_rows_update(float* table0, float* m0, float* v0, int32_t d0, float
   const size_t seg_bytes = segreduce_workspace_bytes(n, d0 + d1);
   void* seg_ws = cv.take<char>(seg_bytes);
   prof_mark(MR_PHASE_SORT, st);
-  int rc = launch_sort_pairs(row_ids, n, bits_for(num_rows), skeys, sidx, sort_ws, sort_bytes, st);
+  int rc = sort_row_ids(row_ids, n, num_rows, skeys, sidx, sort_ws, sort_bytes, st);
   if (rc != MR_OK) return rc;
   RowUpdate u{};
   u.mode = MR_TABLES_SPARSE;
@@ -1910,9 +1918,13 @@ int mr_dp_reduce_apply(const float* const* grad_peers, float* const* param_peers
                        float* v, int64_t lo, int64_t hi, int32_t optimizer, float lr_t, float beta_1, float beta_2,
                        float epsilon, float l2, const float* grad_multicast, float* param_multicast, void* stream) {
   MR_REQUIRE(grad_peers && param_peers, "dp_reduce_apply: NULL pointer array");
-  MR_REQUIRE(world >= 1 && rank >= 0 && rank < world, "dp_reduce_apply: rank %d of %d", rank, world);
+  MR_REQUIRE((world >= 1 && world <= 8) || world == 16, "dp_reduce_apply: world size %d (1..8 or 16 ranks of one box)",
+             world);
+  MR_REQUIRE(rank >= 0 && rank < world, "dp_reduce_apply: rank %d of %d", rank, world);
   MR_REQUIRE(lo >= 0 && hi >= lo && (lo & 3) == 0 && (hi & 3) == 0, "dp_reduce_apply: [lo, hi) must be multiples of 4");
   MR_REQUIRE(optimizer == MR_OPT_SGD || (m && v), "dp_reduce_apply: Adam needs m and v");
+  MR_REQUIRE(optimizer == MR_OPT_SGD || ((reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v)) & 15) == 0,
+             "dp_reduce_apply: m and v must be 16-byte aligned");
   for (int r = 0; r < world; ++r)
     MR_REQUIRE(grad_peers[r] && param_peers[r] && ((reinterpret_cast<uintptr_t>(grad_peers[r]) |
                                                      reinterpret_cast<uintptr_t>(param_peers[r])) & 15) == 0,

@@ -74,6 +74,19 @@ __device__ __forceinline__ float4 ld_stream4(const float* p) {
   return r;
 }
 
+// One element of the dense optimizer sweeps (legacy-Keras Adam, SGD, the l2 gradient term) with every rounding
+// spelled out.  Left to itself the compiler contracts a * b + c into FMAs differently in each loop, so the vector and
+// scalar paths of the flat sweep and the data-parallel exchange kernel used to differ in the last bit; with these
+// they compute the same bits for the same inputs.
+__device__ __forceinline__ void adam_step(float& p, float g, float& m, float& v, float lr_t, float b1, float b2,
+                                          float eps) {
+  m = __fmaf_rn(b1, m, __fmul_rn(1.f - b1, g));
+  v = __fmaf_rn(b2, v, __fmul_rn(__fmul_rn(1.f - b2, g), g));
+  p = __fsub_rn(p, __fdiv_rn(__fmul_rn(lr_t, m), __fadd_rn(__fsqrt_rn(v), eps)));
+}
+__device__ __forceinline__ float sgd_step(float p, float g, float lr) { return __fmaf_rn(-lr, g, p); }
+__device__ __forceinline__ float plus_l2(float g, float p, float c2) { return __fmaf_rn(c2, p, g); }  // g + 2 l2 p
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

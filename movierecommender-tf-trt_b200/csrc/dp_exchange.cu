@@ -31,12 +31,13 @@ struct DpPeers {
   float* p[kDpMaxWorld];
 };
 
+// the element arithmetic of mr_optimizer_flat (common.cuh): the exchange's step is bit-identical to the flat sweep's
 __device__ __forceinline__ void adam4(float4& p, const float4& g, float4& m, float4& v, float lr_t, float b1, float b2,
                                       float eps) {
-  m.x = b1 * m.x + (1.f - b1) * g.x; v.x = b2 * v.x + (1.f - b2) * g.x * g.x; p.x = p.x - lr_t * m.x / (sqrtf(v.x) + eps);
-  m.y = b1 * m.y + (1.f - b1) * g.y; v.y = b2 * v.y + (1.f - b2) * g.y * g.y; p.y = p.y - lr_t * m.y / (sqrtf(v.y) + eps);
-  m.z = b1 * m.z + (1.f - b1) * g.z; v.z = b2 * v.z + (1.f - b2) * g.z * g.z; p.z = p.z - lr_t * m.z / (sqrtf(v.z) + eps);
-  m.w = b1 * m.w + (1.f - b1) * g.w; v.w = b2 * v.w + (1.f - b2) * g.w * g.w; p.w = p.w - lr_t * m.w / (sqrtf(v.w) + eps);
+  adam_step(p.x, g.x, m.x, v.x, lr_t, b1, b2, eps);
+  adam_step(p.y, g.y, m.y, v.y, lr_t, b1, b2, eps);
+  adam_step(p.z, g.z, m.z, v.z, lr_t, b1, b2, eps);
+  adam_step(p.w, g.w, m.w, v.w, lr_t, b1, b2, eps);
 }
 
 // NVSwitch multicast (NVLS): one load that the switch answers with the SUM of the word in every replica of a
@@ -97,14 +98,16 @@ __global__ void __launch_bounds__(kDpThreads) dp_reduce_apply_kernel(const DpPee
       const int64_t i = i0 + u * nth;
       if (i < hi4) {
         if (l2 != 0.f) {
-          g[u].x += c2 * pv[u].x; g[u].y += c2 * pv[u].y; g[u].z += c2 * pv[u].z; g[u].w += c2 * pv[u].w;
+          g[u].x = plus_l2(g[u].x, pv[u].x, c2); g[u].y = plus_l2(g[u].y, pv[u].y, c2);
+          g[u].z = plus_l2(g[u].z, pv[u].z, c2); g[u].w = plus_l2(g[u].w, pv[u].w, c2);
         }
         if (ADAM) {
           adam4(pv[u], g[u], mv[u], vv[u], lr_t, b1, b2, eps);
           reinterpret_cast<float4*>(m)[i] = mv[u];
           reinterpret_cast<float4*>(v)[i] = vv[u];
         } else {
-          pv[u].x -= lr_t * g[u].x; pv[u].y -= lr_t * g[u].y; pv[u].z -= lr_t * g[u].z; pv[u].w -= lr_t * g[u].w;
+          pv[u].x = sgd_step(pv[u].x, g[u].x, lr_t); pv[u].y = sgd_step(pv[u].y, g[u].y, lr_t);
+          pv[u].z = sgd_step(pv[u].z, g[u].z, lr_t); pv[u].w = sgd_step(pv[u].w, g[u].w, lr_t);
         }
         if (WORLD == 0) {
           multimem_st(mc_p + i, pv[u]);

@@ -40,8 +40,11 @@ int launch_gather_rows(const float* table, int64_t rows, int dim, const int32_t*
 
 // ---- radix_sort.cu ---------------------------------------------------------------------------
 size_t sort_workspace_bytes(int64_t n);
+// num_rows >= 0: every key outside [0, num_rows) is replaced by the sentinel num_rows as it is loaded (out_keys then
+// holds the sentinel), so an out-of-range id sorts after all valid ids instead of among the valid id that shares its
+// low key_bits bits.  key_bits must then cover num_rows itself.
 int launch_sort_pairs(const int32_t* keys, int64_t n, int key_bits, int32_t* out_keys, int32_t* out_index,
-                      void* ws, size_t ws_bytes, cudaStream_t st);
+                      void* ws, size_t ws_bytes, cudaStream_t st, int32_t num_rows = -1);
 
 // ---- segreduce.cu ----------------------------------------------------------------------------
 struct RowUpdate {       // what to do with each reduced row gradient

@@ -2,17 +2,11 @@
 // App. A-4):  Adam  m = b1*m + (1-b1)*g ; v = b2*v + (1-b2)*g^2 ; p -= lr_t * m / (sqrt(v) + eps)
 // with lr_t = lr*sqrt(1-b2^t)/(1-b1^t) computed on the host;  SGD  p -= lr*g.
 // `l2` adds the regulariser gradient 2*l2*p (embedding tables with layers_l2reg[0] != 0).
+// Every path computes an element with common.cuh's adam_step / sgd_step / plus_l2: the same bits whatever the path.
 // HBM-bound: 28 bytes per element (read p,g,m,v; write p,m,v); 128-bit accesses, grid-stride.
 #include "launchers.h"
 
 namespace mr {
-
-__device__ __forceinline__ void adam1(float& p, float g, float& m, float& v, float lr_t, float b1, float b2,
-                                      float eps) {
-  m = b1 * m + (1.f - b1) * g;
-  v = b2 * v + (1.f - b2) * g * g;
-  p = p - lr_t * m / (sqrtf(v) + eps);
-}
 
 template <bool ADAM>
 __global__ void __launch_bounds__(256) optimizer_flat_kernel(float* __restrict__ p, const float* __restrict__ g,
@@ -28,32 +22,34 @@ __global__ void __launch_bounds__(256) optimizer_flat_kernel(float* __restrict__
       float4 pv = reinterpret_cast<float4*>(p)[i];
       float4 gv = reinterpret_cast<const float4*>(g)[i];
       if (l2 != 0.f) {
-        gv.x += c2 * pv.x; gv.y += c2 * pv.y; gv.z += c2 * pv.z; gv.w += c2 * pv.w;
+        gv.x = plus_l2(gv.x, pv.x, c2); gv.y = plus_l2(gv.y, pv.y, c2);
+        gv.z = plus_l2(gv.z, pv.z, c2); gv.w = plus_l2(gv.w, pv.w, c2);
       }
       if (ADAM) {
         float4 mv = reinterpret_cast<float4*>(m)[i];
         float4 vv = reinterpret_cast<float4*>(v)[i];
-        adam1(pv.x, gv.x, mv.x, vv.x, lr_t, b1, b2, eps);
-        adam1(pv.y, gv.y, mv.y, vv.y, lr_t, b1, b2, eps);
-        adam1(pv.z, gv.z, mv.z, vv.z, lr_t, b1, b2, eps);
-        adam1(pv.w, gv.w, mv.w, vv.w, lr_t, b1, b2, eps);
+        adam_step(pv.x, gv.x, mv.x, vv.x, lr_t, b1, b2, eps);
+        adam_step(pv.y, gv.y, mv.y, vv.y, lr_t, b1, b2, eps);
+        adam_step(pv.z, gv.z, mv.z, vv.z, lr_t, b1, b2, eps);
+        adam_step(pv.w, gv.w, mv.w, vv.w, lr_t, b1, b2, eps);
         reinterpret_cast<float4*>(m)[i] = mv;
         reinterpret_cast<float4*>(v)[i] = vv;
       } else {
-        pv.x -= lr_t * gv.x; pv.y -= lr_t * gv.y; pv.z -= lr_t * gv.z; pv.w -= lr_t * gv.w;
+        pv.x = sgd_step(pv.x, gv.x, lr_t); pv.y = sgd_step(pv.y, gv.y, lr_t);
+        pv.z = sgd_step(pv.z, gv.z, lr_t); pv.w = sgd_step(pv.w, gv.w, lr_t);
       }
       reinterpret_cast<float4*>(p)[i] = pv;
     }
     for (int64_t i = (n4 << 2) + tid; i < n; i += nth) {
-      float gi = g[i] + (l2 != 0.f ? c2 * p[i] : 0.f);
-      if (ADAM) adam1(p[i], gi, m[i], v[i], lr_t, b1, b2, eps);
-      else p[i] -= lr_t * gi;
+      const float gi = l2 != 0.f ? plus_l2(g[i], p[i], c2) : g[i];
+      if (ADAM) adam_step(p[i], gi, m[i], v[i], lr_t, b1, b2, eps);
+      else p[i] = sgd_step(p[i], gi, lr_t);
     }
   } else {
     for (int64_t i = tid; i < n; i += nth) {
-      float gi = g[i] + (l2 != 0.f ? c2 * p[i] : 0.f);
-      if (ADAM) adam1(p[i], gi, m[i], v[i], lr_t, b1, b2, eps);
-      else p[i] -= lr_t * gi;
+      const float gi = l2 != 0.f ? plus_l2(g[i], p[i], c2) : g[i];
+      if (ADAM) adam_step(p[i], gi, m[i], v[i], lr_t, b1, b2, eps);
+      else p[i] = sgd_step(p[i], gi, lr_t);
     }
   }
 }
@@ -80,26 +76,28 @@ __global__ void __launch_bounds__(256) optimizer_regions_kernel(const OptRegions
     float4 pv = reinterpret_cast<float4*>(p)[i];
     float4 gv = reinterpret_cast<const float4*>(g)[i];
     if (l2 != 0.f) {
-      gv.x += c2 * pv.x; gv.y += c2 * pv.y; gv.z += c2 * pv.z; gv.w += c2 * pv.w;
+      gv.x = plus_l2(gv.x, pv.x, c2); gv.y = plus_l2(gv.y, pv.y, c2);
+      gv.z = plus_l2(gv.z, pv.z, c2); gv.w = plus_l2(gv.w, pv.w, c2);
     }
     if (ADAM) {
       float4 mv = reinterpret_cast<float4*>(m)[i];
       float4 vv = reinterpret_cast<float4*>(v)[i];
-      adam1(pv.x, gv.x, mv.x, vv.x, lr_t, b1, b2, eps);
-      adam1(pv.y, gv.y, mv.y, vv.y, lr_t, b1, b2, eps);
-      adam1(pv.z, gv.z, mv.z, vv.z, lr_t, b1, b2, eps);
-      adam1(pv.w, gv.w, mv.w, vv.w, lr_t, b1, b2, eps);
+      adam_step(pv.x, gv.x, mv.x, vv.x, lr_t, b1, b2, eps);
+      adam_step(pv.y, gv.y, mv.y, vv.y, lr_t, b1, b2, eps);
+      adam_step(pv.z, gv.z, mv.z, vv.z, lr_t, b1, b2, eps);
+      adam_step(pv.w, gv.w, mv.w, vv.w, lr_t, b1, b2, eps);
       reinterpret_cast<float4*>(m)[i] = mv;
       reinterpret_cast<float4*>(v)[i] = vv;
     } else {
-      pv.x -= lr_t * gv.x; pv.y -= lr_t * gv.y; pv.z -= lr_t * gv.z; pv.w -= lr_t * gv.w;
+      pv.x = sgd_step(pv.x, gv.x, lr_t); pv.y = sgd_step(pv.y, gv.y, lr_t);
+        pv.z = sgd_step(pv.z, gv.z, lr_t); pv.w = sgd_step(pv.w, gv.w, lr_t);
     }
     reinterpret_cast<float4*>(p)[i] = pv;
   }
   for (int64_t i = (n4 << 2) + tid; i < n; i += nth) {
-    float gi = g[i] + (l2 != 0.f ? c2 * p[i] : 0.f);
-    if (ADAM) adam1(p[i], gi, m[i], v[i], lr_t, b1, b2, eps);
-    else p[i] -= lr_t * gi;
+    const float gi = l2 != 0.f ? plus_l2(g[i], p[i], c2) : g[i];
+    if (ADAM) adam_step(p[i], gi, m[i], v[i], lr_t, b1, b2, eps);
+    else p[i] = sgd_step(p[i], gi, lr_t);
   }
 }
 

@@ -1,6 +1,6 @@
 // Stable LSD radix sort of (row id, sample index) pairs -- the "sort" of the deterministic
 // sort-and-segmented-reduce embedding-gradient path.  8-bit digits; only ceil(key_bits/8) passes run
-// (ids are < num_users / num_items, so 2-3 passes).  Each warp owns a contiguous tile of kKeysPerWarp
+// (ids are <= num_users / num_items once out-of-range ids are mapped to that sentinel, so 2-3 passes).  Each warp owns a contiguous tile of kKeysPerWarp
 // keys and walks it 32 keys at a time in order, ranking equal digits with __match_any_sync, so the
 // sort is stable without any block-level synchronisation and without atomics.
 #include "launchers.h"
@@ -18,10 +18,16 @@ constexpr int kBins = 256;
 
 __device__ __forceinline__ unsigned digit_of(int32_t key, int shift) { return ((unsigned)key >> shift) & 0xFFu; }
 
+// Key as the sort sees it: keys above `sentinel` (unsigned compare, so negative keys too) become `sentinel`.
+// 0xFFFFFFFF leaves every key as it is.
+__device__ __forceinline__ int32_t load_key(const int32_t* keys, int64_t i, unsigned sentinel) {
+  return (int32_t)min((unsigned)__ldg(keys + i), sentinel);
+}
+
 // hist[bin * nwt + wt] = number of keys of warp tile `wt` whose digit is `bin`.
 __global__ void __launch_bounds__(kSortWarps * 32) radix_hist_kernel(const int32_t* __restrict__ keys, int64_t n,
-                                                                     int shift, unsigned* __restrict__ hist,
-                                                                     int64_t nwt) {
+                                                                     int shift, unsigned sentinel,
+                                                                     unsigned* __restrict__ hist, int64_t nwt) {
   __shared__ unsigned cnt[kSortWarps][kBins];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int64_t wt = (int64_t)blockIdx.x * kSortWarps + w;
@@ -33,7 +39,7 @@ __global__ void __launch_bounds__(kSortWarps * 32) radix_hist_kernel(const int32
 #pragma unroll
     for (int q = 0; q < kTileIters; ++q) {
       const int64_t i = base + 32 * q + lane;
-      kreg[q] = i < n ? __ldg(keys + i) : 0;
+      kreg[q] = i < n ? load_key(keys, i, sentinel) : 0;
     }
 #pragma unroll
     for (int q = 0; q < kTileIters; ++q) {
@@ -83,7 +89,7 @@ __global__ void __launch_bounds__(256) radix_rowscan_kernel(unsigned* __restrict
 // Scatter pass: keys (and their payload index) move to their stable position for this digit.
 __global__ void __launch_bounds__(kSortWarps * 32) radix_scatter_kernel(
     const int32_t* __restrict__ keys, const int32_t* __restrict__ index /* null = identity */, int64_t n, int shift,
-    const unsigned* __restrict__ hist, const unsigned* __restrict__ totals, int64_t nwt,
+    unsigned sentinel, const unsigned* __restrict__ hist, const unsigned* __restrict__ totals, int64_t nwt,
     int32_t* __restrict__ out_keys, int32_t* __restrict__ out_index) {
   __shared__ unsigned run[kSortWarps][kBins];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -117,7 +123,7 @@ __global__ void __launch_bounds__(kSortWarps * 32) radix_scatter_kernel(
 #pragma unroll
   for (int q = 0; q < kTileIters; ++q) {
     const int64_t i = base + 32 * q + lane;
-    kreg[q] = i < n ? __ldg(keys + i) : 0;
+    kreg[q] = i < n ? load_key(keys, i, sentinel) : 0;
     vreg[q] = i < n ? (index != nullptr ? __ldg(index + i) : (int32_t)i) : 0;
   }
 #pragma unroll
@@ -150,7 +156,7 @@ size_t sort_workspace_bytes(int64_t n) {
 }
 
 int launch_sort_pairs(const int32_t* keys, int64_t n, int key_bits, int32_t* out_keys, int32_t* out_index,
-                      void* ws, size_t ws_bytes, cudaStream_t st) {
+                      void* ws, size_t ws_bytes, cudaStream_t st, int32_t num_rows) {
   if (n == 0) return MR_OK;
   if (ws_bytes < sort_workspace_bytes(n)) {
     set_error("sort workspace too small: %zu < %zu", ws_bytes, sort_workspace_bytes(n));
@@ -176,11 +182,14 @@ int launch_sort_pairs(const int32_t* keys, int64_t n, int key_bits, int32_t* out
     const bool to_out = ((passes - 1 - p) & 1) == 0;
     int32_t* dst_k = to_out ? out_keys : tmp_keys;
     int32_t* dst_i = to_out ? out_index : tmp_index;
-    radix_hist_kernel<<<blocks, kSortWarps * 32, 0, st>>>(src_k, n, 8 * p, hist, nwt);
+    // the first pass maps out-of-range keys to the sentinel and stores them so; later passes read mapped keys
+    const unsigned sentinel = (p == 0 && num_rows >= 0) ? (unsigned)num_rows : 0xFFFFFFFFu;
+    radix_hist_kernel<<<blocks, kSortWarps * 32, 0, st>>>(src_k, n, 8 * p, sentinel, hist, nwt);
     MR_LAUNCH_CHECK("radix_hist_kernel");
     radix_rowscan_kernel<<<kBins, 256, 0, st>>>(hist, nwt, totals);
     MR_LAUNCH_CHECK("radix_rowscan_kernel");
-    radix_scatter_kernel<<<blocks, kSortWarps * 32, 0, st>>>(src_k, src_i, n, 8 * p, hist, totals, nwt, dst_k, dst_i);
+    radix_scatter_kernel<<<blocks, kSortWarps * 32, 0, st>>>(src_k, src_i, n, 8 * p, sentinel, hist, totals, nwt, dst_k,
+                                                             dst_i);
     MR_LAUNCH_CHECK("radix_scatter_kernel");
     src_k = dst_k;
     src_i = dst_i;

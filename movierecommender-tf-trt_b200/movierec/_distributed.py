@@ -455,14 +455,13 @@ class ShardedNeuMF(object):
         if self._ws is None or self._ws.numel() < nbytes:
             self._ws = torch.empty(nbytes, dtype=torch.uint8, device=e.device)
         adam = self.optimizer == "adam"
-        t = e.iterations + 1
         ptr = lambda x: C.c_void_p(x.data_ptr()) if x is not None else C.c_void_p(0)
         g = tabs["gmf"]
         nat.check(nat.lib.mr_sparse_rows_update(
             ptr(tabs["mlp"]["p"]), ptr(tabs["mlp"]["m"]), ptr(tabs["mlp"]["v"]), d,
             ptr(g["p"] if g else None), ptr(g["m"] if g else None), ptr(g["v"] if g else None), self.f,
             self.shard[side]["rows"], ptr(route["local"]), ptr(grads), n, nat.OPT_ADAM if adam else nat.OPT_SGD,
-            e.lr, e.adam_lr_t(t) if adam else e.lr, e.beta_1, e.beta_2, self._engine_mod.ADAM_EPSILON,
+            e.lr, e.step_lr_t(), e.beta_1, e.beta_2, self._engine_mod.ADAM_EPSILON,
             ptr(self._ws), self._ws.numel(), e._stream()), "mr_sparse_rows_update")
 
     # ---- the step ---------------------------------------------------------------------------------------

@@ -479,10 +479,11 @@ class NeuMFEngine(object):
 
     def apply_dense_only(self):
         """Optimizer update of the dense block alone from g_dense (row-sharded runs: the table rows are
-        updated by their owners through mr_sparse_rows_update)."""
+        updated by their owners through mr_sparse_rows_update).  The step size is step_lr_t(), the one mr_neumf_apply
+        takes, so the dense block moves exactly as in a single-GPU step."""
         t = self.iterations + 1
         adam = self.optimizer == "adam"
-        lr_t = self.adam_lr_t(t) if adam else self.lr
+        lr_t = self.step_lr_t()
         nat.check(nat.lib.mr_optimizer_flat(_ptr(self.dense), _ptr(self.g_dense), _ptr(self.m_dense), _ptr(self.v_dense),
                                             self.dense_count, nat.OPT_ADAM if adam else nat.OPT_SGD, lr_t, self.beta_1,
                                             self.beta_2, ADAM_EPSILON, 0.0, self._stream()), "mr_optimizer_flat")
