@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 101     /* major*100 + minor */
+#define MR_VERSION 102     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
@@ -236,6 +236,42 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
                       const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
                       float* top_scores, int32_t* pos, float* sums, float* scores, void* ws, size_t ws_bytes,
                       void* stream);
+
+/* Top-k of ragged lists of caller-supplied scores: list u is scores[rowptr[u] .. rowptr[u+1]) (device rowptr, U + 1
+ * int64, rowptr[0] = 0, non-decreasing, rowptr[U] = nnz; U and nnz <= INT32_MAX, no rows when U = 0).  Order: the
+ * RankLayer order (descending score, NaN as -inf, -0 == +0, the EARLIER position in the list first among ties), so pos
+ * is exactly mr_rank_scores' position for label_col = target, and with the target last exactly mr_rank_eval's rule
+ * (the positive loses ties).  top_pos / top_scores (U x k, each may be NULL): the k best positions within the list,
+ * -1 / NaN padding beyond the list's length (an empty list is all padding).  targets (U, may be NULL): a position in
+ * the list; pos[u] = the number of candidates ordered before it (the list length for a target outside [0, len));
+ * sums = {hit_sum, dcg_sum} over the U lists (hit = pos < k, dcg = ln2/ln(pos+2)*hit).  pos and sums need targets.
+ * 1 <= k <= MR_MAX_TOPK.  Deterministic (distinct integer keys).  Every list is clamped to [0, nnz), so a malformed
+ * rowptr never makes a kernel read or write outside the arrays; its lists' results are unspecified.
+ * Workspace: 8 bytes per list + 4 per list + about 8 k + 4 bytes per 512 rows (staged partial results of the lists
+ * longer than 1024, which are cut into <= 32 slices), plus alignment.  No host synchronisation, no read-back. */
+size_t mr_topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k);
+int mr_topk_lists(const float* scores, int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
+                  int32_t* top_pos, float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream);
+
+/* The same on the model's probabilities of the pairs (users[u], items[j]), j in list u: batched serving (one request =
+ * one user and its own candidate list, of any length; the reference client's one user x ~1000 candidates,
+ * trt_client.py:47-57) and ranking evaluation with candidate sets of different sizes.  top_items (U x k) =
+ * items[rowptr[u] + top_pos], -1 padding; probs (nnz, may be NULL) receives every pair's probability.  An item may
+ * appear more than once in a list: each copy is a separate candidate.  An out-of-range user gives its list -1 / NaN in
+ * every slot and pos = the list length; an out-of-range item gets probability NaN and ranks as NaN ranks.
+ * The launch sequence is a function of the model alone (never of U or nnz), so a list's outputs do not depend on the
+ * other lists of the call: tensor-core towers with an eligible item projection that is not MR_PROJECTION_OFF (>= 3
+ * layers, mf_dim 32 / 64 / 128) take the projected sequence of mr_rank_eval (item half once per call, user half once
+ * per list); the default tower (mr_uses_small_tower's model, projection and fused kernel not OFF) takes its projected
+ * CUDA-core forward with the user half computed for the call's users only; every other model takes mr_neumf_forward.
+ * A pair then gets the probability mr_rank_eval gives it when both calls take the projected sequence.  Scoring runs in
+ * launches of at most 2^22 rows, so the scoring workspace is bounded by one launch (a few bytes per row) plus, on the
+ * projected paths, the item projection (num_items x layers_sizes[1] floats) and one row of layers_sizes[1] floats (the
+ * default tower: also layers_sizes[0]/2) per list.  On top of mr_topk_lists' workspace: 8 bytes per row. */
+size_t mr_rank_lists_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz, int32_t k);
+int mr_rank_lists(const MrModel* model, const int32_t* users, int64_t U, const int64_t* rowptr, const int32_t* items,
+                  int64_t nnz, int32_t k, const int32_t* targets, int32_t* top_pos, int32_t* top_items, float* top_scores,
+                  int32_t* pos, float* sums, float* probs, void* ws, size_t ws_bytes, void* stream);
 
 /* On-device negative sampler -- replaces _get_random_negatives_and_positive
  * (data_pipeline.py:99-113): for positive p (global index first_index + p, user pos_users[p]) draw

@@ -701,6 +701,87 @@ static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const 
   return MR_OK;
 }
 
+// ---- ragged candidate lists: list u pairs users[u] with items[rowptr[u] .. rowptr[u+1]) ------------------------------
+// The scoring sequence is a function of the model alone -- never of U or nnz -- so that a list's outputs do not depend on
+// the other lists of the call (what a serving batcher needs):
+//  LISTS_TC: the tensor-core tower with the projected first layer (eligible models, projection not OFF): Pi once per
+//            call, Zu once per list, the second layer's producers read relu(Pi[item] + Zu[seg[row]]), the last layer
+//            dots with the output weights, and the partial-logit head adds the GMF term;
+//  LISTS_SMALL: the default tower: Pi over the item table, Pu over the call's users, the thread-per-row forward;
+//  LISTS_FORWARD: per-row user ids and the plain forward.
+enum { LISTS_TC = 0, LISTS_SMALL = 1, LISTS_FORWARD = 2 };
+constexpr int64_t kAnyRows = INT64_MAX / 4;  // "eligible at any row count" for the row-count rules of AUTO
+static int lists_path(const MrModel& m) {
+  if (m.n_layers >= 3 && catalogue_head_supported(m) && item_proj_ok(m, kAnyRows)) return LISTS_TC;
+  if (small_eval_ok(m, kAnyRows)) return LISTS_SMALL;
+  return LISTS_FORWARD;
+}
+
+// Rows per scoring launch: the call's rows in whole 128-row tiles, up to the ranking eval's 2^22 -- or the forward's
+// own 2^21 on the plain-forward path, whose workspace then grows with the rows up to that cap and stays there.
+static int64_t lists_sub_batch(const MrModel& m, int64_t nnz) {
+  const int64_t cap = lists_path(m) == LISTS_FORWARD ? kTcSubBatchCap : kEvalSubBatchCap;
+  const int64_t r = (nnz + 127) / 128 * 128;
+  return r < 128 ? 128 : (r < cap ? r : cap);
+}
+
+struct ListsTcWs {
+  float *pack_fu, *pack_fi, *Pi, *Zu;
+  float* pack_f[MR_MAX_LAYERS];
+  float* H[MR_MAX_LAYERS];  // H[2 .. n-2]: sb x L[l]; H[n-1]: sb floats (the partial logits)
+  size_t total;
+};
+static ListsTcWs carve_lists_tc(const MrModel& m, int64_t U, int64_t sb, void* ws) {
+  ListsTcWs t{};
+  Carver cv(ws);
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+  t.pack_fu = cv.take<float>((size_t)2 * d_u * m.L[1]);
+  t.pack_fi = cv.take<float>((size_t)2 * d_i * m.L[1]);
+  t.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
+  t.Zu = cv.take<float>((size_t)(U < 1 ? 1 : U) * m.L[1]);
+  for (int l = 2; l < m.n_layers; ++l) {
+    t.pack_f[l] = cv.take<float>((size_t)2 * m.L[l - 1] * m.L[l]);
+    t.H[l] = cv.take<float>((size_t)sb * (l == m.n_layers - 1 ? 1 : m.L[l]));
+  }
+  t.total = cv.off;
+  return t;
+}
+
+struct ListsSmallWs {
+  float *Pi, *Eu, *Pu;
+  size_t total;
+};
+static ListsSmallWs carve_lists_small(const MrModel& m, int64_t U, void* ws) {
+  ListsSmallWs w{};
+  Carver cv(ws);
+  const size_t Ul = (size_t)(U < 1 ? 1 : U);
+  w.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
+  w.Eu = cv.take<float>(Ul * (m.L[0] / 2));
+  w.Pu = cv.take<float>(Ul * m.L[1]);
+  w.total = cv.off;
+  return w;
+}
+
+static size_t lists_scoring_bytes(const MrModel& m, int64_t U, int64_t nnz) {
+  const int64_t sb = lists_sub_batch(m, nnz);
+  switch (lists_path(m)) {
+    case LISTS_TC: return carve_lists_tc(m, U, sb, nullptr).total;
+    case LISTS_SMALL: return carve_lists_small(m, U, nullptr).total;
+    default: return mr_forward_workspace_bytes(&m, sb);
+  }
+}
+
+static int lists_check(int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
+                       const int32_t* pos, const float* sums) {
+  MR_REQUIRE(U >= 0 && U <= INT32_MAX && nnz >= 0 && nnz <= INT32_MAX, "lists: bad U=%lld nnz=%lld", (long long)U,
+             (long long)nnz);
+  MR_REQUIRE(U > 0 || nnz == 0, "lists: nnz=%lld rows in no list", (long long)nnz);
+  MR_REQUIRE(k >= 1 && k <= MR_MAX_TOPK, "lists: k=%d out of [1,%d]", k, MR_MAX_TOPK);
+  MR_REQUIRE(targets != nullptr || (pos == nullptr && sums == nullptr), "lists: pos / sums need targets");
+  MR_REQUIRE(U == 0 || rowptr != nullptr, "lists: rowptr is NULL");
+  return MR_OK;
+}
+
 }  // namespace mr
 
 using namespace mr;
@@ -1747,6 +1828,189 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
     prof_mark(MR_PHASE_RANK, st);
     rc = launch_topk_metrics(pos, U, k, sums, st);
   }
+  prof_mark(-1, st);
+  return rc;
+}
+
+size_t mr_topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k) {
+  if (U < 0 || U > INT32_MAX || nnz < 0 || nnz > INT32_MAX || k < 1 || k > MR_MAX_TOPK) return 0;
+  return topk_lists_workspace_bytes(U, nnz, k) + 256;
+}
+
+int mr_topk_lists(const float* scores, int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
+                  int32_t* top_pos, float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream) {
+  int rc = lists_check(U, rowptr, nnz, k, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  MR_REQUIRE(nnz == 0 || scores != nullptr, "topk_lists: scores is NULL");
+  MR_REQUIRE(ws != nullptr, "topk_lists: workspace is NULL");
+  if (ws_bytes < mr_topk_lists_workspace_bytes(U, nnz, k)) {
+    set_error("topk_lists workspace too small: %zu < %zu", ws_bytes, mr_topk_lists_workspace_bytes(U, nnz, k));
+    return MR_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  TopkListsArgs a{};
+  a.scores = scores;
+  a.rowptr = rowptr;
+  a.U = U;
+  a.nnz = nnz;
+  a.k = k;
+  a.targets = targets;
+  a.top_pos = top_pos;
+  a.top_scores = top_scores;
+  a.pos = pos;
+  prof_mark(MR_PHASE_RANK, st);
+  rc = launch_topk_lists(a, sums, ws, st);
+  prof_mark(-1, st);
+  return rc;
+}
+
+size_t mr_rank_lists_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz, int32_t k) {
+  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
+      model->num_users < 1 || model->L[0] < 2)
+    return 0;
+  const size_t sel = mr_topk_lists_workspace_bytes(U, nnz, k);
+  if (sel == 0) return 0;
+  return sel + align_up((size_t)nnz * sizeof(int32_t), 256) + align_up((size_t)nnz * sizeof(float), 256) +
+         lists_scoring_bytes(*model, U, nnz) + 256;
+}
+
+int mr_rank_lists(const MrModel* model, const int32_t* users, int64_t U, const int64_t* rowptr, const int32_t* items,
+                  int64_t nnz, int32_t k, const int32_t* targets, int32_t* top_pos, int32_t* top_items, float* top_scores,
+                  int32_t* pos, float* sums, float* probs, void* ws, size_t ws_bytes, void* stream) {
+  int rc = check_model(model);
+  if (rc != MR_OK) return rc;
+  rc = lists_check(U, rowptr, nnz, k, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  MR_REQUIRE(U == 0 || users != nullptr, "rank_lists: users is NULL");
+  MR_REQUIRE(nnz == 0 || items != nullptr, "rank_lists: items is NULL");
+  MR_REQUIRE(ws != nullptr, "rank_lists: workspace is NULL");
+  if (ws_bytes < mr_rank_lists_workspace_bytes(model, U, nnz, k)) {
+    set_error("rank_lists workspace too small: %zu < %zu", ws_bytes, mr_rank_lists_workspace_bytes(model, U, nnz, k));
+    return MR_ERR_WORKSPACE;
+  }
+  const MrModel& m = *model;
+  cudaStream_t st = (cudaStream_t)stream;
+  Carver cv(ws);
+  void* sel_ws = cv.take<char>(topk_lists_workspace_bytes(U, nnz, k));
+  int32_t* seg = cv.take<int32_t>((size_t)nnz);
+  float* probs_buf = cv.take<float>((size_t)nnz);
+  void* score_ws = static_cast<char*>(ws) + cv.off;
+  float* pr = probs != nullptr ? probs : probs_buf;
+  const int path = lists_path(m);
+  const int64_t sb = lists_sub_batch(m, nnz);
+  if (nnz > 0) {
+    prof_mark(MR_PHASE_MISC, st);
+    // seg: the list of each row (TC / default tower), or the user of each row (plain forward)
+    rc = launch_list_rows(rowptr, U, nnz, path == LISTS_FORWARD ? users : nullptr, seg, st);
+    if (rc != MR_OK) return rc;
+  }
+  if (nnz > 0 && path == LISTS_TC) {
+    const ListsTcWs t = carve_lists_tc(m, U, sb, score_ws);
+    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+    rc = launch_pack_weights(m.W[1], d_u, m.L[1], 0, t.pack_fu, st);
+    if (rc == MR_OK) rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], d_i, m.L[1], 0, t.pack_fi, st);
+    for (int l = 2; rc == MR_OK && l < m.n_layers; ++l) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, t.pack_f[l], st);
+    if (rc != MR_OK) return rc;
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    TcWs tw{};
+    tw.pack_fi = t.pack_fi;
+    tw.Pi = t.Pi;
+    rc = tc_project_items(m, tw, st);
+    if (rc != MR_OK) return rc;
+    {  // Zu = E_user[users[u]] . W1[user rows] + b1, one row per list (zero row for an out-of-range user)
+      TcDenseArgs a{};
+      a.gather = true;
+      a.user_tab = m.user_mlp;
+      a.users = users;
+      a.num_users = m.num_users;
+      a.num_items = m.num_items;
+      a.d_u = d_u;
+      a.user_div = 1;
+      a.user_mul = 1;
+      a.b_packed = t.pack_fu;
+      a.N = m.L[1];
+      a.K = d_u;
+      a.rows = U;
+      a.row0 = 0;
+      a.epilogue = TC_EPI_BIAS_RELU;
+      a.bias = m.b[1];
+      a.linear = true;
+      a.out = t.Zu;
+      rc = launch_tc_dense(a, st);
+      if (rc != MR_OK) return rc;
+    }
+    for (int64_t r0 = 0; r0 < nnz; r0 += sb) {
+      const int64_t r1 = r0 + sb < nnz ? r0 + sb : nnz;
+      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+      for (int l = 2; l < m.n_layers; ++l) {
+        TcDenseArgs a{};
+        a.a_dense = l == 2 ? nullptr : t.H[l - 1];
+        a.items = items;
+        a.num_users = m.num_users;
+        a.num_items = m.num_items;
+        a.b_packed = t.pack_f[l];
+        a.N = m.L[l];
+        a.K = m.L[l - 1];
+        a.rows = r1 - r0;
+        a.row0 = r0;
+        a.epilogue = TC_EPI_BIAS_RELU;
+        a.bias = m.b[l];
+        a.out = t.H[l];
+        if (l == 2) {  // the producers compute relu(Pi[items[row]] + Zu[seg[row]])
+          a.proj_i = t.Pi;
+          a.proj_u = t.Zu;
+          a.proj_ids = seg;
+          a.proj_u_rows = (int32_t)U;
+        }
+        if (l == m.n_layers - 1) {
+          a.epilogue = TC_EPI_HEAD_DOT;
+          a.head_w = m.w_out + m.mf_dim;
+        }
+        rc = launch_tc_dense(a, st);
+        if (rc != MR_OK) return rc;
+      }
+      prof_mark(MR_PHASE_HEAD, st);
+      rc = launch_lists_head(m, t.H[m.n_layers - 1], users, U, seg, items, r0, r1 - r0, pr, st);
+      if (rc != MR_OK) return rc;
+    }
+  } else if (nnz > 0 && path == LISTS_SMALL) {
+    const ListsSmallWs w = carve_lists_small(m, U, score_ws);
+    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, w.Pi, st);
+    if (rc == MR_OK) rc = launch_gather_rows(m.user_mlp, m.num_users, d_u, users, U, w.Eu, st);  // NaN rows: bad users
+    if (rc == MR_OK) rc = launch_small_rows_gemm(w.Eu, U, d_u, m.W[1], L1, L1, false, m.b[1], w.Pu, st);
+    prof_mark(MR_PHASE_FUSED_TILE, st);
+    for (int64_t r0 = 0; rc == MR_OK && r0 < nnz; r0 += sb) {
+      const int64_t r1 = r0 + sb < nnz ? r0 + sb : nnz;
+      rc = launch_small_tower_forward(m, w.Pi, w.Pu, users, items + r0, r1 - r0, 1, pr + r0, st, seg + r0, U);
+    }
+    if (rc != MR_OK) return rc;
+  } else if (nnz > 0) {
+    const size_t fwd_bytes = mr_forward_workspace_bytes(model, sb);
+    for (int64_t r0 = 0; r0 < nnz; r0 += sb) {
+      const int64_t r1 = r0 + sb < nnz ? r0 + sb : nnz;
+      rc = mr_neumf_forward(model, seg + r0, items + r0, r1 - r0, 1, nullptr, pr + r0, nullptr, nullptr, score_ws,
+                            fwd_bytes, stream);
+      if (rc != MR_OK) return rc;
+    }
+  }
+  TopkListsArgs a{};
+  a.scores = pr;
+  a.rowptr = rowptr;
+  a.U = U;
+  a.nnz = nnz;
+  a.k = k;
+  a.targets = targets;
+  a.users = users;
+  a.num_users = m.num_users;
+  a.items = items;
+  a.top_pos = top_pos;
+  a.top_items = top_items;
+  a.top_scores = top_scores;
+  a.pos = pos;
+  prof_mark(MR_PHASE_RANK, st);
+  rc = launch_topk_lists(a, sums, sel_ws, st);
   prof_mark(-1, st);
   return rc;
 }

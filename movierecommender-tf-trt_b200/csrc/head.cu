@@ -680,10 +680,15 @@ __global__ void __launch_bounds__(kHeadThreads) head_rank_warp_kernel(const Head
 // user against the whole catalogue per `group` rows).  Row-parallel -- a group here is tens of thousands of rows, far
 // beyond the warp-per-group kernel's shared-memory slice -- with the per-row arithmetic of head_rank_warp_kernel
 // (gmf_head_prob).  Four rows per warp step, KS steps in flight.
-template <int NV>
+// RAGGED (candidate lists): row r is global row row0 + r, pairing users[seg[row0 + r]] with items[row0 + r]; h_dot is
+// launch-local; an out-of-range user, item or list index gives NaN.
+template <int NV, bool RAGGED>
 __global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrModel m, const float* __restrict__ h_dot,
                                                                       const int32_t* __restrict__ users, int64_t rows,
-                                                                      int group, float* __restrict__ probs) {
+                                                                      int group, float* __restrict__ probs,
+                                                                      const int32_t* __restrict__ seg,
+                                                                      const int32_t* __restrict__ items, int64_t row0,
+                                                                      int64_t num_lists) {
   constexpr int f = 32 * NV, KS = NV >= 4 ? 1 : 2;  // (KS = 4 spills at NV = 1 and needs 170 registers at NV = 4)
   const int lane = threadIdx.x & 31;
   const int sub = lane & 7, quad = lane >> 3;
@@ -701,11 +706,20 @@ __global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrMo
     for (int k = 0; k < KS; ++k) {
       int64_t row = r0 + 4 * k + quad;
       if (row >= rows) row = rows - 1;  // dead slots re-read the last row
-      const int64_t slot = row / group;
-      const int it = (int)(row - slot * group);
-      int u = __ldg(users + slot);
-      bad[k] = (unsigned)u >= (unsigned)m.num_users;
-      if (bad[k]) u = 0;
+      int u, it;
+      if (RAGGED) {
+        const int sg = __ldg(seg + row0 + row);
+        u = (unsigned)sg < (uint64_t)num_lists ? __ldg(users + sg) : -1;
+        it = __ldg(items + row0 + row);
+        bad[k] = (unsigned)u >= (unsigned)m.num_users || (unsigned)it >= (unsigned)m.num_items;
+        if (bad[k]) u = it = 0;
+      } else {
+        const int64_t slot = row / group;
+        it = (int)(row - slot * group);
+        u = __ldg(users + slot);
+        bad[k] = (unsigned)u >= (unsigned)m.num_users;
+        if (bad[k]) u = 0;
+      }
       z[k] = __ldg(h_dot + row);
 #pragma unroll
       for (int v = 0; v < NV; ++v) {
@@ -718,7 +732,7 @@ __global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrMo
     for (int k = 0; k < KS; ++k) {
       const int64_t row = r0 + 4 * k + quad;
       const float pr = gmf_head_prob<NV>(wu[k], gi[k], z[k], b_out, bad[k]);
-      if (sub == 0 && row < rows) probs[row] = pr;
+      if (sub == 0 && row < rows) probs[(RAGGED ? row0 : 0) + row] = pr;
     }
   }
 }
@@ -864,11 +878,31 @@ int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* u
   const int64_t cap = (int64_t)sm_count() * 8;
   const unsigned grid = (unsigned)(want < cap ? want : cap);
   if (m.mf_dim == 32)
-    catalogue_head_kernel<1><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs);
+    catalogue_head_kernel<1, false><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, nullptr, nullptr, 0, 0);
   else if (m.mf_dim == 64)
-    catalogue_head_kernel<2><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs);
+    catalogue_head_kernel<2, false><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, nullptr, nullptr, 0, 0);
   else
-    catalogue_head_kernel<4><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs);
+    catalogue_head_kernel<4, false><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, nullptr, nullptr, 0, 0);
+  MR_LAUNCH_CHECK("catalogue_head_kernel");
+  return MR_OK;
+}
+
+int launch_lists_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t num_lists, const int32_t* seg,
+                      const int32_t* items, int64_t row0, int64_t rows, float* probs, cudaStream_t st) {
+  if (!catalogue_head_supported(m)) {
+    set_error("lists head: needs mf_dim 32, 64 or 128 and 16-byte aligned GMF tables / output weights");
+    return MR_ERR_INVALID;
+  }
+  if (rows == 0) return MR_OK;
+  const int64_t want = (rows + 4 * (kHeadThreads / 32) - 1) / (4 * (kHeadThreads / 32));
+  const int64_t cap = (int64_t)sm_count() * 8;
+  const unsigned grid = (unsigned)(want < cap ? want : cap);
+  if (m.mf_dim == 32)
+    catalogue_head_kernel<1, true><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, 1, probs, seg, items, row0, num_lists);
+  else if (m.mf_dim == 64)
+    catalogue_head_kernel<2, true><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, 1, probs, seg, items, row0, num_lists);
+  else
+    catalogue_head_kernel<4, true><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, 1, probs, seg, items, row0, num_lists);
   MR_LAUNCH_CHECK("catalogue_head_kernel");
   return MR_OK;
 }

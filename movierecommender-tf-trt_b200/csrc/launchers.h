@@ -106,6 +106,28 @@ size_t topk_workspace_bytes(int64_t U, int32_t N, int32_t k);  // per chunk of U
 int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st);
 // sums = {hit_sum, dcg_sum} of pos[0, U) in a fixed order, no workspace
 int launch_topk_metrics(const int32_t* pos, int64_t U, int k, float* sums, cudaStream_t st);
+// Ragged lists: list u is scores[rowptr[u] .. rowptr[u+1]) (segments clamped to [0, nnz)); keys carry the position
+// in the list, so ties go to the earlier position.  Outputs per list u (each may be NULL): top_pos / top_items
+// (items[start + pos]) / top_scores (U x k, -1 / NaN padding), pos[u] (needs targets: positions in the list).
+struct TopkListsArgs {
+  const float* scores;
+  const int64_t* rowptr;
+  int64_t U, nnz;
+  int32_t k;
+  const int32_t* targets;
+  const int32_t* users;  // optional: a list whose users[u] lies outside [0, num_users) gets -1 / NaN and pos = len
+  int32_t num_users;
+  const int32_t* items;  // needed with top_items
+  int32_t* top_pos;
+  int32_t* top_items;
+  float* top_scores;
+  int32_t* pos;
+};
+size_t topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k);
+// sums (may be NULL, needs targets) = {hit_sum, dcg_sum} of the U lists' positions
+int launch_topk_lists(const TopkListsArgs& a, float* sums, void* ws, cudaStream_t st);
+// seg[r] = the list holding row r (in [0, U)), or users[that list] when users != NULL
+int launch_list_rows(const int64_t* rowptr, int64_t U, int64_t nnz, const int32_t* users, int32_t* seg, cudaStream_t st);
 // out[r] = r % N for r < rows
 int launch_tile_iota(int32_t* out, int64_t rows, int32_t N, cudaStream_t st);
 
@@ -207,6 +229,10 @@ int launch_head_rank(const HeadArgs& a, int group, int32_t* pos, float* probs, c
 bool catalogue_head_supported(const MrModel& m);
 int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t rows, int group,
                           float* probs, cudaStream_t st);
+// the same for candidate lists: global row row0 + r pairs users[seg[row0 + r]] (seg < num_lists) with items[row0 + r];
+// h_dot launch-local, probs global
+int launch_lists_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t num_lists, const int32_t* seg,
+                      const int32_t* items, int64_t row0, int64_t rows, float* probs, cudaStream_t st);
 // metric sums from positions (rank.cu): sums = {hit_sum, dcg_sum}
 int launch_rank_metrics(const int32_t* pos, int64_t G, int k, float* sums, float* partials, cudaStream_t st);
 
@@ -239,9 +265,11 @@ struct SmallTowerArgs {
 };
 bool small_tower_supported(const MrModel& m, int group);
 int launch_small_tower_train(const SmallTowerArgs& a, cudaStream_t st, int* grid_out);
-// forward of the same tower: probs[row] for rows whose user is users[row / group]
+// forward of the same tower: probs[row] for rows whose user is users[row / group]; with seg (candidate lists), row r
+// belongs to list seg[r] < num_lists, whose user is users[seg[r]] and whose Pu row is seg[r]
 int launch_small_tower_forward(const MrModel& m, const float* Pi, const float* Pu, const int32_t* users,
-                               const int32_t* items, int64_t rows, int group, float* probs, cudaStream_t st);
+                               const int32_t* items, int64_t rows, int group, float* probs, cudaStream_t st,
+                               const int32_t* seg = nullptr, int64_t num_lists = 0);
 // out = A (rows x K) . W (K x N, or its transpose read from an N x K array when `transpose`) (+ bias)
 int launch_small_rows_gemm(const float* A, int64_t rows, int K, const float* W, int ldw, int N, bool transpose,
                            const float* bias, float* out, cudaStream_t st);

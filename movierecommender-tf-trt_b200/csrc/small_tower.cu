@@ -303,18 +303,28 @@ __global__ void __launch_bounds__(kThreads, MR_ST_CTAS) small_tower_train_kernel
 // Ranking eval / forward: thread = candidate row, `group` consecutive rows share users[row / group].  The row's Pi and
 // Pu are read as eight 16-byte pieces (the user's row hits L1 for the group's other candidates), layers 2-3 and the
 // output unit run in registers on constant-bank weights, one probability is stored per row (NaN for a bad id).
+// RAGGED (candidate lists): row r belongs to list seg[r] of num_lists; its user is users[seg[r]] and its Pu row is
+// seg[r] (Pu holds one row per list).
+template <bool RAGGED>
 __global__ void __launch_bounds__(256) small_tower_forward_kernel(const float* __restrict__ Pi, const float* __restrict__ Pu,
                                                                   const float* __restrict__ gmf_u,
                                                                   const float* __restrict__ gmf_i,
                                                                   const int32_t* __restrict__ users,
                                                                   const int32_t* __restrict__ items, int64_t rows, int group,
-                                                                  int num_users, int num_items, float* __restrict__ probs) {
+                                                                  int num_users, int num_items, float* __restrict__ probs,
+                                                                  const int32_t* __restrict__ seg, int64_t num_lists) {
   for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < rows; row += (int64_t)gridDim.x * blockDim.x) {
-    int u = __ldg(users + row / group), it = __ldg(items + row);
+    int u, pr, it = __ldg(items + row);
+    if (RAGGED) {
+      pr = __ldg(seg + row);
+      u = (unsigned)pr < (uint64_t)num_lists ? __ldg(users + pr) : -1;
+    } else {
+      pr = u = __ldg(users + row / group);
+    }
     const bool bad = (unsigned)u >= (unsigned)num_users || (unsigned)it >= (unsigned)num_items;
-    if (bad) u = it = 0;
+    if (bad) pr = u = it = 0;
     const float4* pi4 = reinterpret_cast<const float4*>(Pi + (size_t)it * L1);
-    const float4* pu4 = reinterpret_cast<const float4*>(Pu + (size_t)u * L1);
+    const float4* pu4 = reinterpret_cast<const float4*>(Pu + (size_t)pr * L1);
     float z2[L2];
 #pragma unroll
     for (int o = 0; o < L2; ++o) z2[o] = c_w[cB2 + o];
@@ -487,7 +497,8 @@ int launch_small_tower_train(const SmallTowerArgs& a, cudaStream_t stream, int* 
 }
 
 int launch_small_tower_forward(const MrModel& m, const float* Pi, const float* Pu, const int32_t* users,
-                               const int32_t* items, int64_t rows, int group, float* probs, cudaStream_t stream) {
+                               const int32_t* items, int64_t rows, int group, float* probs, cudaStream_t stream,
+                               const int32_t* seg, int64_t num_lists) {
   if (rows == 0) return MR_OK;
   int64_t grid = (rows + 255) / 256;
   const int64_t cap = (int64_t)sm_count() * 8;
@@ -496,8 +507,14 @@ int launch_small_tower_forward(const MrModel& m, const float* Pi, const float* P
   cudaEvent_t g_const_free = nullptr;
   int rc = upload_weights(m, stream, &g_const_free);
   if (rc != MR_OK) return rc;
-  st::small_tower_forward_kernel<<<(unsigned)grid, 256, 0, stream>>>(Pi, Pu, m.user_gmf, m.item_gmf, users, items, rows,
-                                                                     group, m.num_users, m.num_items, probs);
+  if (seg != nullptr)
+    st::small_tower_forward_kernel<true><<<(unsigned)grid, 256, 0, stream>>>(Pi, Pu, m.user_gmf, m.item_gmf, users, items,
+                                                                           rows, 1, m.num_users, m.num_items, probs, seg,
+                                                                           num_lists);
+  else
+    st::small_tower_forward_kernel<false><<<(unsigned)grid, 256, 0, stream>>>(Pi, Pu, m.user_gmf, m.item_gmf, users, items,
+                                                                            rows, group, m.num_users, m.num_items, probs,
+                                                                            nullptr, 0);
   const cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "small_tower_forward_kernel");
   count_launch();

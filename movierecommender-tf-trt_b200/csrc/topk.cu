@@ -24,12 +24,14 @@ constexpr int kTopkMinSlice = 1024;
 constexpr int kTopkMaxSlices = 32;  // one merge lane per slice
 constexpr unsigned long long kNoKey = ~0ull;
 
-static int topk_slice_len(int32_t N) {
+__host__ __device__ static int topk_slice_len(int32_t N) {
   int64_t s = ((int64_t)N + kTopkMaxSlices - 1) / kTopkMaxSlices;
   s = (s + 31) / 32 * 32;
   return (int)(s < kTopkMinSlice ? kTopkMinSlice : s);
 }
-static int topk_slices(int32_t N) { return (int)(((int64_t)N + topk_slice_len(N) - 1) / topk_slice_len(N)); }
+__host__ __device__ static int topk_slices(int32_t N) {
+  return (int)(((int64_t)N + topk_slice_len(N) - 1) / topk_slice_len(N));
+}
 static int topk_cap(int k) {  // buffer entries: a power of two >= k + 32 (room for one more warp-wide append)
   int c = 64;
   while (c < k + 32) c <<= 1;
@@ -65,6 +67,44 @@ __device__ int topk_flush(unsigned long long* buf, int n, int cap, int k, int la
     }
   }
   return n < k ? n : k;
+}
+
+// Appends the lanes' keys below the running threshold thr to the warp's buffer (n entries), sorting and cutting the
+// buffer to k first when a full warp might not fit; thr becomes the k-th best key once k keys are known.
+__device__ __forceinline__ void topk_push(unsigned long long* buf, int& n, unsigned long long& thr,
+                                          unsigned long long key, int cap, int k, int lane) {
+  if (n + 32 > cap) {
+    n = topk_flush(buf, n, cap, k, lane);
+    if (n == k) thr = buf[k - 1];
+  }
+  const bool pass = key < thr;
+  const uint32_t pm = __ballot_sync(0xffffffffu, pass);
+  if (pass) buf[n + __popc(pm & ((1u << lane) - 1u))] = key;
+  n += __popc(pm);
+  __syncwarp();
+}
+
+// Merges S <= 32 ascending lists of k keys (list j at lists + j * k, kNoKey-padded) into the k smallest: k rounds of a
+// warp minimum over the lists' heads (lane = list).  Keys are distinct, so each round has one winner.  emit(i, key)
+// runs on lane i % 32 for i = 0 .. k-1 (key = kNoKey past the last entry).
+template <class Emit>
+__device__ __forceinline__ void topk_merge_warp(const unsigned long long* lists, int S, int k, int lane, Emit emit) {
+  const unsigned long long* mine = lists + (size_t)lane * k;
+  int cur = 0;
+  unsigned long long head = lane < S ? mine[0] : kNoKey;
+  for (int i = 0; i < k; ++i) {
+    unsigned long long m = head;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long x = __shfl_xor_sync(0xffffffffu, m, o);
+      m = x < m ? x : m;
+    }
+    if (m != kNoKey && head == m) {
+      ++cur;
+      head = cur < k ? mine[cur] : kNoKey;
+    }
+    if (lane == (i & 31)) emit(i, m);
+  }
 }
 
 __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs a, int S, int slice, int cap,
@@ -116,15 +156,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs
     const bool cand = item < hi && (!((xmask >> lane) & 1u) || item == t);  // the target is never excluded
     const unsigned long long key = cand ? topk_key(__ldg(row + item), item) : kNoKey;
     below += (has_t && key < key_t) ? 1 : 0;
-    if (n + 32 > cap) {
-      n = topk_flush(buf, n, cap, k, lane);
-      if (n == k) thr = buf[k - 1];
-    }
-    const bool pass = key < thr;
-    const uint32_t pm = __ballot_sync(0xffffffffu, pass);
-    if (pass) buf[n + __popc(pm & ((1u << lane) - 1u))] = key;
-    n += __popc(pm);
-    __syncwarp();
+    topk_push(buf, n, thr, key, cap, k, lane);
   }
   n = topk_flush(buf, n, cap, k, lane);
   unsigned long long* out = lists + (size_t)w * k;
@@ -142,26 +174,11 @@ __global__ void __launch_bounds__(kTopkThreads) topk_merge_kernel(const TopkArgs
   const int64_t gu = a.u0 + u;
   const int k = a.k, N = a.N;
   const bool bad_u = a.users != nullptr && (unsigned)__ldg(a.users + gu) >= (unsigned)a.num_users;
-  const unsigned long long* mine = lists + ((size_t)u * S + lane) * k;
-  int cur = 0;
-  unsigned long long head = lane < S ? mine[0] : kNoKey;
-  for (int i = 0; i < k; ++i) {
-    unsigned long long m = head;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const unsigned long long x = __shfl_xor_sync(0xffffffffu, m, o);
-      m = x < m ? x : m;
-    }
-    if (m != kNoKey && head == m) {  // keys are distinct: one winner
-      ++cur;
-      head = cur < k ? mine[cur] : kNoKey;
-    }
-    if (lane == (i & 31)) {
-      const int item = (m == kNoKey || bad_u) ? -1 : (int)(uint32_t)m;
-      if (a.top_items != nullptr) a.top_items[gu * k + i] = item;
-      if (a.top_scores != nullptr) a.top_scores[gu * k + i] = item < 0 ? nanf("") : __ldg(a.scores + u * N + item);
-    }
-  }
+  topk_merge_warp(lists + (size_t)u * S * k, S, k, lane, [&](int i, unsigned long long m) {
+    const int item = (m == kNoKey || bad_u) ? -1 : (int)(uint32_t)m;
+    if (a.top_items != nullptr) a.top_items[gu * k + i] = item;
+    if (a.top_scores != nullptr) a.top_scores[gu * k + i] = item < 0 ? nanf("") : __ldg(a.scores + u * N + item);
+  });
   if (a.pos != nullptr) {
     int c = lane < S ? counts[u * S + lane] : 0;
     c = warp_sum_int(c);
@@ -182,6 +199,234 @@ int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st) {
   MR_LAUNCH_CHECK("topk_slice_kernel");
   topk_merge_kernel<<<(unsigned)((a.U + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, S, lists, counts);
   MR_LAUNCH_CHECK("topk_merge_kernel");
+  return MR_OK;
+}
+
+// ---- ragged lists: list u is scores[rowptr[u] .. rowptr[u+1]) ---------------------------------------------------
+// The same keys with the POSITION in the list as the low half: ascending keys = descending score, the earlier position
+// first among ties.  A short list (<= one slice of kTopkMinSlice) is one warp from scores to final outputs.  A long list
+// is cut into topk_slices(len) <= 32 slices whose warps stage k keys each, and one merge warp per long list finishes it.
+// Work items: warp w < U takes slice 0 of list w; the slices 1.. of the long lists follow at U + (their rank among all
+// such slices), found by a binary search over a device scan of the per-list counts -- no read-back, and the host
+// bound U + ceil(nnz / 1024) covers them (a long list has fewer than len / 1024 slices beyond its first).
+// Only long lists stage: fewer than 2 nnz / 1024 slices of 8 k bytes, i.e. < nnz k / 64 bytes.
+// Segments are clamped to [0, nnz), so a malformed rowptr cannot make any kernel leave its arrays.
+
+__device__ __forceinline__ void list_bounds(const int64_t* __restrict__ rowptr, int64_t u, int64_t nnz, int64_t& b,
+                                            int64_t& e) {
+  b = __ldg(rowptr + u);
+  e = __ldg(rowptr + u + 1);
+  b = b < 0 ? 0 : (b > nnz ? nnz : b);
+  e = e < b ? b : (e > nnz ? nnz : e);
+}
+
+// off[u] (u = 0 .. U): low 32 bits = staged slices of the long lists before u, high 32 bits = long lists before u; the
+// slices 1.. of long list u are then work items U + (low - high) ..  One CTA, 4096 lists per round.
+__global__ void __launch_bounds__(1024) topk_lists_scan_kernel(const int64_t* __restrict__ rowptr, int64_t U, int64_t nnz,
+                                                               unsigned long long* __restrict__ off) {
+  __shared__ unsigned long long warp_tot[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned long long carry = 0;
+  for (int64_t base = 0; base <= U; base += 4 * 1024) {
+    unsigned long long v[4], t = 0;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int64_t u = base + 4 * threadIdx.x + q;
+      v[q] = 0;
+      if (u < U) {
+        int64_t b, e;
+        list_bounds(rowptr, u, nnz, b, e);
+        if (e - b > kTopkMinSlice) v[q] = (1ull << 32) | (unsigned)topk_slices((int32_t)(e - b));
+      }
+      t += v[q];
+    }
+    unsigned long long x = t;  // inclusive warp scan of the thread totals
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (lane == 31) warp_tot[warp] = x;
+    __syncthreads();
+    if (warp == 0) {
+      unsigned long long w = warp_tot[lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long y = __shfl_up_sync(0xffffffffu, w, o);
+        if (lane >= o) w += y;
+      }
+      warp_tot[lane] = w;  // inclusive over warps
+    }
+    __syncthreads();
+    unsigned long long run = carry + (warp > 0 ? warp_tot[warp - 1] : 0ull) + x - t;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int64_t u = base + 4 * threadIdx.x + q;
+      if (u <= U) off[u] = run;
+      run += v[q];
+    }
+    carry += warp_tot[31];
+    __syncthreads();
+  }
+}
+
+__device__ __forceinline__ int64_t lists_extra(unsigned long long o) { return (int64_t)(uint32_t)o - (int64_t)(o >> 32); }
+
+// Final outputs of slot i of list u (list start b, length len) from key m.
+__device__ __forceinline__ void lists_emit(const TopkListsArgs& a, int64_t u, int64_t b, int i, unsigned long long m,
+                                           bool bad_u) {
+  const int p = (m == kNoKey || bad_u) ? -1 : (int)(uint32_t)m;
+  const size_t o = (size_t)u * a.k + i;
+  if (a.top_pos != nullptr) a.top_pos[o] = p;
+  if (a.top_items != nullptr) a.top_items[o] = p < 0 ? -1 : __ldg(a.items + b + p);
+  if (a.top_scores != nullptr) a.top_scores[o] = p < 0 ? nanf("") : __ldg(a.scores + b + p);
+}
+
+__global__ void __launch_bounds__(kTopkThreads) topk_lists_slice_kernel(const TopkListsArgs a, int cap,
+                                                                        const unsigned long long* __restrict__ off,
+                                                                        unsigned long long* __restrict__ stage,
+                                                                        int32_t* __restrict__ counts, int32_t* __restrict__ pos) {
+  extern __shared__ unsigned long long topk_smem[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned long long* buf = topk_smem + (size_t)warp * cap;
+  const int64_t w = (int64_t)blockIdx.x * (kTopkThreads / 32) + warp;
+  const int64_t U = a.U;
+  int64_t u;
+  int s;
+  if (w < U) {
+    u = w;
+    s = 0;
+  } else {  // slice >= 1 of a long list: the last u whose extra slices start at or before e (warp-uniform search)
+    const int64_t e = w - U;
+    if (e >= lists_extra(off[U])) return;
+    int64_t lo = 0, hi = U - 1;
+    while (lo < hi) {
+      const int64_t mid = (lo + hi + 1) >> 1;
+      if (lists_extra(off[mid]) <= e) lo = mid;
+      else hi = mid - 1;
+    }
+    u = lo;
+    s = 1 + (int)(e - lists_extra(off[u]));
+  }
+  int64_t b, e;
+  list_bounds(a.rowptr, u, a.nnz, b, e);
+  const int len = (int)(e - b), k = a.k;
+  const bool is_long = len > kTopkMinSlice;
+  const int slice = is_long ? topk_slice_len(len) : kTopkMinSlice;
+  const int lo = s * slice, hi = min(len, lo + slice);
+  const float* sc = a.scores + b;
+  const int t = a.targets != nullptr ? __ldg(a.targets + u) : -1;
+  const bool has_t = (unsigned)t < (unsigned)len;
+  const unsigned long long key_t = has_t ? topk_key(__ldg(sc + t), t) : 0ull;
+  int below = 0, n = 0;
+  unsigned long long thr = kNoKey;
+  for (int c = lo; c < hi; c += 32) {
+    const int j = c + lane;
+    const unsigned long long key = j < hi ? topk_key(__ldg(sc + j), j) : kNoKey;
+    below += (has_t && key < key_t) ? 1 : 0;
+    topk_push(buf, n, thr, key, cap, k, lane);
+  }
+  n = topk_flush(buf, n, cap, k, lane);
+  below = warp_sum_int(below);
+  if (is_long) {
+    const size_t slot = (uint32_t)off[u] + s;
+    unsigned long long* out = stage + slot * k;
+    for (int i = lane; i < k; i += 32) out[i] = i < n ? buf[i] : kNoKey;
+    if (lane == 0) counts[slot] = below;
+    return;
+  }
+  const bool bad_u = a.users != nullptr && (unsigned)__ldg(a.users + u) >= (unsigned)a.num_users;
+  for (int i = lane; i < k; i += 32) lists_emit(a, u, b, i, i < n ? buf[i] : kNoKey, bad_u);
+  if (pos != nullptr && lane == 0) pos[u] = (bad_u || !has_t) ? len : below;
+}
+
+__global__ void __launch_bounds__(kTopkThreads) topk_lists_merge_kernel(const TopkListsArgs a,
+                                                                        const unsigned long long* __restrict__ off,
+                                                                        const unsigned long long* __restrict__ stage,
+                                                                        const int32_t* __restrict__ counts,
+                                                                        int32_t* __restrict__ pos) {
+  const int lane = threadIdx.x & 31;
+  const int64_t u = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (u >= a.U) return;  // warp-uniform
+  int64_t b, e;
+  list_bounds(a.rowptr, u, a.nnz, b, e);
+  const int len = (int)(e - b);
+  if (len <= kTopkMinSlice) return;  // finished by its slice warp
+  const int S = topk_slices(len), k = a.k;
+  const size_t slot0 = (uint32_t)off[u];
+  const bool bad_u = a.users != nullptr && (unsigned)__ldg(a.users + u) >= (unsigned)a.num_users;
+  topk_merge_warp(stage + slot0 * k, S, k, lane, [&](int i, unsigned long long m) { lists_emit(a, u, b, i, m, bad_u); });
+  if (pos != nullptr) {
+    const int c = warp_sum_int(lane < S ? counts[slot0 + lane] : 0);
+    const int t = a.targets != nullptr ? __ldg(a.targets + u) : -1;
+    if (lane == 0) pos[u] = (bad_u || (unsigned)t >= (unsigned)len) ? len : c;
+  }
+}
+
+static int64_t lists_stage_slots(int64_t nnz) { return (nnz + 511) / 512; }  // > the staged slices of any rowptr
+
+size_t topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k) {
+  const size_t slots = (size_t)lists_stage_slots(nnz);
+  return align_up((size_t)(U + 1) * sizeof(unsigned long long), 256) + align_up((size_t)U * sizeof(int32_t), 256) +
+         align_up(slots * k * sizeof(unsigned long long), 256) + align_up(slots * sizeof(int32_t), 256);
+}
+
+int launch_topk_lists(const TopkListsArgs& a, float* sums, void* ws, cudaStream_t st) {
+  Carver cv(ws);
+  unsigned long long* off = cv.take<unsigned long long>((size_t)a.U + 1);
+  int32_t* pos_buf = cv.take<int32_t>((size_t)a.U);
+  const size_t slots = (size_t)lists_stage_slots(a.nnz);
+  unsigned long long* stage = cv.take<unsigned long long>(slots * a.k);
+  int32_t* counts = cv.take<int32_t>(slots);
+  int32_t* pos = a.pos != nullptr ? a.pos : (sums != nullptr ? pos_buf : nullptr);
+  if (a.U > 0) {
+    const int cap = topk_cap(a.k), wpc = kTopkThreads / 32;
+    const size_t smem = (size_t)wpc * cap * sizeof(unsigned long long);
+    const int64_t warps = a.U + (a.nnz + kTopkMinSlice - 1) / kTopkMinSlice;
+    topk_lists_scan_kernel<<<1, 1024, 0, st>>>(a.rowptr, a.U, a.nnz, off);
+    MR_LAUNCH_CHECK("topk_lists_scan_kernel");
+    topk_lists_slice_kernel<<<(unsigned)((warps + wpc - 1) / wpc), kTopkThreads, smem, st>>>(a, cap, off, stage, counts,
+                                                                                             pos);
+    MR_LAUNCH_CHECK("topk_lists_slice_kernel");
+    topk_lists_merge_kernel<<<(unsigned)((a.U + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, off, stage, counts, pos);
+    MR_LAUNCH_CHECK("topk_lists_merge_kernel");
+  }
+  return launch_topk_metrics(pos, a.U, a.k, sums, st);
+}
+
+// seg[r] = the list holding row r (the last u with rowptr[u] <= r, clamped to [0, U)), or users[that list] when
+// `users` is given.  One CTA per 1024 rows: two searches bound the lists of the CTA's rows, then each thread searches
+// only between them.
+__device__ __forceinline__ int64_t list_of_row(const int64_t* __restrict__ rowptr, int64_t lo, int64_t hi, int64_t r) {
+  while (lo < hi) {  // the last u in [lo, hi] with rowptr[u] <= r (lo when none)
+    const int64_t mid = (lo + hi + 1) >> 1;
+    if (__ldg(rowptr + mid) <= r) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(1024) list_rows_kernel(const int64_t* __restrict__ rowptr, int64_t U, int64_t nnz,
+                                                         const int32_t* __restrict__ users, int32_t* __restrict__ seg) {
+  __shared__ int64_t bounds[2];
+  const int64_t r0 = (int64_t)blockIdx.x * 1024, r1 = min(nnz, r0 + 1024) - 1;
+  if (threadIdx.x < 2) bounds[threadIdx.x] = list_of_row(rowptr, 0, U - 1, threadIdx.x == 0 ? r0 : r1);
+  __syncthreads();
+  const int64_t r = r0 + threadIdx.x;
+  if (r > r1) return;
+  int64_t lo = bounds[0], hi = bounds[1];
+  if (hi < lo) {  // (only a malformed rowptr)
+    lo = 0;
+    hi = U - 1;
+  }
+  const int64_t u = list_of_row(rowptr, lo, hi, r);
+  seg[r] = users != nullptr ? __ldg(users + u) : (int32_t)u;
+}
+
+int launch_list_rows(const int64_t* rowptr, int64_t U, int64_t nnz, const int32_t* users, int32_t* seg, cudaStream_t st) {
+  if (nnz == 0 || U == 0) return MR_OK;
+  list_rows_kernel<<<(unsigned)((nnz + 1023) / 1024), 1024, 0, st>>>(rowptr, U, nnz, users, seg);
+  MR_LAUNCH_CHECK("list_rows_kernel");
   return MR_OK;
 }
 

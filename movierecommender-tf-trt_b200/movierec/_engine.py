@@ -560,6 +560,48 @@ class NeuMFEngine(object):
         self.last_catalogue_bad = bad
         return top_items, top_scores, pos, sums, full
 
+    def rank_lists(self, users, lists, k, targets=None, want_probs=False):
+        """Score and rank ragged candidate lists in one call (mr_rank_lists): list u pairs users[u] with
+        items[rowptr[u]:rowptr[u + 1]].  lists = (rowptr int64 (U + 1,), items int32 (nnz,)), host or device; targets
+        (U,) are positions in the lists.  Returns device tensors (items (U, k) int32, scores (U, k) float32, top_pos
+        (U, k) int32 -- positions within the list --, pos (U,) int32 or None, sums (2,) float32 [hit_sum, dcg_sum] or
+        None, probs (nnz,) float32 or None); pos / sums need targets.  Order: descending probability, the earlier
+        position first among ties; slots beyond a list's length hold -1 / NaN.  Raises ValueError on a malformed
+        rowptr before any launch.  Leaves in `self.last_lists_bad` a one-element device tensor, non-zero when a user
+        or item id (or a target) was out of range."""
+        dev = self.device
+        users = as_device_i32(users, dev)
+        U = users.numel()
+        rowptr, items = _check_lists(lists, U, dev)
+        nnz = items.numel()
+        k = int(k)
+        t = as_device_i32(targets, dev) if targets is not None else None
+        if t is not None and t.numel() != U:
+            raise ValueError("targets ({}) and users ({}) differ in length".format(t.numel(), U))
+        top_pos = torch.empty((U, k), dtype=torch.int32, device=dev)
+        top_items = torch.empty((U, k), dtype=torch.int32, device=dev)
+        top_scores = torch.empty((U, k), dtype=torch.float32, device=dev)
+        pos = torch.empty(U, dtype=torch.int32, device=dev) if t is not None else None
+        sums = torch.zeros(2, dtype=torch.float32, device=dev) if t is not None else None
+        probs = torch.empty(nnz, dtype=torch.float32, device=dev) if want_probs else None
+        nbytes = int(nat.lib.mr_rank_lists_workspace_bytes(C.byref(self._model), U, nnz, k))
+        if nbytes == 0:
+            raise ValueError("rank_lists: bad sizes U={} nnz={} k={}".format(U, nnz, k))
+        ws = self._workspace(nbytes)
+        nat.check(nat.lib.mr_rank_lists(C.byref(self._model), _ptr(users), U, _ptr(rowptr), _ptr(items), nnz, k, _ptr(t),
+                                        _ptr(top_pos), _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums),
+                                        _ptr(probs), _ptr(ws), ws.numel(), self._stream()), "mr_rank_lists")
+        bad = torch.zeros(1, dtype=torch.float32, device=dev)
+        if U:
+            bad = bad + ((users.min() < 0) | (users.max() >= self.num_users)).to(torch.float32).reshape(1)
+        if nnz:
+            bad = bad + ((items.min() < 0) | (items.max() >= self.num_items)).to(torch.float32).reshape(1)
+        if t is not None and U:
+            lens = rowptr[1:] - rowptr[:-1]
+            bad = bad + ((t < 0) | (t.to(torch.int64) >= lens)).any().to(torch.float32).reshape(1)
+        self.last_lists_bad = bad
+        return top_items, top_scores, top_pos, pos, sums, probs
+
     def _ids_out_of_range(self, users, items):
         if users.numel() == 0:
             return torch.zeros(1, dtype=torch.float32, device=self.device)
@@ -705,6 +747,57 @@ def topk_scores(scores, k, exclude=None, excl_ids=None, targets=None, device=Non
                                      _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(ws), nbytes, st),
               "mr_topk_scores")
     return top_items, top_scores, pos, sums
+
+
+def _check_lists(lists, U, device):
+    """(rowptr, items) host or device -> device (int64 rowptr, int32 items); ValueError unless rowptr has U + 1 entries,
+    starts at 0, never decreases and ends at len(items)."""
+    rp, it = lists
+    items = as_device_i32(it, device)
+    nnz = items.numel()
+    if isinstance(rp, torch.Tensor) and rp.is_cuda:
+        rowptr = rp.reshape(-1).to(device, torch.int64).contiguous()
+        n = rowptr.numel()
+        ok = n == U + 1 and (n == 0 or bool(((rowptr[0] == 0) & (rowptr[-1] == nnz) &
+                                             ~(rowptr[1:] < rowptr[:-1]).any()).item()))
+    else:
+        h = (rp.numpy() if isinstance(rp, torch.Tensor) else np.asarray(rp)).reshape(-1).astype(np.int64)
+        ok = h.size == U + 1 and h[0] == 0 and h[-1] == nnz and bool(np.all(h[1:] >= h[:-1]))
+        rowptr = torch.from_numpy(np.ascontiguousarray(h)).to(device)
+    if not ok:
+        raise ValueError("lists: rowptr must have U + 1 = {} entries, start at 0, never decrease and end at len(items) = "
+                         "{}".format(U + 1, nnz))
+    return rowptr, items
+
+
+def topk_lists(scores, rowptr, k, targets=None, device=None):
+    """Top-k of ragged lists of scores (mr_topk_lists): list u is scores[rowptr[u]:rowptr[u + 1]], ordered by
+    descending score (NaN last, the earlier position first among ties).  targets (U,) are positions in the lists.
+    Returns device tensors (top_pos (U, k) int32, top_scores (U, k) float32, pos (U,) int32 or None, sums (2,) or
+    None); slots beyond a list's length hold -1 / NaN.  Raises ValueError on a malformed rowptr."""
+    require_cuda()
+    device = torch.device(device if device is not None else "cuda:{}".format(torch.cuda.current_device()))
+    s = as_device_f32(scores, device)
+    n = (rowptr.numel() if isinstance(rowptr, torch.Tensor) else np.asarray(rowptr).size)
+    U = max(int(n) - 1, 0)
+    rp, _ = _check_lists((rowptr, np.zeros(s.numel(), np.int32)), U, device)
+    nnz = s.numel()
+    k = int(k)
+    t = as_device_i32(targets, device) if targets is not None else None
+    if t is not None and t.numel() != U:
+        raise ValueError("targets ({}) and lists ({}) differ in length".format(t.numel(), U))
+    top_pos = torch.empty((U, k), dtype=torch.int32, device=device)
+    top_scores = torch.empty((U, k), dtype=torch.float32, device=device)
+    pos = torch.empty(U, dtype=torch.int32, device=device) if t is not None else None
+    sums = torch.zeros(2, dtype=torch.float32, device=device) if t is not None else None
+    nbytes = int(nat.lib.mr_topk_lists_workspace_bytes(U, nnz, k))
+    if nbytes == 0:
+        raise ValueError("topk_lists: bad sizes U={} nnz={} k={}".format(U, nnz, k))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+    nat.check(nat.lib.mr_topk_lists(_ptr(s), U, _ptr(rp), nnz, k, _ptr(t), _ptr(top_pos), _ptr(top_scores), _ptr(pos),
+                                    _ptr(sums), _ptr(ws), nbytes, st), "mr_topk_lists")
+    return top_pos, top_scores, pos, sums
 
 
 def gather_rows(table, idx):

@@ -90,6 +90,11 @@ SIGNATURES = {
     "mr_topk_scores": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_catalogue_topk_workspace_bytes": (_sz, [_PM, _i64, _i32]),
     "mr_catalogue_topk": (C.c_int, [_PM, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mr_topk_lists_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "mr_topk_lists": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mr_rank_lists_workspace_bytes": (_sz, [_PM, _i64, _i64, _i32]),
+    "mr_rank_lists": (C.c_int, [_PM, _vp, _i64, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                _vp]),
     "mr_sample_negatives": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i64, _i32, _u64, _u64, _vp, _vp, _vp, _vp]),
     "mr_sort_workspace_bytes": (_sz, [_i64]),
     "mr_sort_pairs": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _sz, _vp]),

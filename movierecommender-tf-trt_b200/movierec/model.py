@@ -178,6 +178,27 @@ class NeuMFModel(object):
         self._raise_on_bad_ids(float(eng.last_catalogue_bad.item()))
         return items.cpu().numpy(), scores.cpu().numpy()
 
+    def recommend_batch(self, users, candidate_lists, top_k=10):
+        """recommend() for many requests at once: user users[u] against its own candidate list, of any length.
+        candidate_lists: a list (or other sequence) of 1-D item arrays, one per user, or a tuple (rowptr, items) of
+        CSR offsets (U + 1) and concatenated items.  Returns NumPy (items (U, top_k) int32, scores (U, top_k) float32)
+        in the RankLayer order (descending score, the earlier candidate first among ties); slots beyond a list's
+        length hold -1 / NaN.  Raises IndexError on an out-of-range user or item.  Host offsets are cut into device
+        calls of whole lists of at most 2^22 candidates (a longer list is a call of its own)."""
+        users = np.asarray(users, dtype=np.int32).reshape(-1)
+        rowptr, items = _candidate_csr(candidate_lists, users.size)
+        eng = self.engine
+        self._raise_on_bad_ids(_ids_outside(users, eng.num_users) or _ids_outside(items, eng.num_items))
+        k = int(top_k)
+        out_items = np.full((users.size, k), -1, np.int32)
+        out_scores = np.full((users.size, k), np.nan, np.float32)
+        for lo, hi in _list_chunks(rowptr):
+            r0, r1 = int(rowptr[lo]), int(rowptr[hi])
+            top, sc, _, _, _, _ = eng.rank_lists(users[lo:hi], (rowptr[lo:hi + 1] - r0, items[r0:r1]), k)
+            out_items[lo:hi] = top.cpu().numpy()
+            out_scores[lo:hi] = sc.cpu().numpy()
+        return out_items, out_scores
+
     def _step_logs(self, out, rows, group):
         loss = out[0] / rows + out[3]
         return {"loss": loss, OUTPUT_PRED + "_loss": out[0] / rows,
@@ -596,6 +617,68 @@ class MovierecModel(object):
         self.model._raise_on_bad_ids(s[2])
         G = max(int(pos.numel()), 1)
         return s[0] / G, s[1] / G
+
+    def evaluate_candidate_lists(self, users, candidate_lists, targets, k=None):
+        """Ranking evaluation with a candidate list of its own size per user (e.g. users with fewer unseen items than
+        the negative count, or candidates from a retrieval stage): for user users[u], the candidate at position
+        targets[u] of its list is ranked among the whole list.  candidate_lists as NeuMFModel.recommend_batch.
+        Returns (hr, ndcg) at k (default: the model's k), like evaluate().  Raises IndexError on an out-of-range user,
+        item or target position."""
+        k = self._k if k is None else k
+        import torch
+        users = np.asarray(users, dtype=np.int32).reshape(-1)
+        targets = np.asarray(targets, dtype=np.int32).reshape(-1)
+        if targets.size != users.size:
+            raise ValueError("targets ({}) and users ({}) differ in length".format(targets.size, users.size))
+        rowptr, items = _candidate_csr(candidate_lists, users.size)
+        eng = self.model.engine
+        self.model._raise_on_bad_ids(_ids_outside(users, eng.num_users) or _ids_outside(items, eng.num_items) or
+                                     bool(np.any((targets < 0) | (targets >= rowptr[1:] - rowptr[:-1]))))
+        sums = []
+        for lo, hi in _list_chunks(rowptr):
+            r0, r1 = int(rowptr[lo]), int(rowptr[hi])
+            sums.append(eng.rank_lists(users[lo:hi], (rowptr[lo:hi + 1] - r0, items[r0:r1]), k,
+                                       targets=targets[lo:hi])[4])
+        total = torch.stack(sums).cpu().numpy().astype(np.float64).sum(axis=0)  # chunk order
+        G = max(int(users.size), 1)
+        return total[0] / G, total[1] / G
+
+
+LISTS_CALL_ROWS = 1 << 22  # candidates per device call of recommend_batch / evaluate_candidate_lists
+
+
+def _candidate_csr(candidate_lists, U):
+    """A (rowptr, items) tuple or a sequence of 1-D item arrays -> host (rowptr int64 (U + 1,), items int32)."""
+    if isinstance(candidate_lists, tuple) and len(candidate_lists) == 2:
+        rp, it = candidate_lists
+        rowptr = np.asarray(rp.cpu() if hasattr(rp, "cpu") else rp, dtype=np.int64).reshape(-1)
+        items = np.asarray(it.cpu() if hasattr(it, "cpu") else it, dtype=np.int32).reshape(-1)
+    else:
+        parts = [np.asarray(x, dtype=np.int32).reshape(-1) for x in candidate_lists]
+        rowptr = np.zeros(len(parts) + 1, np.int64)
+        rowptr[1:] = np.cumsum([p.size for p in parts])
+        items = np.concatenate(parts) if parts else np.zeros(0, np.int32)
+    if rowptr.size != U + 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
+        raise ValueError("candidate lists: expected {} lists with offsets starting at 0, never decreasing and ending at "
+                         "{}".format(U, items.size))
+    return rowptr, items
+
+
+def _ids_outside(ids, limit):
+    return bool(ids.size) and bool(ids.min() < 0 or ids.max() >= limit)
+
+
+def _list_chunks(rowptr, max_rows=None):
+    """[lo, hi) ranges of whole lists of at most max_rows candidates each (a longer list alone)."""
+    max_rows = LISTS_CALL_ROWS if max_rows is None else max_rows
+    U = rowptr.size - 1
+    out, lo = [], 0
+    while lo < U:
+        hi = int(np.searchsorted(rowptr, rowptr[lo] + max_rows, side="right")) - 1
+        hi = min(max(hi, lo + 1), U)
+        out.append((lo, hi))
+        lo = hi
+    return out or [(0, 0)]
 
 
 def _exclusion_lists(exclude):
