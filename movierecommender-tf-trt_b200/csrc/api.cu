@@ -332,79 +332,82 @@ static TcWs carve_tc(const MrModel& m, bool train, int64_t B, void* ws) {
   return t;
 }
 
+// First layer of a grouped batch, rows [r0, r1): the user half once per group, Zu = E_user[user of the group] .
+// W1[user rows] + b1, and the item half per row.  A train workspace (ReLU bits) writes H1 and its bits; an eval
+// workspace has no Pu.  The cases:
+//  - eval with Pi: Zu, then the second layer's producers read relu(Pi[item] + Zu[group]) (H1 never exists in memory);
+//  - train with Pu: H1 = relu(Pi[item] + Pu[user]), the user half once per USER;
+//  - train with Pi only: Zu, then H1 = relu(Pi[item] + Zu[group]);
+//  - eval or train without Pi: Zu, then H1 = relu(E_item[item] . W1[item rows] + Zu[group]).
+static int tc_grouped_first_layer(const MrModel& m, const TcWs& t, const int32_t* users, const int32_t* items, int64_t r0,
+                                  int64_t r1, int group, bool users_per_group, cudaStream_t st) {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+  const bool train = t.bits[1] != nullptr;
+  if (train && t.Pu != nullptr) {
+    prof_mark(MR_PHASE_H1_GATHER, st);
+    const int rc = launch_h1_from_projection(t.Pi, m.num_items, items, r0, r1 - r0, t.Pu, group, users, m.num_users,
+                                             m.L[1], t.H[1], t.bits[1], st);
+    if (rc == MR_OK) prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    return rc;
+  }
+  TcDenseArgs a{};
+  a.gather = true;
+  a.user_tab = m.user_mlp;
+  a.users = users;
+  a.num_users = m.num_users;
+  a.num_items = m.num_items;
+  a.d_u = d_u;
+  a.user_div = 1;
+  a.user_mul = users_per_group ? 1 : group;  // `users` holds one id per group, or one per row
+  a.b_packed = t.pack_fu;
+  a.N = m.L[1];
+  a.K = d_u;
+  a.rows = (r1 - r0) / group;
+  a.row0 = r0 / group;
+  a.epilogue = TC_EPI_BIAS_RELU;
+  a.bias = m.b[1];
+  a.linear = true;
+  a.out = t.Zu;
+  int rc = launch_tc_dense(a, st);
+  if (rc != MR_OK || (!train && t.Pi != nullptr)) return rc;
+  if (t.Pi != nullptr) {
+    prof_mark(MR_PHASE_H1_GATHER, st);
+    rc = launch_h1_from_projection(t.Pi, m.num_items, items, r0, r1 - r0, t.Zu, group, nullptr, 0, m.L[1], t.H[1],
+                                   t.bits[1], st);
+    if (rc == MR_OK) prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    return rc;
+  }
+  TcDenseArgs b{};
+  b.gather = true;
+  b.item_tab = m.item_mlp;
+  b.items = items;
+  b.num_users = m.num_users;
+  b.num_items = m.num_items;
+  b.d_u = 0;
+  b.user_div = 1;
+  b.b_packed = t.pack_fi;
+  b.N = m.L[1];
+  b.K = d_i;
+  b.rows = r1 - r0;
+  b.row0 = r0;
+  b.epilogue = TC_EPI_BIAS_RELU;
+  b.addend = t.Zu;
+  b.addend_div = group;
+  b.out = t.H[1];
+  b.bits_out = t.bits[1];
+  return launch_tc_dense(b, st);
+}
+
 // Forward of rows [r0, r1) on the tensor cores; leaves H[1..n-1] of the sub-batch in the workspace.
 static int tc_forward_rows(const MrModel& m, const TcWs& t, const int32_t* users, const int32_t* items, int user_div,
                            int64_t r0, int64_t r1, cudaStream_t st, int group = 0, bool users_per_group = false,
                            bool head_dot = false) {
   const int d_u = m.L[0] / 2;
-  bool proj_in_producer = false;
+  // the eval case of the grouped first layer whose H1 the second layer's producers compute
+  const bool proj_in_producer = group > 0 && t.bits[1] == nullptr && t.Pi != nullptr;
   if (group > 0) {
-    // grouped batch: Zu = E_user[user of the group] . W1[user rows] + b1 once per group, then
-    // H1 = relu(E_item[item] . W1[item rows] + Zu[row / group]) per row
-    const int d_i = m.L[0] - d_u;
-    // ranking eval: the producers of the second layer compute the projected first layer, H1 never exists in memory;
-    // the (unfused) train step keeps the separate gather kernel, which also writes the ReLU bits of H1
-    const bool train_rows = t.bits[1] != nullptr;
-    const bool fuse_h1 = t.Pi != nullptr && m.n_layers >= 3 && !train_rows;
-    proj_in_producer = fuse_h1;
-    if (fuse_h1 && t.Pu != nullptr) {
-    } else if (t.Pu != nullptr) {  // user- and item-projected first layer: H1 = relu(Pi[item] + Pu[user])
-      prof_mark(MR_PHASE_H1_GATHER, st);
-      const int rc = launch_h1_from_projection(t.Pi, m.num_items, items, r0, r1 - r0, t.Pu, group, users, m.num_users, m.L[1],
-                                               t.H[1], t.bits[1], st);
-      if (rc != MR_OK) return rc;
-      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    } else {
-    TcDenseArgs a{};
-    a.gather = true;
-    a.user_tab = m.user_mlp;
-    a.users = users;
-    a.num_users = m.num_users;
-    a.num_items = m.num_items;
-    a.d_u = d_u;
-    a.user_div = 1;
-    a.user_mul = users_per_group ? 1 : group;  // `users` holds one id per group, or one per row
-    a.b_packed = t.pack_fu;
-    a.N = m.L[1];
-    a.K = d_u;
-    a.rows = (r1 - r0) / group;
-    a.row0 = r0 / group;
-    a.epilogue = TC_EPI_BIAS_RELU;
-    a.bias = m.b[1];
-    a.linear = true;
-    a.out = t.Zu;
-    int rc = launch_tc_dense(a, st);
+    const int rc = tc_grouped_first_layer(m, t, users, items, r0, r1, group, users_per_group, st);
     if (rc != MR_OK) return rc;
-    if (fuse_h1) {
-    } else if (t.Pi != nullptr) {  // item-projected first layer: H1 = relu(Pi[item] + Zu[group])
-      prof_mark(MR_PHASE_H1_GATHER, st);
-      rc = launch_h1_from_projection(t.Pi, m.num_items, items, r0, r1 - r0, t.Zu, group, nullptr, 0, m.L[1], t.H[1],
-                                     t.bits[1], st);
-      if (rc != MR_OK) return rc;
-      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    } else {
-    TcDenseArgs b{};
-    b.gather = true;
-    b.item_tab = m.item_mlp;
-    b.items = items;
-    b.num_users = m.num_users;
-    b.num_items = m.num_items;
-    b.d_u = 0;
-    b.user_div = 1;
-    b.b_packed = t.pack_fi;
-    b.N = m.L[1];
-    b.K = d_i;
-    b.rows = r1 - r0;
-    b.row0 = r0;
-    b.epilogue = TC_EPI_BIAS_RELU;
-    b.addend = t.Zu;
-    b.addend_div = group;
-    b.out = t.H[1];
-    b.bits_out = t.bits[1];
-    rc = launch_tc_dense(b, st);
-    if (rc != MR_OK) return rc;
-    }
-    }
   }
   for (int l = group > 0 ? 2 : 1; l < m.n_layers; ++l) {
     TcDenseArgs a{};
@@ -432,11 +435,6 @@ static int tc_forward_rows(const MrModel& m, const TcWs& t, const int32_t* users
       a.proj_i = t.Pi;
       a.proj_u = t.Zu;
       a.proj_div = group;
-      if (t.Pu != nullptr) {  // one row per USER
-        a.proj_u = t.Pu;
-        a.proj_ids = users;
-        a.proj_u_rows = m.num_users;
-      }
     }
     if (head_dot && l == m.n_layers - 1) {  // H[l] then holds one float per row: relu(.) . w_out[MLP columns]
       a.epilogue = TC_EPI_HEAD_DOT;
@@ -478,6 +476,39 @@ static int tc_project_users(const MrModel& m, const TcWs& t, cudaStream_t st) {
   a.linear = true;
   a.out = t.Pu;
   return launch_tc_dense(a, st);
+}
+
+// Backward of one half of the first layer over its whole table E (rows x d), on the per-row sums S (rows x L1):
+// dE = S . W1h^T (pack_b: the packed backward operand of that half of W[1]), and d W1h = E^T . S plus, with db_partial,
+// d b1 = colsum(S) into the dense partial rows.  mark_phases: attribute the two launches to their phases on st.
+static int tc_table_backward(const MrModel& m, const float* E, const float* S, int64_t rows, int d, const float* pack_b,
+                             float* dE, float* dw_partial, float* db_partial, int64_t partial_stride, bool mark_phases,
+                             cudaStream_t st) {
+  if (mark_phases) prof_mark(MR_PHASE_TC_DENSE_BWD, st);
+  TcDenseArgs a{};
+  a.a_dense = S;
+  a.b_packed = pack_b;
+  a.N = d;
+  a.K = m.L[1];
+  a.rows = rows;
+  a.row0 = 0;
+  a.epilogue = TC_EPI_BIAS_RELU;
+  a.linear = true;
+  a.out = dE;
+  const int rc = launch_tc_dense(a, st);
+  if (rc != MR_OK) return rc;
+  if (mark_phases) prof_mark(MR_PHASE_TC_WGRAD, st);
+  TcWgradArgs w{};
+  w.a_dense = E;
+  w.z = S;
+  w.Fa = d;
+  w.Fb = m.L[1];
+  w.rows = rows;
+  w.row0 = 0;
+  w.dw_partial = dw_partial;
+  w.db_partial = db_partial;
+  w.partial_stride = partial_stride;
+  return launch_tc_wgrad(w, st);
 }
 
 struct TrainWs {
@@ -565,6 +596,596 @@ static int check_opt(const MrModel& m, const MrOptState* o, const MrGrads* g) {
     MR_REQUIRE(m.l2[0] == 0.f, "layers_l2reg[0] != 0 makes embedding gradients dense; use MR_TABLES_DENSE");
   }
   return MR_OK;
+}
+
+// ---- train step ----------------------------------------------------------------------------------------------------
+// Every launch-sequence choice of a step, made once by TrainStep::plan.  The tower runs as the projected tensor-core
+// tower's fused kernel, the tensor-core sub-batch loop, the default tower's projected step on CUDA cores, or the
+// generic tile kernel.
+enum { TRAIN_TC_FUSED = 0, TRAIN_TC = 1, TRAIN_SMALL = 2, TRAIN_TILES = 3 };
+struct TrainPlan {
+  int path;             // TRAIN_*
+  bool grouped;         // one user per group: the user side runs once per group (promise checked on the device)
+  bool proj, uproj;     // item / user half of the first layer once per item / user (item_proj_ok, user_proj_ok)
+  int64_t n_user_rows;  // staged user-gradient rows: one per group or one per row
+  // where the segmented reductions put the MLP part of their rows (dense table mode): the per-user / per-item sums
+  // of dZ[1] (L1 wide) on a projected side, the gradient table otherwise
+  float *user_sums, *item_sums;
+  TcWs tc;              // TRAIN_TC_FUSED, TRAIN_TC: Pi / Si and Pu / Su NULL on a side that is not projected
+  SmallWs small;        // TRAIN_SMALL
+};
+
+// One train step: the call's arguments, workspace, streams and plan.  Its parts run as prologue, tower, epilogue.
+struct TrainStep {
+  const MrModel& m;
+  const MrOptState& opt;
+  const MrGrads& grads;
+  const int32_t *users, *items;
+  const float* labels;
+  int64_t B;
+  int group, k, flags;
+  float inv_batch;
+  float* step_out;
+  TrainWs t;
+  SideStream* side;  // NULL when it could not be created: its work then runs on st
+  cudaStream_t st;
+  TrainPlan p;
+
+  TrainPlan plan() const;
+  int prologue() const;
+  int tower_tc() const;
+  int tc_sub_batches() const;
+  int tc_grouped_first_layer_backward(int64_t r0, int64_t r1) const;
+  template <class UserTables, class ItemTables>
+  int projected_backward(UserTables user_tables, ItemTables item_tables) const;
+  int tower_small() const;
+  int tower_tiles() const;
+  int epilogue() const;
+};
+
+TrainPlan TrainStep::plan() const {
+  const bool dense = opt.table_mode == MR_TABLES_DENSE;
+  const bool users_grouped = (flags & MR_TRAIN_USERS_GROUPED) != 0;
+  TrainPlan q{};
+  if (use_tc(m)) {
+    q.grouped = users_grouped && tc_grouped_ok(m, B, group);
+    q.proj = q.grouped && dense && item_proj_ok(m, B);
+    q.uproj = q.proj && user_proj_ok(m, B, group);
+    // The per-row work of the projected step in ONE kernel (tc_fused.cu): H1, the second layer forward, the head,
+    // the second layer's weight gradient and backward, the staged rows and their group sums never leave the SM.
+    const bool fused = q.uproj && m.fused_train != MR_FUSED_OFF && fused_train_supported(m, group);
+    q.path = fused ? TRAIN_TC_FUSED : TRAIN_TC;
+    q.tc = carve_tc(m, true, B, t.tc_ws);
+    if (!q.proj) q.tc.Pi = q.tc.Si = nullptr;
+    if (!q.uproj) q.tc.Pu = q.tc.Su = nullptr;
+  } else if (users_grouped && dense && small_proj_ok(m, B, group)) {
+    // default tower: both projections on CUDA cores, thread per group (small_tower.cu)
+    q.path = TRAIN_SMALL;
+    q.grouped = q.proj = q.uproj = true;
+    q.small = carve_small(m, t.small_ws);
+  } else {
+    q.path = TRAIN_TILES;
+  }
+  const bool small = q.path == TRAIN_SMALL;
+  q.user_sums = q.uproj ? (small ? q.small.Su : q.tc.Su) : grads.user_mlp;
+  q.item_sums = q.proj ? (small ? q.small.Si : q.tc.Si) : grads.item_mlp;
+  q.n_user_rows = q.grouped ? B / group : B;
+  return q;
+}
+
+// The l2 penalty, then on the side stream the clears of what the segmented reductions add into, the group check and
+// the stable sorts of the ids (the reductions' keys): they do not depend on the tower, so they run under it (phase
+// timing then sees only the launch cost of this block on the caller's stream).
+int TrainStep::prologue() const {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+  int rc = MR_OK;
+  prof_mark(MR_PHASE_MISC, st);
+  MR_CUDA(cudaMemsetAsync(t.flags, 0, 256, st));
+  MR_CUDA(cudaMemsetAsync(step_out, 0, MR_STEP_OUT_FLOATS * sizeof(float), st));
+  // l2 penalty of the step's weights: first, so that nothing reads the tables after grads->user_tables_ready
+  if (any_l2(m)) {
+    float* pen = step_out + MR_OUT_L2_PENALTY;
+    if (m.l2[0] != 0.f) {
+      rc = launch_l2_penalty(m.user_mlp, (int64_t)m.num_users * d_u, m.l2[0], pen, st);
+      if (rc == MR_OK) rc = launch_l2_penalty(m.item_mlp, (int64_t)m.num_items * d_i, m.l2[0], pen, st);
+      if (rc == MR_OK && m.mf_dim > 0) rc = launch_l2_penalty(m.user_gmf, (int64_t)m.num_users * m.mf_dim, m.l2[0], pen, st);
+      if (rc == MR_OK && m.mf_dim > 0) rc = launch_l2_penalty(m.item_gmf, (int64_t)m.num_items * m.mf_dim, m.l2[0], pen, st);
+      if (rc != MR_OK) return rc;
+    }
+    for (int l = 1; l < m.n_layers; ++l)
+      if (m.l2[l] != 0.f) {
+        rc = launch_l2_penalty(m.W[l], (int64_t)m.L[l - 1] * m.L[l], m.l2[l], pen, st);
+        if (rc != MR_OK) return rc;
+      }
+  }
+  cudaStream_t ss = st;
+  if (side != nullptr) {
+    MR_CUDA(cudaEventRecord(side->fork, st));
+    MR_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
+    ss = side->stream;
+  }
+  prof_mark(MR_PHASE_SORT, st);
+  if (opt.table_mode == MR_TABLES_DENSE) {  // (on a projected side a GEMM on the sums then writes the MLP table whole)
+    MR_CUDA(cudaMemsetAsync(p.user_sums, 0, (size_t)m.num_users * (p.uproj ? m.L[1] : d_u) * sizeof(float), ss));
+    MR_CUDA(cudaMemsetAsync(p.item_sums, 0, (size_t)m.num_items * (p.proj ? m.L[1] : d_i) * sizeof(float), ss));
+    if (m.mf_dim > 0) {
+      MR_CUDA(cudaMemsetAsync(grads.user_gmf, 0, (size_t)m.num_users * m.mf_dim * sizeof(float), ss));
+      MR_CUDA(cudaMemsetAsync(grads.item_gmf, 0, (size_t)m.num_items * m.mf_dim * sizeof(float), ss));
+    }
+  }
+  if (p.grouped) {
+    rc = launch_check_grouped(users, B, group, t.flags + 1, ss);
+    if (rc == MR_OK) rc = launch_group_heads(users, B / group, group, t.group_users, ss);
+    if (rc != MR_OK) return rc;
+  }
+  rc = sort_row_ids(p.grouped ? t.group_users : users, p.n_user_rows, m.num_users, t.sorted_keys, t.sorted_index,
+                    t.sort_ws, t.sort_ws_bytes, ss);
+  if (rc == MR_OK)
+    rc = sort_row_ids(items, B, m.num_items, t.sorted_keys_i, t.sorted_index_i, t.sort_ws, t.sort_ws_bytes, ss);
+  if (rc != MR_OK) return rc;
+  if (side != nullptr) MR_CUDA(cudaEventRecord(side->join, ss));
+  prof_mark(MR_PHASE_MISC, st);
+  return MR_OK;
+}
+
+// Backward of the projected first layer after the tower's per-row work: segment sums of the staged rows [dZ1 | GMF row
+// gradient] per item (the GMF part straight into its gradient table), then the tower's GEMMs over the item table on
+// them (item_tables, caller's stream); the same per user when the user half is projected (user_tables).  The two
+// chains are independent (disjoint buffers and columns of the dense partial rows): the user chain runs on the side
+// stream, so the latency-bound upper levels of one run under the other, and the user-side gradient tables (83 % of the table-gradient bytes at the ML-20M shape) are final while
+// the item side is still being reduced: a data-parallel caller starts their all-reduce on grads->user_tables_ready.
+template <class UserTables, class ItemTables>
+int TrainStep::projected_backward(UserTables user_tables, ItemTables item_tables) const {
+  if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join, 0));  // sorted keys, cleared sums and GMF tables
+  RowUpdate u{};
+  u.mode = MR_TABLES_DENSE;
+  u.optimizer = opt.optimizer;
+  u.d0 = m.L[1];
+  u.d1 = m.mf_dim;
+  if (p.uproj) {
+    cudaStream_t su = st;
+    if (side != nullptr) {
+      MR_CUDA(cudaEventRecord(side->fork2, st));
+      MR_CUDA(cudaStreamWaitEvent(side->stream, side->fork2, 0));
+      su = side->stream;
+    }
+    u.num_rows = m.num_users;
+    u.g0 = p.user_sums;
+    u.g1 = grads.user_gmf;
+    int rc = launch_segreduce(t.sorted_keys, t.sorted_index, p.n_user_rows, t.stage_u, u, t.seg_ws_u, t.seg_ws_u_bytes, su);
+    if (rc != MR_OK) return rc;
+    // user_gmf: gradients final, table last read by the tower
+    if (grads.user_gmf_ready != nullptr) MR_CUDA(cudaEventRecord((cudaEvent_t)grads.user_gmf_ready, su));
+    rc = user_tables(su);  // the step's last read of the user table, so it goes before the event
+    if (rc != MR_OK) return rc;
+    if (grads.user_tables_ready != nullptr) MR_CUDA(cudaEventRecord((cudaEvent_t)grads.user_tables_ready, su));
+    if (side != nullptr) MR_CUDA(cudaEventRecord(side->join2, su));
+  }
+  prof_mark(MR_PHASE_SEGREDUCE, st);
+  u.num_rows = m.num_items;
+  u.g0 = p.item_sums;
+  u.g1 = grads.item_gmf;
+  int rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, u, t.seg_ws, t.seg_ws_bytes, st);
+  if (rc == MR_OK) rc = item_tables();
+  if (rc != MR_OK) return rc;
+  if (p.uproj && side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join2, 0));
+  return MR_OK;
+}
+
+// First layer's backward of a grouped sub-batch, rows [r0, r1): the item half per row, the user half per group on
+// S1 = the group sums of dZ[1].  A projected half only stages its rows here; it runs on the per-item / per-user sums.
+int TrainStep::tc_grouped_first_layer_backward(int64_t r0, int64_t r1) const {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, f = m.mf_dim;
+  const TcWs& tw = p.tc;
+  const int64_t ng = (r1 - r0) / group, g0 = r0 / group;
+  int rc = MR_OK;
+  prof_mark(MR_PHASE_MISC, st);
+  if (p.uproj)
+    rc = launch_group_sum_rows(t.stage_i + (size_t)r0 * (d_i + f), ng, group, m.L[1],
+                               t.stage_u + (size_t)g0 * (d_u + f), st, d_i + f, d_u + f);
+  else if (p.proj)  // (columns [0, L1) of the item staging rows, stride d_i + f)
+    rc = launch_group_sum_rows(t.stage_i + (size_t)r0 * (d_i + f), ng, group, m.L[1], tw.S1, st, d_i + f);
+  else
+    rc = launch_group_sum_rows(tw.dZ[1], ng, group, m.L[1], tw.S1, st);
+  if (rc != MR_OK) return rc;
+  prof_mark(MR_PHASE_TC_WGRAD, st);
+  if (!p.proj) {
+    TcWgradArgs wi{};
+    wi.gather = true;
+    wi.item_tab = m.item_mlp;
+    wi.items = items;
+    wi.num_users = m.num_users;
+    wi.num_items = m.num_items;
+    wi.d_u = 0;
+    wi.z = tw.dZ[1];
+    wi.Fa = d_i;
+    wi.Fb = m.L[1];
+    wi.rows = r1 - r0;
+    wi.row0 = r0;
+    wi.dw_partial = t.dense_partial + (m.W[1] - m.dense) + (size_t)d_u * m.L[1];
+    wi.db_partial = t.dense_partial + (m.b[1] - m.dense);
+    wi.partial_stride = t.dense_stride;
+    rc = launch_tc_wgrad(wi, st);
+    if (rc != MR_OK) return rc;
+  }
+  if (p.uproj) return MR_OK;
+  TcWgradArgs wu{};
+  wu.gather = true;
+  wu.user_tab = m.user_mlp;
+  wu.users = users;
+  wu.num_users = m.num_users;
+  wu.num_items = m.num_items;
+  wu.d_u = d_u;
+  wu.user_mul = group;
+  wu.z = tw.S1;
+  wu.Fa = d_u;
+  wu.Fb = m.L[1];
+  wu.rows = ng;
+  wu.row0 = g0;
+  wu.dw_partial = t.dense_partial + (m.W[1] - m.dense);
+  // the bias gradient (column sums of dZ[1]) comes with the item half, or from the group sums when the item half runs
+  // per item
+  wu.db_partial = p.proj ? t.dense_partial + (m.b[1] - m.dense) : nullptr;
+  wu.partial_stride = t.dense_stride;
+  rc = launch_tc_wgrad(wu, st);
+  if (rc != MR_OK) return rc;
+  prof_mark(MR_PHASE_TC_DENSE_BWD, st);
+  if (!p.proj) {
+    TcDenseArgs bi{};
+    bi.a_dense = tw.dZ[1];
+    bi.d_u = 0;  // every output column belongs to the item row
+    bi.b_packed = tw.pack_bi;
+    bi.N = d_i;
+    bi.K = m.L[1];
+    bi.rows = r1 - r0;
+    bi.row0 = r0;
+    bi.epilogue = TC_EPI_STAGE;
+    bi.stage_u = t.stage_u;
+    bi.stage_i = t.stage_i;
+    bi.su = d_u + f;
+    bi.si = d_i + f;
+    rc = launch_tc_dense(bi, st);
+    if (rc != MR_OK) return rc;
+  }
+  TcDenseArgs bu{};
+  bu.a_dense = tw.S1;
+  bu.d_u = d_u;  // every output column belongs to the user row of the group
+  bu.b_packed = tw.pack_bu;
+  bu.N = d_u;
+  bu.K = m.L[1];
+  bu.rows = ng;
+  bu.row0 = g0;
+  bu.epilogue = TC_EPI_STAGE;
+  bu.stage_u = t.stage_u;
+  bu.stage_i = t.stage_i;
+  bu.su = d_u + f;
+  bu.si = d_i + f;
+  return launch_tc_dense(bu, st);
+}
+
+// Per sub-batch: forward layers -> head -> per layer weight gradient + backward.
+int TrainStep::tc_sub_batches() const {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, n = m.n_layers, f = m.mf_dim;
+  const TcWs& tw = p.tc;
+  const int gdiv = p.grouped ? group : 0;
+  const int64_t sb = tc_sub_batch(B);
+  for (int64_t r0 = 0; r0 < B; r0 += sb) {
+    const int64_t r1 = r0 + sb < B ? r0 + sb : B;
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    int rc = tc_forward_rows(m, tw, users, items, 1, r0, r1, st, gdiv);
+    if (rc != MR_OK) return rc;
+    prof_mark(MR_PHASE_HEAD, st);
+    HeadArgs h{};
+    h.model = &m;
+    h.h_last = tw.H[n - 1];
+    h.users = users;
+    h.items = items;
+    h.labels = labels;
+    h.rows = r1 - r0;
+    h.row0 = r0;
+    h.user_div = 1;
+    h.group = gdiv;
+    h.inv_batch = inv_batch;
+    h.probs = t.probs;
+    h.dz_last = tw.dZ[n - 1];
+    h.stage_u = t.stage_u;
+    h.stage_i = t.stage_i;
+    h.head_partial = tw.head_partial;
+    h.flags = t.flags;
+    rc = launch_head(h, st);
+    if (rc != MR_OK) return rc;
+    for (int l = n - 1; l >= (p.grouped ? 2 : 1); --l) {
+      prof_mark(MR_PHASE_TC_WGRAD, st);
+      TcWgradArgs w{};
+      w.gather = (l == 1);
+      w.a_dense = (l == 1) ? nullptr : tw.H[l - 1];
+      w.user_tab = m.user_mlp;
+      w.item_tab = m.item_mlp;
+      w.users = users;
+      w.items = items;
+      w.num_users = m.num_users;
+      w.num_items = m.num_items;
+      w.d_u = d_u;
+      w.z = tw.dZ[l];
+      w.Fa = m.L[l - 1];
+      w.Fb = m.L[l];
+      w.rows = r1 - r0;
+      w.row0 = r0;
+      w.dw_partial = t.dense_partial + (m.W[l] - m.dense);
+      w.db_partial = t.dense_partial + (m.b[l] - m.dense);
+      w.partial_stride = t.dense_stride;
+      rc = launch_tc_wgrad(w, st);
+      if (rc != MR_OK) return rc;
+      prof_mark(MR_PHASE_TC_DENSE_BWD, st);
+      TcDenseArgs a{};
+      a.gather = false;
+      a.a_dense = tw.dZ[l];
+      a.d_u = d_u;
+      a.b_packed = tw.pack_b[l];
+      a.N = m.L[l - 1];
+      a.K = m.L[l];
+      a.rows = r1 - r0;
+      a.row0 = r0;
+      if (l - 1 >= 1) {
+        a.epilogue = TC_EPI_MASK;
+        a.mask_bits = tw.bits[l - 1];
+        a.out = tw.dZ[l - 1];
+        if (p.proj && l - 1 == 1) {  // dZ[1] goes straight into the item staging rows: the keys of its per-item sums
+          a.out = t.stage_i + (size_t)r0 * (d_i + f);
+          a.out_ld = d_i + f;
+        }
+      } else {
+        a.epilogue = TC_EPI_STAGE;
+        a.stage_u = t.stage_u;
+        a.stage_i = t.stage_i;
+        a.su = d_u + f;
+        a.si = d_i + f;
+      }
+      rc = launch_tc_dense(a, st);
+      if (rc != MR_OK) return rc;
+    }
+    if (p.grouped) {
+      rc = tc_grouped_first_layer_backward(r0, r1);
+      if (rc != MR_OK) return rc;
+    }
+  }
+  return MR_OK;
+}
+
+// ---- tensor-core tower: the fused kernel or the sub-batch loop, then the projected first layer's backward on its
+// per-item / per-user sums and the reductions of the dense partial rows
+int TrainStep::tower_tc() const {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, n = m.n_layers, f = m.mf_dim;
+  const TcWs& tw = p.tc;
+  const bool fused = p.path == TRAIN_TC_FUSED;
+  const int P = sm_count();  // rows of the partial buffer = CTAs of the weight-gradient kernel
+  int rc = MR_OK;
+  MR_CUDA(cudaMemsetAsync(t.dense_partial, 0, (size_t)P * t.dense_stride * sizeof(float), st));
+  if (!fused) {  // (the fused kernel packs its own operand image of W[2] and keeps the head's sums itself)
+    MR_CUDA(cudaMemsetAsync(tw.head_partial, 0, head_partial_floats(m) * sizeof(float), st));
+    for (int l = p.grouped ? 2 : 1; l < n; ++l) {
+      rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, tw.pack_f[l], st);
+      if (rc == MR_OK) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 1, tw.pack_b[l], st);
+      if (rc != MR_OK) return rc;
+    }
+  }
+  if (p.grouped) {  // W[1] is (L0, L1) row-major: rows [0, d_u) multiply the user row, rows [d_u, L0) the item row
+    const float* Wu = m.W[1];
+    const float* Wi = m.W[1] + (size_t)d_u * m.L[1];
+    rc = launch_pack_weights(Wu, d_u, m.L[1], 0, tw.pack_fu, st);
+    if (rc == MR_OK) rc = launch_pack_weights(Wi, d_i, m.L[1], 0, tw.pack_fi, st);
+    if (rc == MR_OK) rc = launch_pack_weights(Wu, d_u, m.L[1], 1, tw.pack_bu, st);
+    if (rc == MR_OK) rc = launch_pack_weights(Wi, d_i, m.L[1], 1, tw.pack_bi, st);
+    if (rc != MR_OK) return rc;
+  }
+  if (p.proj) {
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    rc = tc_project_items(m, tw, st);
+    if (rc == MR_OK && p.uproj) rc = tc_project_users(m, tw, st);
+    if (rc != MR_OK) return rc;
+  }
+  int fused_grid = 0;
+  if (fused) {
+    prof_mark(MR_PHASE_FUSED_TILE, st);
+    FusedTrainArgs fa{};
+    fa.Pi = tw.Pi;
+    fa.Pu = tw.Pu;
+    fa.user_gmf = m.user_gmf;
+    fa.item_gmf = m.item_gmf;
+    fa.users = users;
+    fa.items = items;
+    fa.labels = labels;
+    fa.num_users = m.num_users;
+    fa.num_items = m.num_items;
+    fa.rows = B;
+    fa.group = group;
+    fa.W2 = m.W[2];
+    fa.w2_image = tw.w2_image;
+    fa.b2 = m.b[2];
+    fa.w_out = m.w_out;
+    fa.b_out = m.b_out;
+    fa.inv_batch = inv_batch;
+    fa.probs = t.probs;
+    fa.stage_i = t.stage_i;
+    fa.stage_u = t.stage_u;
+    fa.si = d_i + f;
+    fa.su = d_u + f;
+    fa.partial = t.dense_partial;
+    fa.partial_stride = t.dense_stride;
+    fa.off_w2 = m.W[2] - m.dense;
+    fa.off_b2 = m.b[2] - m.dense;
+    fa.off_wout = m.w_out - m.dense;
+    fa.off_bout = m.b_out - m.dense;
+    fa.loss_partial = t.loss_partial;
+    fa.flags = t.flags;
+    rc = launch_fused_train(fa, st, &fused_grid);
+  } else {
+    rc = tc_sub_batches();
+  }
+  if (rc != MR_OK) return rc;
+  if (p.proj) {
+    float* dw1 = t.dense_partial + (m.W[1] - m.dense);
+    rc = projected_backward(
+        [&](cudaStream_t su) {
+          return tc_table_backward(m, m.user_mlp, tw.Su, m.num_users, d_u, tw.pack_bu, grads.user_mlp, dw1,
+                                   t.dense_partial + (m.b[1] - m.dense), t.dense_stride, false, su);
+        },
+        [&] {
+          return tc_table_backward(m, m.item_mlp, tw.Si, m.num_items, d_i, tw.pack_bi, grads.item_mlp,
+                                   dw1 + (size_t)d_u * m.L[1], nullptr, t.dense_stride, true, st);
+        });
+    if (rc != MR_OK) return rc;
+  }
+  prof_mark(MR_PHASE_MISC, st);
+  if (fused)  // (its d w_out / d b_out partials sit in the CTAs' rows of the dense partial buffer already)
+    rc = launch_sum_partials(t.loss_partial, fused_grid, step_out + MR_OUT_LOSS_SUM, st);
+  else
+    rc = launch_head_reduce(m, tw.head_partial, t.dense_partial + (m.w_out - m.dense),
+                            t.dense_partial + (m.b_out - m.dense), step_out + MR_OUT_LOSS_SUM, st);
+  if (rc != MR_OK) return rc;
+  return launch_dense_reduce(m, t.dense_partial, t.dense_stride, P, grads.dense, st, !(flags & MR_TRAIN_NO_DENSE_L2));
+}
+
+// ---- default tower, projected: Pi / Pu over the tables, one thread-per-group kernel for everything per row,
+// segment sums of the staged rows per item / per user, then the first layer's backward on the sums
+int TrainStep::tower_small() const {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1], cap = max_tile_ctas();
+  const SmallWs& w = p.small;
+  const float* W1u = m.W[1];
+  const float* W1i = m.W[1] + (size_t)d_u * L1;
+  MR_CUDA(cudaMemsetAsync(t.dense_partial, 0, (size_t)cap * t.dense_stride * sizeof(float), st));
+  prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+  int rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, W1i, L1, L1, false, nullptr, w.Pi, st);
+  if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, W1u, L1, L1, false, m.b[1], w.Pu, st);
+  if (rc != MR_OK) return rc;
+  SmallTowerArgs a{};
+  a.model = &m;
+  a.Pi = w.Pi;
+  a.Pu = w.Pu;
+  a.users = users;
+  a.items = items;
+  a.labels = labels;
+  a.B = B;
+  a.inv_batch = inv_batch;
+  a.probs = t.probs;
+  a.stage_i = t.stage_i;
+  a.stage_u = t.stage_u;
+  a.dense_partial = t.dense_partial;
+  a.dense_stride = t.dense_stride;
+  a.loss_partial = t.loss_partial;
+  a.flags = t.flags;
+  a.max_ctas = cap;
+  int grid = 0, grid_i = 0, grid_u = 0;
+  prof_mark(MR_PHASE_FUSED_TILE, st);
+  rc = launch_small_tower_train(a, st, &grid);
+  if (rc != MR_OK) return rc;
+  rc = projected_backward(
+      [&](cudaStream_t su) {  // d E_user = Su . W1u^T, d W1u = E_user^T . Su, d b1 = colsum(Su)
+        int r = launch_small_rows_gemm(w.Su, m.num_users, L1, W1u, L1, d_u, true, nullptr, grads.user_mlp, su);
+        if (r == MR_OK)
+          r = launch_small_table_wgrad(m.user_mlp, w.Su, m.num_users, t.dense_partial + (W1u - m.dense),
+                                       t.dense_partial + (m.b[1] - m.dense), t.dense_stride, cap, su, &grid_u);
+        return r;
+      },
+      [&] {
+        prof_mark(MR_PHASE_TC_DENSE_BWD, st);  // d E_item = Si . W1i^T over the table
+        int r = launch_small_rows_gemm(w.Si, m.num_items, L1, W1i, L1, d_i, true, nullptr, grads.item_mlp, st);
+        if (r != MR_OK) return r;
+        prof_mark(MR_PHASE_TC_WGRAD, st);  // d W1i = E_item^T . Si
+        return launch_small_table_wgrad(m.item_mlp, w.Si, m.num_items, t.dense_partial + (W1i - m.dense), nullptr,
+                                        t.dense_stride, cap, st, &grid_i);
+      });
+  if (rc != MR_OK) return rc;
+  prof_mark(MR_PHASE_MISC, st);
+  const int nrows = grid > grid_i ? (grid > grid_u ? grid : grid_u) : (grid_i > grid_u ? grid_i : grid_u);
+  rc = launch_dense_reduce(m, t.dense_partial, t.dense_stride, nrows, grads.dense, st, !(flags & MR_TRAIN_NO_DENSE_L2));
+  if (rc != MR_OK) return rc;
+  return launch_sum_partials(t.loss_partial, grid, step_out + MR_OUT_LOSS_SUM, st);
+}
+
+// ---- generic tile kernel: the whole per-row step on CUDA cores
+int TrainStep::tower_tiles() const {
+  int rc = launch_transpose_kernels(m, t.wt, st);
+  if (rc != MR_OK) return rc;
+  TileLaunch a{};
+  a.model = &m;
+  a.train = true;
+  a.wt = t.wt;
+  a.users = users;
+  a.items = items;
+  a.labels = labels;
+  a.B = B;
+  a.user_div = 1;
+  a.inv_batch = inv_batch;
+  a.probs = t.probs;
+  a.loss_partial = t.loss_partial;
+  a.dense_partial = t.dense_partial;
+  a.dense_stride = t.dense_stride;
+  a.stage_u = t.stage_u;
+  a.stage_i = t.stage_i;
+  a.flags = t.flags;
+  int grid = 0;
+  prof_mark(MR_PHASE_TILE_TRAIN, st);
+  rc = launch_neumf_tiles(a, st, &grid);
+  prof_mark(MR_PHASE_MISC, st);
+  if (rc != MR_OK) return rc;
+  rc = launch_dense_reduce(m, t.dense_partial, t.dense_stride, grid, grads.dense, st, !(flags & MR_TRAIN_NO_DENSE_L2));
+  if (rc != MR_OK) return rc;
+  return launch_sum_partials(t.loss_partial, grid, step_out + MR_OUT_LOSS_SUM, st);
+}
+
+// The bad-id flag, the ranking of grouped batches, the embedding rows of the sides not projected (stable sort by row
+// id, segmented reduce in batch order, row update) and, unless a projected user side recorded them, the events.
+int TrainStep::epilogue() const {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+  int rc = MR_OK;
+  if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join, 0));  // sorts and the group check are done
+  flag_to_float_kernel<<<1, 1, 0, st>>>(t.flags, step_out + MR_OUT_BAD_IDS);
+  MR_LAUNCH_CHECK("flag_to_float_kernel");
+
+  if (group > 0) {
+    prof_mark(MR_PHASE_RANK, st);
+    // label column = argmax of the group's labels (model.py:447-448): any layout of the positive is ranked right
+    rc = launch_rank_scores(t.probs, B / group, group, k, nullptr, nullptr, t.pos, step_out + MR_OUT_HIT_SUM,
+                            t.rank_partials, st, labels);
+    if (rc != MR_OK) return rc;
+  }
+  prof_mark(MR_PHASE_MISC, st);
+
+  RowUpdate u{};
+  u.mode = opt.table_mode;
+  u.optimizer = opt.optimizer;
+  u.lr = opt.lr;
+  u.lr_t = opt.optimizer == MR_OPT_ADAM ? adam_lr_t(opt, opt.iterations + 1) : opt.lr;
+  u.beta_1 = opt.beta_1;
+  u.beta_2 = opt.beta_2;
+  u.epsilon = opt.epsilon;
+  // users
+  u.d0 = d_u;
+  u.d1 = m.mf_dim;
+  u.num_rows = m.num_users;
+  u.p0 = m.user_mlp; u.m0 = opt.m_user_mlp; u.v0 = opt.v_user_mlp; u.g0 = grads.user_mlp;
+  u.p1 = m.user_gmf; u.m1 = opt.m_user_gmf; u.v1 = opt.v_user_gmf; u.g1 = grads.user_gmf;
+  if (!p.uproj) {
+    prof_mark(MR_PHASE_SEGREDUCE, st);
+    rc = launch_segreduce(t.sorted_keys, t.sorted_index, p.n_user_rows, t.stage_u, u, t.seg_ws, t.seg_ws_bytes, st);
+    if (rc != MR_OK) return rc;
+  }
+  // items
+  u.d0 = d_i;
+  u.num_rows = m.num_items;
+  u.p0 = m.item_mlp; u.m0 = opt.m_item_mlp; u.v0 = opt.v_item_mlp; u.g0 = grads.item_mlp;
+  u.p1 = m.item_gmf; u.m1 = opt.m_item_gmf; u.v1 = opt.v_item_gmf; u.g1 = grads.item_gmf;
+  if (!p.proj) {
+    prof_mark(MR_PHASE_SEGREDUCE, st);
+    rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, u, t.seg_ws, t.seg_ws_bytes, st);
+  }
+  if (!p.uproj) {  // the user side's gradients are final only now
+    if (grads.user_gmf_ready != nullptr) MR_CUDA(cudaEventRecord((cudaEvent_t)grads.user_gmf_ready, st));
+    if (grads.user_tables_ready != nullptr) MR_CUDA(cudaEventRecord((cudaEvent_t)grads.user_tables_ready, st));
+  }
+  prof_mark(-1, st);
+  return rc;
 }
 
 // ---- fused ranking evaluation on the tensor-core path -----------------------------------------------------
@@ -920,640 +1541,18 @@ int mr_neumf_train_grads(MrModel* model, MrOptState* opt, MrGrads* grads, const 
     set_error("train workspace too small: %zu < %zu", ws_bytes, mr_train_workspace_bytes(model, B));
     return MR_ERR_WORKSPACE;
   }
-  const MrModel& m = *model;
-  cudaStream_t st = (cudaStream_t)stream;
-  TrainWs t = carve_train(m, B, ws);
-  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
-  bool user_event_recorded = false;  // grads->user_tables_ready: recorded early where the launch sequence allows
-  bool user_gmf_event_recorded = false;  // grads->user_gmf_ready likewise
-
-  prof_mark(MR_PHASE_MISC, st);
-  MR_CUDA(cudaMemsetAsync(t.flags, 0, 256, st));
-  MR_CUDA(cudaMemsetAsync(step_out, 0, MR_STEP_OUT_FLOATS * sizeof(float), st));
-  // l2 penalty of the step's weights: first, so that nothing reads the tables after grads->user_tables_ready
-  if (any_l2(m)) {
-    float* pen = step_out + MR_OUT_L2_PENALTY;
-    if (m.l2[0] != 0.f) {
-      rc = launch_l2_penalty(m.user_mlp, (int64_t)m.num_users * d_u, m.l2[0], pen, st);
-      if (rc == MR_OK) rc = launch_l2_penalty(m.item_mlp, (int64_t)m.num_items * d_i, m.l2[0], pen, st);
-      if (rc == MR_OK && m.mf_dim > 0) rc = launch_l2_penalty(m.user_gmf, (int64_t)m.num_users * m.mf_dim, m.l2[0], pen, st);
-      if (rc == MR_OK && m.mf_dim > 0) rc = launch_l2_penalty(m.item_gmf, (int64_t)m.num_items * m.mf_dim, m.l2[0], pen, st);
-      if (rc != MR_OK) return rc;
-    }
-    for (int l = 1; l < m.n_layers; ++l)
-      if (m.l2[l] != 0.f) {
-        rc = launch_l2_penalty(m.W[l], (int64_t)m.L[l - 1] * m.L[l], m.l2[l], pen, st);
-        if (rc != MR_OK) return rc;
-      }
-  }
-
-  // grouped batch (MR_TRAIN_USERS_GROUPED): user-only work once per group; the promise is checked on the device
-  const bool grouped = (flags & MR_TRAIN_USERS_GROUPED) && use_tc(m) && tc_grouped_ok(m, B, group);
-  const int gdiv = grouped ? group : 0;
-  // item-projected first layer: item half of the first layer once per item (see item_proj_ok)
-  const bool proj = grouped && opt->table_mode == MR_TABLES_DENSE && item_proj_ok(m, B);
-  const bool uproj = proj && user_proj_ok(m, B, group);
-  // default tower: both projections on CUDA cores, thread per group (small_tower.cu)
-  const bool small = (flags & MR_TRAIN_USERS_GROUPED) && opt->table_mode == MR_TABLES_DENSE && small_proj_ok(m, B, group);
-  const bool by_group = grouped || small;
-  const int64_t n_user_rows = by_group ? B / group : B;  // staged user-gradient rows: one per group or one per row
-  // stable sorts of the ids (keys of the segmented reductions below) on the side stream, under the tower
-  // (phase timing then sees only the launch cost of this block on the main stream)
-  SideStream* side = side_stream();
-  {
-    cudaStream_t ss = st;
-    if (side != nullptr) {
-      MR_CUDA(cudaEventRecord(side->fork, st));
-      MR_CUDA(cudaStreamWaitEvent(side->stream, side->fork, 0));
-      ss = side->stream;
-    }
-    prof_mark(MR_PHASE_SORT, st);
-    if (opt->table_mode == MR_TABLES_DENSE) {  // the gradient tables the segmented reductions write into
-      if (uproj)
-        MR_CUDA(cudaMemsetAsync(carve_tc(m, true, B, t.tc_ws).Su, 0, (size_t)m.num_users * m.L[1] * sizeof(float), ss));
-      else if (small)
-        MR_CUDA(cudaMemsetAsync(carve_small(m, t.small_ws).Su, 0, (size_t)m.num_users * m.L[1] * sizeof(float), ss));
-      else
-        MR_CUDA(cudaMemsetAsync(grads->user_mlp, 0, (size_t)m.num_users * d_u * sizeof(float), ss));
-      if (proj)  // the per-item sums of dZ[1]; grads->item_mlp is then written whole by a GEMM on them
-        MR_CUDA(cudaMemsetAsync(carve_tc(m, true, B, t.tc_ws).Si, 0, (size_t)m.num_items * m.L[1] * sizeof(float), ss));
-      else if (small)
-        MR_CUDA(cudaMemsetAsync(carve_small(m, t.small_ws).Si, 0, (size_t)m.num_items * m.L[1] * sizeof(float), ss));
-      else
-        MR_CUDA(cudaMemsetAsync(grads->item_mlp, 0, (size_t)m.num_items * d_i * sizeof(float), ss));
-      if (m.mf_dim > 0) {
-        MR_CUDA(cudaMemsetAsync(grads->user_gmf, 0, (size_t)m.num_users * m.mf_dim * sizeof(float), ss));
-        MR_CUDA(cudaMemsetAsync(grads->item_gmf, 0, (size_t)m.num_items * m.mf_dim * sizeof(float), ss));
-      }
-    }
-    if (by_group) {
-      rc = launch_check_grouped(users, B, group, t.flags + 1, ss);
-      if (rc == MR_OK) rc = launch_group_heads(users, B / group, group, t.group_users, ss);
-      if (rc != MR_OK) return rc;
-    }
-    rc = sort_row_ids(by_group ? t.group_users : users, n_user_rows, m.num_users, t.sorted_keys, t.sorted_index,
-                      t.sort_ws, t.sort_ws_bytes, ss);
-    if (rc == MR_OK)
-      rc = sort_row_ids(items, B, m.num_items, t.sorted_keys_i, t.sorted_index_i, t.sort_ws, t.sort_ws_bytes, ss);
-    if (rc != MR_OK) return rc;
-    if (side != nullptr) MR_CUDA(cudaEventRecord(side->join, ss));
-    prof_mark(MR_PHASE_MISC, st);
-  }
-  if (use_tc(m)) {
-    // ---- tensor-core path: per sub-batch, forward layers -> head -> per layer weight gradient + backward
-    const int P = sm_count();  // rows of the partial buffer = CTAs of the weight-gradient kernel
-    const int n = m.n_layers, f = m.mf_dim;
-    TcWs tw = carve_tc(m, true, B, t.tc_ws);
-    if (!proj) tw.Pi = tw.Si = nullptr;
-    if (!uproj) tw.Pu = tw.Su = nullptr;
-    // The per-row work of the projected step in ONE kernel (tc_fused.cu): H1, the second layer forward, the head,
-    // the second layer's weight gradient and backward, the staged rows and their group sums never leave the SM.
-    const bool fused = uproj && m.fused_train != MR_FUSED_OFF && fused_train_supported(m, group);
-    MR_CUDA(cudaMemsetAsync(t.dense_partial, 0, (size_t)P * t.dense_stride * sizeof(float), st));
-    if (!fused) {  // (the fused kernel packs its own operand image of W[2] and keeps the head's sums itself)
-      MR_CUDA(cudaMemsetAsync(tw.head_partial, 0, head_partial_floats(m) * sizeof(float), st));
-      for (int l = grouped ? 2 : 1; l < n; ++l) {
-        rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, tw.pack_f[l], st);
-        if (rc == MR_OK) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 1, tw.pack_b[l], st);
-        if (rc != MR_OK) return rc;
-      }
-    }
-    if (grouped) {  // W[1] is (L0, L1) row-major: rows [0, d_u) multiply the user row, rows [d_u, L0) the item row
-      const float* Wu = m.W[1];
-      const float* Wi = m.W[1] + (size_t)d_u * m.L[1];
-      rc = launch_pack_weights(Wu, d_u, m.L[1], 0, tw.pack_fu, st);
-      if (rc == MR_OK) rc = launch_pack_weights(Wi, d_i, m.L[1], 0, tw.pack_fi, st);
-      if (rc == MR_OK) rc = launch_pack_weights(Wu, d_u, m.L[1], 1, tw.pack_bu, st);
-      if (rc == MR_OK) rc = launch_pack_weights(Wi, d_i, m.L[1], 1, tw.pack_bi, st);
-      if (rc != MR_OK) return rc;
-    }
-    if (proj) {
-      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-      rc = tc_project_items(m, tw, st);
-      if (rc == MR_OK && uproj) rc = tc_project_users(m, tw, st);
-      if (rc != MR_OK) return rc;
-    }
-    int fused_grid = 0;
-    if (fused) {
-      prof_mark(MR_PHASE_FUSED_TILE, st);
-      FusedTrainArgs fa{};
-      fa.Pi = tw.Pi;
-      fa.Pu = tw.Pu;
-      fa.user_gmf = m.user_gmf;
-      fa.item_gmf = m.item_gmf;
-      fa.users = users;
-      fa.items = items;
-      fa.labels = labels;
-      fa.num_users = m.num_users;
-      fa.num_items = m.num_items;
-      fa.rows = B;
-      fa.group = group;
-      fa.W2 = m.W[2];
-      fa.w2_image = tw.w2_image;
-      fa.b2 = m.b[2];
-      fa.w_out = m.w_out;
-      fa.b_out = m.b_out;
-      fa.inv_batch = inv_global_batch;
-      fa.probs = t.probs;
-      fa.stage_i = t.stage_i;
-      fa.stage_u = t.stage_u;
-      fa.si = d_i + f;
-      fa.su = d_u + f;
-      fa.partial = t.dense_partial;
-      fa.partial_stride = t.dense_stride;
-      fa.off_w2 = m.W[2] - m.dense;
-      fa.off_b2 = m.b[2] - m.dense;
-      fa.off_wout = m.w_out - m.dense;
-      fa.off_bout = m.b_out - m.dense;
-      fa.loss_partial = t.loss_partial;
-      fa.flags = t.flags;
-      rc = launch_fused_train(fa, st, &fused_grid);
-      if (rc != MR_OK) return rc;
-    }
-    const int64_t sb = tc_sub_batch(B);
-    for (int64_t r0 = 0; r0 < B && !fused; r0 += sb) {
-      const int64_t r1 = r0 + sb < B ? r0 + sb : B;
-      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-      rc = tc_forward_rows(m, tw, users, items, 1, r0, r1, st, gdiv);
-      if (rc != MR_OK) return rc;
-      prof_mark(MR_PHASE_HEAD, st);
-      HeadArgs h{};
-      h.model = model;
-      h.h_last = tw.H[n - 1];
-      h.users = users;
-      h.items = items;
-      h.labels = labels;
-      h.rows = r1 - r0;
-      h.row0 = r0;
-      h.user_div = 1;
-      h.group = gdiv;
-      h.inv_batch = inv_global_batch;
-      h.probs = t.probs;
-      h.dz_last = tw.dZ[n - 1];
-      h.stage_u = t.stage_u;
-      h.stage_i = t.stage_i;
-      h.head_partial = tw.head_partial;
-      h.flags = t.flags;
-      rc = launch_head(h, st);
-      if (rc != MR_OK) return rc;
-      for (int l = n - 1; l >= 1; --l) {
-        if (grouped && l == 1) {
-          // first layer of a grouped batch: item half per row, user half per group on S1 = group sums of dZ[1]
-          const int64_t ng = (r1 - r0) / group, g0 = r0 / group;
-          prof_mark(MR_PHASE_MISC, st);
-          if (uproj)  // ... and their group sums go to the user staging rows: the user half runs on per-user sums
-            rc = launch_group_sum_rows(t.stage_i + (size_t)r0 * (d_i + f), ng, group, m.L[1],
-                                       t.stage_u + (size_t)g0 * (d_u + f), st, d_i + f, d_u + f);
-          else if (proj)  // dZ[1] of these rows sits in the item staging rows (columns [0, L1), stride d_i + f)
-            rc = launch_group_sum_rows(t.stage_i + (size_t)r0 * (d_i + f), ng, group, m.L[1], tw.S1, st, d_i + f);
-          else
-            rc = launch_group_sum_rows(tw.dZ[1], ng, group, m.L[1], tw.S1, st);
-          if (rc != MR_OK) return rc;
-          prof_mark(MR_PHASE_TC_WGRAD, st);
-          if (!proj) {
-          TcWgradArgs wi{};
-          wi.gather = true;
-          wi.item_tab = m.item_mlp;
-          wi.items = items;
-          wi.num_users = m.num_users;
-          wi.num_items = m.num_items;
-          wi.d_u = 0;
-          wi.z = tw.dZ[1];
-          wi.Fa = d_i;
-          wi.Fb = m.L[1];
-          wi.rows = r1 - r0;
-          wi.row0 = r0;
-          wi.dw_partial = t.dense_partial + (m.W[1] - m.dense) + (size_t)d_u * m.L[1];
-          wi.db_partial = t.dense_partial + (m.b[1] - m.dense);
-          wi.partial_stride = t.dense_stride;
-          rc = launch_tc_wgrad(wi, st);
-          if (rc != MR_OK) return rc;
-          }
-          if (uproj) continue;
-          TcWgradArgs wu{};
-          wu.gather = true;
-          wu.user_tab = m.user_mlp;
-          wu.users = users;
-          wu.num_users = m.num_users;
-          wu.num_items = m.num_items;
-          wu.d_u = d_u;
-          wu.user_mul = group;
-          wu.z = tw.S1;
-          wu.Fa = d_u;
-          wu.Fb = m.L[1];
-          wu.rows = ng;
-          wu.row0 = g0;
-          wu.dw_partial = t.dense_partial + (m.W[1] - m.dense);
-          // the bias gradient (column sums of dZ[1]) comes with the item half, or from the group sums when the
-          // item half runs per item
-          wu.db_partial = proj ? t.dense_partial + (m.b[1] - m.dense) : nullptr;
-          wu.partial_stride = t.dense_stride;
-          rc = launch_tc_wgrad(wu, st);
-          if (rc != MR_OK) return rc;
-          prof_mark(MR_PHASE_TC_DENSE_BWD, st);
-          if (!proj) {
-          TcDenseArgs bi{};
-          bi.a_dense = tw.dZ[1];
-          bi.d_u = 0;  // every output column belongs to the item row
-          bi.b_packed = tw.pack_bi;
-          bi.N = d_i;
-          bi.K = m.L[1];
-          bi.rows = r1 - r0;
-          bi.row0 = r0;
-          bi.epilogue = TC_EPI_STAGE;
-          bi.stage_u = t.stage_u;
-          bi.stage_i = t.stage_i;
-          bi.su = d_u + f;
-          bi.si = d_i + f;
-          rc = launch_tc_dense(bi, st);
-          if (rc != MR_OK) return rc;
-          }
-          TcDenseArgs bu{};
-          bu.a_dense = tw.S1;
-          bu.d_u = d_u;  // every output column belongs to the user row of the group
-          bu.b_packed = tw.pack_bu;
-          bu.N = d_u;
-          bu.K = m.L[1];
-          bu.rows = ng;
-          bu.row0 = g0;
-          bu.epilogue = TC_EPI_STAGE;
-          bu.stage_u = t.stage_u;
-          bu.stage_i = t.stage_i;
-          bu.su = d_u + f;
-          bu.si = d_i + f;
-          rc = launch_tc_dense(bu, st);
-          if (rc != MR_OK) return rc;
-          continue;
-        }
-        prof_mark(MR_PHASE_TC_WGRAD, st);
-        TcWgradArgs w{};
-        w.gather = (l == 1);
-        w.a_dense = (l == 1) ? nullptr : tw.H[l - 1];
-        w.user_tab = m.user_mlp;
-        w.item_tab = m.item_mlp;
-        w.users = users;
-        w.items = items;
-        w.num_users = m.num_users;
-        w.num_items = m.num_items;
-        w.d_u = d_u;
-        w.z = tw.dZ[l];
-        w.Fa = m.L[l - 1];
-        w.Fb = m.L[l];
-        w.rows = r1 - r0;
-        w.row0 = r0;
-        w.dw_partial = t.dense_partial + (m.W[l] - m.dense);
-        w.db_partial = t.dense_partial + (m.b[l] - m.dense);
-        w.partial_stride = t.dense_stride;
-        rc = launch_tc_wgrad(w, st);
-        if (rc != MR_OK) return rc;
-        prof_mark(MR_PHASE_TC_DENSE_BWD, st);
-        TcDenseArgs a{};
-        a.gather = false;
-        a.a_dense = tw.dZ[l];
-        a.d_u = d_u;
-        a.b_packed = tw.pack_b[l];
-        a.N = m.L[l - 1];
-        a.K = m.L[l];
-        a.rows = r1 - r0;
-        a.row0 = r0;
-        if (l - 1 >= 1) {
-          a.epilogue = TC_EPI_MASK;
-          a.mask_bits = tw.bits[l - 1];
-          a.out = tw.dZ[l - 1];
-          if (proj && l - 1 == 1) {  // dZ[1] goes straight into the item staging rows: the keys of its per-item sums
-            a.out = t.stage_i + (size_t)r0 * (d_i + f);
-            a.out_ld = d_i + f;
-          }
-        } else {
-          a.epilogue = TC_EPI_STAGE;
-          a.stage_u = t.stage_u;
-          a.stage_i = t.stage_i;
-          a.su = d_u + f;
-          a.si = d_i + f;
-        }
-        rc = launch_tc_dense(a, st);
-        if (rc != MR_OK) return rc;
-      }
-    }
-    if (proj) {
-      // item half of the first layer's backward on per-item sums: Si = segment sums of [dZ1 | GMF row gradient] by
-      // item (GMF part straight into its gradient table), then d E_item = Si . W1i^T and d W1i = E_item^T . Si
-      if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join, 0));
-      RowUpdate ui{};
-      ui.mode = MR_TABLES_DENSE;
-      ui.optimizer = opt->optimizer;
-      ui.d0 = m.L[1];
-      ui.d1 = f;
-      ui.num_rows = m.num_items;
-      ui.g0 = tw.Si;
-      ui.g1 = grads->item_gmf;
-      // the two reductions are independent: the user side runs on the side stream, so the latency-bound upper
-      // levels of one chain (20 us launches of a few CTAs) run under the other chain
-      cudaStream_t su_st = st;
-      if (uproj && side != nullptr) {
-        MR_CUDA(cudaEventRecord(side->fork2, st));
-        MR_CUDA(cudaStreamWaitEvent(side->stream, side->fork2, 0));
-        su_st = side->stream;
-      }
-      if (uproj && su_st != st) {
-        RowUpdate uu{};
-        uu.mode = MR_TABLES_DENSE;
-        uu.optimizer = opt->optimizer;
-        uu.d0 = m.L[1];
-        uu.d1 = f;
-        uu.num_rows = m.num_users;
-        uu.g0 = tw.Su;
-        uu.g1 = grads->user_gmf;
-        rc = launch_segreduce(t.sorted_keys, t.sorted_index, n_user_rows, t.stage_u, uu, t.seg_ws_u, t.seg_ws_u_bytes, su_st);
-        if (rc != MR_OK) return rc;
-        if (grads->user_gmf_ready != nullptr) {  // user_gmf: gradients final, table last read by the fused kernel
-          MR_CUDA(cudaEventRecord((cudaEvent_t)grads->user_gmf_ready, su_st));
-          user_gmf_event_recorded = true;
-        }
-        // d E_user = Su . W1u^T right behind it on the side stream: both user-side gradient tables (83 % of the
-        // table-gradient bytes at the ML-20M shape) are then final while the item side is still being reduced, and
-        // a data-parallel caller starts their all-reduce on grads->user_tables_ready
-        TcDenseArgs bu{};
-        bu.a_dense = tw.Su;
-        bu.b_packed = tw.pack_bu;
-        bu.N = d_u;
-        bu.K = m.L[1];
-        bu.rows = m.num_users;
-        bu.row0 = 0;
-        bu.epilogue = TC_EPI_BIAS_RELU;
-        bu.linear = true;
-        bu.out = grads->user_mlp;
-        rc = launch_tc_dense(bu, su_st);
-        if (rc != MR_OK) return rc;
-        // d W1u = E_user^T . Su, d b1 = colsum(Su): the step's last read of the user table, so it goes before the event
-        // (its columns of the partial buffer are disjoint from the item half's, which the caller's stream adds to)
-        TcWgradArgs wu{};
-        wu.a_dense = m.user_mlp;
-        wu.z = tw.Su;
-        wu.Fa = d_u;
-        wu.Fb = m.L[1];
-        wu.rows = m.num_users;
-        wu.row0 = 0;
-        wu.dw_partial = t.dense_partial + (m.W[1] - m.dense);
-        wu.db_partial = t.dense_partial + (m.b[1] - m.dense);
-        wu.partial_stride = t.dense_stride;
-        rc = launch_tc_wgrad(wu, su_st);
-        if (rc != MR_OK) return rc;
-        if (grads->user_tables_ready != nullptr) {
-          MR_CUDA(cudaEventRecord((cudaEvent_t)grads->user_tables_ready, su_st));
-          user_event_recorded = true;
-        }
-        MR_CUDA(cudaEventRecord(side->join2, su_st));
-      }
-      prof_mark(MR_PHASE_SEGREDUCE, st);
-      rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, ui, t.seg_ws, t.seg_ws_bytes, st);
-      if (rc != MR_OK) return rc;
-      if (uproj && su_st == st) {  // per-user sums of [group sums of dZ1 | GMF row gradient]
-        RowUpdate uu{};
-        uu.mode = MR_TABLES_DENSE;
-        uu.optimizer = opt->optimizer;
-        uu.d0 = m.L[1];
-        uu.d1 = f;
-        uu.num_rows = m.num_users;
-        uu.g0 = tw.Su;
-        uu.g1 = grads->user_gmf;
-        prof_mark(MR_PHASE_SEGREDUCE, st);
-        rc = launch_segreduce(t.sorted_keys, t.sorted_index, n_user_rows, t.stage_u, uu, t.seg_ws, t.seg_ws_bytes, st);
-        if (rc != MR_OK) return rc;
-      }
-      prof_mark(MR_PHASE_TC_DENSE_BWD, st);
-      TcDenseArgs bi{};
-      bi.a_dense = tw.Si;
-      bi.b_packed = tw.pack_bi;
-      bi.N = d_i;
-      bi.K = m.L[1];
-      bi.rows = m.num_items;
-      bi.row0 = 0;
-      bi.epilogue = TC_EPI_BIAS_RELU;
-      bi.linear = true;
-      bi.out = grads->item_mlp;
-      rc = launch_tc_dense(bi, st);
-      if (rc != MR_OK) return rc;
-      prof_mark(MR_PHASE_TC_WGRAD, st);
-      TcWgradArgs wi{};
-      wi.a_dense = m.item_mlp;
-      wi.z = tw.Si;
-      wi.Fa = d_i;
-      wi.Fb = m.L[1];
-      wi.rows = m.num_items;
-      wi.row0 = 0;
-      wi.dw_partial = t.dense_partial + (m.W[1] - m.dense) + (size_t)d_u * m.L[1];
-      wi.db_partial = nullptr;
-      wi.partial_stride = t.dense_stride;
-      rc = launch_tc_wgrad(wi, st);
-      if (rc != MR_OK) return rc;
-      if (uproj && su_st != st) MR_CUDA(cudaStreamWaitEvent(st, side->join2, 0));
-      if (uproj && su_st == st) {  // without a side stream: d E_user = Su . W1u^T, d W1u = E_user^T . Su, d b1 here
-        {
-          prof_mark(MR_PHASE_TC_DENSE_BWD, st);
-          TcDenseArgs bu{};
-          bu.a_dense = tw.Su;
-          bu.b_packed = tw.pack_bu;
-          bu.N = d_u;
-          bu.K = m.L[1];
-          bu.rows = m.num_users;
-          bu.row0 = 0;
-          bu.epilogue = TC_EPI_BIAS_RELU;
-          bu.linear = true;
-          bu.out = grads->user_mlp;
-          rc = launch_tc_dense(bu, st);
-          if (rc != MR_OK) return rc;
-        }
-        prof_mark(MR_PHASE_TC_WGRAD, st);
-        TcWgradArgs wu{};
-        wu.a_dense = m.user_mlp;
-        wu.z = tw.Su;
-        wu.Fa = d_u;
-        wu.Fb = m.L[1];
-        wu.rows = m.num_users;
-        wu.row0 = 0;
-        wu.dw_partial = t.dense_partial + (m.W[1] - m.dense);
-        wu.db_partial = t.dense_partial + (m.b[1] - m.dense);
-        wu.partial_stride = t.dense_stride;
-        rc = launch_tc_wgrad(wu, st);
-        if (rc != MR_OK) return rc;
-      }
-    }
-    prof_mark(MR_PHASE_MISC, st);
-    if (fused)  // (its d w_out / d b_out partials sit in the CTAs' rows of the dense partial buffer already)
-      rc = launch_sum_partials(t.loss_partial, fused_grid, step_out + MR_OUT_LOSS_SUM, st);
-    else
-      rc = launch_head_reduce(m, tw.head_partial, t.dense_partial + (m.w_out - m.dense),
-                              t.dense_partial + (m.b_out - m.dense), step_out + MR_OUT_LOSS_SUM, st);
-    if (rc != MR_OK) return rc;
-    rc = launch_dense_reduce(m, t.dense_partial, t.dense_stride, P, grads->dense, st, !(flags & MR_TRAIN_NO_DENSE_L2));
-    if (rc != MR_OK) return rc;
-  } else if (small) {
-    // ---- default tower, projected: Pi / Pu over the tables, one thread-per-group kernel for everything per row,
-    // segment sums of the staged rows per item / per user, then the first layer's backward on the sums
-    const int L1 = m.L[1], f = m.mf_dim, cap = max_tile_ctas();
-    const SmallWs w = carve_small(m, t.small_ws);
-    const float* W1u = m.W[1];
-    const float* W1i = m.W[1] + (size_t)d_u * L1;
-    MR_CUDA(cudaMemsetAsync(t.dense_partial, 0, (size_t)cap * t.dense_stride * sizeof(float), st));
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, W1i, L1, L1, false, nullptr, w.Pi, st);
-    if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, W1u, L1, L1, false, m.b[1], w.Pu, st);
-    if (rc != MR_OK) return rc;
-    SmallTowerArgs a{};
-    a.model = model;
-    a.Pi = w.Pi;
-    a.Pu = w.Pu;
-    a.users = users;
-    a.items = items;
-    a.labels = labels;
-    a.B = B;
-    a.inv_batch = inv_global_batch;
-    a.probs = t.probs;
-    a.stage_i = t.stage_i;
-    a.stage_u = t.stage_u;
-    a.dense_partial = t.dense_partial;
-    a.dense_stride = t.dense_stride;
-    a.loss_partial = t.loss_partial;
-    a.flags = t.flags;
-    a.max_ctas = cap;
-    int grid = 0, grid_i = 0, grid_u = 0;
-    prof_mark(MR_PHASE_FUSED_TILE, st);
-    rc = launch_small_tower_train(a, st, &grid);
-    if (rc != MR_OK) return rc;
-    if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join, 0));  // sorted keys, cleared Si / Su / GMF tables
-    // the user-side chain (per-user sums, d E_user, d W1u / d b1) runs on the side stream next to the item-side one:
-    // both are short launches whose cost is latency, not bytes
-    cudaStream_t su_st = st;
-    if (side != nullptr) {
-      MR_CUDA(cudaEventRecord(side->fork2, st));
-      MR_CUDA(cudaStreamWaitEvent(side->stream, side->fork2, 0));
-      su_st = side->stream;
-    }
-    RowUpdate ru{};
-    ru.mode = MR_TABLES_DENSE;
-    ru.optimizer = opt->optimizer;
-    ru.d0 = L1;
-    ru.d1 = f;
-    ru.num_rows = m.num_users;
-    ru.g0 = w.Su;
-    ru.g1 = grads->user_gmf;
-    rc = launch_segreduce(t.sorted_keys, t.sorted_index, n_user_rows, t.stage_u, ru, t.seg_ws_u, t.seg_ws_u_bytes, su_st);
-    if (rc == MR_OK && su_st != st && grads->user_gmf_ready != nullptr) {
-      MR_CUDA(cudaEventRecord((cudaEvent_t)grads->user_gmf_ready, su_st));
-      user_gmf_event_recorded = true;
-    }
-    if (rc == MR_OK) rc = launch_small_rows_gemm(w.Su, m.num_users, L1, W1u, L1, d_u, true, nullptr, grads->user_mlp, su_st);
-    if (rc == MR_OK)
-      rc = launch_small_table_wgrad(m.user_mlp, w.Su, m.num_users, t.dense_partial + (W1u - m.dense),
-                                    t.dense_partial + (m.b[1] - m.dense), t.dense_stride, cap, su_st, &grid_u);
-    if (rc != MR_OK) return rc;
-    if (su_st != st) {
-      if (grads->user_tables_ready != nullptr) {  // gradients final, user tables no longer read
-        MR_CUDA(cudaEventRecord((cudaEvent_t)grads->user_tables_ready, su_st));
-        user_event_recorded = true;
-      }
-      MR_CUDA(cudaEventRecord(side->join2, su_st));
-    }
-    prof_mark(MR_PHASE_SEGREDUCE, st);
-    ru.num_rows = m.num_items;
-    ru.g0 = w.Si;
-    ru.g1 = grads->item_gmf;
-    rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, ru, t.seg_ws, t.seg_ws_bytes, st);
-    if (rc != MR_OK) return rc;
-    prof_mark(MR_PHASE_TC_DENSE_BWD, st);  // d E_item = Si . W1i^T over the table
-    rc = launch_small_rows_gemm(w.Si, m.num_items, L1, W1i, L1, d_i, true, nullptr, grads->item_mlp, st);
-    if (rc != MR_OK) return rc;
-    prof_mark(MR_PHASE_TC_WGRAD, st);  // d W1i = E_item^T . Si
-    rc = launch_small_table_wgrad(m.item_mlp, w.Si, m.num_items, t.dense_partial + (W1i - m.dense), nullptr,
-                                  t.dense_stride, cap, st, &grid_i);
-    if (rc != MR_OK) return rc;
-    if (su_st != st) MR_CUDA(cudaStreamWaitEvent(st, side->join2, 0));
-    prof_mark(MR_PHASE_MISC, st);
-    const int nrows = grid > grid_i ? (grid > grid_u ? grid : grid_u) : (grid_i > grid_u ? grid_i : grid_u);
-    rc = launch_dense_reduce(m, t.dense_partial, t.dense_stride, nrows, grads->dense, st, !(flags & MR_TRAIN_NO_DENSE_L2));
-    if (rc != MR_OK) return rc;
-    rc = launch_sum_partials(t.loss_partial, grid, step_out + MR_OUT_LOSS_SUM, st);
-    if (rc != MR_OK) return rc;
-  } else {
-  rc = launch_transpose_kernels(m, t.wt, st);
+  TrainStep s{*model, *opt, *grads, users, items, labels, B, group, k, flags, inv_global_batch, step_out,
+               carve_train(*model, B, ws), side_stream(), (cudaStream_t)stream};
+  s.p = s.plan();
+  rc = s.prologue();
   if (rc != MR_OK) return rc;
-
-  TileLaunch a{};
-  a.model = model;
-  a.train = true;
-  a.wt = t.wt;
-  a.users = users;
-  a.items = items;
-  a.labels = labels;
-  a.B = B;
-  a.user_div = 1;
-  a.inv_batch = inv_global_batch;
-  a.probs = t.probs;
-  a.loss_partial = t.loss_partial;
-  a.dense_partial = t.dense_partial;
-  a.dense_stride = t.dense_stride;
-  a.stage_u = t.stage_u;
-  a.stage_i = t.stage_i;
-  a.flags = t.flags;
-  int grid = 0;
-  prof_mark(MR_PHASE_TILE_TRAIN, st);
-  rc = launch_neumf_tiles(a, st, &grid);
-  prof_mark(MR_PHASE_MISC, st);
+  switch (s.p.path) {
+    case TRAIN_SMALL: rc = s.tower_small(); break;
+    case TRAIN_TILES: rc = s.tower_tiles(); break;
+    default: rc = s.tower_tc(); break;
+  }
   if (rc != MR_OK) return rc;
-  rc = launch_dense_reduce(m, t.dense_partial, t.dense_stride, grid, grads->dense, st, !(flags & MR_TRAIN_NO_DENSE_L2));
-  if (rc != MR_OK) return rc;
-  rc = launch_sum_partials(t.loss_partial, grid, step_out + MR_OUT_LOSS_SUM, st);
-  if (rc != MR_OK) return rc;
-  }
-  if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join, 0));  // sorts and the group check are done
-  flag_to_float_kernel<<<1, 1, 0, st>>>(t.flags, step_out + MR_OUT_BAD_IDS);
-  MR_LAUNCH_CHECK("flag_to_float_kernel");
-
-  if (group > 0) {
-    prof_mark(MR_PHASE_RANK, st);
-    // label column = argmax of the group's labels (model.py:447-448): any layout of the positive is ranked right
-    rc = launch_rank_scores(t.probs, B / group, group, k, nullptr, nullptr, t.pos, step_out + MR_OUT_HIT_SUM,
-                            t.rank_partials, st, labels);
-    if (rc != MR_OK) return rc;
-  }
-  prof_mark(MR_PHASE_MISC, st);
-
-  // ---- embedding rows: stable sort by row id, segmented reduce in batch order, row update -------
-  RowUpdate u{};
-  u.mode = opt->table_mode;
-  u.optimizer = opt->optimizer;
-  u.lr = opt->lr;
-  u.lr_t = opt->optimizer == MR_OPT_ADAM ? adam_lr_t(*opt, opt->iterations + 1) : opt->lr;
-  u.beta_1 = opt->beta_1;
-  u.beta_2 = opt->beta_2;
-  u.epsilon = opt->epsilon;
-  // users
-  u.d0 = d_u;
-  u.d1 = m.mf_dim;
-  u.num_rows = m.num_users;
-  u.p0 = m.user_mlp; u.m0 = opt->m_user_mlp; u.v0 = opt->v_user_mlp; u.g0 = grads->user_mlp;
-  u.p1 = m.user_gmf; u.m1 = opt->m_user_gmf; u.v1 = opt->v_user_gmf; u.g1 = grads->user_gmf;
-  if (!uproj && !small) {
-    prof_mark(MR_PHASE_SEGREDUCE, st);
-    rc = launch_segreduce(t.sorted_keys, t.sorted_index, n_user_rows, t.stage_u, u, t.seg_ws, t.seg_ws_bytes, st);
-    if (rc != MR_OK) return rc;
-  }
-  // items
-  u.d0 = d_i;
-  u.num_rows = m.num_items;
-  u.p0 = m.item_mlp; u.m0 = opt->m_item_mlp; u.v0 = opt->v_item_mlp; u.g0 = grads->item_mlp;
-  u.p1 = m.item_gmf; u.m1 = opt->m_item_gmf; u.v1 = opt->v_item_gmf; u.g1 = grads->item_gmf;
-  if (!proj && !small) {  // (the item-projected step reduced the item rows before its per-item GEMMs)
-    prof_mark(MR_PHASE_SEGREDUCE, st);
-    rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, u, t.seg_ws, t.seg_ws_bytes, st);
-  }
-  if (grads->user_gmf_ready != nullptr && !user_gmf_event_recorded)  // other launch sequences: final at the end
-    MR_CUDA(cudaEventRecord((cudaEvent_t)grads->user_gmf_ready, st));
-  if (grads->user_tables_ready != nullptr && !user_event_recorded)
-    MR_CUDA(cudaEventRecord((cudaEvent_t)grads->user_tables_ready, st));
-  prof_mark(-1, st);
-  return rc;
+  return s.epilogue();
 }
 
 int mr_neumf_apply(MrModel* model, MrOptState* opt, const MrGrads* grads, void* stream) {
