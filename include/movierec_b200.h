@@ -29,11 +29,12 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 102     /* major*100 + minor */
+#define MR_VERSION 103     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
 #define MR_MAX_TOPK 256    /* k of the catalogue top-k calls */
+#define MR_MAX_CUTOFFS 8   /* cutoffs of one mr_targets_scores / mr_catalogue_targets call */
 
 typedef enum MrStatus {
   MR_OK = 0,
@@ -236,6 +237,43 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
                       const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
                       float* top_scores, int32_t* pos, float* sums, float* scores, void* ws, size_t ws_bytes,
                       void* stream);
+
+/* Many held-out items per row, ranked against the whole catalogue (a per-user last-20 % or temporal split, all of a
+ * user's future ratings): row u's targets are tgt_items[tgt_rowptr[u] .. tgt_rowptr[u+1]) (device tgt_rowptr, U + 1
+ * int64; lists strictly ascending, as mr_build_user_csr writes them; every segment is clamped to [0, nnz_t), so a
+ * malformed rowptr or an unsorted list never makes a kernel leave its arrays -- that list's results are unspecified).
+ * U, nnz_t <= INT32_MAX.  Exclusion lists as mr_topk_scores.  Candidates of row u: every item of [0, N) not excluded,
+ * plus every target (a target is never excluded).  Order: mr_topk_scores' (descending score, NaN as -inf, -0 == +0,
+ * the lower item id first among ties).
+ * tpos (nnz_t int32, list order, may be NULL): the number of candidates ordered before the target -- the other targets
+ * count as candidates; N for a target outside [0, N) and for every target of an out-of-range user.  With one target
+ * per row this is mr_topk_scores' pos, bit for bit.
+ * sums (device floats, may be NULL; not both NULL with tpos): for the rows with n >= 1 targets, sorted positions
+ * p_1 <= .. <= p_n, cutoff k, h = #{p_j < k} and gain g(p) = ln2 / ln(p + 2):
+ *   hit = [p_1 < k], precision = h / k, recall = h / n, ndcg = sum_{p_j < k} g(p_j) / sum_{i < min(k, n)} g(i),
+ *   map = sum_{p_j < k} j / (p_j + 1) / min(k, n) (j 1-based), mrr = 1 / (p_1 + 1) (no cutoff).
+ * Targets outside [0, N) count in n; rows with an empty list contribute nothing and are not counted.  Accumulated in
+ * double in a fixed order that depends on U alone (never on chunking).  ks [host]: 1 <= n_ks <= MR_MAX_CUTOFFS cutoffs,
+ * each >= 1 (k > N allowed).  Layout below: 2 + 5 n_ks floats.
+ * Deterministic (integer counts, no float atomics).  No host synchronisation, no read-back.  Workspace: one chunk of
+ * rows (4 bytes per row) plus about 24 bytes per target, plus a fixed 43 KB. */
+enum { MR_TGT_USERS = 0,      /* rows with at least one target */
+       MR_TGT_MRR = 1,        /* sum of 1 / (p_1 + 1) */
+       MR_TGT_CUTOFF0 = 2,    /* sums[MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * c + m]: metric m at cutoff ks[c] */
+       MR_TGT_HIT = 0, MR_TGT_PRECISION = 1, MR_TGT_RECALL = 2, MR_TGT_NDCG = 3, MR_TGT_MAP = 4,
+       MR_TGT_PER_CUTOFF = 5 };
+size_t mr_targets_scores_workspace_bytes(int64_t U, int32_t N, int64_t nnz_t);
+int mr_targets_scores(const float* scores, int64_t U, int32_t N, const int32_t* excl_ids, int32_t excl_rows,
+                      const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
+                      const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks /*[host]*/, int32_t n_ks,
+                      int32_t* tpos, float* sums, void* ws, size_t ws_bytes, void* stream);
+/* The same on the model's probabilities of every (users[u], item) pair, scored in chunks exactly as mr_catalogue_topk
+ * scores them (so a pair's probability is the same in both calls).  Exclusion lists are indexed by user id. */
+size_t mr_catalogue_targets_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz_t);
+int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, int32_t excl_rows,
+                         const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
+                         const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks /*[host]*/, int32_t n_ks,
+                         int32_t* tpos, float* sums, void* ws, size_t ws_bytes, void* stream);
 
 /* Top-k of ragged lists of caller-supplied scores: list u is scores[rowptr[u] .. rowptr[u+1]) (device rowptr, U + 1
  * int64, rowptr[0] = 0, non-decreasing, rowptr[U] = nnz; U and nnz <= INT32_MAX, no rows when U = 0).  Order: the

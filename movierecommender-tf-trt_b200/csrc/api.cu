@@ -1322,6 +1322,79 @@ static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const 
   return MR_OK;
 }
 
+// The chunk loop of the catalogue calls: per chunk of C users, the probabilities of every (user, item) pair through the
+// model's catalogue_path sequence, then select(u0, users in the chunk, probabilities) under MR_PHASE_RANK.  The
+// probabilities go to scores + u0 * N when scores is given, else to probs_buf (C x N).  mr_catalogue_topk and
+// mr_catalogue_targets both score through here, so a pair's probability is the same in both by construction.
+template <class Select>
+static int catalogue_sweep(const MrModel& m, const int32_t* users, int64_t U, int64_t C, int32_t* iota, float* probs_buf,
+                           float* scores, void* score_ws, cudaStream_t st, Select select) {
+  const int32_t N = m.num_items;
+  const int64_t Cmax = catalogue_chunk_users(N);
+  const int path = catalogue_path(m);
+  TcWs t{};
+  float *Pi = nullptr, *Pu = nullptr;
+  size_t fwd_bytes = 0;
+  prof_mark(MR_PHASE_MISC, st);
+  int rc = launch_tile_iota(iota, C * N, N, st);
+  if (rc != MR_OK) return rc;
+  if (path == CAT_TC) {
+    t = carve_eval(m, N, Cmax * N, score_ws, C * N);
+    rc = eval_prepare(m, t, st);
+  } else if (path == CAT_SMALL) {  // Pi, Pu over the tables, as mr_rank_eval's default-tower path
+    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
+    Carver cs(score_ws);
+    Pi = cs.take<float>((size_t)m.num_items * L1);
+    Pu = cs.take<float>((size_t)m.num_users * L1);
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, Pi, st);
+    if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, m.W[1], L1, L1, false, m.b[1], Pu, st);
+  } else {
+    fwd_bytes = mr_forward_workspace_bytes(&m, C * N);
+  }
+  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
+    const int64_t c = U - u0 < C ? U - u0 : C;
+    const int64_t rows = c * N;
+    float* out = scores != nullptr ? scores + u0 * N : probs_buf;
+    if (path == CAT_TC) {
+      // each chunk starts at row 0 of its own users: one group = one user, Zu once per user
+      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+      rc = tc_forward_rows(m, t, users + u0, iota, 1, 0, rows, st, N, true, true);
+      if (rc == MR_OK) {
+        prof_mark(MR_PHASE_HEAD, st);
+        rc = launch_catalogue_head(m, t.H[m.n_layers - 1], users + u0, rows, N, out, st);
+      }
+    } else if (path == CAT_SMALL) {
+      prof_mark(MR_PHASE_FUSED_TILE, st);
+      rc = launch_small_tower_forward(m, Pi, Pu, users + u0, iota, rows, N, out, st);
+    } else {
+      rc = mr_neumf_forward(&m, users + u0, iota, rows, N, nullptr, out, nullptr, nullptr, score_ws, fwd_bytes, st);
+    }
+    if (rc != MR_OK) break;
+    prof_mark(MR_PHASE_RANK, st);
+    rc = select(u0, c, out);
+  }
+  return rc;
+}
+
+static int targets_check(int64_t U, int32_t N, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_items,
+                         const int64_t* tgt_rowptr, const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks,
+                         int32_t n_ks, const int32_t* tpos, const float* sums, TargetCutoffs& cut) {
+  MR_REQUIRE(U >= 0 && U <= INT32_MAX && N >= 1 && nnz_t >= 0 && nnz_t <= INT32_MAX, "targets: bad U=%lld N=%d nnz_t=%lld",
+             (long long)U, N, (long long)nnz_t);
+  MR_REQUIRE(U > 0 || nnz_t == 0, "targets: nnz_t=%lld targets in no list", (long long)nnz_t);
+  MR_REQUIRE(ks != nullptr && n_ks >= 1 && n_ks <= MR_MAX_CUTOFFS, "targets: n_ks=%d out of [1,%d]", n_ks, MR_MAX_CUTOFFS);
+  for (int c = 0; c < n_ks; ++c) {
+    MR_REQUIRE(ks[c] >= 1, "targets: cutoff ks[%d]=%d < 1", c, ks[c]);
+    cut.k[c] = ks[c];
+  }
+  cut.n = n_ks;
+  MR_REQUIRE(excl_rows >= 0 && (excl_rowptr == nullptr || excl_items != nullptr), "targets: bad exclusion lists");
+  MR_REQUIRE(nnz_t == 0 || (tgt_rowptr != nullptr && tgt_items != nullptr), "targets: tgt_rowptr / tgt_items is NULL");
+  MR_REQUIRE(tpos != nullptr || sums != nullptr, "targets: tpos and sums are both NULL");
+  return MR_OK;
+}
+
 // ---- ragged candidate lists: list u pairs users[u] with items[rowptr[u] .. rowptr[u+1]) ------------------------------
 // The scoring sequence is a function of the model alone -- never of U or nnz -- so that a list's outputs do not depend on
 // the other lists of the call (what a serving batcher needs):
@@ -1756,35 +1829,13 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
     set_error("catalogue_topk workspace too small: %zu < %zu", ws_bytes, mr_catalogue_topk_workspace_bytes(model, U, k));
     return MR_ERR_WORKSPACE;
   }
-  const int64_t Cmax = catalogue_chunk_users(N);
-  const int64_t C = clamp_users(U, Cmax);
+  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
   Carver cv(ws);
   int32_t* iota = cv.take<int32_t>((size_t)C * N);
   float* probs_buf = cv.take<float>((size_t)C * N);
   const size_t topk_bytes = topk_workspace_bytes(C, N, k);
   void* topk_ws = cv.take<char>(topk_bytes);
   void* score_ws = static_cast<char*>(ws) + cv.off;
-  const int path = catalogue_path(m);
-  TcWs t{};
-  float *Pi = nullptr, *Pu = nullptr;
-  size_t fwd_bytes = 0;
-  prof_mark(MR_PHASE_MISC, st);
-  rc = launch_tile_iota(iota, C * N, N, st);
-  if (rc != MR_OK) return rc;
-  if (path == CAT_TC) {
-    t = carve_eval(m, N, Cmax * N, score_ws, C * N);
-    rc = eval_prepare(m, t, st);
-  } else if (path == CAT_SMALL) {  // Pi, Pu over the tables, as mr_rank_eval's default-tower path
-    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
-    Carver cs(score_ws);
-    Pi = cs.take<float>((size_t)m.num_items * L1);
-    Pu = cs.take<float>((size_t)m.num_users * L1);
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, Pi, st);
-    if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, m.W[1], L1, L1, false, m.b[1], Pu, st);
-  } else {
-    fwd_bytes = mr_forward_workspace_bytes(model, C * N);
-  }
   TopkArgs a{};
   a.N = N;
   a.k = k;
@@ -1798,34 +1849,127 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
   a.top_items = top_items;
   a.top_scores = top_scores;
   a.pos = pos;
-  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
-    const int64_t c = U - u0 < C ? U - u0 : C;
-    const int64_t rows = c * N;
-    float* out = scores != nullptr ? scores + u0 * N : probs_buf;
-    if (path == CAT_TC) {
-      // each chunk starts at row 0 of its own users: one group = one user, Zu once per user
-      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-      rc = tc_forward_rows(m, t, users + u0, iota, 1, 0, rows, st, N, true, true);
-      if (rc == MR_OK) {
-        prof_mark(MR_PHASE_HEAD, st);
-        rc = launch_catalogue_head(m, t.H[m.n_layers - 1], users + u0, rows, N, out, st);
-      }
-    } else if (path == CAT_SMALL) {
-      prof_mark(MR_PHASE_FUSED_TILE, st);
-      rc = launch_small_tower_forward(m, Pi, Pu, users + u0, iota, rows, N, out, st);
-    } else {
-      rc = mr_neumf_forward(model, users + u0, iota, rows, N, nullptr, out, nullptr, nullptr, score_ws, fwd_bytes, stream);
-    }
-    if (rc != MR_OK) break;
-    prof_mark(MR_PHASE_RANK, st);
+  rc = catalogue_sweep(m, users, U, C, iota, probs_buf, scores, score_ws, st, [&](int64_t u0, int64_t c, const float* out) {
     a.u0 = u0;
     a.U = c;
     a.scores = out;
-    rc = launch_topk(a, topk_ws, st);
-  }
+    return launch_topk(a, topk_ws, st);
+  });
   if (rc == MR_OK) {
     prof_mark(MR_PHASE_RANK, st);
     rc = launch_topk_metrics(pos, U, k, sums, st);
+  }
+  prof_mark(-1, st);
+  return rc;
+}
+
+size_t mr_targets_scores_workspace_bytes(int64_t U, int32_t N, int64_t nnz_t) {
+  if (U < 0 || U > INT32_MAX || N < 1 || nnz_t < 0 || nnz_t > INT32_MAX) return 0;
+  return targets_workspace_bytes(clamp_users(U, catalogue_chunk_users(N)), nnz_t) + 256;
+}
+
+int mr_targets_scores(const float* scores, int64_t U, int32_t N, const int32_t* excl_ids, int32_t excl_rows,
+                      const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
+                      const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks, int32_t n_ks, int32_t* tpos,
+                      float* sums, void* ws, size_t ws_bytes, void* stream) {
+  TargetCutoffs cut{};
+  int rc = targets_check(U, N, excl_rows, excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums,
+                         cut);
+  if (rc != MR_OK) return rc;
+  MR_REQUIRE(U == 0 || scores != nullptr, "targets_scores: scores is NULL");
+  MR_REQUIRE(ws != nullptr, "targets_scores: workspace is NULL");
+  if (ws_bytes < mr_targets_scores_workspace_bytes(U, N, nnz_t)) {
+    set_error("targets_scores workspace too small: %zu < %zu", ws_bytes, mr_targets_scores_workspace_bytes(U, N, nnz_t));
+    return MR_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t C = catalogue_chunk_users(N);
+  const TargetsWs w = carve_targets(ws, clamp_users(U, C), nnz_t);
+  TargetsArgs a{};
+  a.N = N;
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_items;
+  a.tgt_rowptr = tgt_rowptr;
+  a.tgt_items = tgt_items;
+  a.nnz_t = nnz_t;
+  a.tpos = tpos;
+  prof_mark(MR_PHASE_RANK, st);
+  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
+    a.u0 = u0;
+    a.U = U - u0 < C ? U - u0 : C;
+    a.scores = scores + u0 * N;
+    rc = launch_targets_chunk(a, w, st);
+  }
+  if (rc == MR_OK) rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
+  prof_mark(-1, st);
+  return rc;
+}
+
+size_t mr_catalogue_targets_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz_t) {
+  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
+      model->num_users < 1 || model->L[0] < 2)
+    return 0;
+  const MrModel& m = *model;
+  const size_t sel = mr_targets_scores_workspace_bytes(U, m.num_items, nnz_t);
+  if (sel == 0) return 0;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(m.num_items));
+  const size_t rows = (size_t)C * m.num_items;
+  return align_up(rows * sizeof(int32_t), 256) + align_up(rows * sizeof(float), 256) + align_up(sel, 256) +
+         catalogue_scoring_bytes(m, C) + 512;
+}
+
+int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, int32_t excl_rows,
+                         const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
+                         const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks, int32_t n_ks, int32_t* tpos,
+                         float* sums, void* ws, size_t ws_bytes, void* stream) {
+  int rc = check_model(model);
+  if (rc != MR_OK) return rc;
+  const MrModel& m = *model;
+  const int32_t N = m.num_items;
+  TargetCutoffs cut{};
+  rc = targets_check(U, N, excl_rows, excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums, cut);
+  if (rc != MR_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (U == 0) {
+    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, (MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * n_ks) * sizeof(float), st));
+    return MR_OK;
+  }
+  MR_REQUIRE(users != nullptr, "catalogue_targets: users is NULL");
+  MR_REQUIRE(ws != nullptr, "catalogue_targets: workspace is NULL");
+  if (ws_bytes < mr_catalogue_targets_workspace_bytes(model, U, nnz_t)) {
+    set_error("catalogue_targets workspace too small: %zu < %zu", ws_bytes,
+              mr_catalogue_targets_workspace_bytes(model, U, nnz_t));
+    return MR_ERR_WORKSPACE;
+  }
+  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
+  Carver cv(ws);
+  int32_t* iota = cv.take<int32_t>((size_t)C * N);
+  float* probs_buf = cv.take<float>((size_t)C * N);
+  const TargetsWs w = carve_targets(cv.take<char>(mr_targets_scores_workspace_bytes(U, N, nnz_t)), C, nnz_t);
+  void* score_ws = static_cast<char*>(ws) + cv.off;
+  TargetsArgs a{};
+  a.N = N;
+  a.excl_ids = users;  // exclusion lists are indexed by user id
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_items;
+  a.tgt_rowptr = tgt_rowptr;
+  a.tgt_items = tgt_items;
+  a.nnz_t = nnz_t;
+  a.users = users;
+  a.num_users = m.num_users;
+  a.tpos = tpos;
+  rc = catalogue_sweep(m, users, U, C, iota, probs_buf, nullptr, score_ws, st, [&](int64_t u0, int64_t c, const float* out) {
+    a.u0 = u0;
+    a.U = c;
+    a.scores = out;
+    return launch_targets_chunk(a, w, st);
+  });
+  if (rc == MR_OK) {
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
   }
   prof_mark(-1, st);
   return rc;

@@ -130,6 +130,44 @@ int launch_topk_lists(const TopkListsArgs& a, float* sums, void* ws, cudaStream_
 int launch_list_rows(const int64_t* rowptr, int64_t U, int64_t nnz, const int32_t* users, int32_t* seg, cudaStream_t st);
 // out[r] = r % N for r < rows
 int launch_tile_iota(int32_t* out, int64_t rows, int32_t N, cudaStream_t st);
+// Positions of many targets per row: row u's targets are tgt_items[tgt_rowptr[u] .. tgt_rowptr[u+1]) (segments clamped
+// to [0, nnz_t)); candidates, order and exclusion lists as TopkArgs, a target never excluded.
+struct TargetsArgs {
+  const float* scores;  // the chunk's rows: U x N, row 0 = global row u0
+  int64_t U, u0;
+  int32_t N;
+  // every array below is indexed by the GLOBAL row u0 + u
+  const int32_t* excl_ids;
+  int32_t excl_rows;
+  const int64_t* excl_rowptr;
+  const int32_t* excl_items;
+  const int64_t* tgt_rowptr;
+  const int32_t* tgt_items;
+  int64_t nnz_t;
+  const int32_t* users;  // optional: a row whose users[u] lies outside [0, num_users) gives every target position N
+  int32_t num_users;
+  int32_t* tpos;  // may be NULL
+};
+constexpr int kTgtSumsMax = MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * MR_MAX_CUTOFFS;
+struct TargetCutoffs {
+  int32_t k[MR_MAX_CUTOFFS];
+  int32_t n;
+};
+// Workspace of one call: sorted keys, merge scratch and positions (in sorted order) per target, histogram bins per
+// target plus one per row of a chunk (C rows), per-block metric partials.
+struct TargetsWs {
+  unsigned long long *keys, *tmp;
+  int32_t *hist, *spos;
+  double* partials;
+  size_t total;
+};
+TargetsWs carve_targets(void* ws, int64_t C, int64_t nnz_t);
+size_t targets_workspace_bytes(int64_t C, int64_t nnz_t);
+// The chunk's positions: w.spos (ascending per row) and a.tpos (list order)
+int launch_targets_chunk(const TargetsArgs& a, const TargetsWs& w, cudaStream_t st);
+// sums (MR_TGT_* layout, may be NULL) from the positions of all U rows, in a fixed order
+int launch_targets_metrics(const int64_t* tgt_rowptr, int64_t U, int64_t nnz_t, const int32_t* spos,
+                           const TargetCutoffs& ks, float* sums, double* partials, cudaStream_t st);
 
 // ---- sampler.cu ------------------------------------------------------------------------------
 int launch_sample_negatives(const int64_t* rowptr, const int32_t* csr_items, int32_t num_items,

@@ -107,6 +107,47 @@ __device__ __forceinline__ void topk_merge_warp(const unsigned long long* lists,
   }
 }
 
+// The first index of the ascending list items[b, e) whose entry is >= v (e when none).
+__device__ __forceinline__ int64_t list_lower_bound(const int32_t* __restrict__ items, int64_t b, int64_t e, int v) {
+  while (b < e) {
+    const int64_t mid = (b + e) >> 1;
+    if (__ldg(items + mid) < v) b = mid + 1;
+    else e = mid;
+  }
+  return b;
+}
+
+// A warp's cursor [ep, ee) into the exclusion list of global row gu, from the first entry >= lo (empty when the row
+// has no list).
+__device__ __forceinline__ void excl_cursor(const int32_t* __restrict__ excl_ids, int32_t excl_rows,
+                                            const int64_t* __restrict__ excl_rowptr, const int32_t* __restrict__ excl_items,
+                                            int64_t gu, int lo, int64_t& ep, int64_t& ee) {
+  ep = ee = 0;
+  if (excl_rowptr == nullptr) return;
+  const int64_t r = excl_ids != nullptr ? (int64_t)__ldg(excl_ids + gu) : gu;
+  if (r >= 0 && r < excl_rows) {
+    ee = excl_rowptr[r + 1];
+    ep = list_lower_bound(excl_items, excl_rowptr[r], ee, lo);
+  }
+}
+
+// Bit i = items[ep, ee) holds c + i, for a warp walking its items 32 at a time in ascending c; advances ep past the
+// entries below c + 32.  Warp-uniform: lists are sorted, so the entries below c + 32 are a prefix of the lanes.
+__device__ __forceinline__ uint32_t list_mask(const int32_t* __restrict__ items, int64_t& ep, int64_t ee, int c,
+                                              int lane) {
+  uint32_t mask = 0;
+  for (;;) {
+    const int64_t i = ep + lane;
+    const int e = i < ee ? __ldg(items + i) : INT_MAX;
+    const bool in = e < c + 32;
+    const int nin = __popc(__ballot_sync(0xffffffffu, in));
+    mask |= __reduce_or_sync(0xffffffffu, (in && e >= c) ? 1u << (e - c) : 0u);
+    ep += nin;
+    if (nin < 32) break;
+  }
+  return mask;
+}
+
 __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs a, int S, int slice, int cap,
                                                                   unsigned long long* __restrict__ lists,
                                                                   int32_t* __restrict__ counts) {
@@ -121,37 +162,15 @@ __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs
   const int N = a.N, k = a.k;
   const float* row = a.scores + u * N;
   const int lo = s * slice, hi = min(N, lo + slice);
-  // exclusion list: [ep, ee) from the first entry >= lo
-  int64_t ep = 0, ee = 0;
-  if (a.excl_rowptr != nullptr) {
-    const int64_t r = a.excl_ids != nullptr ? (int64_t)__ldg(a.excl_ids + gu) : gu;
-    if (r >= 0 && r < a.excl_rows) {
-      int64_t b = a.excl_rowptr[r], e = a.excl_rowptr[r + 1];
-      ee = e;
-      while (b < e) {
-        const int64_t mid = (b + e) >> 1;
-        if (__ldg(a.excl_items + mid) < lo) b = mid + 1;
-        else e = mid;
-      }
-      ep = b;
-    }
-  }
+  int64_t ep, ee;  // exclusion list: [ep, ee) from the first entry >= lo
+  excl_cursor(a.excl_ids, a.excl_rows, a.excl_rowptr, a.excl_items, gu, lo, ep, ee);
   const int t = a.targets != nullptr ? __ldg(a.targets + gu) : -1;
   const bool has_t = (unsigned)t < (unsigned)N;
   const unsigned long long key_t = has_t ? topk_key(__ldg(row + t), t) : 0ull;
   int below = 0, n = 0;
   unsigned long long thr = kNoKey;
   for (int c = lo; c < hi; c += 32) {
-    uint32_t xmask = 0;  // excluded items of [c, c + 32)
-    for (;;) {           // warp-uniform: lists are sorted, so the entries below c + 32 are a prefix of the lanes
-      const int64_t i = ep + lane;
-      const int e = i < ee ? __ldg(a.excl_items + i) : INT_MAX;
-      const bool in = e < c + 32;
-      const int nin = __popc(__ballot_sync(0xffffffffu, in));
-      xmask |= __reduce_or_sync(0xffffffffu, (in && e >= c) ? 1u << (e - c) : 0u);
-      ep += nin;
-      if (nin < 32) break;
-    }
+    const uint32_t xmask = list_mask(a.excl_items, ep, ee, c, lane);  // excluded items of [c, c + 32)
     const int item = c + lane;
     const bool cand = item < hi && (!((xmask >> lane) & 1u) || item == t);  // the target is never excluded
     const unsigned long long key = cand ? topk_key(__ldg(row + item), item) : kNoKey;
@@ -485,6 +504,328 @@ int launch_tile_iota(int32_t* out, int64_t rows, int32_t N, cudaStream_t st) {
   if (grid > cap) grid = cap;
   tile_iota_kernel<<<(unsigned)grid, 256, 0, st>>>(out, rows, N);
   MR_LAUNCH_CHECK("tile_iota_kernel");
+  return MR_OK;
+}
+
+// ---- positions of many targets per row: row u's targets are tgt_items[tgt_rowptr[u] .. tgt_rowptr[u+1]) ----------
+// Candidates of a row: the items not excluded plus every target (a target is never excluded); order: topk_key.  The
+// position of a target = the candidates with a smaller key.  Per chunk of rows:
+//  sort:     one CTA per row sorts the keys of the row's targets ascending (targets outside [0, N) as kNoKey, last):
+//            a block bitonic sort in shared memory up to kTgtTile keys; longer lists sort tiles of kTgtTile, then merge
+//            them in global memory (each key's output place = its place in its run + its rank in the other run).
+//            It also zeroes the row's histogram, n + 1 integer bins.
+//  count:    one warp per (row, slice), the slices of topk_slice_kernel: the warp walks its slice next to the
+//            exclusion list and the target list, and every candidate that is not a target adds 1 to bin b = the
+//            number of target keys below its own (a binary search over the sorted keys, in shared memory for lists of
+//            at most kTgtSmemKeys targets, else in global memory).  Integer counts: the order of the additions is
+//            irrelevant.
+//  finalize: one warp per row: the sorted target j has j targets and sum_{b <= j} hist[b] other candidates below it.
+//            The positions land in sorted order in spos (ascending per row) and in list order in tpos.
+// After the last chunk one fixed-order pass turns spos into metric sums (below), so chunking never shows in them.
+// Bytes per row: 4 N (scores) + 4 x (exclusion list) + 4 t (target list) read; about 24 t of workspace traffic.
+constexpr int kTgtSortThreads = 256;
+constexpr int kTgtTile = 2048;     // keys a sort CTA sorts in shared memory (16 KB)
+constexpr int kTgtSmemKeys = 512;  // lists up to this length are searched and counted in shared memory
+constexpr int kMetricBlocks = 128, kMetricThreads = 256;
+
+TargetsWs carve_targets(void* ws, int64_t C, int64_t nnz_t) {
+  TargetsWs w{};
+  Carver cv(ws);
+  const size_t t = (size_t)(nnz_t < 1 ? 1 : nnz_t);
+  w.keys = cv.take<unsigned long long>(t);
+  w.tmp = cv.take<unsigned long long>(t);
+  w.hist = cv.take<int32_t>(t + (size_t)(C < 1 ? 1 : C));
+  w.spos = cv.take<int32_t>(t);
+  w.partials = cv.take<double>((size_t)kMetricBlocks * kTgtSumsMax);
+  w.total = cv.off;
+  return w;
+}
+
+size_t targets_workspace_bytes(int64_t C, int64_t nnz_t) { return carve_targets(nullptr, C, nnz_t).total; }
+
+__device__ __forceinline__ bool targets_bad_user(const TargetsArgs& a, int64_t gu) {
+  return a.users != nullptr && (unsigned)__ldg(a.users + gu) >= (unsigned)a.num_users;
+}
+
+// Ascending bitonic sort of buf[0, cap) (cap a power of two) by the whole block.
+__device__ void block_bitonic(unsigned long long* buf, int cap) {
+  for (int size = 2; size <= cap; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int i = threadIdx.x; i < cap / 2; i += blockDim.x) {
+        const int x0 = 2 * i - (i & (stride - 1)), x1 = x0 + stride;
+        const unsigned long long x = buf[x0], y = buf[x1];
+        if ((x > y) == ((x0 & size) == 0)) {
+          buf[x0] = y;
+          buf[x1] = x;
+        }
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// Entries of the ascending v[b, e) below x (upper = false) or not above x (upper = true).
+__device__ __forceinline__ int64_t keys_rank(const unsigned long long* v, int64_t b, int64_t e, unsigned long long x,
+                                             bool upper) {
+  while (b < e) {
+    const int64_t mid = (b + e) >> 1;
+    if (v[mid] < x || (upper && v[mid] == x)) b = mid + 1;
+    else e = mid;
+  }
+  return b;
+}
+
+__global__ void __launch_bounds__(kTgtSortThreads) targets_sort_kernel(const TargetsArgs a, const TargetsWs w) {
+  __shared__ unsigned long long tile[kTgtTile];
+  const int64_t u = blockIdx.x, gu = a.u0 + u;
+  int64_t tb, te;
+  list_bounds(a.tgt_rowptr, gu, a.nnz_t, tb, te);
+  const int64_t n = te - tb;
+  int32_t* hist = w.hist + tb + u;
+  for (int64_t i = threadIdx.x; i <= n; i += blockDim.x) hist[i] = 0;
+  if (n == 0 || targets_bad_user(a, gu)) return;  // block-uniform; finalize gives a bad row's targets N
+  const int N = a.N;
+  const float* row = a.scores + u * N;
+  const int32_t* items = a.tgt_items + tb;
+  auto key_of = [&](int64_t i) {
+    const int t = __ldg(items + i);
+    return (unsigned)t < (unsigned)N ? topk_key(__ldg(row + t), t) : kNoKey;
+  };
+  unsigned long long* keys = w.keys + tb;
+  if (n <= kTgtTile) {
+    int cap = 64;
+    while (cap < n) cap <<= 1;
+    for (int i = threadIdx.x; i < cap; i += blockDim.x) tile[i] = i < n ? key_of(i) : kNoKey;
+    __syncthreads();
+    block_bitonic(tile, cap);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) keys[i] = tile[i];
+    return;
+  }
+  unsigned long long *src = keys, *dst = w.tmp + tb;
+  for (int64_t t0 = 0; t0 < n; t0 += kTgtTile) {
+    const int m = (int)(n - t0 < kTgtTile ? n - t0 : kTgtTile);
+    for (int i = threadIdx.x; i < kTgtTile; i += blockDim.x) tile[i] = i < m ? key_of(t0 + i) : kNoKey;
+    __syncthreads();
+    block_bitonic(tile, kTgtTile);
+    for (int i = threadIdx.x; i < m; i += blockDim.x) src[t0 + i] = tile[i];
+    __syncthreads();
+  }
+  for (int64_t width = kTgtTile; width < n; width <<= 1) {  // merge runs of `width` pairwise: src -> dst
+    for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
+      const int64_t s = i / (2 * width) * (2 * width);
+      const int64_t mid = s + width < n ? s + width : n, end = s + 2 * width < n ? s + 2 * width : n;
+      const unsigned long long x = src[i];
+      // equal keys (only kNoKey) keep the left run first, so every output place is taken once
+      const int64_t p = i < mid ? (i - s) + keys_rank(src, mid, end, x, false) - mid
+                                : (i - mid) + keys_rank(src, s, mid, x, true) - s;
+      dst[s + p] = x;
+    }
+    __syncthreads();
+    unsigned long long* t = src;
+    src = dst;
+    dst = t;
+  }
+  if (src != keys) {
+    for (int64_t i = threadIdx.x; i < n; i += blockDim.x) keys[i] = src[i];
+  }
+}
+
+__global__ void __launch_bounds__(kTopkThreads) targets_count_kernel(const TargetsArgs a, int S, int slice,
+                                                                     const TargetsWs w) {
+  __shared__ unsigned long long skeys[kTopkThreads / 32][kTgtSmemKeys];
+  __shared__ int32_t shist[kTopkThreads / 32][kTgtSmemKeys + 1];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t wi = (int64_t)blockIdx.x * (kTopkThreads / 32) + warp;
+  if (wi >= a.U * S) return;  // warp-uniform
+  const int64_t u = wi / S;
+  const int s = (int)(wi - u * S);
+  const int64_t gu = a.u0 + u;
+  int64_t tb, te;
+  list_bounds(a.tgt_rowptr, gu, a.nnz_t, tb, te);
+  const int64_t n = te - tb;
+  if (n == 0 || targets_bad_user(a, gu)) return;
+  const int N = a.N;
+  const float* row = a.scores + u * N;
+  const int lo = s * slice, hi = min(N, lo + slice);
+  int64_t ep, ee;
+  excl_cursor(a.excl_ids, a.excl_rows, a.excl_rowptr, a.excl_items, gu, lo, ep, ee);
+  int64_t tp = list_lower_bound(a.tgt_items, tb, te, lo);
+  const bool local = n <= kTgtSmemKeys;
+  const unsigned long long* keys = w.keys + tb;
+  int32_t* hist = w.hist + tb + u;
+  if (local) {
+    for (int i = lane; i < n; i += 32) skeys[warp][i] = keys[i];
+    for (int i = lane; i <= n; i += 32) shist[warp][i] = 0;
+    keys = skeys[warp];
+    hist = shist[warp];
+    __syncwarp();
+  }
+  int64_t top = 1;
+  while (2 * top <= n) top <<= 1;
+  for (int c = lo; c < hi; c += 32) {
+    const uint32_t skip = list_mask(a.excl_items, ep, ee, c, lane) | list_mask(a.tgt_items, tp, te, c, lane);
+    const int item = c + lane;
+    if (item < hi && !((skip >> lane) & 1u)) {  // a candidate that is not a target
+      const unsigned long long key = topk_key(__ldg(row + item), item);
+      int64_t b = 0;  // target keys below key
+      for (int64_t step = top; step > 0; step >>= 1)
+        if (b + step <= n && keys[b + step - 1] < key) b += step;
+      atomicAdd(hist + b, 1);
+    }
+  }
+  if (local) {
+    __syncwarp();
+    for (int i = lane; i <= n; i += 32) {
+      const int v = shist[warp][i];
+      if (v != 0) atomicAdd(w.hist + tb + u + i, v);
+    }
+  }
+}
+
+__global__ void __launch_bounds__(kTopkThreads) targets_finalize_kernel(const TargetsArgs a, const TargetsWs w) {
+  const int lane = threadIdx.x & 31;
+  const int64_t u = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (u >= a.U) return;  // warp-uniform
+  const int64_t gu = a.u0 + u;
+  int64_t tb, te;
+  list_bounds(a.tgt_rowptr, gu, a.nnz_t, tb, te);
+  const int64_t n = te - tb;
+  const int N = a.N;
+  const bool bad_u = targets_bad_user(a, gu);
+  const int32_t* hist = w.hist + tb + u;
+  int64_t run = 0;  // sum of hist[0, base)
+  for (int64_t base = 0; base < n; base += 32) {
+    const int64_t j = base + lane;
+    int64_t x = (j < n && !bad_u) ? hist[j] : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int64_t y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (j < n) {
+      const unsigned long long key = bad_u ? kNoKey : w.keys[tb + j];
+      const int p = key == kNoKey ? N : (int)(j + run + x);
+      w.spos[tb + j] = p;
+      if (a.tpos != nullptr && key != kNoKey) {
+        const int64_t i = list_lower_bound(a.tgt_items, tb, te, (int)(uint32_t)key);
+        if (i < te) a.tpos[i] = p;
+      }
+    }
+    run += __shfl_sync(0xffffffffu, x, 31);
+  }
+  if (a.tpos != nullptr) {  // targets outside [0, N), every target of a bad row
+    for (int64_t i = tb + lane; i < te; i += 32)
+      if (bad_u || (unsigned)__ldg(a.tgt_items + i) >= (unsigned)N) a.tpos[i] = N;
+  }
+}
+
+int launch_targets_chunk(const TargetsArgs& a, const TargetsWs& w, cudaStream_t st) {
+  if (a.U == 0 || a.tgt_rowptr == nullptr) return MR_OK;
+  const int S = topk_slices(a.N), slice = topk_slice_len(a.N), wpc = kTopkThreads / 32;
+  targets_sort_kernel<<<(unsigned)a.U, kTgtSortThreads, 0, st>>>(a, w);
+  MR_LAUNCH_CHECK("targets_sort_kernel");
+  targets_count_kernel<<<(unsigned)((a.U * S + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, S, slice, w);
+  MR_LAUNCH_CHECK("targets_count_kernel");
+  targets_finalize_kernel<<<(unsigned)((a.U + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, w);
+  MR_LAUNCH_CHECK("targets_finalize_kernel");
+  return MR_OK;
+}
+
+// Sum of v over the block in a fixed order; the result is valid in thread 0.
+__device__ double block_sum_double(double v, double* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();  // red may still be read from the previous call
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+  if (threadIdx.x == 0)
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += red[i];
+  return t;
+}
+
+__device__ __forceinline__ double dcg_gain(int p) {  // topk_metric_kernel's gain, ln2 / ln(p + 2) in float
+  return (double)(logf(2.f) / logf((float)p + 2.f));
+}
+
+// Per-block partial sums: users are assigned to threads by their index alone (thread-strided over a fixed grid), each
+// thread adds its users in index order and the block its threads in a fixed tree, so the sums depend on U only.
+__global__ void __launch_bounds__(kMetricThreads) targets_metric_kernel(const int64_t* __restrict__ rowptr, int64_t U,
+                                                                        int64_t nnz_t, const int32_t* __restrict__ spos,
+                                                                        const TargetCutoffs ks,
+                                                                        double* __restrict__ partials) {
+  __shared__ double red[kMetricThreads / 32];
+  double* out = partials + (size_t)blockIdx.x * kTgtSumsMax;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x, first = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  double users = 0.0, mrr = 0.0;
+  for (int64_t u = first; u < U; u += stride) {
+    int64_t b, e;
+    list_bounds(rowptr, u, nnz_t, b, e);
+    if (e == b) continue;
+    users += 1.0;
+    mrr += 1.0 / ((double)spos[b] + 1.0);
+  }
+  double t = block_sum_double(users, red);
+  if (threadIdx.x == 0) out[MR_TGT_USERS] = t;
+  t = block_sum_double(mrr, red);
+  if (threadIdx.x == 0) out[MR_TGT_MRR] = t;
+  for (int c = 0; c < ks.n; ++c) {
+    int k = ks.k[0];  // (a constant index per step keeps the parameter array out of local memory)
+#pragma unroll
+    for (int i = 1; i < MR_MAX_CUTOFFS; ++i)
+      if (c == i) k = ks.k[i];
+    double hit = 0.0, prec = 0.0, rec = 0.0, ndcg = 0.0, map = 0.0;
+    for (int64_t u = first; u < U; u += stride) {
+      int64_t b, e;
+      list_bounds(rowptr, u, nnz_t, b, e);
+      const int64_t n = e - b;
+      if (n == 0) continue;
+      double h = 0.0, dcg = 0.0, ap = 0.0;
+      for (int64_t j = 0; j < n; ++j) {  // positions ascend: stop at the first one outside the cutoff
+        const int p = spos[b + j];
+        if (p >= k) break;
+        h += 1.0;
+        dcg += dcg_gain(p);
+        ap += (double)(j + 1) / ((double)p + 1.0);
+      }
+      const int64_t m = n < k ? n : k;
+      double idcg = 0.0;
+      for (int64_t i = 0; i < m; ++i) idcg += dcg_gain((int)i);
+      hit += h > 0.0 ? 1.0 : 0.0;
+      prec += h / (double)k;
+      rec += h / (double)n;
+      ndcg += dcg / idcg;
+      map += ap / (double)m;
+    }
+    const double v[MR_TGT_PER_CUTOFF] = {hit, prec, rec, ndcg, map};
+#pragma unroll
+    for (int m = 0; m < MR_TGT_PER_CUTOFF; ++m) {
+      t = block_sum_double(v[m], red);
+      if (threadIdx.x == 0) out[MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * c + m] = t;
+    }
+  }
+}
+
+__global__ void targets_metric_reduce_kernel(const double* __restrict__ partials, int nm, float* __restrict__ sums) {
+  const int m = threadIdx.x;
+  if (m >= nm) return;
+  double t = 0.0;
+  for (int b = 0; b < kMetricBlocks; ++b) t += partials[(size_t)b * kTgtSumsMax + m];
+  sums[m] = (float)t;
+}
+
+int launch_targets_metrics(const int64_t* tgt_rowptr, int64_t U, int64_t nnz_t, const int32_t* spos,
+                           const TargetCutoffs& ks, float* sums, double* partials, cudaStream_t st) {
+  if (sums == nullptr) return MR_OK;
+  const int nm = MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * ks.n;
+  if (U == 0 || tgt_rowptr == nullptr) {
+    MR_CUDA(cudaMemsetAsync(sums, 0, nm * sizeof(float), st));
+    return MR_OK;
+  }
+  targets_metric_kernel<<<kMetricBlocks, kMetricThreads, 0, st>>>(tgt_rowptr, U, nnz_t, spos, ks, partials);
+  MR_LAUNCH_CHECK("targets_metric_kernel");
+  targets_metric_reduce_kernel<<<1, 64, 0, st>>>(partials, nm, sums);
+  MR_LAUNCH_CHECK("targets_metric_reduce_kernel");
   return MR_OK;
 }
 

@@ -533,16 +533,7 @@ class NeuMFEngine(object):
         t = as_device_i32(targets, dev) if targets is not None else None
         if t is not None and t.numel() != U:
             raise ValueError("targets ({}) and users ({}) differ in length".format(t.numel(), U))
-        rowptr = items = None
-        excl_rows = 0
-        if exclude is not None:
-            rp, it = exclude
-            rowptr = (rp if isinstance(rp, torch.Tensor) else torch.from_numpy(np.asarray(rp, dtype=np.int64)))
-            rowptr = rowptr.reshape(-1).to(dev, torch.int64).contiguous()
-            items = as_device_i32(it, dev)
-            if items.numel() == 0:  # every list empty: the library still wants a pointer
-                items = torch.zeros(1, dtype=torch.int32, device=dev)
-            excl_rows = max(rowptr.numel() - 1, 0)
+        rowptr, items, excl_rows = _exclusion_on_device(exclude, dev)
         top_items = torch.empty((U, k), dtype=torch.int32, device=dev)
         top_scores = torch.empty((U, k), dtype=torch.float32, device=dev)
         pos = torch.empty(U, dtype=torch.int32, device=dev) if t is not None else None
@@ -601,6 +592,40 @@ class NeuMFEngine(object):
             bad = bad + ((t < 0) | (t.to(torch.int64) >= lens)).any().to(torch.float32).reshape(1)
         self.last_lists_bad = bad
         return top_items, top_scores, top_pos, pos, sums, probs
+
+    def catalogue_targets(self, users, targets, ks, exclude=None):
+        """Place of every held-out item of a user among the whole catalogue (mr_catalogue_targets): user users[u] has
+        the ascending target list items[rowptr[u]:rowptr[u + 1]] of targets = (rowptr int64 (U + 1,), items int32),
+        host or device, and its candidates are every item not on its exclusion list plus its targets.  exclude: as
+        catalogue_topk.  ks: 1 to MR_MAX_CUTOFFS cutoffs >= 1.  Returns device tensors (tpos (nnz,) int32 in list
+        order, sums (2 + 5 len(ks),) float32: [users with a target, mrr sum] then per cutoff [hit, precision, recall,
+        ndcg, map] sums).  Raises ValueError on a malformed rowptr or bad cutoffs before any launch.  Leaves in
+        `self.last_catalogue_bad` a one-element device tensor, non-zero when a user or target id was out of range
+        (such targets get position num_items)."""
+        dev = self.device
+        users = as_device_i32(users, dev)
+        U = users.numel()
+        rowptr, items = _check_lists(targets, U, dev)
+        nnz = items.numel()
+        kbuf, n_ks = _cutoffs(ks)
+        excl_rowptr, excl_items, excl_rows = _exclusion_on_device(exclude, dev)
+        tpos = torch.empty(nnz, dtype=torch.int32, device=dev)
+        sums = torch.zeros(nat.TGT_CUTOFF0 + nat.TGT_PER_CUTOFF * n_ks, dtype=torch.float32, device=dev)
+        nbytes = int(nat.lib.mr_catalogue_targets_workspace_bytes(C.byref(self._model), U, nnz))
+        if nbytes == 0:
+            raise ValueError("catalogue_targets: bad sizes U={} nnz={}".format(U, nnz))
+        ws = self._workspace(nbytes)
+        nat.check(nat.lib.mr_catalogue_targets(C.byref(self._model), _ptr(users), U, excl_rows, _ptr(excl_rowptr),
+                                               _ptr(excl_items), _ptr(rowptr), _ptr(items if nnz else None), nnz, kbuf,
+                                               n_ks, _ptr(tpos if nnz else None), _ptr(sums), _ptr(ws), ws.numel(),
+                                               self._stream()), "mr_catalogue_targets")
+        bad = torch.zeros(1, dtype=torch.float32, device=dev)
+        if U:
+            bad = bad + ((users.min() < 0) | (users.max() >= self.num_users)).to(torch.float32).reshape(1)
+        if nnz:
+            bad = bad + ((items.min() < 0) | (items.max() >= self.num_items)).to(torch.float32).reshape(1)
+        self.last_catalogue_bad = bad
+        return tpos, sums
 
     def _ids_out_of_range(self, users, items):
         if users.numel() == 0:
@@ -726,16 +751,7 @@ def topk_scores(scores, k, exclude=None, excl_ids=None, targets=None, device=Non
     k = int(k)
     ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
     t = as_device_i32(targets, device) if targets is not None else None
-    rowptr = items = None
-    excl_rows = 0
-    if exclude is not None:
-        rp, it = exclude
-        rowptr = (rp if isinstance(rp, torch.Tensor) else torch.from_numpy(np.asarray(rp, dtype=np.int64)))
-        rowptr = rowptr.reshape(-1).to(device, torch.int64).contiguous()
-        items = as_device_i32(it, device)
-        if items.numel() == 0:
-            items = torch.zeros(1, dtype=torch.int32, device=device)
-        excl_rows = max(rowptr.numel() - 1, 0)
+    rowptr, items, excl_rows = _exclusion_on_device(exclude, device)
     top_items = torch.empty((U, k), dtype=torch.int32, device=device)
     top_scores = torch.empty((U, k), dtype=torch.float32, device=device)
     pos = torch.empty(U, dtype=torch.int32, device=device) if t is not None else None
@@ -798,6 +814,59 @@ def topk_lists(scores, rowptr, k, targets=None, device=None):
     nat.check(nat.lib.mr_topk_lists(_ptr(s), U, _ptr(rp), nnz, k, _ptr(t), _ptr(top_pos), _ptr(top_scores), _ptr(pos),
                                     _ptr(sums), _ptr(ws), nbytes, st), "mr_topk_lists")
     return top_pos, top_scores, pos, sums
+
+
+def _cutoffs(ks):
+    """Cutoffs -> (host int32 array for the C ABI, count); ValueError unless 1..MR_MAX_CUTOFFS values, each >= 1."""
+    ks = [int(k) for k in np.asarray(ks).reshape(-1)]
+    if not 1 <= len(ks) <= nat.MR_MAX_CUTOFFS or min(ks) < 1:
+        raise ValueError("cutoffs must be 1 to {} values >= 1, got {}".format(nat.MR_MAX_CUTOFFS, ks))
+    return (C.c_int32 * len(ks))(*ks), len(ks)
+
+
+def _exclusion_on_device(exclude, device):
+    """None | (rowptr, items) host or device -> (device rowptr int64 or None, device items int32 or None, rows)."""
+    if exclude is None:
+        return None, None, 0
+    rp, it = exclude
+    rowptr = (rp if isinstance(rp, torch.Tensor) else torch.from_numpy(np.asarray(rp, dtype=np.int64)))
+    rowptr = rowptr.reshape(-1).to(device, torch.int64).contiguous()
+    items = as_device_i32(it, device)
+    if items.numel() == 0:  # every list empty: the library still wants a pointer
+        items = torch.zeros(1, dtype=torch.int32, device=device)
+    return rowptr, items, max(rowptr.numel() - 1, 0)
+
+
+def targets_scores(scores, targets, ks, exclude=None, excl_ids=None, device=None):
+    """Positions of many targets per row of a (U, N) score matrix (mr_targets_scores): row u's ascending targets are
+    items[rowptr[u]:rowptr[u + 1]] of targets = (rowptr, items); candidates are the items not on the row's exclusion
+    list (exclude / excl_ids as topk_scores) plus the row's targets; order as topk_scores.  Returns device tensors
+    (tpos (nnz,) int32 in list order, sums (2 + 5 len(ks),) float32 laid out as NeuMFEngine.catalogue_targets').
+    Raises ValueError on a malformed rowptr or bad cutoffs before any launch."""
+    require_cuda()
+    device = torch.device(device if device is not None else "cuda:{}".format(torch.cuda.current_device()))
+    s = scores if isinstance(scores, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(scores)))
+    if s.dim() != 2:
+        raise ValueError("scores must be (U, N), got shape {}".format(tuple(s.shape)))
+    U, N = int(s.shape[0]), int(s.shape[1])
+    s = s.to(device, torch.float32).contiguous()
+    rowptr, items = _check_lists(targets, U, device)
+    nnz = items.numel()
+    kbuf, n_ks = _cutoffs(ks)
+    ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
+    excl_rowptr, excl_items, excl_rows = _exclusion_on_device(exclude, device)
+    tpos = torch.empty(nnz, dtype=torch.int32, device=device)
+    sums = torch.zeros(nat.TGT_CUTOFF0 + nat.TGT_PER_CUTOFF * n_ks, dtype=torch.float32, device=device)
+    nbytes = int(nat.lib.mr_targets_scores_workspace_bytes(U, N, nnz))
+    if nbytes == 0:
+        raise ValueError("targets_scores: bad sizes U={} N={} nnz={}".format(U, N, nnz))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+    nat.check(nat.lib.mr_targets_scores(_ptr(s), U, N, _ptr(ids), excl_rows, _ptr(excl_rowptr), _ptr(excl_items),
+                                        _ptr(rowptr), _ptr(items if nnz else None), nnz, kbuf, n_ks,
+                                        _ptr(tpos if nnz else None), _ptr(sums), _ptr(ws), nbytes, st),
+              "mr_targets_scores")
+    return tpos, sums
 
 
 def gather_rows(table, idx):

@@ -13,6 +13,10 @@ MR_MAX_LAYERS = 8
 MR_MAX_WIDTH = 1024
 MR_MAX_NEGS = 1023
 MR_MAX_TOPK = 256
+MR_MAX_CUTOFFS = 8
+# sums of mr_targets_scores / mr_catalogue_targets: [users, mrr] then TGT_PER_CUTOFF metrics per cutoff
+TGT_USERS, TGT_MRR, TGT_CUTOFF0, TGT_PER_CUTOFF = 0, 1, 2, 5
+TGT_METRICS = ("hr", "precision", "recall", "ndcg", "map")  # MR_TGT_HIT .. MR_TGT_MAP
 MR_STEP_OUT_FLOATS = 8
 OUT_LOSS_SUM, OUT_HIT_SUM, OUT_DCG_SUM, OUT_L2_PENALTY, OUT_BAD_IDS = 0, 1, 2, 3, 4
 TRAIN_USERS_GROUPED = 1  # MR_TRAIN_USERS_GROUPED
@@ -90,6 +94,12 @@ SIGNATURES = {
     "mr_topk_scores": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_catalogue_topk_workspace_bytes": (_sz, [_PM, _i64, _i32]),
     "mr_catalogue_topk": (C.c_int, [_PM, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mr_targets_scores_workspace_bytes": (_sz, [_i64, _i32, _i64]),
+    "mr_targets_scores": (C.c_int, [_vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _sz,
+                                    _vp]),
+    "mr_catalogue_targets_workspace_bytes": (_sz, [_PM, _i64, _i64]),
+    "mr_catalogue_targets": (C.c_int, [_PM, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _sz,
+                                       _vp]),
     "mr_topk_lists_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "mr_topk_lists": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_rank_lists_workspace_bytes": (_sz, [_PM, _i64, _i64, _i32]),

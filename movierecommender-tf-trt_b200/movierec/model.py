@@ -643,8 +643,62 @@ class MovierecModel(object):
         G = max(int(users.size), 1)
         return total[0] / G, total[1] / G
 
+    def evaluate_full_catalogue_sets(self, test, exclude=None, ks=None):
+        """All-items ranking evaluation with several held-out items per user (a per-user last-20 % or temporal split,
+        all of a user's future ratings): each held-out item is ranked among every item not on the user's exclusion list
+        plus the user's held-out items (which are never excluded).  test: a ratings DataFrame (user / item columns) or
+        a (rowptr, items) CSR indexed by user id with ascending lists; the users evaluated are those with a non-empty
+        list.  exclude: as evaluate_full_catalogue -- typically the training generator.  ks: cutoffs (default: the
+        model's k).  Returns the means over the users evaluated: {"mrr", "hr@k", "precision@k", "recall@k", "ndcg@k",
+        "map@k"} for every cutoff k.  Raises IndexError on an out-of-range user or item."""
+        ks = (self._k,) if ks is None else tuple(int(k) for k in np.asarray(ks).reshape(-1))
+        import torch
+        eng = self.model.engine
+        nu, ni = eng.num_users, eng.num_items
+        if hasattr(test, "columns"):
+            from . import data_pipeline as dp
+            u = np.asarray(test[dp.COL_USER_ID], dtype=np.int64)
+            i = np.asarray(test[dp.COL_ITEM_ID], dtype=np.int64)
+            self.model._raise_on_bad_ids(_ids_outside(u, nu) or _ids_outside(i, ni))
+            rowptr, items = np.zeros(nu + 1, np.int64), np.zeros(0, np.int32)
+            if u.size:
+                rp, it = _engine_module().build_user_csr(u.astype(np.int32), i.astype(np.int32), nu, ni)
+                rowptr, items = rp.cpu().numpy(), it.cpu().numpy()
+        else:
+            rp, it = test
+            rowptr = np.asarray(rp.cpu() if hasattr(rp, "cpu") else rp, dtype=np.int64).reshape(-1)
+            items = np.asarray(it.cpu() if hasattr(it, "cpu") else it, dtype=np.int64).reshape(-1)
+            if rowptr.size < 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
+                raise ValueError("test lists: offsets must start at 0, never decrease and end at {}".format(items.size))
+            self.model._raise_on_bad_ids(_ids_outside(items, ni) or bool(np.any(rowptr[nu + 1:] > rowptr[nu])))
+            inner = np.ones(max(items.size - 1, 0), bool)
+            inner[rowptr[1:-1][(rowptr[1:-1] > 0) & (rowptr[1:-1] < items.size)] - 1] = False
+            if np.any((items[1:] <= items[:-1]) & inner):
+                raise ValueError("test lists: every user's items must be strictly ascending")
+            items = items.astype(np.int32)
+        users = np.flatnonzero(rowptr[1:] > rowptr[:-1]).astype(np.int32)
+        total = np.zeros(2 + 5 * len(ks), np.float64)  # [users, mrr] + 5 per cutoff: MR_TGT_* of movierec_b200.h
+        if users.size:
+            r0, r1 = int(rowptr[users[0]]), int(rowptr[users[-1] + 1])
+            sub_rowptr = np.append(rowptr[users], r1) - r0
+            sub_items = items[r0:r1]
+            excl = _exclusion_lists(exclude)
+            sums = []
+            for lo, hi in _list_chunks(sub_rowptr, TARGETS_CALL_ROWS):
+                a, b = int(sub_rowptr[lo]), int(sub_rowptr[hi])
+                sums.append(eng.catalogue_targets(users[lo:hi], (sub_rowptr[lo:hi + 1] - a, sub_items[a:b]), ks,
+                                                  exclude=excl)[1])
+            total = torch.stack(sums).cpu().numpy().astype(np.float64).sum(axis=0)  # call order
+        G = max(total[0], 1.0)
+        out = {"mrr": total[1] / G}
+        for c, k in enumerate(ks):
+            for m, name in enumerate(("hr", "precision", "recall", "ndcg", "map")):
+                out["{}@{}".format(name, k)] = total[2 + 5 * c + m] / G
+        return out
+
 
 LISTS_CALL_ROWS = 1 << 22  # candidates per device call of recommend_batch / evaluate_candidate_lists
+TARGETS_CALL_ROWS = (1 << 31) - 1  # held-out items per device call of evaluate_full_catalogue_sets (int32 counts)
 
 
 def _candidate_csr(candidate_lists, U):
