@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 103     /* major*100 + minor */
+#define MR_VERSION 104     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
@@ -310,6 +310,41 @@ size_t mr_rank_lists_workspace_bytes(const MrModel* model, int64_t U, int64_t nn
 int mr_rank_lists(const MrModel* model, const int32_t* users, int64_t U, const int64_t* rowptr, const int32_t* items,
                   int64_t nnz, int32_t k, const int32_t* targets, int32_t* top_pos, int32_t* top_items, float* top_scores,
                   int32_t* pos, float* sums, float* probs, void* ws, size_t ws_bytes, void* stream);
+
+/* Fold-in of new users (or of known users whose history has grown): the item tables and the dense block stay frozen
+ * and only each user's two embedding rows (MLP, GMF) are optimised against the user's history and sampled negatives --
+ * the standard answer for embedding models with no closed-form user solve, and the protocol of "strong generalisation"
+ * evaluation.  The results are plain (U, dim) tables: a copy of the MrModel whose user_mlp / user_gmf point at them
+ * and whose num_users = U is served and evaluated by every call above, unchanged.
+ * Histories: a CSR over the U new users (device rowptr U + 1 int64, rowptr[0] = 0, non-decreasing, rowptr[U] = nnz;
+ * device items, each list strictly ascending, ids in [0, num_items), no list covering every item -- the format of the
+ * exclusion lists).  init_users (device, U, may be NULL = all -1): the model row user u starts from, -1 = zero rows.
+ * The model is never written.  For user u, with list S of n items, and step t = 0 .. steps-1:
+ *   1. the positive at position j of S draws `negs` negatives from the items not in S with mr_sample_negatives' rule
+ *      (index = j, epoch = t, seed; with fewer candidates than negs, with replacement) -- n (negs + 1) rows;
+ *   2. forward and BCE over those rows, loss = their mean;
+ *   3. the gradient with respect to u's MLP and GMF rows only, plus 2 l2[0] row;
+ *   4. one legacy-Keras Adam step (per-user m and v from zero, step size lr sqrt(1-b2^(t+1)) / (1-b1^(t+1))) or SGD.
+ * A user's result depends only on the model, its list, its initial rows and cfg (never on the other users of the call
+ * or their order) and is bit-identical run to run: fixed summation orders, no float atomics.
+ * out_loss (U, may be NULL): the mean BCE of the last step, before its update; NaN when steps = 0 or the list is
+ * empty.  Validation: the sizes and cfg on the host; then one small kernel checks the CSR, the item ids and
+ * init_users and the call reads back one word (the only synchronisation) before any other launch -- MR_ERR_INVALID
+ * for a malformed rowptr, an unsorted list, an id out of range or a list covering every item.
+ * Workspace: the item half of the first layer over the item table (num_items x layers_sizes[1] floats; none without
+ * a hidden layer), the transposed dense block and the sort of the users by history length. */
+typedef struct MrFoldIn {     /* [host] */
+  int32_t steps;              /* optimisation steps per user (0 = return the initial rows) */
+  int32_t negs;               /* negatives per positive per step, 1..MR_MAX_NEGS */
+  int32_t optimizer;          /* MrOptimizer */
+  float lr, beta_1, beta_2, epsilon;
+  uint64_t seed;
+} MrFoldIn;
+size_t mr_fold_in_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz);
+int mr_fold_in_users(const MrModel* model, const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz,
+                     const int32_t* init_users, const MrFoldIn* cfg /*[host]*/, float* out_user_mlp /* (U, L[0]/2) */,
+                     float* out_user_gmf /* (U, mf_dim), NULL when mf_dim == 0 */, float* out_loss, void* ws,
+                     size_t ws_bytes, void* stream);
 
 /* On-device negative sampler -- replaces _get_random_negatives_and_positive
  * (data_pipeline.py:99-113): for positive p (global index first_index + p, user pos_users[p]) draw

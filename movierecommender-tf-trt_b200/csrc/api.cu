@@ -2171,6 +2171,118 @@ int mr_sample_negatives(const int64_t* csr_rowptr, const int32_t* csr_items, int
   return rc;
 }
 
+// ---- fold-in: the item half of the first layer once per call (the tensor-core table GEMM on the towers whose item
+// projection it already computes, else a per-element kernel), the users sorted by history length, one kernel ----------
+static bool fold_in_tc_pi(const MrModel& m) {
+  const int d_i = m.L[0] - m.L[0] / 2;
+  return use_tc(m) && m.n_layers >= 3 && d_i % 128 == 0 && d_i <= 256 && m.L[1] == d_i;
+}
+
+struct FoldWs {
+  int32_t *flags, *keys, *sorted_keys, *order;
+  void* sort_ws;
+  size_t sort_ws_bytes;
+  float *wt, *Pi, *pack_fi;
+  size_t total;
+};
+
+static FoldWs carve_fold_in(const MrModel& m, int64_t U, void* ws) {
+  FoldWs w{};
+  Carver cv(ws);
+  const int d_i = m.L[0] - m.L[0] / 2;
+  w.flags = cv.take<int32_t>(64);
+  w.keys = cv.take<int32_t>(U);
+  w.sorted_keys = cv.take<int32_t>(U);
+  w.order = cv.take<int32_t>(U);
+  w.sort_ws_bytes = sort_workspace_bytes(U);
+  w.sort_ws = cv.take<char>(w.sort_ws_bytes);
+  w.wt = cv.take<float>(m.dense_count);
+  if (m.n_layers > 1) w.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
+  if (fold_in_tc_pi(m)) w.pack_fi = cv.take<float>((size_t)2 * d_i * m.L[1]);
+  w.total = cv.off;
+  return w;
+}
+
+size_t mr_fold_in_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz) {
+  if (check_model(model) != MR_OK || U < 0 || U > INT32_MAX || nnz < 0 || nnz > INT32_MAX) return 0;
+  return carve_fold_in(*model, U, nullptr).total;
+}
+
+int mr_fold_in_users(const MrModel* model, const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz,
+                     const int32_t* init_users, const MrFoldIn* cfg, float* out_user_mlp, float* out_user_gmf,
+                     float* out_loss, void* ws, size_t ws_bytes, void* stream) {
+  int rc = check_model(model);
+  if (rc != MR_OK) return rc;
+  const MrModel& m = *model;
+  cudaStream_t st = (cudaStream_t)stream;
+  MR_REQUIRE(cfg != nullptr, "fold_in: cfg is NULL");
+  MR_REQUIRE(cfg->steps >= 0, "fold_in: steps=%d must be >= 0", cfg->steps);
+  MR_REQUIRE(cfg->negs >= 1 && cfg->negs <= MR_MAX_NEGS, "fold_in: negs=%d out of [1,%d]", cfg->negs, MR_MAX_NEGS);
+  MR_REQUIRE(cfg->optimizer == MR_OPT_ADAM || cfg->optimizer == MR_OPT_SGD, "fold_in: unknown optimizer %d",
+             cfg->optimizer);
+  MR_REQUIRE(isfinite(cfg->lr), "fold_in: lr must be finite");
+  if (cfg->optimizer == MR_OPT_ADAM)
+    MR_REQUIRE(cfg->beta_1 >= 0.f && cfg->beta_1 < 1.f && cfg->beta_2 >= 0.f && cfg->beta_2 < 1.f && cfg->epsilon > 0.f,
+               "fold_in: Adam needs beta_1, beta_2 in [0, 1) and epsilon > 0");
+  MR_REQUIRE(U >= 0 && U <= INT32_MAX && nnz >= 0 && nnz <= INT32_MAX, "fold_in: bad sizes U=%lld nnz=%lld",
+             (long long)U, (long long)nnz);
+  MR_REQUIRE(rowptr != nullptr, "fold_in: rowptr is NULL");
+  MR_REQUIRE(nnz == 0 || items != nullptr, "fold_in: items is NULL");
+  MR_REQUIRE(U == 0 || out_user_mlp != nullptr, "fold_in: out_user_mlp is NULL");
+  MR_REQUIRE(U == 0 || m.mf_dim == 0 || out_user_gmf != nullptr, "fold_in: out_user_gmf is NULL but mf_dim > 0");
+  MR_REQUIRE(fold_in_supported(m), "fold_in: layer widths too large for the kernel's shared memory");
+  const FoldWs w = carve_fold_in(m, U, ws);
+  if (ws == nullptr || ws_bytes < w.total) {
+    set_error("fold_in: workspace %zu bytes < %zu", ws_bytes, w.total);
+    return MR_ERR_WORKSPACE;
+  }
+  if (U == 0) return MR_OK;
+
+  // the histories are checked before any other work: one small kernel and a one-word read-back
+  MR_CUDA(cudaMemsetAsync(w.flags, 0, sizeof(int32_t), st));
+  rc = launch_fold_in_check(rowptr, items, U, nnz, m.num_items, init_users, m.num_users, w.keys, w.flags, st);
+  if (rc != MR_OK) return rc;
+  int32_t bad = 0;
+  MR_CUDA(cudaMemcpyAsync(&bad, w.flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  MR_CUDA(cudaStreamSynchronize(st));
+  MR_REQUIRE(!(bad & 1), "fold_in: rowptr must start at 0, never decrease and end at nnz, and every list must be "
+             "strictly ascending");
+  MR_REQUIRE(!(bad & 2), "fold_in: an item id lies outside [0, %d)", m.num_items);
+  MR_REQUIRE(!(bad & 4), "fold_in: an init user lies outside [-1, %d)", m.num_users);
+  MR_REQUIRE(!(bad & 8), "fold_in: a history covers every item: no negatives to draw");
+
+  rc = launch_sort_pairs(w.keys, U, bits_for((int64_t)m.num_items + 1), w.sorted_keys, w.order, w.sort_ws,
+                         w.sort_ws_bytes, st);
+  if (rc == MR_OK) rc = launch_transpose_kernels(m, w.wt, st);
+  if (rc == MR_OK && m.n_layers > 1) {
+    if (fold_in_tc_pi(m)) {
+      TcWs t{};
+      t.pack_fi = w.pack_fi;
+      t.Pi = w.Pi;
+      const int d_u = m.L[0] / 2;
+      rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], m.L[0] - d_u, m.L[1], 0, t.pack_fi, st);
+      if (rc == MR_OK) rc = tc_project_items(m, t, st);
+    } else {
+      rc = launch_fold_in_project(m, w.Pi, st);
+    }
+  }
+  if (rc != MR_OK) return rc;
+  FoldInArgs a{};
+  a.model = model;
+  a.wt = w.wt;
+  a.Pi = w.Pi;
+  a.rowptr = rowptr;
+  a.items = items;
+  a.init_users = init_users;
+  a.order = w.order;
+  a.U = U;
+  a.cfg = *cfg;
+  a.out_mlp = out_user_mlp;
+  a.out_gmf = out_user_gmf;
+  a.out_loss = out_loss;
+  return launch_fold_in(a, st);
+}
+
 int mr_users_grouped(const int32_t* users, int64_t n, int32_t group, int32_t* flag, void* stream) {
   MR_REQUIRE(users != nullptr && flag != nullptr, "users_grouped: NULL pointer");
   MR_REQUIRE(n >= 0 && group >= 1, "users_grouped: bad sizes");

@@ -175,6 +175,30 @@ int launch_sample_negatives(const int64_t* rowptr, const int32_t* csr_items, int
                             int negs, uint64_t seed, uint64_t epoch, int32_t* out_users, int32_t* out_items,
                             float* out_labels, cudaStream_t st);
 
+// ---- fold_in.cu: per-user optimisation of the user rows against a history, everything else frozen ----------------
+struct FoldInArgs {
+  const MrModel* model;
+  const float* wt;          // transposed hidden kernels, dense-block layout
+  const float* Pi;          // (num_items x L1) item half of the first layer; NULL without a hidden layer
+  const int64_t* rowptr;
+  const int32_t* items;
+  const int32_t* init_users;
+  const int32_t* order;     // the U users, longest history first
+  int64_t U;
+  MrFoldIn cfg;
+  float* out_mlp;
+  float* out_gmf;
+  float* out_loss;
+};
+bool fold_in_supported(const MrModel& m);
+int launch_fold_in(const FoldInArgs& a, cudaStream_t st);
+// Pi = E_item . W1[item rows] with one thread per output (any widths)
+int launch_fold_in_project(const MrModel& m, float* Pi, cudaStream_t st);
+// flags[0] |= 1 malformed rowptr or unsorted list, 2 item out of range, 4 init user out of range, 8 a list covering
+// every item; keys[u] = num_items - length of list u (the longest history sorts first)
+int launch_fold_in_check(const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz, int32_t num_items,
+                         const int32_t* init_users, int32_t num_users, int32_t* keys, int32_t* flags, cudaStream_t st);
+
 // ---- tc_dense.cu / tc_wgrad.cu / head.cu: tensor-core path of the train step ------------------------
 enum { TC_EPI_BIAS_RELU = 0, TC_EPI_MASK = 1, TC_EPI_STAGE = 2, TC_EPI_HEAD_DOT = 3 };
 struct TcDenseArgs {

@@ -281,6 +281,10 @@ class NeuMFEngine(object):
 
     # ---- C structs ------------------------------------------------------------------------------
     def _structs(self):
+        self._model_struct()
+        self._opt_structs()
+
+    def _model_struct(self):
         m = nat.MrModel()
         m.user_mlp, m.item_mlp = self.user_mlp.data_ptr(), self.item_mlp.data_ptr()
         m.user_gmf = self.user_gmf.data_ptr() if self.mf_dim else None
@@ -302,6 +306,8 @@ class NeuMFEngine(object):
         m.mf_dim = self.mf_dim
         m.compute_path, m.item_projection, m.fused_train = self.compute_path, self.item_projection, self.fused_train
         self._model = m
+
+    def _opt_structs(self):
 
         o = nat.MrOptState()
         o.optimizer = nat.OPT_ADAM if self.optimizer == "adam" else nat.OPT_SGD
@@ -627,6 +633,57 @@ class NeuMFEngine(object):
         self.last_catalogue_bad = bad
         return tpos, sums
 
+    def fold_in(self, histories, steps, lr, negs, seed=0, init_users=None, optimizer=None, beta_1=None, beta_2=None):
+        """Fold-in of U new users (mr_fold_in_users): the item tables and the dense block stay frozen and only each
+        user's MLP and GMF rows are optimised, `steps` times, against the user's history and `negs` sampled negatives
+        per positive per step.  histories: (rowptr, items) with ascending lists, host or device, or a list of item
+        arrays (sorted and de-duplicated here).  init_users (U,): the row of this model a user starts from, -1 = zero
+        rows (default: all zero).  optimizer / beta_1 / beta_2 default to the engine's.  Returns device tensors
+        (user_mlp (U, d_u), user_gmf (U, mf_dim) or None, loss (U,): the mean BCE of each user's last step before its
+        update, NaN for steps = 0 or an empty history).  Raises IndexError on an item or init user out of range and
+        ValueError on a malformed CSR or a history that covers every item, before any launch."""
+        dev = self.device
+        rowptr, items = fold_in_histories(histories, self.num_items)
+        U, nnz = rowptr.size - 1, items.size
+        init = None
+        if init_users is not None:
+            init = np.asarray(init_users.cpu() if hasattr(init_users, "cpu") else init_users, np.int64).reshape(-1)
+            if init.size != U:
+                raise ValueError("init_users ({}) and histories ({}) differ in length".format(init.size, U))
+            if init.size and (init.min() < -1 or init.max() >= self.num_users):
+                raise IndexError("init_users: a user lies outside [-1, {})".format(self.num_users))
+        optimizer = self.optimizer if optimizer is None else optimizer
+        if optimizer not in ("adam", "sgd"):
+            raise ValueError("optimizer must be 'adam' or 'sgd', found {!r}".format(optimizer))
+        cfg = nat.MrFoldIn()
+        cfg.steps, cfg.negs = int(steps), int(negs)
+        cfg.optimizer = nat.OPT_ADAM if optimizer == "adam" else nat.OPT_SGD
+        cfg.lr = float(lr)
+        cfg.beta_1 = float(self.beta_1 if beta_1 is None else beta_1)
+        cfg.beta_2 = float(self.beta_2 if beta_2 is None else beta_2)
+        cfg.epsilon = ADAM_EPSILON
+        cfg.seed = int(seed) & (2 ** 64 - 1)
+        d_rowptr = torch.from_numpy(rowptr).to(dev)
+        d_items = torch.from_numpy(items if nnz else np.zeros(1, np.int32)).to(dev)
+        d_init = torch.from_numpy(init.astype(np.int32)).to(dev) if init is not None and U else None
+        f32 = torch.float32
+        out_mlp = torch.empty((U, self.d_u), dtype=f32, device=dev)
+        out_gmf = torch.empty((U, self.mf_dim), dtype=f32, device=dev) if self.mf_dim else None
+        loss = torch.empty(U, dtype=f32, device=dev)
+        nbytes = int(nat.lib.mr_fold_in_workspace_bytes(C.byref(self._model), U, nnz))
+        ws = self._workspace(max(nbytes, 256))
+        nat.check(nat.lib.mr_fold_in_users(C.byref(self._model), _ptr(d_rowptr), _ptr(d_items), U, nnz, _ptr(d_init),
+                                           C.byref(cfg), _ptr(out_mlp), _ptr(out_gmf), _ptr(loss), _ptr(ws), ws.numel(),
+                                           self._stream()), "mr_fold_in_users")
+        return out_mlp, out_gmf, loss
+
+    def user_view(self, user_mlp, user_gmf=None):
+        """An engine whose users are the rows of user_mlp (U, d_u) / user_gmf (U, mf_dim) -- typically fold_in's
+        output -- and which shares this engine's item tables and dense block (not copies: later updates of this
+        engine show through).  Every scoring and evaluation call works on it with user id u = row u; training it,
+        changing its weights or reading optimizer state raises."""
+        return UserViewEngine(self, user_mlp, user_gmf)
+
     def _ids_out_of_range(self, users, items):
         if users.numel() == 0:
             return torch.zeros(1, dtype=torch.float32, device=self.device)
@@ -681,6 +738,75 @@ class NeuMFEngine(object):
         if check_ids:
             self.last_eval_bad = self._ids_out_of_range(d_users, d_items)
         return pos, sums.sum(dim=0), None, None
+
+
+class UserViewEngine(NeuMFEngine):
+    """NeuMFEngine.user_view: other user tables in front of a model's item tables and dense block.  Scoring only."""
+
+    def __init__(self, base, user_mlp, user_gmf=None):
+        self.__dict__.update({k: v for k, v in base.__dict__.items() if k in _VIEW_SHARED})
+        f32 = torch.float32
+        user_mlp = user_mlp.to(self.device, f32).contiguous()
+        if user_mlp.dim() != 2 or user_mlp.shape[1] != self.d_u or user_mlp.shape[0] < 1:
+            raise ValueError("user_mlp must be (U >= 1, {}), got {}".format(self.d_u, tuple(user_mlp.shape)))
+        if self.mf_dim:
+            if user_gmf is None:
+                raise ValueError("the model has a GMF branch: user_gmf (U, {}) is required".format(self.mf_dim))
+            user_gmf = user_gmf.to(self.device, f32).contiguous()
+            if tuple(user_gmf.shape) != (user_mlp.shape[0], self.mf_dim):
+                raise ValueError("user_gmf must be ({}, {}), got {}".format(user_mlp.shape[0], self.mf_dim,
+                                                                           tuple(user_gmf.shape)))
+        else:
+            user_gmf = None
+        self.num_users = int(user_mlp.shape[0])
+        self.user_mlp, self.user_gmf = user_mlp, user_gmf
+        self._tables = dict(base._tables)
+        self._tables[K_USER] = user_mlp
+        if self.mf_dim:
+            self._tables[K_GMF_USER] = user_gmf
+        self._ws = None
+        self._model_struct()
+
+    def _scoring_only(self, *args, **kwargs):
+        raise RuntimeError("a user view only scores: train, update or save the model it was made from")
+
+    train_step = train_grads = apply = apply_region = finish_apply = apply_dense_only = _scoring_only
+    set_weights = initialize = get_optimizer_state = set_optimizer_state = rebind_flat = _scoring_only
+    gradient_tensors = gradient_parts = gradient_regions = _scoring_only
+
+
+# what a user view shares with its base engine (the item tables and dense block by reference, the description by value)
+_VIEW_SHARED = ("compute_path", "item_projection", "fused_train", "device", "num_items", "L", "l2", "mf_dim", "d_u", "d_i",
+                "optimizer", "lr", "beta_1", "beta_2", "table_mode", "iterations", "_dense_slices", "dense_count",
+                "item_mlp", "item_gmf", "dense")
+
+
+def fold_in_histories(histories, num_items):
+    """Histories of fold_in -> host (rowptr int64 (U + 1,), items int32).  (rowptr, items) with ascending lists (host or
+    device tensors or arrays) is checked as is; a list of item arrays is sorted and de-duplicated per user.  Raises
+    IndexError on an item outside [0, num_items) and ValueError on a malformed rowptr, a list that is not strictly
+    ascending or a list that covers every item."""
+    host = lambda x: np.asarray(x.cpu() if hasattr(x, "cpu") else x)
+    if isinstance(histories, tuple) and len(histories) == 2:
+        rowptr = host(histories[0]).astype(np.int64).reshape(-1)
+        items = host(histories[1]).astype(np.int64).reshape(-1)
+    else:
+        parts = [np.unique(host(h).astype(np.int64).reshape(-1)) for h in histories]
+        rowptr = np.zeros(len(parts) + 1, np.int64)
+        rowptr[1:] = np.cumsum([p.size for p in parts])
+        items = np.concatenate(parts) if parts else np.zeros(0, np.int64)
+    if rowptr.size < 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
+        raise ValueError("histories: offsets must start at 0, never decrease and end at len(items) = {}".format(items.size))
+    if items.size and (items.min() < 0 or items.max() >= num_items):
+        raise IndexError("histories: an item lies outside [0, {})".format(num_items))
+    inner = np.ones(max(items.size - 1, 0), bool)  # pairs of neighbours inside one list
+    starts = rowptr[1:-1]
+    inner[starts[(starts > 0) & (starts < items.size)] - 1] = False
+    if np.any((items[1:] <= items[:-1]) & inner):
+        raise ValueError("histories: every user's items must be strictly ascending")
+    if np.any(rowptr[1:] - rowptr[:-1] >= num_items):
+        raise ValueError("histories: a history covers every item, so there is no negative to draw")
+    return rowptr, items.astype(np.int32)
 
 
 # Kernel selection is part of the model description handed to the library (MrModel), not library state.  These

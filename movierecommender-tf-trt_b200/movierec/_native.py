@@ -71,9 +71,16 @@ class MrGrads(C.Structure):
                 ("user_gmf_ready", C.c_void_p)]
 
 
+class MrFoldIn(C.Structure):
+    _fields_ = [("steps", C.c_int32), ("negs", C.c_int32), ("optimizer", C.c_int32),
+                ("lr", C.c_float), ("beta_1", C.c_float), ("beta_2", C.c_float), ("epsilon", C.c_float),
+                ("seed", C.c_uint64)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/movierec_b200.h
 _vp, _i32, _i64, _u64, _f, _sz = C.c_void_p, C.c_int32, C.c_int64, C.c_uint64, C.c_float, C.c_size_t
 _PM, _PO, _PG = C.POINTER(MrModel), C.POINTER(MrOptState), C.POINTER(MrGrads)
+_PF = C.POINTER(MrFoldIn)
 SIGNATURES = {
     "mr_version": (C.c_int, []),
     "mr_last_error": (C.c_char_p, []),
@@ -105,6 +112,8 @@ SIGNATURES = {
     "mr_rank_lists_workspace_bytes": (_sz, [_PM, _i64, _i64, _i32]),
     "mr_rank_lists": (C.c_int, [_PM, _vp, _i64, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
                                 _vp]),
+    "mr_fold_in_workspace_bytes": (_sz, [_PM, _i64, _i64]),
+    "mr_fold_in_users": (C.c_int, [_PM, _vp, _vp, _i64, _i64, _vp, _PF, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_sample_negatives": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i64, _i32, _u64, _u64, _vp, _vp, _vp, _vp]),
     "mr_sort_workspace_bytes": (_sz, [_i64]),
     "mr_sort_pairs": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _sz, _vp]),

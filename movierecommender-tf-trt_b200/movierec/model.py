@@ -50,6 +50,14 @@ METRIC_VAL_DCG = "val_{}_{}".format(OUTPUT_PRED, DCG)
 
 EARLY_STOPPING_PATIENCE = 5  # model.py:324
 
+# Fold-in defaults (MovierecModel.fold_in), from the planted-cluster grid of tools/fold_in_bench.py --quality
+# (profiles/r06_fold_in_quality.json, Adam, 4 negatives): recall@10 of the folded-in users is flat at 0.28-0.30 for lr
+# 0.03-0.3 at 5-100 steps, and the mean loss still falls up to about 30 steps; lr 0.01 needs >= 20 steps, and the
+# training lr 0.001 reaches the plateau only at 100 steps (0.04 at 30).  30 steps at 0.05 sits inside the plateau on
+# both axes.
+FOLD_IN_STEPS = 30
+FOLD_IN_LR = 0.05
+
 
 def _engine_module():
     # imported lazily so that parameter validation (pure host logic) works without a GPU;
@@ -198,6 +206,17 @@ class NeuMFModel(object):
             out_items[lo:hi] = top.cpu().numpy()
             out_scores[lo:hi] = sc.cpu().numpy()
         return out_items, out_scores
+
+    def recommend_for_histories(self, histories, top_k=10, **fold_in_args):
+        """Top-k for users the model has not seen, from their rating histories alone: one fold-in of every history
+        (MovierecModel.fold_in, whose keyword arguments fold_in_args takes) and one full-catalogue top-k call on the
+        folded rows, with each history as that user's exclusion list.  histories as MovierecModel.fold_in.  Returns
+        NumPy (items (U, top_k) int32, scores (U, top_k) float32) like recommend_for_users."""
+        eng = self.engine
+        rowptr, items = _engine_module().fold_in_histories(histories, eng.num_items)
+        view = self._owner.fold_in((rowptr, items), **fold_in_args)
+        return view.model.recommend_for_users(np.arange(rowptr.size - 1, dtype=np.int32), top_k,
+                                              exclude=(rowptr, items))
 
     def _step_logs(self, out, rows, group):
         loss = out[0] / rows + out[3]
@@ -587,6 +606,22 @@ class MovierecModel(object):
                                         validation_data=validation_data_generator,
                                         epochs=epochs, callbacks=callbacks, verbose=self.verbose)
 
+    def fold_in(self, histories, steps=None, lr=None, negs=None, seed=0, init_users=None):
+        """Fold-in of users the model was not trained on (or of known users whose history has grown): the item tables
+        and the dense block stay frozen and only each user's two embedding rows are optimised, on the device, against
+        the user's history and sampled negatives.  histories: a list of item arrays (one per user, any order) or a
+        (rowptr, items) CSR of ascending lists.  steps / lr default to FOLD_IN_STEPS / FOLD_IN_LR, negs to the model's
+        num_negs_per_pos; the optimiser is the model's.  init_users: per user, the model row to start from (-1 = zero
+        rows, the default).  Returns a FoldedModel whose user id u is new user u: recommend_for_users, recommend_batch,
+        evaluate_full_catalogue and evaluate_full_catalogue_sets work on it unchanged; .user_weights() gives the rows
+        and .loss each user's last-step loss.  Raises IndexError on an out-of-range item or init user and ValueError on
+        a malformed CSR or a history that covers every item."""
+        eng = self.model.engine
+        mlp, gmf, loss = eng.fold_in(histories, FOLD_IN_STEPS if steps is None else steps,
+                                     FOLD_IN_LR if lr is None else lr,
+                                     self._num_negs_per_pos if negs is None else negs, seed=seed, init_users=init_users)
+        return FoldedModel(self, mlp, gmf, loss)
+
     def evaluate(self, users, items, k=None):
         """Full-sweep ranking evaluation (BASELINE config 4): one user id per group and
         (negs_eval+1) candidate items per user with the positive last.  Returns (hr, dcg)."""
@@ -695,6 +730,35 @@ class MovierecModel(object):
             for m, name in enumerate(("hr", "precision", "recall", "ndcg", "map")):
                 out["{}@{}".format(name, k)] = total[2 + 5 * c + m] / G
         return out
+
+
+class FoldedModel(MovierecModel):
+    """MovierecModel.fold_in's result: user id u is new user u, items and dense block are the model's (shared).
+    Scoring and evaluation work as on the model; training and saving raise."""
+
+    def __init__(self, base, user_mlp, user_gmf, loss):
+        self.__dict__.update(base.__dict__)
+        view = base.model.engine.user_view(user_mlp, user_gmf)
+        self._num_users = view.num_users
+        self.model = _FoldedNeuMF(self, view)
+        self.loss = loss.cpu().numpy()
+
+    def user_weights(self):
+        """The folded rows as NumPy: (user_mlp (U, L[0]/2), user_gmf (U, mf_dim) or None)."""
+        e = self.model.engine
+        return e.user_mlp.cpu().numpy(), (e.user_gmf.cpu().numpy() if e.user_gmf is not None else None)
+
+    def _no_training(self, *args, **kwargs):
+        raise RuntimeError("a folded-in model only scores: train or save the model it was folded into")
+
+    fit_generator = save = _no_training
+
+
+class _FoldedNeuMF(NeuMFModel):
+    def _no_training(self, *args, **kwargs):
+        raise RuntimeError("a folded-in model only scores: train or save the model it was folded into")
+
+    train_on_batch = fit_generator = save_weights = load_weights = set_weights = _no_training
 
 
 LISTS_CALL_ROWS = 1 << 22  # candidates per device call of recommend_batch / evaluate_candidate_lists
