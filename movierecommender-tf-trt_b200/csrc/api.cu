@@ -195,12 +195,12 @@ static bool use_tc(const MrModel& m) { return m.compute_path != MR_PATH_SIMT && 
 // GEMM and of the weight gradient run on num_items rows instead of `rows`.  Same values up to summation order.
 // Needs L1 == d_i so that the staged item rows keep their width d_i + f, and dense gradient tables.
 // (selector: MrModel.item_projection -- part of the model description, so that workspace sizing and the launch
-// sequence of every call on that model agree)
-static bool item_proj_ok(const MrModel& m, int64_t rows) {
+// sequence of every call on that model agree).  any_rows: a choice of the model alone, AUTO as at any row count.
+static bool item_proj_ok(const MrModel& m, int64_t rows, bool any_rows = false) {
   if (m.item_projection == MR_PROJECTION_OFF || !use_tc(m) || m.n_layers < 3) return false;
   const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
   if (d_i % 128 || d_i > 256 || m.L[1] != d_i) return false;
-  if (m.item_projection == MR_PROJECTION_ON) return true;
+  if (m.item_projection == MR_PROJECTION_ON || any_rows) return true;
   return 2 * (int64_t)m.num_items <= rows;  // three GEMMs over num_items rows replace three over `rows` rows
 }
 
@@ -224,10 +224,10 @@ static bool small_proj_ok(const MrModel& m, int64_t rows, int group) {
 }
 
 // ranking eval of the default tower: one user id per group of candidates, Pi / Pu over the tables first
-static bool small_eval_ok(const MrModel& m, int64_t rows) {
+static bool small_eval_ok(const MrModel& m, int64_t rows, bool any_rows = false) {
   if (use_tc(m) || m.item_projection == MR_PROJECTION_OFF || m.fused_train == MR_FUSED_OFF) return false;
   if (!small_tower_supported(m, 5)) return false;
-  if (m.item_projection == MR_PROJECTION_ON) return true;
+  if (m.item_projection == MR_PROJECTION_ON || any_rows) return true;
   return 2 * ((int64_t)m.num_items + m.num_users) <= rows;
 }
 
@@ -339,6 +339,30 @@ static TcWs carve_tc(const MrModel& m, bool train, int64_t B, void* ws) {
 //  - train with Pu: H1 = relu(Pi[item] + Pu[user]), the user half once per USER;
 //  - train with Pi only: Zu, then H1 = relu(Pi[item] + Zu[group]);
 //  - eval or train without Pi: Zu, then H1 = relu(E_item[item] . W1[item rows] + Zu[group]).
+// Zu rows [0, rows) = E_user[users[(row0 + r) * user_mul]] . W1[user rows] + b1 (a zero row for an out-of-range user).
+static int tc_user_half(const MrModel& m, const TcWs& t, const int32_t* users, int user_mul, int64_t row0, int64_t rows,
+                        cudaStream_t st) {
+  TcDenseArgs a{};
+  a.gather = true;
+  a.user_tab = m.user_mlp;
+  a.users = users;
+  a.num_users = m.num_users;
+  a.num_items = m.num_items;
+  a.d_u = m.L[0] / 2;
+  a.user_div = 1;
+  a.user_mul = user_mul;
+  a.b_packed = t.pack_fu;
+  a.N = m.L[1];
+  a.K = m.L[0] / 2;
+  a.rows = rows;
+  a.row0 = row0;
+  a.epilogue = TC_EPI_BIAS_RELU;
+  a.bias = m.b[1];
+  a.linear = true;
+  a.out = t.Zu;
+  return launch_tc_dense(a, st);
+}
+
 static int tc_grouped_first_layer(const MrModel& m, const TcWs& t, const int32_t* users, const int32_t* items, int64_t r0,
                                   int64_t r1, int group, bool users_per_group, cudaStream_t st) {
   const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
@@ -350,25 +374,8 @@ static int tc_grouped_first_layer(const MrModel& m, const TcWs& t, const int32_t
     if (rc == MR_OK) prof_mark(MR_PHASE_TC_DENSE_FWD, st);
     return rc;
   }
-  TcDenseArgs a{};
-  a.gather = true;
-  a.user_tab = m.user_mlp;
-  a.users = users;
-  a.num_users = m.num_users;
-  a.num_items = m.num_items;
-  a.d_u = d_u;
-  a.user_div = 1;
-  a.user_mul = users_per_group ? 1 : group;  // `users` holds one id per group, or one per row
-  a.b_packed = t.pack_fu;
-  a.N = m.L[1];
-  a.K = d_u;
-  a.rows = (r1 - r0) / group;
-  a.row0 = r0 / group;
-  a.epilogue = TC_EPI_BIAS_RELU;
-  a.bias = m.b[1];
-  a.linear = true;
-  a.out = t.Zu;
-  int rc = launch_tc_dense(a, st);
+  // `users` holds one id per group, or one per row
+  int rc = tc_user_half(m, t, users, users_per_group ? 1 : group, r0 / group, (r1 - r0) / group, st);
   if (rc != MR_OK || (!train && t.Pi != nullptr)) return rc;
   if (t.Pi != nullptr) {
     prof_mark(MR_PHASE_H1_GATHER, st);
@@ -398,18 +405,22 @@ static int tc_grouped_first_layer(const MrModel& m, const TcWs& t, const int32_t
   return launch_tc_dense(b, st);
 }
 
-// Forward of rows [r0, r1) on the tensor cores; leaves H[1..n-1] of the sub-batch in the workspace.
+// Forward of rows [r0, r1) on the tensor cores; leaves H[1..n-1] of the sub-batch in the workspace.  group > 0: a
+// grouped batch, whose first layer tc_grouped_first_layer runs.  proj_ids (candidate lists): t.Zu already holds
+// proj_u_rows user halves and row r reads Zu[proj_ids[r]].  head_dot: H[n-1] holds one float per row, the last
+// layer's output dotted with w_out[MLP columns].
 static int tc_forward_rows(const MrModel& m, const TcWs& t, const int32_t* users, const int32_t* items, int user_div,
                            int64_t r0, int64_t r1, cudaStream_t st, int group = 0, bool users_per_group = false,
-                           bool head_dot = false) {
+                           bool head_dot = false, const int32_t* proj_ids = nullptr, int32_t proj_u_rows = 0) {
   const int d_u = m.L[0] / 2;
-  // the eval case of the grouped first layer whose H1 the second layer's producers compute
-  const bool proj_in_producer = group > 0 && t.bits[1] == nullptr && t.Pi != nullptr;
+  const bool split_first = group > 0 || proj_ids != nullptr;  // the first layer's user half is Zu
+  // the eval case of the split first layer, whose H1 the second layer's producers compute
+  const bool proj_in_producer = split_first && t.bits[1] == nullptr && t.Pi != nullptr;
   if (group > 0) {
     const int rc = tc_grouped_first_layer(m, t, users, items, r0, r1, group, users_per_group, st);
     if (rc != MR_OK) return rc;
   }
-  for (int l = group > 0 ? 2 : 1; l < m.n_layers; ++l) {
+  for (int l = split_first ? 2 : 1; l < m.n_layers; ++l) {
     TcDenseArgs a{};
     a.gather = (l == 1);
     a.a_dense = (l == 1) ? nullptr : t.H[l - 1];
@@ -435,8 +446,10 @@ static int tc_forward_rows(const MrModel& m, const TcWs& t, const int32_t* users
       a.proj_i = t.Pi;
       a.proj_u = t.Zu;
       a.proj_div = group;
+      a.proj_ids = proj_ids;
+      a.proj_u_rows = proj_u_rows;
     }
-    if (head_dot && l == m.n_layers - 1) {  // H[l] then holds one float per row: relu(.) . w_out[MLP columns]
+    if (head_dot && l == m.n_layers - 1) {
       a.epilogue = TC_EPI_HEAD_DOT;
       a.head_w = m.w_out + m.mf_dim;
     }
@@ -447,18 +460,18 @@ static int tc_forward_rows(const MrModel& m, const TcWs& t, const int32_t* users
 }
 
 // Pi = E_item . W1[item rows] over the whole item table (pack_fi must hold the packed item rows of W[1]).
-static int tc_project_items(const MrModel& m, const TcWs& t, cudaStream_t st) {
+static int tc_project_items(const MrModel& m, const float* pack_fi, float* Pi, cudaStream_t st) {
   const int d_u = m.L[0] / 2;
   TcDenseArgs a{};
   a.a_dense = m.item_mlp;
-  a.b_packed = t.pack_fi;
+  a.b_packed = pack_fi;
   a.N = m.L[1];
   a.K = m.L[0] - d_u;
   a.rows = m.num_items;
   a.row0 = 0;
   a.epilogue = TC_EPI_BIAS_RELU;
   a.linear = true;
-  a.out = t.Pi;
+  a.out = Pi;
   return launch_tc_dense(a, st);
 }
 
@@ -980,7 +993,7 @@ int TrainStep::tower_tc() const {
   }
   if (p.proj) {
     prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = tc_project_items(m, tw, st);
+    rc = tc_project_items(m, tw.pack_fi, tw.Pi, st);
     if (rc == MR_OK && p.uproj) rc = tc_project_users(m, tw, st);
     if (rc != MR_OK) return rc;
   }
@@ -1188,9 +1201,9 @@ int TrainStep::epilogue() const {
   return rc;
 }
 
-// ---- fused ranking evaluation on the tensor-core path -----------------------------------------------------
-// Rows per launch: whole groups and whole 128-row tiles, at most 2^22 rows (the ML-20M sweep of 13.8 M rows: 14
-// launches of 2^20 rows 4.60 ms, 7 of 2^21 4.41 ms, 4 of 2^22 4.33 ms).
+// ---- evaluation: one plan per scoring call ---------------------------------------------------------------
+// Rows per launch of mr_rank_eval's tensor-core tower: whole groups and whole 128-row tiles, at most 2^22 rows (the
+// ML-20M sweep of 13.8 M rows: 14 launches of 2^20 rows 4.60 ms, 7 of 2^21 4.41 ms, 4 of 2^22 4.33 ms).
 static int64_t eval_sub_batch(int group) {
   int64_t a = 128, b = group;
   while (b) { const int64_t t = a % b; a = b; b = t; }
@@ -1201,85 +1214,12 @@ static int64_t eval_sub_batch(int group) {
 
 static bool eval_fused_ok(const MrModel& m, int group) {
   return use_tc(m) && (head_rank_supported(m) || (m.n_layers >= 3 && head_rank_takes_dot(m, group))) && m.n_layers >= 2 &&
-         group <= 256 && eval_sub_batch(group) > 0;
+         group >= 2 && group <= 256 && eval_sub_batch(group) > 0;
 }
 
-// sb_rows > 0: rows per launch chosen by the caller (the catalogue sweep: whole users, no alignment rule)
-static TcWs carve_eval(const MrModel& m, int group, int64_t rows, void* ws, int64_t sb_rows = 0) {
-  TcWs t{};
-  Carver cv(ws);
-  int64_t sb = sb_rows > 0 ? sb_rows : eval_sub_batch(group);
-  if (sb_rows <= 0 && rows < sb) sb = (rows + 127) / 128 * 128;
-  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
-  t.pack_fu = cv.take<float>((size_t)2 * d_u * m.L[1]);
-  t.pack_fi = cv.take<float>((size_t)2 * d_i * m.L[1]);
-  t.Zu = cv.take<float>((size_t)(sb / group + 1) * m.L[1]);
-  if (item_proj_ok(m, rows)) t.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
-  for (int l = 1; l < m.n_layers; ++l) {
-    if (l >= 2) t.pack_f[l] = cv.take<float>((size_t)2 * m.L[l - 1] * m.L[l]);
-    t.H[l] = cv.take<float>((size_t)sb * m.L[l]);
-  }
-  t.total = cv.off;
-  return t;
-}
-
-// Once per eval call: the first layer's two halves and the later layers packed as MMA operands, and Pi when the
-// item projection is on.
-static int eval_prepare(const MrModel& m, const TcWs& t, cudaStream_t st) {
-  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
-  int rc = launch_pack_weights(m.W[1], d_u, m.L[1], 0, t.pack_fu, st);
-  if (rc == MR_OK) rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], d_i, m.L[1], 0, t.pack_fi, st);
-  for (int l = 2; rc == MR_OK && l < m.n_layers; ++l) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, t.pack_f[l], st);
-  if (rc != MR_OK) return rc;
-  if (t.Pi != nullptr) {
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = tc_project_items(m, t, st);
-  }
-  return rc;
-}
-
-// users: one id per group; items: G * group, the positive last.  Forward with the user half of the first layer
-// once per user, then the fused score + position kernel.
-static int rank_eval_fused(const MrModel& m, const int32_t* users, const int32_t* items, int64_t G, int group, int k,
-                           int32_t* pos, float* probs, float* sums, int32_t* flags, float* partials, void* tc_ws,
-                           cudaStream_t st) {
-  const int64_t rows = G * group;
-  TcWs t = carve_eval(m, group, rows, tc_ws);
-  prof_mark(MR_PHASE_MISC, st);
-  MR_CUDA(cudaMemsetAsync(flags, 0, 256, st));
-  int rc = eval_prepare(m, t, st);
-  if (rc != MR_OK) return rc;
-  const int64_t sb = eval_sub_batch(group);
-  for (int64_t r0 = 0; r0 < rows; r0 += sb) {
-    const int64_t r1 = r0 + sb < rows ? r0 + sb : rows;
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    // the last hidden layer's epilogue dots its output with the output unit's weights when the score kernel has
-    // the matching variant (a plain layer must precede it: l >= 2 of the grouped sequence)
-    const bool head_dot = m.n_layers >= 3 && head_rank_takes_dot(m, group);
-    rc = tc_forward_rows(m, t, users, items, 1, r0, r1, st, group, true, head_dot);
-    if (rc != MR_OK) return rc;
-    prof_mark(MR_PHASE_HEAD, st);
-    HeadArgs h{};
-    h.model = &m;
-    h.h_is_dot = head_dot;
-    h.h_last = t.H[m.n_layers - 1];
-    h.users = users;
-    h.items = items;
-    h.rows = r1 - r0;
-    h.row0 = r0;
-    h.flags = flags;
-    rc = launch_head_rank(h, group, pos, probs, st);
-    if (rc != MR_OK) return rc;
-  }
-  prof_mark(MR_PHASE_RANK, st);
-  rc = launch_rank_metrics(pos, G, k, sums, partials, st);
-  prof_mark(-1, st);
-  return rc;
-}
-
-// ---- catalogue top-k: every user against every item, in chunks of whole users --------------------------------
-// Users per chunk: about kEvalSubBatchCap rows (the ranking eval's launch size), at least one user, and at most
-// kCatalogueMaxChunkUsers so that the selection's per-slice lists stay bounded when the catalogue is tiny.
+// Catalogue calls score in chunks of whole users: about kEvalSubBatchCap rows (the ranking eval's launch size), at
+// least one user, and at most kCatalogueMaxChunkUsers so that the selection's per-slice lists stay bounded when the
+// catalogue is tiny.
 constexpr int64_t kCatalogueMaxChunkUsers = 16384;
 
 static int64_t catalogue_chunk_users(int32_t N) {
@@ -1288,30 +1228,136 @@ static int64_t catalogue_chunk_users(int32_t N) {
   return c < 1 ? 1 : c;
 }
 
-// The scoring sequence of a chunk, the one mr_rank_eval takes for the model with each user as one group of width
-// num_items: the tensor-core tower with the projected first layer in the second layer's producers and the partial-
-// logit head (>= 3 layers), the default tower's projected tables, or the plain forward.  Decided on the full chunk
-// size so that the choice does not depend on how many users a call has.
-enum { CAT_TC = 0, CAT_SMALL = 1, CAT_FORWARD = 2 };
-static int catalogue_path(const MrModel& m) {
-  const int64_t rows = catalogue_chunk_users(m.num_items) * m.num_items;
-  if (use_tc(m) && m.n_layers >= 3 && catalogue_head_supported(m)) return CAT_TC;
-  if (small_eval_ok(m, rows)) return CAT_SMALL;
-  return CAT_FORWARD;
-}
+// The tower an eval call scores with: the tensor-core tower with the first layer split into its user half Zu and its
+// item half (Pi, or the gathered item rows), the default tower's projected tables on CUDA cores (small_tower.cu), or
+// the plain forward (mr_neumf_forward).
+enum { EVAL_TC = 0, EVAL_SMALL = 1, EVAL_FORWARD = 2 };
+// The shape of the call: G groups of `group` rows with one user each (mr_rank_eval), chunks of C users against the
+// whole catalogue (catalogue calls, group = num_items), or U ragged lists of nnz rows in all (mr_rank_lists).
+enum { SCORE_GROUPS = 0, SCORE_CATALOGUE = 1, SCORE_LISTS = 2 };
+struct EvalPlan {
+  int tower;           // EVAL_*
+  bool proj;           // Pi = E_item . W1[item rows] over the item table (always on EVAL_SMALL)
+  bool head_dot;       // EVAL_TC: the last hidden layer ends in its dot with w_out[MLP columns] (one float per row) and
+                       // the head adds the GMF term; else the head reads the last layer whole
+  bool call_users;     // the user half once per call over the call's users (SCORE_LISTS: Zu, or Pu of the gathered
+                       // rows); else Zu per launch, one row per group, or Pu over the user table
+  int64_t user_rows;   // rows of Zu (EVAL_TC) or Pu (EVAL_SMALL)
+  int64_t sb;          // rows per scoring launch (EVAL_TC; SCORE_LISTS); EVAL_FORWARD: rows per forward call
+};
 
-static size_t catalogue_scoring_bytes(const MrModel& m, int64_t C) {
-  const int64_t rows = C * m.num_items;
-  switch (catalogue_path(m)) {
-    case CAT_TC: return carve_eval(m, m.num_items, catalogue_chunk_users(m.num_items) * m.num_items, nullptr, rows).total;
-    case CAT_SMALL:
-      return align_up((size_t)m.num_items * m.L[1] * sizeof(float), 256) +
-             align_up((size_t)m.num_users * m.L[1] * sizeof(float), 256);
-    default: return mr_forward_workspace_bytes(&m, rows);
+// Every launch-sequence choice of an eval call, made once.  users / group / rows: G, group, G * group (SCORE_GROUPS);
+// C, num_items, C * num_items (SCORE_CATALOGUE); U, -, nnz (SCORE_LISTS).  fused_head: mr_rank_eval's tensor-core
+// tower ends in the fused score + position head, which writes no ranks.  AUTO's row-count rules judge the call's rows,
+// the catalogue's full chunk (so that the choice does not depend on how many users a call has), or for lists nothing:
+// their sequence is a function of the model alone, so that a list's outputs do not depend on the other lists.
+static EvalPlan eval_plan(const MrModel& m, int shape, int64_t users, int group, int64_t rows, bool fused_head = true) {
+  const bool lists = shape == SCORE_LISTS;
+  const int64_t auto_rows = shape == SCORE_CATALOGUE ? catalogue_chunk_users(m.num_items) * m.num_items : rows;
+  EvalPlan p{};
+  p.call_users = lists;
+  const bool tc = shape == SCORE_GROUPS
+                      ? fused_head && eval_fused_ok(m, group)
+                      : m.n_layers >= 3 && catalogue_head_supported(m) && (lists ? item_proj_ok(m, 0, true) : use_tc(m));
+  if (tc) {
+    p.tower = EVAL_TC;
+    // the catalogue's tower without Pi runs the unprojected grouped first layer
+    p.proj = item_proj_ok(m, auto_rows, lists);
+    p.head_dot = shape != SCORE_GROUPS || (m.n_layers >= 3 && head_rank_takes_dot(m, group));
+  } else {
+    p.tower = small_eval_ok(m, auto_rows, lists) ? EVAL_SMALL : EVAL_FORWARD;
+    p.proj = p.tower == EVAL_SMALL;
   }
+  const int64_t tiles = (rows + 127) / 128 * 128;
+  if (lists) {  // the call's rows in whole tiles, up to the ranking eval's 2^22 -- or the forward's own 2^21
+    const int64_t cap = p.tower == EVAL_FORWARD ? kTcSubBatchCap : kEvalSubBatchCap;
+    p.sb = tiles < 128 ? 128 : (tiles < cap ? tiles : cap);
+  } else if (shape == SCORE_GROUPS && tc) {
+    p.sb = eval_sub_batch(group) < tiles ? eval_sub_batch(group) : tiles;
+  } else {
+    p.sb = rows;
+  }
+  if (lists) p.user_rows = users < 1 ? 1 : users;
+  else p.user_rows = tc ? p.sb / group + 1 : m.num_users;
+  return p;
 }
 
+struct EvalWs {
+  TcWs t;            // EVAL_TC: the packed weights, Zu and H; Pi (proj); EVAL_SMALL: Pu
+  float* Eu;         // EVAL_SMALL with call_users: the call's users' MLP rows
+  void* fwd;         // EVAL_FORWARD: mr_neumf_forward's workspace
+  size_t fwd_bytes;
+  size_t total;
+};
+
+// The scoring workspace of a plan; the workspace queries take its size from here (ws = NULL).  H[1] exists only when
+// the first layer writes it (with Pi the second layer's producers compute it), and H[n-1] holds one float per row when
+// the plan ends in head_dot.
+static EvalWs eval_carve(const MrModel& m, const EvalPlan& p, void* ws) {
+  EvalWs w{};
+  Carver cv(ws);
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
+  if (p.tower == EVAL_TC) {
+    w.t.pack_fu = cv.take<float>((size_t)2 * d_u * L1);
+    w.t.pack_fi = cv.take<float>((size_t)2 * d_i * L1);
+    for (int l = 2; l < m.n_layers; ++l) w.t.pack_f[l] = cv.take<float>((size_t)2 * m.L[l - 1] * m.L[l]);
+    w.t.Zu = cv.take<float>((size_t)p.user_rows * L1);
+    for (int l = p.proj ? 2 : 1; l < m.n_layers; ++l)
+      w.t.H[l] = cv.take<float>((size_t)p.sb * (p.head_dot && l == m.n_layers - 1 ? 1 : m.L[l]));
+  }
+  if (p.proj) w.t.Pi = cv.take<float>((size_t)m.num_items * L1);
+  if (p.tower == EVAL_SMALL) {
+    if (p.call_users) w.Eu = cv.take<float>((size_t)p.user_rows * d_u);
+    w.t.Pu = cv.take<float>((size_t)p.user_rows * L1);
+  }
+  if (p.tower == EVAL_FORWARD) {
+    w.fwd_bytes = mr_forward_workspace_bytes(&m, p.sb);
+    w.fwd = cv.take<char>(w.fwd_bytes);
+  }
+  w.total = cv.off;
+  return w;
+}
+
+// Once per call, what the plan's tower reads besides the tables: the packed weights (EVAL_TC), Pi, then the user half
+// that is not per launch -- Pu over the user table or over the call's users (EVAL_SMALL), Zu of the call's users
+// (EVAL_TC with call_users).  users: the call's users, p.user_rows of them when p.call_users.
+static int eval_prepare(const MrModel& m, const EvalPlan& p, const EvalWs& w, const int32_t* users, cudaStream_t st) {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
+  const bool tc = p.tower == EVAL_TC;
+  int rc = MR_OK;
+  if (tc) {
+    rc = launch_pack_weights(m.W[1], d_u, L1, 0, w.t.pack_fu, st);
+    if (rc == MR_OK) rc = launch_pack_weights(m.W[1] + (size_t)d_u * L1, d_i, L1, 0, w.t.pack_fi, st);
+    for (int l = 2; rc == MR_OK && l < m.n_layers; ++l) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, w.t.pack_f[l], st);
+  }
+  if (rc == MR_OK && p.proj) {
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    rc = tc ? tc_project_items(m, w.t.pack_fi, w.t.Pi, st)
+            : launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr,
+                                     w.t.Pi, st);
+  }
+  if (rc != MR_OK) return rc;
+  if (tc && p.call_users) return tc_user_half(m, w.t, users, 1, 0, p.user_rows, st);
+  if (p.tower != EVAL_SMALL) return MR_OK;
+  if (!p.call_users) return launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, m.W[1], L1, L1, false, m.b[1], w.t.Pu, st);
+  rc = launch_gather_rows(m.user_mlp, m.num_users, d_u, users, p.user_rows, w.Eu, st);  // NaN rows: bad users
+  if (rc == MR_OK) rc = launch_small_rows_gemm(w.Eu, p.user_rows, d_u, m.W[1], L1, L1, false, m.b[1], w.t.Pu, st);
+  return rc;
+}
+
+// ---- catalogue calls: every user against every item, in chunks of whole users --------------------------------
 static int64_t clamp_users(int64_t U, int64_t C) { return U < 1 ? 1 : (U < C ? U : C); }
+
+static EvalPlan catalogue_plan(const MrModel& m, int64_t C) {
+  return eval_plan(m, SCORE_CATALOGUE, C, m.num_items, C * m.num_items);
+}
+
+// The sweep's workspace (chunks of C users): the item of every row of a chunk, the chunk's probabilities, the scoring.
+static size_t catalogue_sweep_bytes(const MrModel& m, int64_t C) {
+  const size_t rows = (size_t)C * m.num_items;
+  return align_up(rows * sizeof(int32_t), 256) + align_up(rows * sizeof(float), 256) +
+         eval_carve(m, catalogue_plan(m, C), nullptr).total;
+}
 
 static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const int64_t* excl_rowptr,
                       const int32_t* excl_items, const int32_t* targets, const int32_t* pos, const float* sums) {
@@ -1323,52 +1369,39 @@ static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const 
 }
 
 // The chunk loop of the catalogue calls: per chunk of C users, the probabilities of every (user, item) pair through the
-// model's catalogue_path sequence, then select(u0, users in the chunk, probabilities) under MR_PHASE_RANK.  The
-// probabilities go to scores + u0 * N when scores is given, else to probs_buf (C x N).  mr_catalogue_topk and
-// mr_catalogue_targets both score through here, so a pair's probability is the same in both by construction.
+// plan's tower, then select(u0, users in the chunk, probabilities) under MR_PHASE_RANK.  The probabilities go to
+// scores + u0 * N when scores is given, else to the sweep's buffer (C x N).  ws: catalogue_sweep_bytes(m, C) bytes.
+// mr_catalogue_topk and mr_catalogue_targets both score through here, so a pair's probability is the same in both by
+// construction.
 template <class Select>
-static int catalogue_sweep(const MrModel& m, const int32_t* users, int64_t U, int64_t C, int32_t* iota, float* probs_buf,
-                           float* scores, void* score_ws, cudaStream_t st, Select select) {
+static int catalogue_sweep(const MrModel& m, const int32_t* users, int64_t U, int64_t C, float* scores, void* ws,
+                           cudaStream_t st, Select select) {
   const int32_t N = m.num_items;
-  const int64_t Cmax = catalogue_chunk_users(N);
-  const int path = catalogue_path(m);
-  TcWs t{};
-  float *Pi = nullptr, *Pu = nullptr;
-  size_t fwd_bytes = 0;
+  const EvalPlan p = catalogue_plan(m, C);
+  Carver cv(ws);
+  int32_t* iota = cv.take<int32_t>((size_t)C * N);
+  float* probs_buf = cv.take<float>((size_t)C * N);
+  const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
   prof_mark(MR_PHASE_MISC, st);
   int rc = launch_tile_iota(iota, C * N, N, st);
-  if (rc != MR_OK) return rc;
-  if (path == CAT_TC) {
-    t = carve_eval(m, N, Cmax * N, score_ws, C * N);
-    rc = eval_prepare(m, t, st);
-  } else if (path == CAT_SMALL) {  // Pi, Pu over the tables, as mr_rank_eval's default-tower path
-    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
-    Carver cs(score_ws);
-    Pi = cs.take<float>((size_t)m.num_items * L1);
-    Pu = cs.take<float>((size_t)m.num_users * L1);
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, Pi, st);
-    if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, m.W[1], L1, L1, false, m.b[1], Pu, st);
-  } else {
-    fwd_bytes = mr_forward_workspace_bytes(&m, C * N);
-  }
+  if (rc == MR_OK) rc = eval_prepare(m, p, w, users, st);
   for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
     const int64_t c = U - u0 < C ? U - u0 : C;
     const int64_t rows = c * N;
     float* out = scores != nullptr ? scores + u0 * N : probs_buf;
-    if (path == CAT_TC) {
+    if (p.tower == EVAL_TC) {
       // each chunk starts at row 0 of its own users: one group = one user, Zu once per user
       prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-      rc = tc_forward_rows(m, t, users + u0, iota, 1, 0, rows, st, N, true, true);
+      rc = tc_forward_rows(m, w.t, users + u0, iota, 1, 0, rows, st, N, true, p.head_dot);
       if (rc == MR_OK) {
         prof_mark(MR_PHASE_HEAD, st);
-        rc = launch_catalogue_head(m, t.H[m.n_layers - 1], users + u0, rows, N, out, st);
+        rc = launch_catalogue_head(m, w.t.H[m.n_layers - 1], users + u0, rows, N, out, st);
       }
-    } else if (path == CAT_SMALL) {
+    } else if (p.tower == EVAL_SMALL) {
       prof_mark(MR_PHASE_FUSED_TILE, st);
-      rc = launch_small_tower_forward(m, Pi, Pu, users + u0, iota, rows, N, out, st);
+      rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, users + u0, iota, rows, N, out, st);
     } else {
-      rc = mr_neumf_forward(&m, users + u0, iota, rows, N, nullptr, out, nullptr, nullptr, score_ws, fwd_bytes, st);
+      rc = mr_neumf_forward(&m, users + u0, iota, rows, N, nullptr, out, nullptr, nullptr, w.fwd, w.fwd_bytes, st);
     }
     if (rc != MR_OK) break;
     prof_mark(MR_PHASE_RANK, st);
@@ -1396,75 +1429,6 @@ static int targets_check(int64_t U, int32_t N, int32_t excl_rows, const int64_t*
 }
 
 // ---- ragged candidate lists: list u pairs users[u] with items[rowptr[u] .. rowptr[u+1]) ------------------------------
-// The scoring sequence is a function of the model alone -- never of U or nnz -- so that a list's outputs do not depend on
-// the other lists of the call (what a serving batcher needs):
-//  LISTS_TC: the tensor-core tower with the projected first layer (eligible models, projection not OFF): Pi once per
-//            call, Zu once per list, the second layer's producers read relu(Pi[item] + Zu[seg[row]]), the last layer
-//            dots with the output weights, and the partial-logit head adds the GMF term;
-//  LISTS_SMALL: the default tower: Pi over the item table, Pu over the call's users, the thread-per-row forward;
-//  LISTS_FORWARD: per-row user ids and the plain forward.
-enum { LISTS_TC = 0, LISTS_SMALL = 1, LISTS_FORWARD = 2 };
-constexpr int64_t kAnyRows = INT64_MAX / 4;  // "eligible at any row count" for the row-count rules of AUTO
-static int lists_path(const MrModel& m) {
-  if (m.n_layers >= 3 && catalogue_head_supported(m) && item_proj_ok(m, kAnyRows)) return LISTS_TC;
-  if (small_eval_ok(m, kAnyRows)) return LISTS_SMALL;
-  return LISTS_FORWARD;
-}
-
-// Rows per scoring launch: the call's rows in whole 128-row tiles, up to the ranking eval's 2^22 -- or the forward's
-// own 2^21 on the plain-forward path, whose workspace then grows with the rows up to that cap and stays there.
-static int64_t lists_sub_batch(const MrModel& m, int64_t nnz) {
-  const int64_t cap = lists_path(m) == LISTS_FORWARD ? kTcSubBatchCap : kEvalSubBatchCap;
-  const int64_t r = (nnz + 127) / 128 * 128;
-  return r < 128 ? 128 : (r < cap ? r : cap);
-}
-
-struct ListsTcWs {
-  float *pack_fu, *pack_fi, *Pi, *Zu;
-  float* pack_f[MR_MAX_LAYERS];
-  float* H[MR_MAX_LAYERS];  // H[2 .. n-2]: sb x L[l]; H[n-1]: sb floats (the partial logits)
-  size_t total;
-};
-static ListsTcWs carve_lists_tc(const MrModel& m, int64_t U, int64_t sb, void* ws) {
-  ListsTcWs t{};
-  Carver cv(ws);
-  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
-  t.pack_fu = cv.take<float>((size_t)2 * d_u * m.L[1]);
-  t.pack_fi = cv.take<float>((size_t)2 * d_i * m.L[1]);
-  t.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
-  t.Zu = cv.take<float>((size_t)(U < 1 ? 1 : U) * m.L[1]);
-  for (int l = 2; l < m.n_layers; ++l) {
-    t.pack_f[l] = cv.take<float>((size_t)2 * m.L[l - 1] * m.L[l]);
-    t.H[l] = cv.take<float>((size_t)sb * (l == m.n_layers - 1 ? 1 : m.L[l]));
-  }
-  t.total = cv.off;
-  return t;
-}
-
-struct ListsSmallWs {
-  float *Pi, *Eu, *Pu;
-  size_t total;
-};
-static ListsSmallWs carve_lists_small(const MrModel& m, int64_t U, void* ws) {
-  ListsSmallWs w{};
-  Carver cv(ws);
-  const size_t Ul = (size_t)(U < 1 ? 1 : U);
-  w.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
-  w.Eu = cv.take<float>(Ul * (m.L[0] / 2));
-  w.Pu = cv.take<float>(Ul * m.L[1]);
-  w.total = cv.off;
-  return w;
-}
-
-static size_t lists_scoring_bytes(const MrModel& m, int64_t U, int64_t nnz) {
-  const int64_t sb = lists_sub_batch(m, nnz);
-  switch (lists_path(m)) {
-    case LISTS_TC: return carve_lists_tc(m, U, sb, nullptr).total;
-    case LISTS_SMALL: return carve_lists_small(m, U, nullptr).total;
-    default: return mr_forward_workspace_bytes(&m, sb);
-  }
-}
-
 static int lists_check(int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
                        const int32_t* pos, const float* sums) {
   MR_REQUIRE(U >= 0 && U <= INT32_MAX && nnz >= 0 && nnz <= INT32_MAX, "lists: bad U=%lld nnz=%lld", (long long)U,
@@ -1670,18 +1634,18 @@ int mr_neumf_train_step(MrModel* model, MrOptState* opt, MrGrads* grads, const i
   return mr_neumf_apply(model, opt, grads, stream);
 }
 
+// [flags 256 B][partials][probabilities, unless the fused head writes them][scoring]: the larger of the plans with and
+// without ranks
 size_t mr_rank_eval_workspace_bytes(const MrModel* model, int64_t G, int32_t group) {
-  if (G < 0 || group < 1) return 0;
-  size_t fused = 0;
-  if (model != nullptr && model->n_layers >= 1 && model->n_layers <= MR_MAX_LAYERS && tc_eligible(*model) && group >= 2 &&
-      eval_sub_batch(group) > 0 && model->n_layers >= 2)
-    fused = carve_eval(*model, group, G * group, nullptr).total + 512;
-  size_t plain = mr_forward_workspace_bytes(model, G * group) + align_up((size_t)G * group * sizeof(float), 256);
-  if (model != nullptr && model->n_layers >= 1 && model->n_layers <= MR_MAX_LAYERS && !tc_eligible(*model) &&
-      small_tower_supported(*model, 5))  // Pi, Pu of the default-tower eval
-    plain += align_up((size_t)model->num_items * model->L[1] * sizeof(float), 256) +
-             align_up((size_t)model->num_users * model->L[1] * sizeof(float), 256);
-  return (plain > fused ? plain : fused) + align_up(rank_partials_count(G) * sizeof(float), 256) + 512;
+  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || G < 0 || group < 1) return 0;
+  size_t scoring = 0;
+  for (const bool ranks : {false, true}) {
+    const EvalPlan p = eval_plan(*model, SCORE_GROUPS, G, group, G * group, !ranks);
+    const size_t probs = p.tower == EVAL_TC ? 0 : align_up((size_t)G * group * sizeof(float), 256);
+    const size_t n = probs + eval_carve(*model, p, nullptr).total;
+    if (n > scoring) scoring = n;
+  }
+  return 256 + align_up(rank_partials_count(G) * sizeof(float), 256) + scoring;
 }
 
 int mr_rank_eval(const MrModel* model, const int32_t* users, const int32_t* items, int64_t G, int32_t group, int32_t k,
@@ -1701,38 +1665,54 @@ int mr_rank_eval(const MrModel* model, const int32_t* users, const int32_t* item
     if (rc0 != MR_OK) return rc0;
   }
   MR_REQUIRE(users && items, "rank_eval: NULL ids");
-  if (rank == nullptr && eval_fused_ok(*model, group)) {
-    // fused path: [flags 256 B][partials][tensor-core workspace]
-    Carver cvf(ws);
-    int32_t* flags = cvf.take<int32_t>(64);
-    float* partials_f = cvf.take<float>(rank_partials_count(G));
-    return rank_eval_fused(*model, users, items, G, group, k, pos, probs, sums, flags, partials_f,
-                           static_cast<char*>(ws) + cvf.off, (cudaStream_t)stream);
-  }
-  const size_t fwd_bytes = mr_forward_workspace_bytes(model, G * group);
-  Carver cv(static_cast<char*>(ws) + fwd_bytes);
-  float* probs_buf = cv.take<float>((size_t)G * group);
+  const MrModel& m = *model;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t rows = G * group;
+  const EvalPlan p = eval_plan(m, SCORE_GROUPS, G, group, rows, rank == nullptr);
+  Carver cv(ws);
+  int32_t* flags = cv.take<int32_t>(64);
   float* partials = cv.take<float>(rank_partials_count(G));
-  float* pr = probs != nullptr ? probs : probs_buf;
+  float* probs_buf = p.tower == EVAL_TC ? nullptr : cv.take<float>((size_t)rows);
+  const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
   int rc;
-  if (small_eval_ok(*model, G * group)) {  // default tower: projected tables, thread-per-row forward (small_tower.cu)
-    const MrModel& m = *model;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
-    float* Pi = cv.take<float>((size_t)m.num_items * L1);
-    float* Pu = cv.take<float>((size_t)m.num_users * L1);
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, Pi, st);
-    if (rc == MR_OK) rc = launch_small_rows_gemm(m.user_mlp, m.num_users, d_u, m.W[1], L1, L1, false, m.b[1], Pu, st);
-    prof_mark(MR_PHASE_FUSED_TILE, st);
-    if (rc == MR_OK) rc = launch_small_tower_forward(m, Pi, Pu, users, items, G * group, group, pr, st);
+  if (p.tower == EVAL_TC) {  // forward with the user half of the first layer once per group, then the fused head
+    prof_mark(MR_PHASE_MISC, st);
+    MR_CUDA(cudaMemsetAsync(flags, 0, 256, st));
+    rc = eval_prepare(m, p, w, users, st);
+    for (int64_t r0 = 0; r0 < rows && rc == MR_OK; r0 += p.sb) {
+      const int64_t r1 = r0 + p.sb < rows ? r0 + p.sb : rows;
+      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+      rc = tc_forward_rows(m, w.t, users, items, 1, r0, r1, st, group, true, p.head_dot);
+      if (rc != MR_OK) break;
+      prof_mark(MR_PHASE_HEAD, st);
+      HeadArgs h{};
+      h.model = &m;
+      h.h_is_dot = p.head_dot;
+      h.h_last = w.t.H[m.n_layers - 1];
+      h.users = users;
+      h.items = items;
+      h.rows = r1 - r0;
+      h.row0 = r0;
+      h.flags = flags;
+      rc = launch_head_rank(h, group, pos, probs, st);
+    }
+    if (rc != MR_OK) return rc;
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_rank_metrics(pos, G, k, sums, partials, st);
   } else {
-    rc = mr_neumf_forward(model, users, items, G * group, group, nullptr, pr, nullptr, nullptr, ws, fwd_bytes, stream);
+    float* pr = probs != nullptr ? probs : probs_buf;
+    if (p.tower == EVAL_SMALL) {  // thread-per-row forward on the projected tables (small_tower.cu)
+      rc = eval_prepare(m, p, w, users, st);
+      prof_mark(MR_PHASE_FUSED_TILE, st);
+      if (rc == MR_OK) rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, users, items, rows, group, pr, st);
+    } else {
+      rc = mr_neumf_forward(model, users, items, rows, group, nullptr, pr, nullptr, nullptr, w.fwd, w.fwd_bytes, stream);
+    }
+    if (rc != MR_OK) return rc;
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_rank_scores(pr, G, group, k, nullptr, rank, pos, sums, partials, st);
   }
-  if (rc != MR_OK) return rc;
-  prof_mark(MR_PHASE_RANK, (cudaStream_t)stream);
-  rc = launch_rank_scores(pr, G, group, k, nullptr, rank, pos, sums, partials, (cudaStream_t)stream);
-  prof_mark(-1, (cudaStream_t)stream);
+  prof_mark(-1, st);
   return rc;
 }
 
@@ -1804,9 +1784,7 @@ size_t mr_catalogue_topk_workspace_bytes(const MrModel* model, int64_t U, int32_
     return 0;
   const MrModel& m = *model;
   const int64_t C = clamp_users(U, catalogue_chunk_users(m.num_items));
-  const size_t rows = (size_t)C * m.num_items;
-  return align_up(rows * sizeof(int32_t), 256) + align_up(rows * sizeof(float), 256) +
-         align_up(topk_workspace_bytes(C, m.num_items, k), 256) + catalogue_scoring_bytes(m, C) + 512;
+  return align_up(topk_workspace_bytes(C, m.num_items, k), 256) + catalogue_sweep_bytes(m, C) + 512;
 }
 
 int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int32_t k, int32_t excl_rows,
@@ -1831,11 +1809,7 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
   }
   const int64_t C = clamp_users(U, catalogue_chunk_users(N));
   Carver cv(ws);
-  int32_t* iota = cv.take<int32_t>((size_t)C * N);
-  float* probs_buf = cv.take<float>((size_t)C * N);
-  const size_t topk_bytes = topk_workspace_bytes(C, N, k);
-  void* topk_ws = cv.take<char>(topk_bytes);
-  void* score_ws = static_cast<char*>(ws) + cv.off;
+  void* topk_ws = cv.take<char>(topk_workspace_bytes(C, N, k));
   TopkArgs a{};
   a.N = N;
   a.k = k;
@@ -1849,12 +1823,13 @@ int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int
   a.top_items = top_items;
   a.top_scores = top_scores;
   a.pos = pos;
-  rc = catalogue_sweep(m, users, U, C, iota, probs_buf, scores, score_ws, st, [&](int64_t u0, int64_t c, const float* out) {
-    a.u0 = u0;
-    a.U = c;
-    a.scores = out;
-    return launch_topk(a, topk_ws, st);
-  });
+  rc = catalogue_sweep(m, users, U, C, scores, static_cast<char*>(ws) + cv.off, st,
+                       [&](int64_t u0, int64_t c, const float* out) {
+                         a.u0 = u0;
+                         a.U = c;
+                         a.scores = out;
+                         return launch_topk(a, topk_ws, st);
+                       });
   if (rc == MR_OK) {
     prof_mark(MR_PHASE_RANK, st);
     rc = launch_topk_metrics(pos, U, k, sums, st);
@@ -1914,10 +1889,7 @@ size_t mr_catalogue_targets_workspace_bytes(const MrModel* model, int64_t U, int
   const MrModel& m = *model;
   const size_t sel = mr_targets_scores_workspace_bytes(U, m.num_items, nnz_t);
   if (sel == 0) return 0;
-  const int64_t C = clamp_users(U, catalogue_chunk_users(m.num_items));
-  const size_t rows = (size_t)C * m.num_items;
-  return align_up(rows * sizeof(int32_t), 256) + align_up(rows * sizeof(float), 256) + align_up(sel, 256) +
-         catalogue_scoring_bytes(m, C) + 512;
+  return align_up(sel, 256) + catalogue_sweep_bytes(m, clamp_users(U, catalogue_chunk_users(m.num_items))) + 512;
 }
 
 int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, int32_t excl_rows,
@@ -1945,10 +1917,7 @@ int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, 
   }
   const int64_t C = clamp_users(U, catalogue_chunk_users(N));
   Carver cv(ws);
-  int32_t* iota = cv.take<int32_t>((size_t)C * N);
-  float* probs_buf = cv.take<float>((size_t)C * N);
   const TargetsWs w = carve_targets(cv.take<char>(mr_targets_scores_workspace_bytes(U, N, nnz_t)), C, nnz_t);
-  void* score_ws = static_cast<char*>(ws) + cv.off;
   TargetsArgs a{};
   a.N = N;
   a.excl_ids = users;  // exclusion lists are indexed by user id
@@ -1961,12 +1930,13 @@ int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, 
   a.users = users;
   a.num_users = m.num_users;
   a.tpos = tpos;
-  rc = catalogue_sweep(m, users, U, C, iota, probs_buf, nullptr, score_ws, st, [&](int64_t u0, int64_t c, const float* out) {
-    a.u0 = u0;
-    a.U = c;
-    a.scores = out;
-    return launch_targets_chunk(a, w, st);
-  });
+  rc = catalogue_sweep(m, users, U, C, nullptr, static_cast<char*>(ws) + cv.off, st,
+                       [&](int64_t u0, int64_t c, const float* out) {
+                         a.u0 = u0;
+                         a.U = c;
+                         a.scores = out;
+                         return launch_targets_chunk(a, w, st);
+                       });
   if (rc == MR_OK) {
     prof_mark(MR_PHASE_RANK, st);
     rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
@@ -2014,7 +1984,7 @@ size_t mr_rank_lists_workspace_bytes(const MrModel* model, int64_t U, int64_t nn
   const size_t sel = mr_topk_lists_workspace_bytes(U, nnz, k);
   if (sel == 0) return 0;
   return sel + align_up((size_t)nnz * sizeof(int32_t), 256) + align_up((size_t)nnz * sizeof(float), 256) +
-         lists_scoring_bytes(*model, U, nnz) + 256;
+         eval_carve(*model, eval_plan(*model, SCORE_LISTS, U, 0, nnz), nullptr).total + 256;
 }
 
 int mr_rank_lists(const MrModel* model, const int32_t* users, int64_t U, const int64_t* rowptr, const int32_t* items,
@@ -2037,106 +2007,31 @@ int mr_rank_lists(const MrModel* model, const int32_t* users, int64_t U, const i
   void* sel_ws = cv.take<char>(topk_lists_workspace_bytes(U, nnz, k));
   int32_t* seg = cv.take<int32_t>((size_t)nnz);
   float* probs_buf = cv.take<float>((size_t)nnz);
-  void* score_ws = static_cast<char*>(ws) + cv.off;
   float* pr = probs != nullptr ? probs : probs_buf;
-  const int path = lists_path(m);
-  const int64_t sb = lists_sub_batch(m, nnz);
+  const EvalPlan p = eval_plan(m, SCORE_LISTS, U, 0, nnz);
+  const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
   if (nnz > 0) {
     prof_mark(MR_PHASE_MISC, st);
-    // seg: the list of each row (TC / default tower), or the user of each row (plain forward)
-    rc = launch_list_rows(rowptr, U, nnz, path == LISTS_FORWARD ? users : nullptr, seg, st);
-    if (rc != MR_OK) return rc;
-  }
-  if (nnz > 0 && path == LISTS_TC) {
-    const ListsTcWs t = carve_lists_tc(m, U, sb, score_ws);
-    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
-    rc = launch_pack_weights(m.W[1], d_u, m.L[1], 0, t.pack_fu, st);
-    if (rc == MR_OK) rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], d_i, m.L[1], 0, t.pack_fi, st);
-    for (int l = 2; rc == MR_OK && l < m.n_layers; ++l) rc = launch_pack_weights(m.W[l], m.L[l - 1], m.L[l], 0, t.pack_f[l], st);
-    if (rc != MR_OK) return rc;
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    TcWs tw{};
-    tw.pack_fi = t.pack_fi;
-    tw.Pi = t.Pi;
-    rc = tc_project_items(m, tw, st);
-    if (rc != MR_OK) return rc;
-    {  // Zu = E_user[users[u]] . W1[user rows] + b1, one row per list (zero row for an out-of-range user)
-      TcDenseArgs a{};
-      a.gather = true;
-      a.user_tab = m.user_mlp;
-      a.users = users;
-      a.num_users = m.num_users;
-      a.num_items = m.num_items;
-      a.d_u = d_u;
-      a.user_div = 1;
-      a.user_mul = 1;
-      a.b_packed = t.pack_fu;
-      a.N = m.L[1];
-      a.K = d_u;
-      a.rows = U;
-      a.row0 = 0;
-      a.epilogue = TC_EPI_BIAS_RELU;
-      a.bias = m.b[1];
-      a.linear = true;
-      a.out = t.Zu;
-      rc = launch_tc_dense(a, st);
-      if (rc != MR_OK) return rc;
-    }
-    for (int64_t r0 = 0; r0 < nnz; r0 += sb) {
-      const int64_t r1 = r0 + sb < nnz ? r0 + sb : nnz;
-      prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-      for (int l = 2; l < m.n_layers; ++l) {
-        TcDenseArgs a{};
-        a.a_dense = l == 2 ? nullptr : t.H[l - 1];
-        a.items = items;
-        a.num_users = m.num_users;
-        a.num_items = m.num_items;
-        a.b_packed = t.pack_f[l];
-        a.N = m.L[l];
-        a.K = m.L[l - 1];
-        a.rows = r1 - r0;
-        a.row0 = r0;
-        a.epilogue = TC_EPI_BIAS_RELU;
-        a.bias = m.b[l];
-        a.out = t.H[l];
-        if (l == 2) {  // the producers compute relu(Pi[items[row]] + Zu[seg[row]])
-          a.proj_i = t.Pi;
-          a.proj_u = t.Zu;
-          a.proj_ids = seg;
-          a.proj_u_rows = (int32_t)U;
-        }
-        if (l == m.n_layers - 1) {
-          a.epilogue = TC_EPI_HEAD_DOT;
-          a.head_w = m.w_out + m.mf_dim;
-        }
-        rc = launch_tc_dense(a, st);
-        if (rc != MR_OK) return rc;
+    // seg: the list of each row, or the user of each row (plain forward)
+    rc = launch_list_rows(rowptr, U, nnz, p.tower == EVAL_FORWARD ? users : nullptr, seg, st);
+    if (rc == MR_OK) rc = eval_prepare(m, p, w, users, st);
+    if (rc == MR_OK && p.tower == EVAL_SMALL) prof_mark(MR_PHASE_FUSED_TILE, st);
+    for (int64_t r0 = 0; r0 < nnz && rc == MR_OK; r0 += p.sb) {
+      const int64_t r1 = r0 + p.sb < nnz ? r0 + p.sb : nnz;
+      if (p.tower == EVAL_TC) {  // the second layer's producers compute relu(Pi[items[row]] + Zu[seg[row]])
+        prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+        rc = tc_forward_rows(m, w.t, users, items, 1, r0, r1, st, 0, false, p.head_dot, seg, (int32_t)U);
+        if (rc != MR_OK) break;
+        prof_mark(MR_PHASE_HEAD, st);
+        rc = launch_catalogue_head(m, w.t.H[m.n_layers - 1], users, r1 - r0, 1, pr, st, seg, items, r0, U);
+      } else if (p.tower == EVAL_SMALL) {
+        rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, users, items + r0, r1 - r0, 1, pr + r0, st, seg + r0, U);
+      } else {
+        rc = mr_neumf_forward(model, seg + r0, items + r0, r1 - r0, 1, nullptr, pr + r0, nullptr, nullptr, w.fwd,
+                              w.fwd_bytes, stream);
       }
-      prof_mark(MR_PHASE_HEAD, st);
-      rc = launch_lists_head(m, t.H[m.n_layers - 1], users, U, seg, items, r0, r1 - r0, pr, st);
-      if (rc != MR_OK) return rc;
-    }
-  } else if (nnz > 0 && path == LISTS_SMALL) {
-    const ListsSmallWs w = carve_lists_small(m, U, score_ws);
-    const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
-    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr, w.Pi, st);
-    if (rc == MR_OK) rc = launch_gather_rows(m.user_mlp, m.num_users, d_u, users, U, w.Eu, st);  // NaN rows: bad users
-    if (rc == MR_OK) rc = launch_small_rows_gemm(w.Eu, U, d_u, m.W[1], L1, L1, false, m.b[1], w.Pu, st);
-    prof_mark(MR_PHASE_FUSED_TILE, st);
-    for (int64_t r0 = 0; rc == MR_OK && r0 < nnz; r0 += sb) {
-      const int64_t r1 = r0 + sb < nnz ? r0 + sb : nnz;
-      rc = launch_small_tower_forward(m, w.Pi, w.Pu, users, items + r0, r1 - r0, 1, pr + r0, st, seg + r0, U);
     }
     if (rc != MR_OK) return rc;
-  } else if (nnz > 0) {
-    const size_t fwd_bytes = mr_forward_workspace_bytes(model, sb);
-    for (int64_t r0 = 0; r0 < nnz; r0 += sb) {
-      const int64_t r1 = r0 + sb < nnz ? r0 + sb : nnz;
-      rc = mr_neumf_forward(model, seg + r0, items + r0, r1 - r0, 1, nullptr, pr + r0, nullptr, nullptr, score_ws,
-                            fwd_bytes, stream);
-      if (rc != MR_OK) return rc;
-    }
   }
   TopkListsArgs a{};
   a.scores = pr;
@@ -2256,12 +2151,9 @@ int mr_fold_in_users(const MrModel* model, const int64_t* rowptr, const int32_t*
   if (rc == MR_OK) rc = launch_transpose_kernels(m, w.wt, st);
   if (rc == MR_OK && m.n_layers > 1) {
     if (fold_in_tc_pi(m)) {
-      TcWs t{};
-      t.pack_fi = w.pack_fi;
-      t.Pi = w.Pi;
       const int d_u = m.L[0] / 2;
-      rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], m.L[0] - d_u, m.L[1], 0, t.pack_fi, st);
-      if (rc == MR_OK) rc = tc_project_items(m, t, st);
+      rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], m.L[0] - d_u, m.L[1], 0, w.pack_fi, st);
+      if (rc == MR_OK) rc = tc_project_items(m, w.pack_fi, w.Pi, st);
     } else {
       rc = launch_fold_in_project(m, w.Pi, st);
     }

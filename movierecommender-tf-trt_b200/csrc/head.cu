@@ -868,7 +868,8 @@ bool head_rank_takes_dot(const MrModel& m, int group) {
 }
 
 int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t rows, int group,
-                          float* probs, cudaStream_t st) {
+                          float* probs, cudaStream_t st, const int32_t* seg, const int32_t* items, int64_t row0,
+                          int64_t num_lists) {
   if (!catalogue_head_supported(m) || group < 1) {
     set_error("catalogue head: needs mf_dim 32, 64 or 128 and 16-byte aligned GMF tables / output weights");
     return MR_ERR_INVALID;
@@ -877,32 +878,18 @@ int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* u
   const int64_t want = (rows + 4 * (kHeadThreads / 32) - 1) / (4 * (kHeadThreads / 32));
   const int64_t cap = (int64_t)sm_count() * 8;
   const unsigned grid = (unsigned)(want < cap ? want : cap);
-  if (m.mf_dim == 32)
-    catalogue_head_kernel<1, false><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, nullptr, nullptr, 0, 0);
-  else if (m.mf_dim == 64)
-    catalogue_head_kernel<2, false><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, nullptr, nullptr, 0, 0);
-  else
-    catalogue_head_kernel<4, false><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, nullptr, nullptr, 0, 0);
-  MR_LAUNCH_CHECK("catalogue_head_kernel");
-  return MR_OK;
-}
-
-int launch_lists_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t num_lists, const int32_t* seg,
-                      const int32_t* items, int64_t row0, int64_t rows, float* probs, cudaStream_t st) {
-  if (!catalogue_head_supported(m)) {
-    set_error("lists head: needs mf_dim 32, 64 or 128 and 16-byte aligned GMF tables / output weights");
-    return MR_ERR_INVALID;
-  }
-  if (rows == 0) return MR_OK;
-  const int64_t want = (rows + 4 * (kHeadThreads / 32) - 1) / (4 * (kHeadThreads / 32));
-  const int64_t cap = (int64_t)sm_count() * 8;
-  const unsigned grid = (unsigned)(want < cap ? want : cap);
-  if (m.mf_dim == 32)
-    catalogue_head_kernel<1, true><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, 1, probs, seg, items, row0, num_lists);
-  else if (m.mf_dim == 64)
-    catalogue_head_kernel<2, true><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, 1, probs, seg, items, row0, num_lists);
-  else
-    catalogue_head_kernel<4, true><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, 1, probs, seg, items, row0, num_lists);
+#define MR_CATALOGUE_HEAD(RAGGED_)                                                                                  \
+  if (m.mf_dim == 32)                                                                                              \
+    catalogue_head_kernel<1, RAGGED_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
+                                                                     row0, num_lists);                             \
+  else if (m.mf_dim == 64)                                                                                         \
+    catalogue_head_kernel<2, RAGGED_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
+                                                                     row0, num_lists);                             \
+  else                                                                                                             \
+    catalogue_head_kernel<4, RAGGED_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
+                                                                     row0, num_lists);
+  if (seg == nullptr) { MR_CATALOGUE_HEAD(false) } else { MR_CATALOGUE_HEAD(true) }
+#undef MR_CATALOGUE_HEAD
   MR_LAUNCH_CHECK("catalogue_head_kernel");
   return MR_OK;
 }

@@ -287,14 +287,13 @@ bool head_rank_supported(const MrModel& m);
 bool head_rank_takes_dot(const MrModel& m, int group);  // launch_head_rank accepts h_is_dot for this model
 int launch_head_rank(const HeadArgs& a, int group, int32_t* pos, float* probs, cudaStream_t st);
 // catalogue sweep head: probs[r] from the partial logit h_dot[r] (tc_dense TC_EPI_HEAD_DOT) and the GMF term of
-// (users[r / group], item r % group), with the per-row arithmetic of launch_head_rank's partial-logit kernel
+// (users[r / group], item r % group), with the per-row arithmetic of launch_head_rank's partial-logit kernel.  With seg
+// (candidate lists, group 1): global row row0 + r pairs users[seg[row0 + r]] (seg < num_lists) with items[row0 + r];
+// h_dot launch-local, probs global
 bool catalogue_head_supported(const MrModel& m);
 int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t rows, int group,
-                          float* probs, cudaStream_t st);
-// the same for candidate lists: global row row0 + r pairs users[seg[row0 + r]] (seg < num_lists) with items[row0 + r];
-// h_dot launch-local, probs global
-int launch_lists_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t num_lists, const int32_t* seg,
-                      const int32_t* items, int64_t row0, int64_t rows, float* probs, cudaStream_t st);
+                          float* probs, cudaStream_t st, const int32_t* seg = nullptr, const int32_t* items = nullptr,
+                          int64_t row0 = 0, int64_t num_lists = 0);
 // metric sums from positions (rank.cu): sums = {hit_sum, dcg_sum}
 int launch_rank_metrics(const int32_t* pos, int64_t G, int k, float* sums, float* partials, cudaStream_t st);
 

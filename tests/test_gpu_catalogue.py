@@ -102,10 +102,11 @@ def _truth(eng, users, ni):
     return o.forward(w, uu, ii)["p"], o.forward(w64, uu, ii)["p"]
 
 
-@pytest.mark.parametrize("layers,mf", TOWERS, ids=["tc-gmf64", "tc-nogmf", "default-tower", "simt"])
-def test_catalogue_against_oracle(eng_mod, layers, mf):
+@pytest.mark.parametrize("layers,mf,proj", [(L, f, None) for L, f in TOWERS] + [([256, 128, 64], 64, "off")],
+                         ids=["tc-gmf64", "tc-nogmf", "default-tower", "simt", "tc-gmf64-unprojected"])
+def test_catalogue_against_oracle(eng_mod, layers, mf, proj):
     nu, ni, k = 70, 1000, 10
-    eng = _engine(eng_mod, layers, mf, nu, ni)
+    eng = _engine(eng_mod, layers, mf, nu, ni, item_projection=proj)
     rng = np.random.default_rng(5)
     users = rng.integers(0, nu, 40).astype(np.int32)
     rowptr, ex = random_lists(rng, nu, ni)

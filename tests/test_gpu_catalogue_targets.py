@@ -118,10 +118,11 @@ def random_lists(rng, rows, N, most=300):
     return csr([sorted(rng.choice(N, int(rng.integers(0, min(N, most))), replace=False).tolist()) for _ in range(rows)])
 
 
-@pytest.mark.parametrize("layers,mf", TOWERS, ids=TOWER_IDS)
-def test_one_target_per_user_equals_catalogue_topk(eng_mod, layers, mf):
+@pytest.mark.parametrize("layers,mf,proj", [(L, f, None) for L, f in TOWERS] + [([256, 128, 64], 64, "off")],
+                         ids=TOWER_IDS + ["tc-gmf64-unprojected"])
+def test_one_target_per_user_equals_catalogue_topk(eng_mod, layers, mf, proj):
     nu, ni, k = 70, 1000, 10
-    eng = _engine(eng_mod, layers, mf, nu, ni)
+    eng = _engine(eng_mod, layers, mf, nu, ni, item_projection=proj)
     rng = np.random.default_rng(5)
     users = rng.integers(0, nu, 40).astype(np.int32)
     users[7] = nu  # an out-of-range user: every target gets N
