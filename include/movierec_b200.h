@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 104     /* major*100 + minor */
+#define MR_VERSION 105     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
@@ -344,6 +344,36 @@ size_t mr_fold_in_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz);
 int mr_fold_in_users(const MrModel* model, const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz,
                      const int32_t* init_users, const MrFoldIn* cfg /*[host]*/, float* out_user_mlp /* (U, L[0]/2) */,
                      float* out_user_gmf /* (U, mf_dim), NULL when mf_dim == 0 */, float* out_loss, void* ws,
+                     size_t ws_bytes, void* stream);
+
+/* Fold-in of new items (or of known items whose raters have grown): mr_fold_in_users with the roles of the two sides
+ * swapped.  The user tables and the dense block stay frozen and only each new item's MLP row (L[0] - L[0]/2 floats)
+ * and GMF row (mf_dim) are optimised against the item's raters and sampled negative users.  cfg is an MrFoldIn, read
+ * the same way.  Raters: a CSR over the M new items (device rowptr M + 1 int64, rowptr[0] = 0, non-decreasing,
+ * rowptr[M] = nnz; device users, each list strictly ascending, ids in [0, num_users), no list covering every user).
+ * init_items (device, M, may be NULL = all -1): the model row item j starts from, -1 = zero rows; with it a caller
+ * re-folds a known item and writes the row back with its own weights.  The model is never written.  For item j, with
+ * rater list R of n users, and step t = 0 .. steps-1:
+ *   1. the positive at position p of R draws `negs` negative users from the users not in R with mr_sample_negatives'
+ *      rule over num_users candidates (index = p, epoch = t, seed; with fewer candidates than negs, with replacement)
+ *      -- n (negs + 1) rows (user, j);
+ *   2. forward and BCE over those rows, loss = their mean;
+ *   3. the gradient with respect to j's MLP and GMF rows only, plus 2 l2[0] row;
+ *   4. one legacy-Keras Adam step (per-item m and v from zero) or SGD.
+ * For an even L[0] the result equals mr_fold_in_users on the role-swapped model: user and item tables exchanged, the
+ * row blocks of W[1] exchanged ([W1i; W1u]) and, without a hidden layer, the two MLP halves of w_out exchanged.
+ * Determinism, out_loss and validation as mr_fold_in_users: MR_ERR_INVALID for a malformed rowptr, an unsorted list,
+ * a user id or init item out of range, or a list covering every user, before any launch but the check's.
+ * Workspace: the user half of the first layer over the user table (num_users x layers_sizes[1] floats; none without a
+ * hidden layer), the transposed dense block and the sort of the items by list length.
+ * Extended catalogue: a copy of the MrModel whose item_mlp / item_gmf point at [the model's rows; the M new rows]
+ * (contiguous, (num_items + M) rows each) and whose num_items = num_items + M is served and evaluated by every call
+ * above, unchanged, with new item j at id num_items + j. */
+size_t mr_fold_in_items_workspace_bytes(const MrModel* model, int64_t M, int64_t nnz);
+int mr_fold_in_items(const MrModel* model, const int64_t* rowptr, const int32_t* users, int64_t M, int64_t nnz,
+                     const int32_t* init_items, const MrFoldIn* cfg /*[host]*/,
+                     float* out_item_mlp /* (M, L[0] - L[0]/2) */,
+                     float* out_item_gmf /* (M, mf_dim), NULL when mf_dim == 0 */, float* out_loss, void* ws,
                      size_t ws_bytes, void* stream);
 
 /* On-device negative sampler -- replaces _get_random_negatives_and_positive

@@ -459,19 +459,20 @@ static int tc_forward_rows(const MrModel& m, const TcWs& t, const int32_t* users
   return MR_OK;
 }
 
-// Pi = E_item . W1[item rows] over the whole item table (pack_fi must hold the packed item rows of W[1]).
-static int tc_project_items(const MrModel& m, const float* pack_fi, float* Pi, cudaStream_t st) {
-  const int d_u = m.L[0] / 2;
+// P = E . W1h over a whole table E (rows x K), linear, no bias (pack must hold the packed row block W1h (K x L[1]) of
+// W[1]): the item half of the first layer over the item table, or fold-in's other half over the user table.
+static int tc_project_table(const MrModel& m, const float* E, int64_t rows, int K, const float* pack, float* P,
+                            cudaStream_t st) {
   TcDenseArgs a{};
-  a.a_dense = m.item_mlp;
-  a.b_packed = pack_fi;
+  a.a_dense = E;
+  a.b_packed = pack;
   a.N = m.L[1];
-  a.K = m.L[0] - d_u;
-  a.rows = m.num_items;
+  a.K = K;
+  a.rows = rows;
   a.row0 = 0;
   a.epilogue = TC_EPI_BIAS_RELU;
   a.linear = true;
-  a.out = Pi;
+  a.out = P;
   return launch_tc_dense(a, st);
 }
 
@@ -993,7 +994,7 @@ int TrainStep::tower_tc() const {
   }
   if (p.proj) {
     prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = tc_project_items(m, tw.pack_fi, tw.Pi, st);
+    rc = tc_project_table(m, m.item_mlp, m.num_items, d_i, tw.pack_fi, tw.Pi, st);
     if (rc == MR_OK && p.uproj) rc = tc_project_users(m, tw, st);
     if (rc != MR_OK) return rc;
   }
@@ -1332,7 +1333,7 @@ static int eval_prepare(const MrModel& m, const EvalPlan& p, const EvalWs& w, co
   }
   if (rc == MR_OK && p.proj) {
     prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-    rc = tc ? tc_project_items(m, w.t.pack_fi, w.t.Pi, st)
+    rc = tc ? tc_project_table(m, m.item_mlp, m.num_items, d_i, w.t.pack_fi, w.t.Pi, st)
             : launch_small_rows_gemm(m.item_mlp, m.num_items, d_i, m.W[1] + (size_t)d_u * L1, L1, L1, false, nullptr,
                                      w.t.Pi, st);
   }
@@ -2066,25 +2067,24 @@ int mr_sample_negatives(const int64_t* csr_rowptr, const int32_t* csr_items, int
   return rc;
 }
 
-// ---- fold-in: the item half of the first layer once per call (the tensor-core table GEMM on the towers whose item
-// projection it already computes, else a per-element kernel), the users sorted by history length, one kernel ----------
-static bool fold_in_tc_pi(const MrModel& m) {
-  const int d_i = m.L[0] - m.L[0] / 2;
-  return use_tc(m) && m.n_layers >= 3 && d_i % 128 == 0 && d_i <= 256 && m.L[1] == d_i;
+// ---- fold-in: the other side's half of the first layer once per call over its table (the tensor-core table GEMM
+// where the other side's width is the one the eval's item projection takes, else a per-element kernel), the new rows
+// sorted by list length, one kernel.  One path for both directions: FoldSide names the sides. --------------------------
+static bool fold_in_tc_proj(const MrModel& m, const FoldSide& sd) {
+  return use_tc(m) && m.n_layers >= 3 && sd.d_o % 128 == 0 && sd.d_o <= 256 && m.L[1] == sd.d_o;
 }
 
 struct FoldWs {
   int32_t *flags, *keys, *sorted_keys, *order;
   void* sort_ws;
   size_t sort_ws_bytes;
-  float *wt, *Pi, *pack_fi;
+  float *wt, *Po, *pack_fo;
   size_t total;
 };
 
-static FoldWs carve_fold_in(const MrModel& m, int64_t U, void* ws) {
+static FoldWs carve_fold_in(const MrModel& m, const FoldSide& sd, int64_t U, void* ws) {
   FoldWs w{};
   Carver cv(ws);
-  const int d_i = m.L[0] - m.L[0] / 2;
   w.flags = cv.take<int32_t>(64);
   w.keys = cv.take<int32_t>(U);
   w.sorted_keys = cv.take<int32_t>(U);
@@ -2092,87 +2092,120 @@ static FoldWs carve_fold_in(const MrModel& m, int64_t U, void* ws) {
   w.sort_ws_bytes = sort_workspace_bytes(U);
   w.sort_ws = cv.take<char>(w.sort_ws_bytes);
   w.wt = cv.take<float>(m.dense_count);
-  if (m.n_layers > 1) w.Pi = cv.take<float>((size_t)m.num_items * m.L[1]);
-  if (fold_in_tc_pi(m)) w.pack_fi = cv.take<float>((size_t)2 * d_i * m.L[1]);
+  if (m.n_layers > 1) w.Po = cv.take<float>((size_t)sd.num_other * m.L[1]);
+  if (fold_in_tc_proj(m, sd)) w.pack_fo = cv.take<float>((size_t)2 * sd.d_o * m.L[1]);
   w.total = cv.off;
   return w;
 }
 
-size_t mr_fold_in_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz) {
+static size_t fold_in_workspace_bytes(const MrModel* model, bool items, int64_t U, int64_t nnz) {
   if (check_model(model) != MR_OK || U < 0 || U > INT32_MAX || nnz < 0 || nnz > INT32_MAX) return 0;
-  return carve_fold_in(*model, U, nullptr).total;
+  return carve_fold_in(*model, fold_side(*model, items), U, nullptr).total;
 }
 
-int mr_fold_in_users(const MrModel* model, const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz,
-                     const int32_t* init_users, const MrFoldIn* cfg, float* out_user_mlp, float* out_user_gmf,
-                     float* out_loss, void* ws, size_t ws_bytes, void* stream) {
+size_t mr_fold_in_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz) {
+  return fold_in_workspace_bytes(model, false, U, nnz);
+}
+
+size_t mr_fold_in_items_workspace_bytes(const MrModel* model, int64_t M, int64_t nnz) {
+  return fold_in_workspace_bytes(model, true, M, nnz);
+}
+
+// The words of one direction's error messages.
+struct FoldNames {
+  const char *fn, *self, *other_id, *init, *covers;
+};
+static const FoldNames kFoldUsers = {"fold_in", "user", "an item id", "an init user", "a history covers every item"};
+static const FoldNames kFoldItems = {"fold_in_items", "item", "a user id", "an init item",
+                                     "a rater list covers every user"};
+
+static int fold_in_call(const MrModel* model, bool items, const int64_t* rowptr, const int32_t* ids, int64_t U,
+                        int64_t nnz, const int32_t* init_rows, const MrFoldIn* cfg, float* out_mlp, float* out_gmf,
+                        float* out_loss, void* ws, size_t ws_bytes, void* stream) {
   int rc = check_model(model);
   if (rc != MR_OK) return rc;
   const MrModel& m = *model;
+  const FoldNames& nm = items ? kFoldItems : kFoldUsers;
+  const char* fn = nm.fn;
   cudaStream_t st = (cudaStream_t)stream;
-  MR_REQUIRE(cfg != nullptr, "fold_in: cfg is NULL");
-  MR_REQUIRE(cfg->steps >= 0, "fold_in: steps=%d must be >= 0", cfg->steps);
-  MR_REQUIRE(cfg->negs >= 1 && cfg->negs <= MR_MAX_NEGS, "fold_in: negs=%d out of [1,%d]", cfg->negs, MR_MAX_NEGS);
-  MR_REQUIRE(cfg->optimizer == MR_OPT_ADAM || cfg->optimizer == MR_OPT_SGD, "fold_in: unknown optimizer %d",
+  MR_REQUIRE(cfg != nullptr, "%s: cfg is NULL", fn);
+  MR_REQUIRE(cfg->steps >= 0, "%s: steps=%d must be >= 0", fn, cfg->steps);
+  MR_REQUIRE(cfg->negs >= 1 && cfg->negs <= MR_MAX_NEGS, "%s: negs=%d out of [1,%d]", fn, cfg->negs, MR_MAX_NEGS);
+  MR_REQUIRE(cfg->optimizer == MR_OPT_ADAM || cfg->optimizer == MR_OPT_SGD, "%s: unknown optimizer %d", fn,
              cfg->optimizer);
-  MR_REQUIRE(isfinite(cfg->lr), "fold_in: lr must be finite");
+  MR_REQUIRE(isfinite(cfg->lr), "%s: lr must be finite", fn);
   if (cfg->optimizer == MR_OPT_ADAM)
     MR_REQUIRE(cfg->beta_1 >= 0.f && cfg->beta_1 < 1.f && cfg->beta_2 >= 0.f && cfg->beta_2 < 1.f && cfg->epsilon > 0.f,
-               "fold_in: Adam needs beta_1, beta_2 in [0, 1) and epsilon > 0");
-  MR_REQUIRE(U >= 0 && U <= INT32_MAX && nnz >= 0 && nnz <= INT32_MAX, "fold_in: bad sizes U=%lld nnz=%lld",
+               "%s: Adam needs beta_1, beta_2 in [0, 1) and epsilon > 0", fn);
+  MR_REQUIRE(U >= 0 && U <= INT32_MAX && nnz >= 0 && nnz <= INT32_MAX, "%s: bad sizes U=%lld nnz=%lld", fn,
              (long long)U, (long long)nnz);
-  MR_REQUIRE(rowptr != nullptr, "fold_in: rowptr is NULL");
-  MR_REQUIRE(nnz == 0 || items != nullptr, "fold_in: items is NULL");
-  MR_REQUIRE(U == 0 || out_user_mlp != nullptr, "fold_in: out_user_mlp is NULL");
-  MR_REQUIRE(U == 0 || m.mf_dim == 0 || out_user_gmf != nullptr, "fold_in: out_user_gmf is NULL but mf_dim > 0");
-  MR_REQUIRE(fold_in_supported(m), "fold_in: layer widths too large for the kernel's shared memory");
-  const FoldWs w = carve_fold_in(m, U, ws);
+  MR_REQUIRE(rowptr != nullptr, "%s: rowptr is NULL", fn);
+  MR_REQUIRE(nnz == 0 || ids != nullptr, "%s: %s is NULL", fn, items ? "users" : "items");
+  MR_REQUIRE(U == 0 || out_mlp != nullptr, "%s: out_%s_mlp is NULL", fn, nm.self);
+  MR_REQUIRE(U == 0 || m.mf_dim == 0 || out_gmf != nullptr, "%s: out_%s_gmf is NULL but mf_dim > 0", fn, nm.self);
+  const FoldSide sd = fold_side(m, items);
+  MR_REQUIRE(fold_in_supported(m, sd), "%s: layer widths too large for the kernel's shared memory", fn);
+  const FoldWs w = carve_fold_in(m, sd, U, ws);
   if (ws == nullptr || ws_bytes < w.total) {
-    set_error("fold_in: workspace %zu bytes < %zu", ws_bytes, w.total);
+    set_error("%s: workspace %zu bytes < %zu", fn, ws_bytes, w.total);
     return MR_ERR_WORKSPACE;
   }
   if (U == 0) return MR_OK;
 
-  // the histories are checked before any other work: one small kernel and a one-word read-back
+  // the lists are checked before any other work: one small kernel and a one-word read-back
   MR_CUDA(cudaMemsetAsync(w.flags, 0, sizeof(int32_t), st));
-  rc = launch_fold_in_check(rowptr, items, U, nnz, m.num_items, init_users, m.num_users, w.keys, w.flags, st);
+  rc = launch_fold_in_check(rowptr, ids, U, nnz, sd.num_other, init_rows, sd.num_self, w.keys, w.flags, st);
   if (rc != MR_OK) return rc;
   int32_t bad = 0;
   MR_CUDA(cudaMemcpyAsync(&bad, w.flags, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   MR_CUDA(cudaStreamSynchronize(st));
-  MR_REQUIRE(!(bad & 1), "fold_in: rowptr must start at 0, never decrease and end at nnz, and every list must be "
-             "strictly ascending");
-  MR_REQUIRE(!(bad & 2), "fold_in: an item id lies outside [0, %d)", m.num_items);
-  MR_REQUIRE(!(bad & 4), "fold_in: an init user lies outside [-1, %d)", m.num_users);
-  MR_REQUIRE(!(bad & 8), "fold_in: a history covers every item: no negatives to draw");
+  MR_REQUIRE(!(bad & 1), "%s: rowptr must start at 0, never decrease and end at nnz, and every list must be "
+             "strictly ascending", fn);
+  MR_REQUIRE(!(bad & 2), "%s: %s lies outside [0, %d)", fn, nm.other_id, sd.num_other);
+  MR_REQUIRE(!(bad & 4), "%s: %s lies outside [-1, %d)", fn, nm.init, sd.num_self);
+  MR_REQUIRE(!(bad & 8), "%s: %s: no negatives to draw", fn, nm.covers);
 
-  rc = launch_sort_pairs(w.keys, U, bits_for((int64_t)m.num_items + 1), w.sorted_keys, w.order, w.sort_ws,
+  rc = launch_sort_pairs(w.keys, U, bits_for((int64_t)sd.num_other + 1), w.sorted_keys, w.order, w.sort_ws,
                          w.sort_ws_bytes, st);
   if (rc == MR_OK) rc = launch_transpose_kernels(m, w.wt, st);
   if (rc == MR_OK && m.n_layers > 1) {
-    if (fold_in_tc_pi(m)) {
-      const int d_u = m.L[0] / 2;
-      rc = launch_pack_weights(m.W[1] + (size_t)d_u * m.L[1], m.L[0] - d_u, m.L[1], 0, w.pack_fi, st);
-      if (rc == MR_OK) rc = tc_project_items(m, w.pack_fi, w.Pi, st);
+    if (fold_in_tc_proj(m, sd)) {
+      rc = launch_pack_weights(sd.W1o, sd.d_o, m.L[1], 0, w.pack_fo, st);
+      if (rc == MR_OK) rc = tc_project_table(m, sd.other_mlp, sd.num_other, sd.d_o, w.pack_fo, w.Po, st);
     } else {
-      rc = launch_fold_in_project(m, w.Pi, st);
+      rc = launch_fold_in_project(sd.other_mlp, sd.num_other, sd.d_o, sd.W1o, m.L[1], w.Po, st);
     }
   }
   if (rc != MR_OK) return rc;
   FoldInArgs a{};
   a.model = model;
+  a.side = sd;
   a.wt = w.wt;
-  a.Pi = w.Pi;
+  a.Po = w.Po;
   a.rowptr = rowptr;
-  a.items = items;
-  a.init_users = init_users;
+  a.ids = ids;
+  a.init_rows = init_rows;
   a.order = w.order;
   a.U = U;
   a.cfg = *cfg;
-  a.out_mlp = out_user_mlp;
-  a.out_gmf = out_user_gmf;
+  a.out_mlp = out_mlp;
+  a.out_gmf = out_gmf;
   a.out_loss = out_loss;
   return launch_fold_in(a, st);
+}
+
+int mr_fold_in_users(const MrModel* model, const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz,
+                     const int32_t* init_users, const MrFoldIn* cfg, float* out_user_mlp, float* out_user_gmf,
+                     float* out_loss, void* ws, size_t ws_bytes, void* stream) {
+  return fold_in_call(model, false, rowptr, items, U, nnz, init_users, cfg, out_user_mlp, out_user_gmf, out_loss, ws,
+                      ws_bytes, stream);
+}
+
+int mr_fold_in_items(const MrModel* model, const int64_t* rowptr, const int32_t* users, int64_t M, int64_t nnz,
+                     const int32_t* init_items, const MrFoldIn* cfg, float* out_item_mlp, float* out_item_gmf,
+                     float* out_loss, void* ws, size_t ws_bytes, void* stream) {
+  return fold_in_call(model, true, rowptr, users, M, nnz, init_items, cfg, out_item_mlp, out_item_gmf, out_loss, ws,
+                      ws_bytes, stream);
 }
 
 int mr_users_grouped(const int32_t* users, int64_t n, int32_t group, int32_t* flag, void* stream) {

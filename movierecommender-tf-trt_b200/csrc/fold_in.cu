@@ -1,14 +1,17 @@
-// Fold-in of new users (include/movierec_b200.h: mr_fold_in_users): the item tables and the dense block are frozen and
-// only each user's MLP and GMF rows are optimised against the user's history and sampled negatives.
+// Fold-in of new users or new items (include/movierec_b200.h: mr_fold_in_users, mr_fold_in_items): the other side's
+// tables and the dense block are frozen and only each new row pair (MLP, GMF) is optimised against its list (a user's
+// items, an item's raters) and sampled negatives.  NeuMF is symmetric in its two towers, so one kernel serves both
+// directions: a FoldSide set on the host names the folded side's width, W1 row block, init tables and head weights and
+// the other side's tables and count.  Below, "self" is the side being folded in and "other" the frozen side.
 //
-// One persistent CTA per user at a time, all steps inside the kernel; users are taken longest history first.  The
-// user's rows, their Adam moments, the user half of the first layer (Pu = e_u . W1u + b1) and the running gradient
-// sums live in shared memory.  A step walks the user's rows (n positives x (negs + 1)) in chunks of at most kChunkRows:
+// One persistent CTA per new row at a time, all steps inside the kernel; rows are taken longest list first.  The
+// rows, their Adam moments, the self half of the first layer (Ps = e_s . W1s + b1) and the running gradient sums live
+// in shared memory.  A step walks the row's training rows (n positives x (negs + 1)) in chunks of at most kChunkRows:
 // one thread per positive draws the chunk's negatives (negative_draw.cuh, the batch sampler's rule), then tiles of TM
-// rows go through relu(Pi[item] + Pu), the later layers (tile_gemm, weights read through L1), the head with the GMF
+// rows go through relu(Po[other] + Ps), the later layers (tile_gemm, weights read through L1), the head with the GMF
 // product, dz and the backward to the masked dZ1.  Per tile, each column of sum dZ1 and of the GMF row gradient is
 // summed over the tile's rows in row order and added to the running sum in tile order: a fixed order, no atomics.  At
-// the end of the step dE_u = (sum dZ1) . W1u^T + 2 l2[0] e_u, and the rows are updated in shared memory.
+// the end of the step dE_s = (sum dZ1) . W1s^T + 2 l2[0] e_s, and the rows are updated in shared memory.
 #include "launchers.h"
 #include "negative_draw.cuh"
 #include "neumf_tile.cuh"
@@ -21,11 +24,12 @@ constexpr int kChunkRows = 1024;  // rows whose negatives are drawn at once (>= 
 struct FoldParams {
   MrModel m;
   const float* Wt[MR_MAX_LAYERS];  // Wt[l] = W[l]^T, (L[l], L[l-1])
-  const float* Pi;                 // (num_items, L1): E_item . W1[item rows]; NULL without a hidden layer
+  FoldSide side;
+  const float* Po;                 // (num_other, L1): E_other . W1o; NULL without a hidden layer
   const int64_t* rowptr;
-  const int32_t* items;
-  const int32_t* init_users;
-  const int32_t* order;            // users, longest history first
+  const int32_t* ids;              // the lists: ids of the other side
+  const int32_t* init_rows;        // model rows of the folded side to start from, -1 = zero rows
+  const int32_t* order;            // new rows, longest list first
   int64_t U;
   int32_t steps, negs, optimizer;
   float lr, beta_1, beta_2, epsilon;
@@ -40,12 +44,16 @@ struct FoldParams {
   int32_t dz_off, loss_off, ids_off, picked_off;
 };
 
-template <int TM>
+// ITEMS: the direction (FoldSide::items).  The two widths follow from it and L[0]; deriving them here rather than
+// reading them from the descriptor keeps the user direction's code as fast as before the descriptor existed (read
+// from the descriptor, the 256-128-64 tower's user fold-in ran 15 % slower on a B200).
+template <int TM, bool ITEMS>
 __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams p) {
   extern __shared__ __align__(16) float smem[];
   const MrModel& m = p.m;
   const int n = m.n_layers, f = m.mf_dim;
-  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+  const FoldSide& sd = p.side;
+  const int d_s = ITEMS ? m.L[0] - m.L[0] / 2 : m.L[0] / 2, d_o = m.L[0] - d_s;
   const int L1 = n > 1 ? m.L[1] : 0;
   const int Ln = m.L[n - 1];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
@@ -74,15 +82,15 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
     const int u = __ldg(p.order + slot);
     const int64_t lo = __ldg(p.rowptr + u);
     const int len = (int)(__ldg(p.rowptr + u + 1) - lo);
-    const int32_t* hist = p.items + lo;
-    const int init = p.init_users != nullptr ? __ldg(p.init_users + u) : -1;
-    for (int k = tid; k < d_u; k += blockDim.x) {
-      s_e[k] = init >= 0 ? m.user_mlp[(size_t)init * d_u + k] : 0.f;
+    const int32_t* hist = p.ids + lo;
+    const int init = p.init_rows != nullptr ? __ldg(p.init_rows + u) : -1;
+    for (int k = tid; k < d_s; k += blockDim.x) {
+      s_e[k] = init >= 0 ? sd.self_mlp[(size_t)init * d_s + k] : 0.f;
       s_me[k] = 0.f;
       s_ve[k] = 0.f;
     }
     for (int j = tid; j < f; j += blockDim.x) {
-      s_g[j] = init >= 0 ? m.user_gmf[(size_t)init * f + j] : 0.f;
+      s_g[j] = init >= 0 ? sd.self_gmf[(size_t)init * f + j] : 0.f;
       s_mg[j] = 0.f;
       s_vg[j] = 0.f;
     }
@@ -92,10 +100,10 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
     __syncthreads();
 
     for (int t = 0; t < p.steps; ++t) {
-      // ---- once per step: Pu = e_u . W1u + b1, the sums cleared --------------------------------------------------
+      // ---- once per step: Ps = e_s . W1s + b1, the sums cleared --------------------------------------------------
       for (int c = tid; c < L1; c += blockDim.x) {
         float s = 0.f;
-        for (int k = 0; k < d_u; ++k) s = fmaf(s_e[k], __ldg(m.W[1] + (size_t)k * L1 + c), s);
+        for (int k = 0; k < d_s; ++k) s = fmaf(s_e[k], __ldg(sd.W1s + (size_t)k * L1 + c), s);
         s_pu[c] = s + __ldg(m.b[1] + c);
         s_sum[c] = 0.f;
       }
@@ -110,27 +118,27 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
         // ---- the chunk's rows: group j = the negatives of positive g0 + j, then the positive ----------------------
         for (int j = tid; j < ng; j += blockDim.x) {
           int* out = s_ids + j * group;
-          draw_negatives(hist, len, m.num_items, p.negs, (uint64_t)(g0 + j), p.seed, (uint64_t)t,
-                         s_picked + j * p.negs, [&](int q, int item) { out[q] = item; });
+          draw_negatives(hist, len, sd.num_other, p.negs, (uint64_t)(g0 + j), p.seed, (uint64_t)t,
+                         s_picked + j * p.negs, [&](int q, int id) { out[q] = id; });
           out[p.negs] = __ldg(hist + g0 + j);
         }
         __syncthreads();
 
         for (int row0 = 0; row0 < rows; row0 += TM) {
           const int valid = min(TM, rows - row0);
-          // ---- first layer (or nothing without a hidden layer) and the GMF item rows ----------------------------
+          // ---- first layer (or nothing without a hidden layer) and the other side's GMF rows ---------------------
           if (n > 1) {
             float* h1 = smem + p.act_off[1];
             for (int e = tid; e < TM * L1; e += blockDim.x) {
               const int r = e / L1, c = e - r * L1;
               float v = 0.f;
-              if (r < valid) v = fmaxf(__ldg(p.Pi + (size_t)s_ids[row0 + r] * L1 + c) + s_pu[c], 0.f);
+              if (r < valid) v = fmaxf(__ldg(p.Po + (size_t)s_ids[row0 + r] * L1 + c) + s_pu[c], 0.f);
               h1[r * p.ld[1] + c] = v;
             }
           }
           for (int e = tid; e < TM * f; e += blockDim.x) {
             const int r = e / f, c = e - r * f;
-            gi[r * p.ldf + c] = r < valid ? __ldg(m.item_gmf + (size_t)s_ids[row0 + r] * f + c) : 0.f;
+            gi[r * p.ldf + c] = r < valid ? __ldg(sd.other_gmf + (size_t)s_ids[row0 + r] * f + c) : 0.f;
           }
           __syncthreads();
           for (int l = 2; l < n; ++l) {
@@ -141,7 +149,7 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
             __syncthreads();
           }
 
-          // ---- head: z = b + w[:f].(g_u*g_i) + w[f:].x ; sigmoid ; BCE ; dz --------------------------------------
+          // ---- head: z = b + w[:f].(g_s*g_o) + w[f:].x ; sigmoid ; BCE ; dz --------------------------------------
           const int ldL = p.ld[n - 1];
           for (int r = warp; r < TM; r += nwarps) {
             float s = 0.f;
@@ -150,9 +158,9 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
               if (n > 1) {
                 for (int c = lane; c < Ln; c += 32) s = fmaf(__ldg(m.w_out + f + c), actL[r * ldL + c], s);
               } else {
-                const float* ei = m.item_mlp + (size_t)s_ids[row0 + r] * d_i;
-                for (int c = lane; c < d_u; c += 32) s = fmaf(__ldg(m.w_out + f + c), s_e[c], s);
-                for (int c = lane; c < d_i; c += 32) s = fmaf(__ldg(m.w_out + f + d_u + c), __ldg(ei + c), s);
+                const float* eo = sd.other_mlp + (size_t)s_ids[row0 + r] * d_o;
+                for (int c = lane; c < d_s; c += 32) s = fmaf(__ldg(m.w_out + f + sd.ws_off + c), s_e[c], s);
+                for (int c = lane; c < d_o; c += 32) s = fmaf(__ldg(m.w_out + f + sd.wo_off + c), __ldg(eo + c), s);
               }
             }
             s = warp_sum(s);
@@ -224,12 +232,12 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
       const float lr_t = adam ? (float)((double)p.lr * sqrt(1.0 - pow((double)p.beta_2, (double)(t + 1))) /
                                         (1.0 - pow((double)p.beta_1, (double)(t + 1))))
                               : p.lr;
-      for (int k = tid; k < d_u; k += blockDim.x) {
+      for (int k = tid; k < d_s; k += blockDim.x) {
         float d = 0.f;
         if (n > 1) {
-          for (int c = 0; c < L1; ++c) d = fmaf(__ldg(m.W[1] + (size_t)k * L1 + c), s_sum[c], d);
+          for (int c = 0; c < L1; ++c) d = fmaf(__ldg(sd.W1s + (size_t)k * L1 + c), s_sum[c], d);
         } else {
-          d = s_sum[0] * __ldg(m.w_out + f + k);
+          d = s_sum[0] * __ldg(m.w_out + f + sd.ws_off + k);
         }
         const float g = plus_l2(d, s_e[k], c2);
         if (adam) adam_step(s_e[k], g, s_me[k], s_ve[k], lr_t, p.beta_1, p.beta_2, p.epsilon);
@@ -244,35 +252,36 @@ __global__ void __launch_bounds__(kFoldThreads) fold_in_kernel(const FoldParams 
       __syncthreads();
     }
 
-    for (int k = tid; k < d_u; k += blockDim.x) p.out_mlp[(size_t)u * d_u + k] = s_e[k];
+    for (int k = tid; k < d_s; k += blockDim.x) p.out_mlp[(size_t)u * d_s + k] = s_e[k];
     for (int j = tid; j < f; j += blockDim.x) p.out_gmf[(size_t)u * f + j] = s_g[j];
     if (tid == 0 && p.out_loss != nullptr) p.out_loss[u] = last_loss;
     __syncthreads();
   }
 }
 
-// Pi[i][c] = sum_k E_item[i][k] W1[d_u + k][c] for the towers the tensor-core table GEMM does not take (odd widths,
-// small towers): one thread per output, consecutive threads on consecutive columns.
-__global__ void fold_in_project_kernel(MrModel m, float* __restrict__ Pi) {
-  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u, L1 = m.L[1];
-  const float* W1i = m.W[1] + (size_t)d_u * L1;
-  const int64_t total = (int64_t)m.num_items * L1;
+// P[i][c] = sum_k E[i][k] W1h[k][c] over a table E (rows x K) and one row block W1h (K x L1) of W[1], for the towers
+// the tensor-core table GEMM does not take (odd widths, small towers): one thread per output, consecutive threads on
+// consecutive columns.
+__global__ void fold_in_project_kernel(const float* __restrict__ E, int64_t rows, int K, const float* __restrict__ W1h,
+                                       int L1, float* __restrict__ P) {
+  const int64_t total = rows * L1;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int64_t i = e / L1;
     const int c = (int)(e - i * L1);
-    const float* ei = m.item_mlp + i * d_i;
+    const float* ei = E + i * K;
     float s = 0.f;
-    for (int k = 0; k < d_i; ++k) s = fmaf(__ldg(ei + k), __ldg(W1i + (size_t)k * L1 + c), s);
-    Pi[e] = s;
+    for (int k = 0; k < K; ++k) s = fmaf(__ldg(ei + k), __ldg(W1h + (size_t)k * L1 + c), s);
+    P[e] = s;
   }
 }
 
-// Validation of the histories and init rows (flags: bit 0 malformed rowptr or a list not strictly ascending, bit 1
-// an item out of range, bit 2 an init user out of range, bit 3 a list covering every item), and the sort key of each
-// user: num_items - length, so that the stable ascending sort takes the longest history first.
-__global__ void fold_in_check_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ items, int64_t U,
-                                     int64_t nnz, int32_t num_items, const int32_t* __restrict__ init_users,
-                                     int32_t num_users, int32_t* __restrict__ keys, int32_t* __restrict__ flags) {
+// Validation of the lists and init rows (flags: bit 0 malformed rowptr or a list not strictly ascending, bit 1 an id
+// of the other side out of range, bit 2 an init row out of range, bit 3 a list covering the whole other side), and the
+// sort key of each new row: num_other - length, so that the stable ascending sort takes the longest list first.  Named
+// for the user direction; the item direction passes its own sides in the same places.
+__global__ void fold_in_check_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ ids, int64_t U,
+                                     int64_t nnz, int32_t num_other, const int32_t* __restrict__ init_rows,
+                                     int32_t num_self, int32_t* __restrict__ keys, int32_t* __restrict__ flags) {
   for (int64_t u = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; u < U; u += (int64_t)gridDim.x * blockDim.x) {
     int bad = 0;
     const int64_t lo = rowptr[u], hi = rowptr[u + 1];
@@ -282,26 +291,49 @@ __global__ void fold_in_check_kernel(const int64_t* __restrict__ rowptr, const i
       len = hi - lo;
       int prev = -1;
       for (int64_t e = lo; e < hi; ++e) {
-        const int it = items[e];
-        if (it < 0 || it >= num_items) bad |= 2;
+        const int it = ids[e];
+        if (it < 0 || it >= num_other) bad |= 2;
         else if (it <= prev) bad |= 1;
         prev = it;
       }
-      if (len >= num_items) bad |= 8;
+      if (len >= num_other) bad |= 8;
     }
-    if (init_users != nullptr) {
-      const int iu = init_users[u];
-      if (iu < -1 || iu >= num_users) bad |= 4;
+    if (init_rows != nullptr) {
+      const int iu = init_rows[u];
+      if (iu < -1 || iu >= num_self) bad |= 4;
     }
-    keys[u] = (bad != 0 || len > num_items) ? 0 : (int32_t)(num_items - len);
+    keys[u] = (bad != 0 || len > num_other) ? 0 : (int32_t)(num_other - len);
     if (bad) atomicOr(flags, bad);
   }
 }
 
 // ---- host side -----------------------------------------------------------------------------------------------------
 
-static size_t fold_layout(const MrModel& m, int tm, FoldParams* p) {
-  const int n = m.n_layers, f = m.mf_dim, d_u = m.L[0] / 2;
+FoldSide fold_side(const MrModel& m, bool items) {
+  const int d_u = m.L[0] / 2, d_i = m.L[0] - d_u;
+  const int L1 = m.n_layers > 1 ? m.L[1] : 0;
+  const float* W1u = m.n_layers > 1 ? m.W[1] : nullptr;
+  const float* W1i = m.n_layers > 1 ? m.W[1] + (size_t)d_u * L1 : nullptr;
+  FoldSide s{};
+  s.items = items;
+  if (!items) {
+    s.d_s = d_u; s.d_o = d_i;
+    s.W1s = W1u; s.W1o = W1i;
+    s.self_mlp = m.user_mlp; s.self_gmf = m.user_gmf; s.num_self = m.num_users;
+    s.other_mlp = m.item_mlp; s.other_gmf = m.item_gmf; s.num_other = m.num_items;
+    s.ws_off = 0; s.wo_off = d_u;
+  } else {
+    s.d_s = d_i; s.d_o = d_u;
+    s.W1s = W1i; s.W1o = W1u;
+    s.self_mlp = m.item_mlp; s.self_gmf = m.item_gmf; s.num_self = m.num_items;
+    s.other_mlp = m.user_mlp; s.other_gmf = m.user_gmf; s.num_other = m.num_users;
+    s.ws_off = d_u; s.wo_off = 0;
+  }
+  return s;
+}
+
+static size_t fold_layout(const MrModel& m, int d_s, int tm, FoldParams* p) {
+  const int n = m.n_layers, f = m.mf_dim;
   int off = 0;
   auto take = [&](int count) {
     const int o = off;
@@ -319,9 +351,9 @@ static size_t fold_layout(const MrModel& m, int tm, FoldParams* p) {
   p->ldg = pad_ld(gmax);
   p->ga_off = take(n > 1 ? tm * p->ldg : 0);
   p->gb_off = take(n > 1 ? tm * p->ldg : 0);
-  p->e_off = take(d_u);
-  p->me_off = take(d_u);
-  p->ve_off = take(d_u);
+  p->e_off = take(d_s);
+  p->me_off = take(d_s);
+  p->ve_off = take(d_s);
   p->g_off = take(f);
   p->mg_off = take(f);
   p->vg_off = take(f);
@@ -337,21 +369,21 @@ static size_t fold_layout(const MrModel& m, int tm, FoldParams* p) {
 }
 
 // Largest tile whose shared memory lets two CTAs share an SM, else whatever fits (0: none).
-static int fold_tile_rows(const MrModel& m) {
+static int fold_tile_rows(const MrModel& m, int d_s) {
   FoldParams tmp;
   const int cands[4] = {32, 16, 8, 4};
   for (int i = 0; i < 4; ++i)
-    if (fold_layout(m, cands[i], &tmp) <= 112 * 1024) return cands[i];
+    if (fold_layout(m, d_s, cands[i], &tmp) <= 112 * 1024) return cands[i];
   for (int i = 0; i < 4; ++i)
-    if (fold_layout(m, cands[i], &tmp) <= 226 * 1024) return cands[i];
+    if (fold_layout(m, d_s, cands[i], &tmp) <= 226 * 1024) return cands[i];
   return 0;
 }
 
-bool fold_in_supported(const MrModel& m) { return fold_tile_rows(m) > 0; }
+bool fold_in_supported(const MrModel& m, const FoldSide& side) { return fold_tile_rows(m, side.d_s) > 0; }
 
-template <int TM>
+template <int TM, bool ITEMS>
 static int launch_fold(const FoldParams& p, size_t smem, cudaStream_t st) {
-  auto kern = fold_in_kernel<TM>;
+  auto kern = fold_in_kernel<TM, ITEMS>;
   MR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int occ = 0;
   MR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kFoldThreads, smem));
@@ -368,20 +400,21 @@ static int launch_fold(const FoldParams& p, size_t smem, cudaStream_t st) {
 
 int launch_fold_in(const FoldInArgs& a, cudaStream_t st) {
   const MrModel& m = *a.model;
-  const int tm = fold_tile_rows(m);
+  const int tm = fold_tile_rows(m, a.side.d_s);
   if (tm == 0) {
     set_error("fold-in: layer widths too large for the kernel's shared memory");
     return MR_ERR_INVALID;
   }
   if (a.U == 0) return MR_OK;
   FoldParams p{};
-  const size_t smem = fold_layout(m, tm, &p);
+  const size_t smem = fold_layout(m, a.side.d_s, tm, &p);
   p.m = m;
   for (int l = 1; l < m.n_layers; ++l) p.Wt[l] = a.wt + (m.W[l] - m.dense);
-  p.Pi = a.Pi;
+  p.side = a.side;
+  p.Po = a.Po;
   p.rowptr = a.rowptr;
-  p.items = a.items;
-  p.init_users = a.init_users;
+  p.ids = a.ids;
+  p.init_rows = a.init_rows;
   p.order = a.order;
   p.U = a.U;
   p.steps = a.cfg.steps;
@@ -396,32 +429,32 @@ int launch_fold_in(const FoldInArgs& a, cudaStream_t st) {
   p.out_gmf = a.out_gmf;
   p.out_loss = a.out_loss;
   switch (tm) {
-    case 32: return launch_fold<32>(p, smem, st);
-    case 16: return launch_fold<16>(p, smem, st);
-    case 8: return launch_fold<8>(p, smem, st);
-    case 4: return launch_fold<4>(p, smem, st);
+    case 32: return a.side.items ? launch_fold<32, true>(p, smem, st) : launch_fold<32, false>(p, smem, st);
+    case 16: return a.side.items ? launch_fold<16, true>(p, smem, st) : launch_fold<16, false>(p, smem, st);
+    case 8: return a.side.items ? launch_fold<8, true>(p, smem, st) : launch_fold<8, false>(p, smem, st);
+    case 4: return a.side.items ? launch_fold<4, true>(p, smem, st) : launch_fold<4, false>(p, smem, st);
   }
   return MR_ERR_INVALID;
 }
 
-int launch_fold_in_project(const MrModel& m, float* Pi, cudaStream_t st) {
-  const int64_t total = (int64_t)m.num_items * m.L[1];
+int launch_fold_in_project(const float* E, int64_t rows, int K, const float* W1h, int L1, float* P, cudaStream_t st) {
+  const int64_t total = rows * L1;
   int64_t blocks = (total + 255) / 256;
   const int64_t cap = (int64_t)sm_count() * 16;
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
-  fold_in_project_kernel<<<(unsigned)blocks, 256, 0, st>>>(m, Pi);
+  fold_in_project_kernel<<<(unsigned)blocks, 256, 0, st>>>(E, rows, K, W1h, L1, P);
   MR_LAUNCH_CHECK("fold_in_project_kernel");
   return MR_OK;
 }
 
-int launch_fold_in_check(const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz, int32_t num_items,
-                         const int32_t* init_users, int32_t num_users, int32_t* keys, int32_t* flags, cudaStream_t st) {
+int launch_fold_in_check(const int64_t* rowptr, const int32_t* ids, int64_t U, int64_t nnz, int32_t num_other,
+                         const int32_t* init_rows, int32_t num_self, int32_t* keys, int32_t* flags, cudaStream_t st) {
   if (U == 0) return MR_OK;
   int64_t blocks = (U + 127) / 128;
   const int64_t cap = (int64_t)sm_count() * 8;
   if (blocks > cap) blocks = cap;
-  fold_in_check_kernel<<<(unsigned)blocks, 128, 0, st>>>(rowptr, items, U, nnz, num_items, init_users, num_users, keys,
+  fold_in_check_kernel<<<(unsigned)blocks, 128, 0, st>>>(rowptr, ids, U, nnz, num_other, init_rows, num_self, keys,
                                                          flags);
   MR_LAUNCH_CHECK("fold_in_check_kernel");
   return MR_OK;

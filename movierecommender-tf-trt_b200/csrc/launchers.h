@@ -175,29 +175,44 @@ int launch_sample_negatives(const int64_t* rowptr, const int32_t* csr_items, int
                             int negs, uint64_t seed, uint64_t epoch, int32_t* out_users, int32_t* out_items,
                             float* out_labels, cudaStream_t st);
 
-// ---- fold_in.cu: per-user optimisation of the user rows against a history, everything else frozen ----------------
+// ---- fold_in.cu: per-row optimisation of new user (or item) rows against a list, everything else frozen -----------
+// The side being folded in ("self") and the frozen side ("other"): users against the item tables, or items against
+// the user tables.  Pointers into the model; the W1 blocks are NULL without a hidden layer.
+struct FoldSide {
+  bool items;                           // folding items in (users otherwise)
+  int d_s, d_o;                         // MLP row widths of the folded side and of the other side
+  const float* W1s;                     // the folded side's row block of W[1] (d_s x L1)
+  const float* W1o;                     // the other side's row block (d_o x L1), for its projection over its table
+  const float *self_mlp, *self_gmf;     // the folded side's model tables: init rows
+  int32_t num_self;
+  const float *other_mlp, *other_gmf;   // the other side's model tables
+  int32_t num_other;                    // the negatives' candidates, the ids' range and the sort key's base
+  int ws_off, wo_off;                   // the two sides' MLP parts in w_out, past its GMF part (no hidden layer)
+};
+FoldSide fold_side(const MrModel& m, bool items);
 struct FoldInArgs {
   const MrModel* model;
+  FoldSide side;
   const float* wt;          // transposed hidden kernels, dense-block layout
-  const float* Pi;          // (num_items x L1) item half of the first layer; NULL without a hidden layer
+  const float* Po;          // (num_other x L1) other half of the first layer, no bias; NULL without a hidden layer
   const int64_t* rowptr;
-  const int32_t* items;
-  const int32_t* init_users;
-  const int32_t* order;     // the U users, longest history first
+  const int32_t* ids;       // the lists: ids of the other side
+  const int32_t* init_rows; // model rows of the folded side to start from, -1 = zero rows (NULL = all -1)
+  const int32_t* order;     // the U new rows, longest list first
   int64_t U;
   MrFoldIn cfg;
   float* out_mlp;
   float* out_gmf;
   float* out_loss;
 };
-bool fold_in_supported(const MrModel& m);
+bool fold_in_supported(const MrModel& m, const FoldSide& side);
 int launch_fold_in(const FoldInArgs& a, cudaStream_t st);
-// Pi = E_item . W1[item rows] with one thread per output (any widths)
-int launch_fold_in_project(const MrModel& m, float* Pi, cudaStream_t st);
-// flags[0] |= 1 malformed rowptr or unsorted list, 2 item out of range, 4 init user out of range, 8 a list covering
-// every item; keys[u] = num_items - length of list u (the longest history sorts first)
-int launch_fold_in_check(const int64_t* rowptr, const int32_t* items, int64_t U, int64_t nnz, int32_t num_items,
-                         const int32_t* init_users, int32_t num_users, int32_t* keys, int32_t* flags, cudaStream_t st);
+// P = E . W1h over a table E (rows x K) and a row block W1h (K x L1) of W[1], one thread per output (any widths)
+int launch_fold_in_project(const float* E, int64_t rows, int K, const float* W1h, int L1, float* P, cudaStream_t st);
+// flags[0] |= 1 malformed rowptr or unsorted list, 2 id out of range, 4 init row out of range, 8 a list covering
+// every candidate; keys[u] = num_other - length of list u (the longest list sorts first)
+int launch_fold_in_check(const int64_t* rowptr, const int32_t* ids, int64_t U, int64_t nnz, int32_t num_other,
+                         const int32_t* init_rows, int32_t num_self, int32_t* keys, int32_t* flags, cudaStream_t st);
 
 // ---- tc_dense.cu / tc_wgrad.cu / head.cu: tensor-core path of the train step ------------------------
 enum { TC_EPI_BIAS_RELU = 0, TC_EPI_MASK = 1, TC_EPI_STAGE = 2, TC_EPI_HEAD_DOT = 3 };

@@ -642,16 +642,33 @@ class NeuMFEngine(object):
         (user_mlp (U, d_u), user_gmf (U, mf_dim) or None, loss (U,): the mean BCE of each user's last step before its
         update, NaN for steps = 0 or an empty history).  Raises IndexError on an item or init user out of range and
         ValueError on a malformed CSR or a history that covers every item, before any launch."""
+        return self._fold_in("users", histories, steps, lr, negs, seed, init_users, optimizer, beta_1, beta_2)
+
+    def fold_in_items(self, raters, steps, lr, negs, seed=0, init_items=None, optimizer=None, beta_1=None, beta_2=None):
+        """Fold-in of M new items (mr_fold_in_items): fold_in with the sides swapped.  The user tables and the dense
+        block stay frozen and only each item's MLP and GMF rows are optimised against the item's raters and `negs`
+        sampled negative users per rater per step.  raters: (rowptr, users) with ascending lists, host or device, or a
+        list of user arrays (sorted and de-duplicated here).  init_items (M,): the row of this model an item starts
+        from, -1 = zero rows (default: all zero).  Returns device tensors (item_mlp (M, d_i), item_gmf (M, mf_dim) or
+        None, loss (M,)); item_view serves them.  Raises IndexError on a user or init item out of range and ValueError
+        on a malformed CSR or a rater list that covers every user, before any launch."""
+        return self._fold_in("items", raters, steps, lr, negs, seed, init_items, optimizer, beta_1, beta_2)
+
+    def _fold_in(self, side, lists, steps, lr, negs, seed, init_rows, optimizer, beta_1, beta_2):
+        items = side == "items"
         dev = self.device
-        rowptr, items = fold_in_histories(histories, self.num_items)
-        U, nnz = rowptr.size - 1, items.size
+        num_self, num_other = (self.num_items, self.num_users) if items else (self.num_users, self.num_items)
+        rowptr, ids = fold_in_histories(lists, num_other, side)
+        U, nnz = rowptr.size - 1, ids.size
         init = None
-        if init_users is not None:
-            init = np.asarray(init_users.cpu() if hasattr(init_users, "cpu") else init_users, np.int64).reshape(-1)
+        if init_rows is not None:
+            init = np.asarray(init_rows.cpu() if hasattr(init_rows, "cpu") else init_rows, np.int64).reshape(-1)
+            init_name, what, lists_name = ("init_items", "an item", "raters") if items else \
+                ("init_users", "a user", "histories")
             if init.size != U:
-                raise ValueError("init_users ({}) and histories ({}) differ in length".format(init.size, U))
-            if init.size and (init.min() < -1 or init.max() >= self.num_users):
-                raise IndexError("init_users: a user lies outside [-1, {})".format(self.num_users))
+                raise ValueError("{} ({}) and {} ({}) differ in length".format(init_name, init.size, lists_name, U))
+            if init.size and (init.min() < -1 or init.max() >= num_self):
+                raise IndexError("{}: {} lies outside [-1, {})".format(init_name, what, num_self))
         optimizer = self.optimizer if optimizer is None else optimizer
         if optimizer not in ("adam", "sgd"):
             raise ValueError("optimizer must be 'adam' or 'sgd', found {!r}".format(optimizer))
@@ -664,17 +681,19 @@ class NeuMFEngine(object):
         cfg.epsilon = ADAM_EPSILON
         cfg.seed = int(seed) & (2 ** 64 - 1)
         d_rowptr = torch.from_numpy(rowptr).to(dev)
-        d_items = torch.from_numpy(items if nnz else np.zeros(1, np.int32)).to(dev)
+        d_ids = torch.from_numpy(ids if nnz else np.zeros(1, np.int32)).to(dev)
         d_init = torch.from_numpy(init.astype(np.int32)).to(dev) if init is not None and U else None
         f32 = torch.float32
-        out_mlp = torch.empty((U, self.d_u), dtype=f32, device=dev)
+        out_mlp = torch.empty((U, self.d_i if items else self.d_u), dtype=f32, device=dev)
         out_gmf = torch.empty((U, self.mf_dim), dtype=f32, device=dev) if self.mf_dim else None
         loss = torch.empty(U, dtype=f32, device=dev)
-        nbytes = int(nat.lib.mr_fold_in_workspace_bytes(C.byref(self._model), U, nnz))
+        name = "mr_fold_in_items" if items else "mr_fold_in_users"
+        query = nat.lib.mr_fold_in_items_workspace_bytes if items else nat.lib.mr_fold_in_workspace_bytes
+        nbytes = int(query(C.byref(self._model), U, nnz))
         ws = self._workspace(max(nbytes, 256))
-        nat.check(nat.lib.mr_fold_in_users(C.byref(self._model), _ptr(d_rowptr), _ptr(d_items), U, nnz, _ptr(d_init),
-                                           C.byref(cfg), _ptr(out_mlp), _ptr(out_gmf), _ptr(loss), _ptr(ws), ws.numel(),
-                                           self._stream()), "mr_fold_in_users")
+        nat.check(getattr(nat.lib, name)(C.byref(self._model), _ptr(d_rowptr), _ptr(d_ids), U, nnz, _ptr(d_init),
+                                         C.byref(cfg), _ptr(out_mlp), _ptr(out_gmf), _ptr(loss), _ptr(ws), ws.numel(),
+                                         self._stream()), name)
         return out_mlp, out_gmf, loss
 
     def user_view(self, user_mlp, user_gmf=None):
@@ -683,6 +702,15 @@ class NeuMFEngine(object):
         engine show through).  Every scoring and evaluation call works on it with user id u = row u; training it,
         changing its weights or reading optimizer state raises."""
         return UserViewEngine(self, user_mlp, user_gmf)
+
+    def item_view(self, item_mlp, item_gmf=None):
+        """An engine whose catalogue is [this engine's items; the rows of item_mlp (M, d_i) / item_gmf (M, mf_dim)] --
+        typically fold_in_items' output -- with new item j at id num_items + j.  It shares this engine's user tables
+        and dense block by reference (later updates of this engine show through), but its item tables are a
+        concatenated COPY: later updates of this engine's item rows do not.  Every scoring and evaluation call works
+        on it, and so do fold_in (a new user's history may hold new items), user_view and item_view; training it,
+        changing its weights or reading optimizer state raises."""
+        return ItemViewEngine(self, item_mlp, item_gmf)
 
     def _ids_out_of_range(self, users, items):
         if users.numel() == 0:
@@ -740,52 +768,83 @@ class NeuMFEngine(object):
         return pos, sums.sum(dim=0), None, None
 
 
-class UserViewEngine(NeuMFEngine):
-    """NeuMFEngine.user_view: other user tables in front of a model's item tables and dense block.  Scoring only."""
+class _ScoringView(NeuMFEngine):
+    """An engine made of another engine's tables with one side replaced or extended: scoring and fold-in only."""
 
-    def __init__(self, base, user_mlp, user_gmf=None):
-        self.__dict__.update({k: v for k, v in base.__dict__.items() if k in _VIEW_SHARED})
+    def _view_rows(self, base, mlp, gmf, d, what, rows):
+        self.__dict__.update({k: v for k, v in base.__dict__.items() if k in _VIEW_DESC})
         f32 = torch.float32
-        user_mlp = user_mlp.to(self.device, f32).contiguous()
-        if user_mlp.dim() != 2 or user_mlp.shape[1] != self.d_u or user_mlp.shape[0] < 1:
-            raise ValueError("user_mlp must be (U >= 1, {}), got {}".format(self.d_u, tuple(user_mlp.shape)))
+        mlp = mlp.to(self.device, f32).contiguous()
+        if mlp.dim() != 2 or mlp.shape[1] != d or mlp.shape[0] < 1:
+            raise ValueError("{}_mlp must be ({} >= 1, {}), got {}".format(what, rows, d, tuple(mlp.shape)))
         if self.mf_dim:
-            if user_gmf is None:
-                raise ValueError("the model has a GMF branch: user_gmf (U, {}) is required".format(self.mf_dim))
-            user_gmf = user_gmf.to(self.device, f32).contiguous()
-            if tuple(user_gmf.shape) != (user_mlp.shape[0], self.mf_dim):
-                raise ValueError("user_gmf must be ({}, {}), got {}".format(user_mlp.shape[0], self.mf_dim,
-                                                                           tuple(user_gmf.shape)))
+            if gmf is None:
+                raise ValueError("the model has a GMF branch: {}_gmf ({}, {}) is required".format(what, rows, self.mf_dim))
+            gmf = gmf.to(self.device, f32).contiguous()
+            if tuple(gmf.shape) != (mlp.shape[0], self.mf_dim):
+                raise ValueError("{}_gmf must be ({}, {}), got {}".format(what, mlp.shape[0], self.mf_dim,
+                                                                         tuple(gmf.shape)))
         else:
-            user_gmf = None
-        self.num_users = int(user_mlp.shape[0])
-        self.user_mlp, self.user_gmf = user_mlp, user_gmf
+            gmf = None
+        return mlp, gmf
+
+    def _set_tables(self, base):
         self._tables = dict(base._tables)
-        self._tables[K_USER] = user_mlp
+        self._tables[K_USER], self._tables[K_ITEM] = self.user_mlp, self.item_mlp
         if self.mf_dim:
-            self._tables[K_GMF_USER] = user_gmf
+            self._tables[K_GMF_USER], self._tables[K_GMF_ITEM] = self.user_gmf, self.item_gmf
         self._ws = None
         self._model_struct()
 
     def _scoring_only(self, *args, **kwargs):
-        raise RuntimeError("a user view only scores: train, update or save the model it was made from")
+        raise RuntimeError("a {} view only scores: train, update or save the model it was made from".format(self._side))
 
     train_step = train_grads = apply = apply_region = finish_apply = apply_dense_only = _scoring_only
     set_weights = initialize = get_optimizer_state = set_optimizer_state = rebind_flat = _scoring_only
     gradient_tensors = gradient_parts = gradient_regions = _scoring_only
 
 
-# what a user view shares with its base engine (the item tables and dense block by reference, the description by value)
-_VIEW_SHARED = ("compute_path", "item_projection", "fused_train", "device", "num_items", "L", "l2", "mf_dim", "d_u", "d_i",
-                "optimizer", "lr", "beta_1", "beta_2", "table_mode", "iterations", "_dense_slices", "dense_count",
-                "item_mlp", "item_gmf", "dense")
+class UserViewEngine(_ScoringView):
+    """NeuMFEngine.user_view: other user tables in front of a model's item tables and dense block.  Scoring only."""
+    _side = "user"
+
+    def __init__(self, base, user_mlp, user_gmf=None):
+        self.user_mlp, self.user_gmf = self._view_rows(base, user_mlp, user_gmf, base.d_u, "user", "U")
+        self.num_users = int(self.user_mlp.shape[0])
+        self.num_items, self.item_mlp, self.item_gmf = base.num_items, base.item_mlp, base.item_gmf
+        self._set_tables(base)
 
 
-def fold_in_histories(histories, num_items):
-    """Histories of fold_in -> host (rowptr int64 (U + 1,), items int32).  (rowptr, items) with ascending lists (host or
-    device tensors or arrays) is checked as is; a list of item arrays is sorted and de-duplicated per user.  Raises
-    IndexError on an item outside [0, num_items) and ValueError on a malformed rowptr, a list that is not strictly
-    ascending or a list that covers every item."""
+class ItemViewEngine(_ScoringView):
+    """NeuMFEngine.item_view: a model's user tables and dense block in front of its item tables extended by new rows
+    (a concatenated copy).  Scoring and fold-in only."""
+    _side = "item"
+
+    def __init__(self, base, item_mlp, item_gmf=None):
+        new_mlp, new_gmf = self._view_rows(base, item_mlp, item_gmf, base.d_i, "item", "M")
+        self.num_users, self.user_mlp, self.user_gmf = base.num_users, base.user_mlp, base.user_gmf
+        self.num_items = base.num_items + int(new_mlp.shape[0])
+        self.item_mlp = torch.cat([base.item_mlp, new_mlp])
+        self.item_gmf = torch.cat([base.item_gmf, new_gmf]) if self.mf_dim else None
+        self._set_tables(base)
+
+
+# what a view takes from its base engine by value: the model description and the dense block (by reference)
+_VIEW_DESC = ("compute_path", "item_projection", "fused_train", "device", "L", "l2", "mf_dim", "d_u", "d_i",
+              "optimizer", "lr", "beta_1", "beta_2", "table_mode", "iterations", "_dense_slices", "dense_count", "dense")
+
+
+_LIST_WORDS = {"users": ("histories", "item", "user's items", "a history covers every item", "items"),
+               "items": ("raters", "user", "item's users", "a rater list covers every user", "users")}
+
+
+def fold_in_histories(histories, num_other, side="users"):
+    """Lists of fold_in (side "users": histories of items) or fold_in_items (side "items": rater lists of users) ->
+    host (rowptr int64 (U + 1,), ids int32).  (rowptr, ids) with ascending lists (host or device tensors or arrays) is
+    checked as is; a list of id arrays is sorted and de-duplicated per list.  num_other: the number of items (users)
+    the ids index.  Raises IndexError on an id outside [0, num_other) and ValueError on a malformed rowptr, a list that
+    is not strictly ascending or a list that covers every id."""
+    name, other, members, covers, ids_name = _LIST_WORDS[side]
     host = lambda x: np.asarray(x.cpu() if hasattr(x, "cpu") else x)
     if isinstance(histories, tuple) and len(histories) == 2:
         rowptr = host(histories[0]).astype(np.int64).reshape(-1)
@@ -796,16 +855,17 @@ def fold_in_histories(histories, num_items):
         rowptr[1:] = np.cumsum([p.size for p in parts])
         items = np.concatenate(parts) if parts else np.zeros(0, np.int64)
     if rowptr.size < 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
-        raise ValueError("histories: offsets must start at 0, never decrease and end at len(items) = {}".format(items.size))
-    if items.size and (items.min() < 0 or items.max() >= num_items):
-        raise IndexError("histories: an item lies outside [0, {})".format(num_items))
+        raise ValueError("{}: offsets must start at 0, never decrease and end at len({}) = {}".format(name, ids_name, items.size))
+    if items.size and (items.min() < 0 or items.max() >= num_other):
+        raise IndexError("{}: {} {} lies outside [0, {})".format(name, "an" if other == "item" else "a", other,
+                                                                 num_other))
     inner = np.ones(max(items.size - 1, 0), bool)  # pairs of neighbours inside one list
     starts = rowptr[1:-1]
     inner[starts[(starts > 0) & (starts < items.size)] - 1] = False
     if np.any((items[1:] <= items[:-1]) & inner):
-        raise ValueError("histories: every user's items must be strictly ascending")
-    if np.any(rowptr[1:] - rowptr[:-1] >= num_items):
-        raise ValueError("histories: a history covers every item, so there is no negative to draw")
+        raise ValueError("{}: every {} must be strictly ascending".format(name, members))
+    if np.any(rowptr[1:] - rowptr[:-1] >= num_other):
+        raise ValueError("{}: {}, so there is no negative to draw".format(name, covers))
     return rowptr, items.astype(np.int32)
 
 

@@ -114,6 +114,8 @@ SIGNATURES = {
                                 _vp]),
     "mr_fold_in_workspace_bytes": (_sz, [_PM, _i64, _i64]),
     "mr_fold_in_users": (C.c_int, [_PM, _vp, _vp, _i64, _i64, _vp, _PF, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "mr_fold_in_items_workspace_bytes": (_sz, [_PM, _i64, _i64]),
+    "mr_fold_in_items": (C.c_int, [_PM, _vp, _vp, _i64, _i64, _vp, _PF, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_sample_negatives": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _i64, _i64, _i32, _u64, _u64, _vp, _vp, _vp, _vp]),
     "mr_sort_workspace_bytes": (_sz, [_i64]),
     "mr_sort_pairs": (C.c_int, [_vp, _i64, _i32, _vp, _vp, _vp, _sz, _vp]),

@@ -55,6 +55,9 @@ EARLY_STOPPING_PATIENCE = 5  # model.py:324
 # 0.03-0.3 at 5-100 steps, and the mean loss still falls up to about 30 steps; lr 0.01 needs >= 20 steps, and the
 # training lr 0.001 reaches the plateau only at 100 steps (0.04 at 30).  30 steps at 0.05 sits inside the plateau on
 # both axes.
+# Item fold-in (MovierecModel.fold_in_items) uses the same defaults: on the planted-cluster grid with held-out items
+# (tools/fold_in_items_bench.py --quality, profiles/r07_fold_in_items_quality.json) recall@10 of the new items is flat
+# at 0.23-0.26 for lr 0.03-0.3 at 30 steps and falls with more steps; no other setting is better on both axes.
 FOLD_IN_STEPS = 30
 FOLD_IN_LR = 0.05
 
@@ -622,6 +625,22 @@ class MovierecModel(object):
                                      self._num_negs_per_pos if negs is None else negs, seed=seed, init_users=init_users)
         return FoldedModel(self, mlp, gmf, loss)
 
+    def fold_in_items(self, raters, steps=None, lr=None, negs=None, seed=0):
+        """Fold-in of items the model was not trained on, such as new releases: fold_in with the sides swapped.  The
+        user tables and the dense block stay frozen and only each new item's two embedding rows are optimised, on the
+        device, against the item's raters and sampled negative users.  raters: a list of user arrays (one per item,
+        any order) or a (rowptr, users) CSR of ascending lists.  steps / lr / negs default as in fold_in.  Returns an
+        ItemFoldedModel whose catalogue is the model's items followed by the new ones (new item j at id
+        num_items + j, listed in .new_item_ids): recommend_for_users, recommend_batch, recommend_for_histories, the
+        evaluate_* calls and fold_in work on it unchanged; .item_weights() gives the new rows and .loss each item's
+        last-step loss.  Raises IndexError on an out-of-range user and ValueError on a malformed CSR or a rater list
+        that covers every user."""
+        eng = self.model.engine
+        mlp, gmf, loss = eng.fold_in_items(raters, FOLD_IN_STEPS if steps is None else steps,
+                                           FOLD_IN_LR if lr is None else lr,
+                                           self._num_negs_per_pos if negs is None else negs, seed=seed)
+        return ItemFoldedModel(self, mlp, gmf, loss)
+
     def evaluate(self, users, items, k=None):
         """Full-sweep ranking evaluation (BASELINE config 4): one user id per group and
         (negs_eval+1) candidate items per user with the positive last.  Returns (hr, dcg)."""
@@ -752,6 +771,28 @@ class FoldedModel(MovierecModel):
         raise RuntimeError("a folded-in model only scores: train or save the model it was folded into")
 
     fit_generator = save = _no_training
+
+
+class ItemFoldedModel(MovierecModel):
+    """MovierecModel.fold_in_items's result: the model's users and dense block (shared) and its catalogue extended by
+    the new items (a copy of the item tables with the new rows appended).  Scoring, evaluation and user fold-in work as
+    on the model; training and saving raise."""
+
+    def __init__(self, base, item_mlp, item_gmf, loss):
+        self.__dict__.update(base.__dict__)
+        view = base.model.engine.item_view(item_mlp, item_gmf)
+        self.new_item_ids = np.arange(self._num_items, view.num_items, dtype=np.int32)
+        self._num_items = view.num_items
+        self.model = _FoldedNeuMF(self, view)
+        self.loss = loss.cpu().numpy()
+        self._new_rows = (item_mlp, item_gmf)
+
+    def item_weights(self):
+        """The new items' rows as NumPy: (item_mlp (M, L[0] - L[0]/2), item_gmf (M, mf_dim) or None)."""
+        mlp, gmf = self._new_rows
+        return mlp.cpu().numpy(), (gmf.cpu().numpy() if gmf is not None else None)
+
+    fit_generator = save = FoldedModel._no_training
 
 
 class _FoldedNeuMF(NeuMFModel):
