@@ -91,6 +91,9 @@ struct SideStream {
   cudaStream_t stream = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;
   cudaEvent_t fork2 = nullptr, join2 = nullptr;  // second excursion of a step: the user-side segmented reduction
+  // the train step's last reads of the user GMF table: the user-side reduction (side stream) and the level 0 of an
+  // item-side reduction that forms the GMF item gradient from it (caller's stream)
+  cudaEvent_t user_sums = nullptr, gmf_read = nullptr;
 };
 static thread_local SideStream g_side;
 
@@ -107,7 +110,9 @@ static SideStream* side_stream() {
         cudaEventCreateWithFlags(&s.fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&s.fork2, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&s.join2, cudaEventDisableTiming) != cudaSuccess) {
+        cudaEventCreateWithFlags(&s.join2, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&s.user_sums, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&s.gmf_read, cudaEventDisableTiming) != cudaSuccess) {
       cudaGetLastError();
       s = SideStream{};
       return nullptr;
@@ -566,6 +571,7 @@ static TrainWs carve_train(const MrModel& m, int64_t B, void* ws) {
   t.loss_partial = cv.take<float>(cap);
   t.probs = cv.take<float>(B);
   t.stage_u = cv.take<float>((size_t)B * (d_u + m.mf_dim));
+  // (the fused train kernel's rows are L1 = d_i wide; its dz per row follows them in the same block: TrainStep::plan)
   t.stage_i = cv.take<float>((size_t)B * (d_i + m.mf_dim));
   t.sorted_keys = cv.take<int32_t>(B);
   t.sorted_index = cv.take<int32_t>(B);
@@ -622,6 +628,9 @@ struct TrainPlan {
   bool grouped;         // one user per group: the user side runs once per group (promise checked on the device)
   bool proj, uproj;     // item / user half of the first layer once per item / user (item_proj_ok, user_proj_ok)
   int64_t n_user_rows;  // staged user-gradient rows: one per group or one per row
+  // TRAIN_TC_FUSED: dz of every row, behind the item staging rows, which then hold dZ1 only (L1 wide); the item-side
+  // reduction forms the GMF item gradient from it (GmfRows).  NULL on the other paths: they stage [dZ1 | d gmf_i].
+  float* dz_rows;
   // where the segmented reductions put the MLP part of their rows (dense table mode): the per-user / per-item sums
   // of dZ[1] (L1 wide) on a projected side, the gradient table otherwise
   float *user_sums, *item_sums;
@@ -669,6 +678,7 @@ TrainPlan TrainStep::plan() const {
     // the second layer's weight gradient and backward, the staged rows and their group sums never leave the SM.
     const bool fused = q.uproj && m.fused_train != MR_FUSED_OFF && fused_train_supported(m, group);
     q.path = fused ? TRAIN_TC_FUSED : TRAIN_TC;
+    if (fused) q.dz_rows = t.stage_i + (size_t)B * m.L[1];
     q.tc = carve_tc(m, true, B, t.tc_ws);
     if (!q.proj) q.tc.Pi = q.tc.Si = nullptr;
     if (!q.uproj) q.tc.Pu = q.tc.Su = nullptr;
@@ -748,16 +758,21 @@ int TrainStep::prologue() const {
 // chains are independent (disjoint buffers and columns of the dense partial rows): the user chain runs on the side
 // stream, so the latency-bound upper levels of one run under the other, and the user-side gradient tables (83 % of the table-gradient bytes at the ML-20M shape) are final while
 // the item side is still being reduced: a data-parallel caller starts their all-reduce on grads->user_tables_ready.
+// A data-parallel caller may also update the user tables from those events on, so they wait for the step's last read
+// of the user GMF table: with GmfRows (TRAIN_TC_FUSED) that is the item-side reduction's level 0.
 template <class UserTables, class ItemTables>
 int TrainStep::projected_backward(UserTables user_tables, ItemTables item_tables) const {
   if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join, 0));  // sorted keys, cleared sums and GMF tables
+  const bool gmf_formed = p.dz_rows != nullptr;
+  const GmfRows gmf{p.dz_rows, t.group_users, group, m.num_users, m.w_out, m.user_gmf};
+  const cudaEvent_t gmf_ready = (cudaEvent_t)grads.user_gmf_ready, tables_ready = (cudaEvent_t)grads.user_tables_ready;
   RowUpdate u{};
   u.mode = MR_TABLES_DENSE;
   u.optimizer = opt.optimizer;
   u.d0 = m.L[1];
   u.d1 = m.mf_dim;
+  cudaStream_t su = st;
   if (p.uproj) {
-    cudaStream_t su = st;
     if (side != nullptr) {
       MR_CUDA(cudaEventRecord(side->fork2, st));
       MR_CUDA(cudaStreamWaitEvent(side->stream, side->fork2, 0));
@@ -768,19 +783,37 @@ int TrainStep::projected_backward(UserTables user_tables, ItemTables item_tables
     u.g1 = grads.user_gmf;
     int rc = launch_segreduce(t.sorted_keys, t.sorted_index, p.n_user_rows, t.stage_u, u, t.seg_ws_u, t.seg_ws_u_bytes, su);
     if (rc != MR_OK) return rc;
-    // user_gmf: gradients final, table last read by the tower
-    if (grads.user_gmf_ready != nullptr) MR_CUDA(cudaEventRecord((cudaEvent_t)grads.user_gmf_ready, su));
-    rc = user_tables(su);  // the step's last read of the user table, so it goes before the event
-    if (rc != MR_OK) return rc;
-    if (grads.user_tables_ready != nullptr) MR_CUDA(cudaEventRecord((cudaEvent_t)grads.user_tables_ready, su));
-    if (side != nullptr) MR_CUDA(cudaEventRecord(side->join2, su));
+    // user_gmf: gradients final, table last read by the tower (or by the item side's level 0 below)
+    if (gmf_ready != nullptr) {
+      if (!gmf_formed) MR_CUDA(cudaEventRecord(gmf_ready, su));
+      else if (side != nullptr) MR_CUDA(cudaEventRecord(side->user_sums, su));
+    }
   }
   prof_mark(MR_PHASE_SEGREDUCE, st);
   u.num_rows = m.num_items;
   u.g0 = p.item_sums;
   u.g1 = grads.item_gmf;
-  int rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, u, t.seg_ws, t.seg_ws_bytes, st);
-  if (rc == MR_OK) rc = item_tables();
+  int rc = launch_segreduce(t.sorted_keys_i, t.sorted_index_i, B, t.stage_i, u, t.seg_ws, t.seg_ws_bytes, st,
+                            gmf_formed ? &gmf : nullptr, [&]() -> int {
+                              if (!gmf_formed) return MR_OK;
+                              if (gmf_ready != nullptr) {
+                                if (side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->user_sums, 0));
+                                MR_CUDA(cudaEventRecord(gmf_ready, st));
+                              }
+                              if (tables_ready != nullptr && side != nullptr) MR_CUDA(cudaEventRecord(side->gmf_read, st));
+                              return MR_OK;
+                            });
+  if (rc != MR_OK) return rc;
+  if (p.uproj) {
+    rc = user_tables(su);  // the step's last read of the user table, so it goes before the event
+    if (rc != MR_OK) return rc;
+    if (tables_ready != nullptr) {
+      if (gmf_formed && side != nullptr) MR_CUDA(cudaStreamWaitEvent(su, side->gmf_read, 0));
+      MR_CUDA(cudaEventRecord(tables_ready, su));
+    }
+    if (side != nullptr) MR_CUDA(cudaEventRecord(side->join2, su));
+  }
+  rc = item_tables();
   if (rc != MR_OK) return rc;
   if (p.uproj && side != nullptr) MR_CUDA(cudaStreamWaitEvent(st, side->join2, 0));
   return MR_OK;
@@ -1021,8 +1054,9 @@ int TrainStep::tower_tc() const {
     fa.inv_batch = inv_batch;
     fa.probs = t.probs;
     fa.stage_i = t.stage_i;
+    fa.dz_rows = p.dz_rows;
     fa.stage_u = t.stage_u;
-    fa.si = d_i + f;
+    fa.si = m.L[1];  // dZ1 only (p.dz_rows)
     fa.su = d_u + f;
     fa.partial = t.dense_partial;
     fa.partial_stride = t.dense_stride;

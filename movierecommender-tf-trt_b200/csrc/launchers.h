@@ -1,6 +1,8 @@
 // Host-side launch functions shared between the .cu files and the C-ABI layer (api.cu).
 #pragma once
 
+#include <functional>
+
 #include "common.cuh"
 
 namespace mr {
@@ -57,9 +59,20 @@ struct RowUpdate {       // what to do with each reduced row gradient
   float *p0, *m0, *v0, *g0;  // table / Adam state / dense gradient table (mode DENSE writes g)
   float *p1, *m1, *v1, *g1;
 };
+// The GMF columns [d0, d0 + d1) of the fused train kernel's item rows, formed at level 0 instead of staged: entry r
+// contributes (dz[r] * w[c]) * user_gmf[group_users[r / group]][c]; the staged rows are then d0 floats apart.
+struct GmfRows {
+  const float* dz;             // [rows]
+  const int32_t* group_users;  // [rows / group]: the user of each group
+  int32_t group, num_users;
+  const float* w;              // [d1]: w_out[:f]
+  const float* user_gmf;       // [num_users x d1]
+};
 size_t segreduce_workspace_bytes(int64_t n, int ld);
+// after_level0 runs once level 0 -- the last reader of `staged` and of gmf->user_gmf -- has been enqueued on st.
 int launch_segreduce(const int32_t* sorted_keys, const int32_t* sorted_index, int64_t n, const float* staged,
-                     const RowUpdate& u, void* ws, size_t ws_bytes, cudaStream_t st);
+                     const RowUpdate& u, void* ws, size_t ws_bytes, cudaStream_t st, const GmfRows* gmf = nullptr,
+                     const std::function<int()>& after_level0 = {});
 
 // ---- optimizer.cu ----------------------------------------------------------------------------
 constexpr int kMaxOptRegions = 5;
@@ -400,7 +413,8 @@ struct FusedTrainArgs {
   const float* b_out;
   float inv_batch;
   float* probs;
-  float* stage_i;         // [rows x si]: dZ1 | d gmf_i
+  float* stage_i;         // [rows x si]: dZ1 (the GMF item gradient is formed from dz_rows by the reduction)
+  float* dz_rows;         // [rows]: dz of every row
   float* stage_u;         // [rows / group x su]: group sums of dZ1 | d gmf_u
   int32_t si, su;
   float* partial;         // dense-gradient partial rows (one per CTA, zeroed by the caller), stride partial_stride

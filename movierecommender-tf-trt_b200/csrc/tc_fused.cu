@@ -6,10 +6,12 @@
 //   z  = w_out . [gmf_u * gmf_i | H2] + b_out, p, BCE    epilogue, thread = row         (model.py:184-188, 213-215)
 //   dZ2 = dz * w_out[f:] * (H2 > 0)                      written back as an MMA operand
 //   dW2 += H1^T . dZ2 ,  dZ1 = (dZ2 . W2^T) * (H1 > 0)   tcgen05 from the SAME shared-memory tiles
-//   staged rows [dZ1 | d gmf_i] per row and [sum_group dZ1 | d gmf_u] per group, d w_out, d b_out, d b2, loss
+//   staged rows dZ1 and dz per row and [sum_group dZ1 | d gmf_u] per group, d w_out, d b_out, d b2, loss
 //
-// so that H1, H2, dZ2 never exist in HBM; the per-row HBM traffic is the two staged gradient rows (which the sorted
-// segmented reduction needs) plus the L2-resident projection / GMF rows.
+// so that H1, H2, dZ2 never exist in HBM; the per-row HBM traffic is the staged gradient rows (which the sorted
+// segmented reduction needs) plus the L2-resident projection / GMF rows.  The GMF item gradient of a row,
+// (dz * w_out[:f]) * gmf_u, is not staged: the item-side reduction forms it from dz and the user's GMF row
+// (segreduce.cu), which saves 256 B written and 256 B read per row.
 //
 // fp32 accuracy on the tensor cores: every operand is split into THREE bf16 parts (round to nearest, x = b1 + b2 + b3
 // up to 2^-24 |x|) and a product keeps the six part products down to 2^-16: b1.b1' + b1.b2' + b2.b1' + b1.b3' + b3.b1'
@@ -124,7 +126,8 @@ struct FusedParams {
   const float* b_out;
   float inv_batch;
   float* probs;           // [rows]
-  float* stage_i;         // [rows x si]: columns [0, 128) dZ1, [128, 192) d gmf_i
+  float* stage_i;         // [rows x si]: columns [0, 128) dZ1
+  float* dz_rows;         // [rows]
   float* stage_u;         // [rows / GROUP x su]: columns [0, 128) group sums of dZ1, [128, 192) d gmf_u
   int32_t si, su;
   float* partial;         // this launch's dense-gradient partial rows: row = CTA, stride partial_stride
@@ -371,7 +374,8 @@ __global__ void __launch_bounds__(kThreads, 1) neumf_fused_train_kernel(const Fu
       if (lane == 0) tc::mbar_arrive(&gmf_ready);
       FZ_T(5)
 
-      // ---- GMF branch, part 2 (after the epilogue has dz): row gradients, straight to the staged rows
+      // ---- GMF branch, part 2 (after the epilogue has dz): dz per row and the group's d gmf_u, straight to the staged
+      // rows, and the d w_out[:f] partials
       tc::mbar_wait(&dz2_full, (uint32_t)(it & 1));
       FZ_T(6)
 #pragma unroll
@@ -386,6 +390,8 @@ __global__ void __launch_bounds__(kThreads, 1) neumf_fused_train_kernel(const Fu
 #pragma unroll
         for (int j = 0; j < GROUP; ++j) {
           const float dz = dz_s[sl0 + j];
+          // (here rather than in epilogue 1, where the store made ptxas spill more of the kernel)
+          if (gvalid && pc == 0) p.dz_rows[grow0 + j] = dz;
           const float4 g = make_float4(dz * wg4.x, dz * wg4.y, dz * wg4.z, dz * wg4.w);
           const float4 u4 = gu[s], i4 = gi[s][j];
           accg.x = fmaf(dz, u4.x * i4.x, accg.x);
@@ -396,9 +402,6 @@ __global__ void __launch_bounds__(kThreads, 1) neumf_fused_train_kernel(const Fu
           ga.y = fmaf(g.y, i4.y, ga.y);
           ga.z = fmaf(g.z, i4.z, ga.z);
           ga.w = fmaf(g.w, i4.w, ga.w);
-          if (gvalid)
-            *reinterpret_cast<float4*>(p.stage_i + (size_t)(grow0 + j) * p.si + kD1 + 4 * pc) =
-                make_float4(g.x * u4.x, g.y * u4.y, g.z * u4.z, g.w * u4.w);
         }
         if (gvalid) *reinterpret_cast<float4*>(p.stage_u + (size_t)(grow0 / GROUP) * p.su + kD1 + 4 * pc) = ga;
       }
@@ -783,6 +786,7 @@ int launch_fused_train(const FusedTrainArgs& a, cudaStream_t st, int* grid_out) 
   p.inv_batch = a.inv_batch;
   p.probs = a.probs;
   p.stage_i = a.stage_i;
+  p.dz_rows = a.dz_rows;
   p.stage_u = a.stage_u;
   p.si = a.si;
   p.su = a.su;
