@@ -275,6 +275,46 @@ int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, 
                          const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks /*[host]*/, int32_t n_ks,
                          int32_t* tpos, float* sums, void* ws, size_t ws_bytes, void* stream);
 
+/* Audiences: the k best users for each item (who to show or notify about a new release), the column-wise counterpart
+ * of mr_topk_scores.  scores is U x M row-major: row u is pool user users[u] (users NULL: user u), column j an item.
+ * users (U, may be NULL) must be strictly ascending (unchecked: otherwise the results are unspecified, but no kernel
+ * leaves its arrays).  Candidates of column j: the pool users with an id >= 0 minus the exclusion list of row
+ * r = excl_ids ? excl_ids[j] : j, i.e. excl_users[excl_rowptr[r] .. excl_rowptr[r+1]) (ascending user ids, the
+ * transpose of mr_build_user_csr's lists); rows r outside [0, excl_rows) and excl_rowptr == NULL mean "nothing
+ * excluded".  Order: descending score, NaN as -inf, -0 == +0, the LOWER USER ID first among ties.  The keys are
+ * distinct, so the result of an item does not depend on chunking, launch order, the other columns of the call or how
+ * the pool is split.  top_users / top_scores (M x k, each may be NULL): the k best candidates in order, -1 / NaN beyond
+ * the number of candidates.  targets (M, may be NULL): one held-out user per column, never excluded; pos[j] = its
+ * 0-based place among the column's candidates when that place is < k, else k (also for a target outside the pool).
+ * The place is clipped at k because an exact place beyond k would need the target's score before the sweep reaches
+ * the target's rows; HR@k and NDCG@k do not need it.  sums = {hit_sum, dcg_sum} over the M columns
+ * (hit = pos < k, dcg = ln2/ln(pos+2)*hit).  pos and sums need targets.  1 <= k <= MR_MAX_TOPK, U <= INT32_MAX.
+ * Columns are selected in chunks of the users of one mr_catalogue_topk chunk of M items (C = min(U, about 2^22 / M,
+ * 16384) rows); per item a running top-k is carried across chunks as S <= 32 lists (S > 1 only for narrow calls:
+ * S = min(32, max(1, 1024 / ceil(M / 32)), ceil(C / 32))).  Workspace: 12 k S bytes per item (keys and raw scores)
+ * + 4 bytes per item, plus alignment: 3.2 MB at M = 26,744, k = 10 (S = 1); 82 MB at k = 256.  Deterministic; no
+ * host synchronisation, no read-back. */
+size_t mr_audience_scores_workspace_bytes(int64_t U, int32_t M, int32_t k);
+int mr_audience_scores(const float* scores, int64_t U, int32_t M, int32_t k, const int32_t* users,
+                       const int32_t* excl_ids, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
+                       const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
+                       void* ws, size_t ws_bytes, void* stream);
+/* The same on the model's probabilities of every (pool user, items[j]) pair: the audience of each item over the whole
+ * user base (users NULL, then U must be num_users) or over a strictly ascending pool users[0, U).  Pool users outside
+ * [0, num_users) are never candidates.  Exclusion lists are indexed by item id (typically the item's training
+ * raters).  An out-of-range item gets -1 / NaN in every slot and pos = k.  scores (U x M, may be NULL) receives the
+ * probabilities (the column of an out-of-range item is unspecified).  The pairs are scored by mr_catalogue_topk's
+ * sweep with the item list tiled over each chunk's users (chunk row r pairs user r / M with items[r % M]): the
+ * tower, the item projection over the whole table and the head are the ones mr_catalogue_topk takes for the model,
+ * so a pair's probability is bit-identical to the one mr_catalogue_topk gives it, whichever items and pool the call
+ * has.  Workspace: mr_audience_scores' plus one sweep chunk of C x M rows (about 8 bytes per row plus the scoring).
+ * No host synchronisation, no read-back. */
+size_t mr_catalogue_audience_workspace_bytes(const MrModel* model, int64_t U, int32_t M, int32_t k);
+int mr_catalogue_audience(const MrModel* model, const int32_t* items, int32_t M, int32_t k, const int32_t* users,
+                          int64_t U, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
+                          const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
+                          float* scores, void* ws, size_t ws_bytes, void* stream);
+
 /* Top-k of ragged lists of caller-supplied scores: list u is scores[rowptr[u] .. rowptr[u+1]) (device rowptr, U + 1
  * int64, rowptr[0] = 0, non-decreasing, rowptr[U] = nnz; U and nnz <= INT32_MAX, no rows when U = 0).  Order: the
  * RankLayer order (descending score, NaN as -inf, -0 == +0, the EARLIER position in the list first among ties), so pos

@@ -1383,15 +1383,19 @@ static int eval_prepare(const MrModel& m, const EvalPlan& p, const EvalWs& w, co
 // ---- catalogue calls: every user against every item, in chunks of whole users --------------------------------
 static int64_t clamp_users(int64_t U, int64_t C) { return U < 1 ? 1 : (U < C ? U : C); }
 
-static EvalPlan catalogue_plan(const MrModel& m, int64_t C) {
-  return eval_plan(m, SCORE_CATALOGUE, C, m.num_items, C * m.num_items);
+// Chunks of C users x M items (M = num_items: the catalogue).  The tower choices judge the catalogue's full chunk
+// whatever M is (eval_plan), so an audience scores a pair with the launch sequence mr_catalogue_topk takes.
+static EvalPlan catalogue_plan(const MrModel& m, int64_t C, int32_t M) {
+  return eval_plan(m, SCORE_CATALOGUE, C, M, C * M);
 }
 
-// The sweep's workspace (chunks of C users): the item of every row of a chunk, the chunk's probabilities, the scoring.
-static size_t catalogue_sweep_bytes(const MrModel& m, int64_t C) {
-  const size_t rows = (size_t)C * m.num_items;
+// The sweep's workspace (chunks of C users x M items): the item of every row of a chunk, the chunk's probabilities, the
+// chunk's user ids when the caller gives none (own_users), the scoring.
+static size_t catalogue_sweep_bytes(const MrModel& m, int64_t C, int32_t M, bool own_users = false) {
+  const size_t rows = (size_t)C * M;
   return align_up(rows * sizeof(int32_t), 256) + align_up(rows * sizeof(float), 256) +
-         eval_carve(m, catalogue_plan(m, C), nullptr).total;
+         (own_users ? align_up((size_t)C * sizeof(int32_t), 256) : 0) +
+         eval_carve(m, catalogue_plan(m, C, M), nullptr).total;
 }
 
 static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const int64_t* excl_rowptr,
@@ -1404,39 +1408,46 @@ static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const 
 }
 
 // The chunk loop of the catalogue calls: per chunk of C users, the probabilities of every (user, item) pair through the
-// plan's tower, then select(u0, users in the chunk, probabilities) under MR_PHASE_RANK.  The probabilities go to
-// scores + u0 * N when scores is given, else to the sweep's buffer (C x N).  ws: catalogue_sweep_bytes(m, C) bytes.
-// mr_catalogue_topk and mr_catalogue_targets both score through here, so a pair's probability is the same in both by
-// construction.
+// plan's tower, then select(u0, users in the chunk, probabilities) under MR_PHASE_RANK.  The items are the catalogue,
+// or with `items` the list items[0, M) (chunk row r pairs user r / M with items[r % M]; the item half of the first
+// layer is still projected once over the whole table).  users == NULL: user u is id u.  The probabilities go to
+// scores + u0 * N (N = the items per user) when scores is given, else to the sweep's buffer (C x N).
+// ws: catalogue_sweep_bytes(m, C, N, users == NULL) bytes.  mr_catalogue_topk, mr_catalogue_targets and
+// mr_catalogue_audience all score through here, so a pair's probability is the same in all of them by construction.
 template <class Select>
 static int catalogue_sweep(const MrModel& m, const int32_t* users, int64_t U, int64_t C, float* scores, void* ws,
-                           cudaStream_t st, Select select) {
-  const int32_t N = m.num_items;
-  const EvalPlan p = catalogue_plan(m, C);
+                           cudaStream_t st, Select select, const int32_t* items = nullptr, int32_t M = 0) {
+  const int32_t N = items != nullptr ? M : m.num_items;
+  const EvalPlan p = catalogue_plan(m, C, N);
   Carver cv(ws);
   int32_t* iota = cv.take<int32_t>((size_t)C * N);
   float* probs_buf = cv.take<float>((size_t)C * N);
+  int32_t* own_users = users == nullptr ? cv.take<int32_t>((size_t)C) : nullptr;
   const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
   prof_mark(MR_PHASE_MISC, st);
-  int rc = launch_tile_iota(iota, C * N, N, st);
+  int rc = items != nullptr ? launch_tile_list(iota, C * N, items, N, st) : launch_tile_iota(iota, C * N, N, st);
   if (rc == MR_OK) rc = eval_prepare(m, p, w, users, st);
   for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
     const int64_t c = U - u0 < C ? U - u0 : C;
     const int64_t rows = c * N;
     float* out = scores != nullptr ? scores + u0 * N : probs_buf;
+    const int32_t* cu = users != nullptr ? users + u0 : own_users;
+    if (own_users != nullptr) rc = launch_iota(own_users, c, u0, st);
+    if (rc != MR_OK) break;
     if (p.tower == EVAL_TC) {
       // each chunk starts at row 0 of its own users: one group = one user, Zu once per user
       prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-      rc = tc_forward_rows(m, w.t, users + u0, iota, 1, 0, rows, st, N, true, p.head_dot);
+      rc = tc_forward_rows(m, w.t, cu, iota, 1, 0, rows, st, N, true, p.head_dot);
       if (rc == MR_OK) {
         prof_mark(MR_PHASE_HEAD, st);
-        rc = launch_catalogue_head(m, w.t.H[m.n_layers - 1], users + u0, rows, N, out, st);
+        rc = launch_catalogue_head(m, w.t.H[m.n_layers - 1], cu, rows, N, out, st, nullptr,
+                                   items != nullptr ? iota : nullptr);
       }
     } else if (p.tower == EVAL_SMALL) {
       prof_mark(MR_PHASE_FUSED_TILE, st);
-      rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, users + u0, iota, rows, N, out, st);
+      rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, cu, iota, rows, N, out, st);
     } else {
-      rc = mr_neumf_forward(&m, users + u0, iota, rows, N, nullptr, out, nullptr, nullptr, w.fwd, w.fwd_bytes, st);
+      rc = mr_neumf_forward(&m, cu, iota, rows, N, nullptr, out, nullptr, nullptr, w.fwd, w.fwd_bytes, st);
     }
     if (rc != MR_OK) break;
     prof_mark(MR_PHASE_RANK, st);
@@ -1819,7 +1830,7 @@ size_t mr_catalogue_topk_workspace_bytes(const MrModel* model, int64_t U, int32_
     return 0;
   const MrModel& m = *model;
   const int64_t C = clamp_users(U, catalogue_chunk_users(m.num_items));
-  return align_up(topk_workspace_bytes(C, m.num_items, k), 256) + catalogue_sweep_bytes(m, C) + 512;
+  return align_up(topk_workspace_bytes(C, m.num_items, k), 256) + catalogue_sweep_bytes(m, C, m.num_items) + 512;
 }
 
 int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int32_t k, int32_t excl_rows,
@@ -1924,7 +1935,8 @@ size_t mr_catalogue_targets_workspace_bytes(const MrModel* model, int64_t U, int
   const MrModel& m = *model;
   const size_t sel = mr_targets_scores_workspace_bytes(U, m.num_items, nnz_t);
   if (sel == 0) return 0;
-  return align_up(sel, 256) + catalogue_sweep_bytes(m, clamp_users(U, catalogue_chunk_users(m.num_items))) + 512;
+  return align_up(sel, 256) + catalogue_sweep_bytes(m, clamp_users(U, catalogue_chunk_users(m.num_items)), m.num_items) +
+         512;
 }
 
 int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, int32_t excl_rows,
@@ -1975,6 +1987,120 @@ int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, 
   if (rc == MR_OK) {
     prof_mark(MR_PHASE_RANK, st);
     rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
+  }
+  prof_mark(-1, st);
+  return rc;
+}
+
+static int audience_check(int64_t U, int32_t M, int32_t k, int32_t excl_rows, const int64_t* excl_rowptr,
+                          const int32_t* excl_users, const int32_t* targets, const int32_t* pos, const float* sums) {
+  MR_REQUIRE(U >= 0 && U <= INT32_MAX && M >= 0, "audience: bad U=%lld M=%d", (long long)U, M);
+  MR_REQUIRE(k >= 1 && k <= MR_MAX_TOPK, "audience: k=%d out of [1,%d]", k, MR_MAX_TOPK);
+  MR_REQUIRE(excl_rows >= 0 && (excl_rowptr == nullptr || excl_users != nullptr), "audience: bad exclusion lists");
+  MR_REQUIRE(targets != nullptr || (pos == nullptr && sums == nullptr), "audience: pos / sums need targets");
+  return MR_OK;
+}
+
+// The selection's workspace for chunks of C users: the running lists of every item.
+static size_t audience_select_bytes(int64_t C, int32_t M, int32_t k) { return carve_audience(nullptr, C, M, k).total; }
+
+size_t mr_audience_scores_workspace_bytes(int64_t U, int32_t M, int32_t k) {
+  if (U < 0 || U > INT32_MAX || M < 0 || k < 1 || k > MR_MAX_TOPK) return 0;
+  return audience_select_bytes(clamp_users(U, catalogue_chunk_users(M)), M, k) + 256;
+}
+
+int mr_audience_scores(const float* scores, int64_t U, int32_t M, int32_t k, const int32_t* users,
+                       const int32_t* excl_ids, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
+                       const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
+                       void* ws, size_t ws_bytes, void* stream) {
+  int rc = audience_check(U, M, k, excl_rows, excl_rowptr, excl_users, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  MR_REQUIRE((U == 0 || M == 0 || scores != nullptr) && ws != nullptr, "audience_scores: scores / ws is NULL");
+  if (ws_bytes < mr_audience_scores_workspace_bytes(U, M, k)) {
+    set_error("audience_scores workspace too small: %zu < %zu", ws_bytes, mr_audience_scores_workspace_bytes(U, M, k));
+    return MR_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
+  const AudienceWs w = carve_audience(ws, C, M, k);
+  AudienceArgs a{};
+  a.M = M;
+  a.k = k;
+  a.users = users;
+  a.num_users = INT32_MAX;  // no model: every id >= 0 is a user
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_users = excl_users;
+  a.targets = targets;
+  prof_mark(MR_PHASE_RANK, st);
+  if (M > 0) rc = launch_audience_init(a, w, st);
+  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
+    a.u0 = u0;
+    a.U = U - u0 < C ? U - u0 : C;
+    a.scores = scores + u0 * M;
+    rc = launch_audience_chunk(a, w, st);
+  }
+  if (rc == MR_OK) rc = launch_audience_final(a, w, nullptr, 0, top_users, top_scores, pos, sums, st);
+  prof_mark(-1, st);
+  return rc;
+}
+
+size_t mr_catalogue_audience_workspace_bytes(const MrModel* model, int64_t U, int32_t M, int32_t k) {
+  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
+      model->num_users < 1 || U < 0 || U > INT32_MAX || M < 0 || k < 1 || k > MR_MAX_TOPK)
+    return 0;
+  const MrModel& m = *model;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
+  return align_up(audience_select_bytes(C, M, k), 256) + catalogue_sweep_bytes(m, C, M < 1 ? 1 : M, true) + 512;
+}
+
+int mr_catalogue_audience(const MrModel* model, const int32_t* items, int32_t M, int32_t k, const int32_t* users,
+                          int64_t U, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
+                          const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
+                          float* scores, void* ws, size_t ws_bytes, void* stream) {
+  int rc = check_model(model);
+  if (rc != MR_OK) return rc;
+  const MrModel& m = *model;
+  rc = audience_check(U, M, k, excl_rows, excl_rowptr, excl_users, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  MR_REQUIRE(users != nullptr || U == m.num_users, "catalogue_audience: without a pool U must be num_users (%d), got %lld",
+             m.num_users, (long long)U);
+  MR_REQUIRE((M == 0 || items != nullptr) && ws != nullptr, "catalogue_audience: items / ws is NULL");
+  if (ws_bytes < mr_catalogue_audience_workspace_bytes(model, U, M, k)) {
+    set_error("catalogue_audience workspace too small: %zu < %zu", ws_bytes,
+              mr_catalogue_audience_workspace_bytes(model, U, M, k));
+    return MR_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
+  Carver cv(ws);
+  const AudienceWs w = carve_audience(cv.take<char>(audience_select_bytes(C, M, k)), C, M, k);
+  AudienceArgs a{};
+  a.M = M;
+  a.k = k;
+  a.users = users;
+  a.num_users = m.num_users;
+  a.excl_ids = items;  // exclusion lists are indexed by item id
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_users = excl_users;
+  a.targets = targets;
+  if (M > 0) {
+    rc = launch_audience_init(a, w, st);
+    if (rc == MR_OK)
+      rc = catalogue_sweep(m, users, U, C, scores, static_cast<char*>(ws) + cv.off, st,
+                           [&](int64_t u0, int64_t c, const float* out) {
+                             a.u0 = u0;
+                             a.U = c;
+                             a.scores = out;
+                             return launch_audience_chunk(a, w, st);
+                           },
+                           items, M);
+  }
+  if (rc == MR_OK) {
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_audience_final(a, w, items, m.num_items, top_users, top_scores, pos, sums, st);
   }
   prof_mark(-1, st);
   return rc;

@@ -680,9 +680,12 @@ __global__ void __launch_bounds__(kHeadThreads) head_rank_warp_kernel(const Head
 // user against the whole catalogue per `group` rows).  Row-parallel -- a group here is tens of thousands of rows, far
 // beyond the warp-per-group kernel's shared-memory slice -- with the per-row arithmetic of head_rank_warp_kernel
 // (gmf_head_prob).  Four rows per warp step, KS steps in flight.
-// RAGGED (candidate lists): row r is global row row0 + r, pairing users[seg[row0 + r]] with items[row0 + r]; h_dot is
-// launch-local; an out-of-range user, item or list index gives NaN.
-template <int NV, bool RAGGED>
+// HEAD_RAGGED (candidate lists): row r is global row row0 + r, pairing users[seg[row0 + r]] with items[row0 + r]; h_dot
+// is launch-local; an out-of-range user, item or list index gives NaN.
+// HEAD_TILED (an item list tiled over the users: audiences): row r pairs users[r / group] with items[r]; an
+// out-of-range user or item gives NaN.
+enum { HEAD_CATALOGUE = 0, HEAD_RAGGED = 1, HEAD_TILED = 2 };
+template <int NV, int MODE>
 __global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrModel m, const float* __restrict__ h_dot,
                                                                       const int32_t* __restrict__ users, int64_t rows,
                                                                       int group, float* __restrict__ probs,
@@ -707,10 +710,15 @@ __global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrMo
       int64_t row = r0 + 4 * k + quad;
       if (row >= rows) row = rows - 1;  // dead slots re-read the last row
       int u, it;
-      if (RAGGED) {
+      if (MODE == HEAD_RAGGED) {
         const int sg = __ldg(seg + row0 + row);
         u = (unsigned)sg < (uint64_t)num_lists ? __ldg(users + sg) : -1;
         it = __ldg(items + row0 + row);
+        bad[k] = (unsigned)u >= (unsigned)m.num_users || (unsigned)it >= (unsigned)m.num_items;
+        if (bad[k]) u = it = 0;
+      } else if (MODE == HEAD_TILED) {
+        u = __ldg(users + row / group);
+        it = __ldg(items + row);
         bad[k] = (unsigned)u >= (unsigned)m.num_users || (unsigned)it >= (unsigned)m.num_items;
         if (bad[k]) u = it = 0;
       } else {
@@ -732,7 +740,7 @@ __global__ void __launch_bounds__(kHeadThreads) catalogue_head_kernel(const MrMo
     for (int k = 0; k < KS; ++k) {
       const int64_t row = r0 + 4 * k + quad;
       const float pr = gmf_head_prob<NV>(wu[k], gi[k], z[k], b_out, bad[k]);
-      if (sub == 0 && row < rows) probs[(RAGGED ? row0 : 0) + row] = pr;
+      if (sub == 0 && row < rows) probs[(MODE == HEAD_RAGGED ? row0 : 0) + row] = pr;
     }
   }
 }
@@ -878,17 +886,19 @@ int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* u
   const int64_t want = (rows + 4 * (kHeadThreads / 32) - 1) / (4 * (kHeadThreads / 32));
   const int64_t cap = (int64_t)sm_count() * 8;
   const unsigned grid = (unsigned)(want < cap ? want : cap);
-#define MR_CATALOGUE_HEAD(RAGGED_)                                                                                  \
-  if (m.mf_dim == 32)                                                                                              \
-    catalogue_head_kernel<1, RAGGED_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
-                                                                     row0, num_lists);                             \
-  else if (m.mf_dim == 64)                                                                                         \
-    catalogue_head_kernel<2, RAGGED_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
-                                                                     row0, num_lists);                             \
-  else                                                                                                             \
-    catalogue_head_kernel<4, RAGGED_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
-                                                                     row0, num_lists);
-  if (seg == nullptr) { MR_CATALOGUE_HEAD(false) } else { MR_CATALOGUE_HEAD(true) }
+#define MR_CATALOGUE_HEAD(MODE_)                                                                                  \
+  if (m.mf_dim == 32)                                                                                            \
+    catalogue_head_kernel<1, MODE_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
+                                                                   row0, num_lists);                             \
+  else if (m.mf_dim == 64)                                                                                       \
+    catalogue_head_kernel<2, MODE_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
+                                                                   row0, num_lists);                             \
+  else                                                                                                           \
+    catalogue_head_kernel<4, MODE_><<<grid, kHeadThreads, 0, st>>>(m, h_dot, users, rows, group, probs, seg, items, \
+                                                                   row0, num_lists);
+  if (seg != nullptr) { MR_CATALOGUE_HEAD(HEAD_RAGGED) }
+  else if (items != nullptr) { MR_CATALOGUE_HEAD(HEAD_TILED) }
+  else { MR_CATALOGUE_HEAD(HEAD_CATALOGUE) }
 #undef MR_CATALOGUE_HEAD
   MR_LAUNCH_CHECK("catalogue_head_kernel");
   return MR_OK;

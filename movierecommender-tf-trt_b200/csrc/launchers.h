@@ -143,6 +143,40 @@ int launch_topk_lists(const TopkListsArgs& a, float* sums, void* ws, cudaStream_
 int launch_list_rows(const int64_t* rowptr, int64_t U, int64_t nnz, const int32_t* users, int32_t* seg, cudaStream_t st);
 // out[r] = r % N for r < rows
 int launch_tile_iota(int32_t* out, int64_t rows, int32_t N, cudaStream_t st);
+// out[r] = items[r % M] for r < rows
+int launch_tile_list(int32_t* out, int64_t rows, const int32_t* items, int32_t M, cudaStream_t st);
+// out[r] = first + r for r < n
+int launch_iota(int32_t* out, int64_t n, int64_t first, cudaStream_t st);
+// Audiences: per item column j of chunks of pool users x M items, the k best candidate users in topk_key(p, user id)
+// order, carried across chunks in the workspace.  Candidates of column j: the chunk's users in [0, num_users) minus
+// the exclusion list of column j, plus targets[j] (never excluded).
+struct AudienceArgs {
+  const float* scores;      // the chunk: U x M row-major, row 0 = pool row u0
+  int64_t U, u0;
+  int32_t M, k;
+  const int32_t* users;     // pool user of pool row r (strictly ascending; NULL: r)
+  int32_t num_users;
+  const int32_t* excl_ids;  // exclusion list of column j = excl_ids[j] (NULL: j); lists outside [0, excl_rows) are empty
+  int32_t excl_rows;
+  const int64_t* excl_rowptr;
+  const int32_t* excl_users;
+  const int32_t* targets;   // (M) or NULL
+};
+struct AudienceWs {
+  unsigned long long* keys;  // M x S x k, ascending per list, kNoKey-padded
+  float* scores;             // the raw score of every key
+  int32_t* pos;              // M: positions when the caller wants sums only
+  int S;                     // lists per item (row splits of a chunk)
+  size_t total;
+};
+// The running state of a call whose chunks have at most C users (ws = NULL: sizes only).
+AudienceWs carve_audience(void* ws, int64_t C, int32_t M, int32_t k);
+int launch_audience_init(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st);
+int launch_audience_chunk(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st);
+// top_users / top_scores (M x k), pos (M; the target's slot, k when absent); items (may be NULL): a column whose
+// items[j] lies outside [0, num_items) gets -1 / NaN and pos = k.  sums (needs targets) = {hit_sum, dcg_sum} at k.
+int launch_audience_final(const AudienceArgs& a, const AudienceWs& w, const int32_t* items, int32_t num_items,
+                          int32_t* top_users, float* top_scores, int32_t* pos, float* sums, cudaStream_t st);
 // Positions of many targets per row: row u's targets are tgt_items[tgt_rowptr[u] .. tgt_rowptr[u+1]) (segments clamped
 // to [0, nnz_t)); candidates, order and exclusion lists as TopkArgs, a target never excluded.
 struct TargetsArgs {
@@ -317,7 +351,8 @@ int launch_head_rank(const HeadArgs& a, int group, int32_t* pos, float* probs, c
 // catalogue sweep head: probs[r] from the partial logit h_dot[r] (tc_dense TC_EPI_HEAD_DOT) and the GMF term of
 // (users[r / group], item r % group), with the per-row arithmetic of launch_head_rank's partial-logit kernel.  With seg
 // (candidate lists, group 1): global row row0 + r pairs users[seg[row0 + r]] (seg < num_lists) with items[row0 + r];
-// h_dot launch-local, probs global
+// h_dot launch-local, probs global.  With items and no seg (an item list tiled over the users): row r pairs
+// users[r / group] with items[r]
 bool catalogue_head_supported(const MrModel& m);
 int launch_catalogue_head(const MrModel& m, const float* h_dot, const int32_t* users, int64_t rows, int group,
                           float* probs, cudaStream_t st, const int32_t* seg = nullptr, const int32_t* items = nullptr,

@@ -829,4 +829,282 @@ int launch_targets_metrics(const int64_t* tgt_rowptr, int64_t U, int64_t nnz_t, 
   return MR_OK;
 }
 
+// ---- audiences: the k best pool users of every item column of (pool users x items) chunks -------------------------
+// Order: topk_key(p, user id), the row selection's order with the user id as the tie-break; keys are distinct, so the
+// top k is unique whatever order the chunks, splits and merges meet in.  Per item the running top-k lives in the
+// workspace as S lists of k keys and k raw scores (kNoKey-padded, keys ascending); split s owns the 32-row tiles
+// s, s + S, s + 2S, .. of every chunk.  Per chunk, one CTA per (32 columns, split): it reads 32 x 32 tiles as 128-byte
+// row segments, transposes them through shared memory, and each warp walks 4 columns, the lanes being 32 users,
+// next to each column's exclusion cursor, appending the keys below the list's k-th key (topk_push).  Only a column
+// with survivors touches its list: survivors and list in one buffer, one flush, and each kept key's raw score from
+// the list (a binary search) or from the chunk.  After the last chunk one warp per item merges its S lists, writes
+// users and scores and looks for the target in the result: pos = its slot, k when absent.
+// S > 1 only when the columns alone give fewer than ~1024 CTAs, so that a narrow call (a few new items) still fills
+// the GPU.  Bytes per pair: the 4-byte score, read once; per (column, chunk, split): one 8-byte threshold read and the
+// cursor's binary search, plus 12 k bytes read and written when the column has survivors.
+constexpr int kAudThreads = 256;
+constexpr int kAudCols = 32;                                 // columns per CTA: one tile wide
+constexpr int kAudColsPerWarp = kAudCols / (kAudThreads / 32);  // 4
+constexpr int kAudTargetCtas = 1024;
+
+static int audience_cap(int k) {  // survivors (<= k after a flush) + the list must fit, and one warp-wide append
+  int c = 64;
+  while (c < k + 32 || c < 2 * k) c <<= 1;
+  return c;
+}
+
+static int audience_splits(int64_t C, int32_t M) {
+  const int64_t blocks = ((int64_t)M + kAudCols - 1) / kAudCols, tiles = (C + 31) / 32;
+  int64_t s = kAudTargetCtas / (blocks < 1 ? 1 : blocks);
+  if (s > 32) s = 32;
+  if (s > tiles) s = tiles;
+  return (int)(s < 1 ? 1 : s);
+}
+
+AudienceWs carve_audience(void* ws, int64_t C, int32_t M, int32_t k) {
+  AudienceWs w{};
+  Carver cv(ws);
+  w.S = audience_splits(C, M);
+  const size_t entries = (size_t)(M < 1 ? 1 : M) * w.S * k;
+  w.keys = cv.take<unsigned long long>(entries);
+  w.scores = cv.take<float>(entries);
+  w.pos = cv.take<int32_t>((size_t)(M < 1 ? 1 : M));
+  w.total = cv.off;
+  return w;
+}
+
+// Bit i = the ascending list items[ep, ee) holds ids[i], for ids ascending over i (INT_MAX past the chunk's end);
+// advances ep past the entries <= ids[31].  The pool's counterpart of list_mask: each list entry finds its place among
+// the 32 ids by a binary search in shared memory.
+__device__ __forceinline__ uint32_t ids_mask(const int32_t* __restrict__ items, int64_t& ep, int64_t ee,
+                                             const int* ids, int lane) {
+  const int last = ids[31];
+  uint32_t mask = 0;
+  for (;;) {
+    const int64_t i = ep + lane;
+    const int e = i < ee ? __ldg(items + i) : 0;
+    const bool in = i < ee && e <= last;
+    const int nin = __popc(__ballot_sync(0xffffffffu, in));
+    uint32_t bit = 0;
+    if (in) {
+      int p = 0;  // ids below e (< 32: e <= last)
+#pragma unroll
+      for (int step = 16; step > 0; step >>= 1)
+        if (ids[p + step - 1] < e) p += step;
+      bit = ids[p] == e ? 1u << p : 0u;
+    }
+    mask |= __reduce_or_sync(0xffffffffu, bit);
+    ep += nin;
+    if (nin < 32) break;
+  }
+  return mask;
+}
+
+// Merges the n survivors in buf into list s of column j (k keys + k scores in the workspace).
+template <bool POOL>
+__device__ void audience_merge(const AudienceArgs& a, const AudienceWs& w, int j, int s, unsigned long long* buf, int n,
+                               int cap, int lane) {
+  const int k = a.k;
+  const size_t base = ((size_t)j * w.S + s) * k;
+  unsigned long long* lk = w.keys + base;
+  float* ls = w.scores + base;
+  n = topk_flush(buf, n, cap, k, lane);
+  for (int i = lane; i < k; i += 32) buf[n + i] = lk[i];
+  __syncwarp();
+  topk_flush(buf, n + k, cap, k, lane);
+  float sc[MR_MAX_TOPK / 32];
+#pragma unroll
+  for (int q = 0; q < MR_MAX_TOPK / 32; ++q) {
+    const int i = lane + 32 * q;
+    sc[q] = 0.f;
+    if (i >= k) continue;
+    const unsigned long long key = buf[i];
+    if (key == kNoKey) continue;
+    int lo = 0, hi = k;  // the key's place in the old list
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (lk[mid] < key) lo = mid + 1;
+      else hi = mid;
+    }
+    if (lo < k && lk[lo] == key) {
+      sc[q] = ls[lo];
+    } else {  // a survivor of this chunk: its row holds the user
+      const int uid = (int)(uint32_t)key;
+      const int64_t r = POOL ? list_lower_bound(a.users, a.u0, a.u0 + a.U, uid) - a.u0 : uid - a.u0;
+      sc[q] = __ldg(a.scores + r * a.M + j);
+    }
+  }
+  __syncwarp();  // every lane has read the old list
+#pragma unroll
+  for (int q = 0; q < MR_MAX_TOPK / 32; ++q) {
+    const int i = lane + 32 * q;
+    if (i < k) {
+      lk[i] = buf[i];
+      ls[i] = sc[q];
+    }
+  }
+}
+
+template <bool POOL>
+__global__ void __launch_bounds__(kAudThreads) audience_chunk_kernel(const AudienceArgs a, const AudienceWs w, int cap) {
+  extern __shared__ unsigned long long aud_smem[];
+  __shared__ float tile[32][33];
+  __shared__ int ids[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int S = w.S, s = blockIdx.y, k = a.k, M = a.M;
+  const int64_t C = a.U, first = (int64_t)s * 32;
+  if (first >= C) return;  // block-uniform: the last chunk may be short
+  const int j0 = blockIdx.x * kAudCols;
+  const int lo_user = POOL ? __ldg(a.users + a.u0 + first) : (int)(a.u0 + first);
+  int n[kAudColsPerWarp], t[kAudColsPerWarp];
+  unsigned long long thr[kAudColsPerWarp];
+  int64_t ep[kAudColsPerWarp], ee[kAudColsPerWarp];
+#pragma unroll
+  for (int q = 0; q < kAudColsPerWarp; ++q) {
+    const int j = j0 + warp * kAudColsPerWarp + q;
+    n[q] = 0;
+    t[q] = -1;
+    thr[q] = kNoKey;
+    ep[q] = ee[q] = 0;
+    if (j < M) {
+      thr[q] = w.keys[((size_t)j * S + s) * k + k - 1];
+      excl_cursor(a.excl_ids, a.excl_rows, a.excl_rowptr, a.excl_users, j, lo_user, ep[q], ee[q]);
+      if (a.targets != nullptr) t[q] = __ldg(a.targets + j);
+    }
+  }
+  for (int64_t r0 = first; r0 < C; r0 += (int64_t)32 * S) {
+    const int col = j0 + lane;
+    for (int rr = warp; rr < 32; rr += kAudThreads / 32) {
+      const int64_t r = r0 + rr;
+      tile[rr][lane] = (r < C && col < M) ? __ldg(a.scores + r * M + col) : 0.f;
+    }
+    if (warp == 0) {
+      const int64_t r = r0 + lane;
+      ids[lane] = r < C ? (POOL ? __ldg(a.users + a.u0 + r) : (int)(a.u0 + r)) : INT_MAX;
+    }
+    __syncthreads();
+    const int uid = ids[lane];
+    const bool ok = r0 + lane < C && uid >= 0 && uid < a.num_users;
+#pragma unroll
+    for (int q = 0; q < kAudColsPerWarp; ++q) {
+      const int c = warp * kAudColsPerWarp + q;
+      if (j0 + c >= M) break;  // warp-uniform
+      const uint32_t x = POOL ? ids_mask(a.excl_users, ep[q], ee[q], ids, lane)
+                              : list_mask(a.excl_users, ep[q], ee[q], (int)(a.u0 + r0), lane);
+      const bool cand = ok && (!((x >> lane) & 1u) || uid == t[q]);  // the target is never excluded
+      const unsigned long long key = cand ? topk_key(tile[lane][c], uid) : kNoKey;
+      topk_push(aud_smem + (size_t)c * cap, n[q], thr[q], key, cap, k, lane);
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int q = 0; q < kAudColsPerWarp; ++q) {
+    const int c = warp * kAudColsPerWarp + q;
+    if (j0 + c < M && n[q] > 0) audience_merge<POOL>(a, w, j0 + c, s, aud_smem + (size_t)c * cap, n[q], cap, lane);
+  }
+}
+
+// One warp per item: the k smallest keys of its S lists (topk_merge_warp's rule, carrying the raw scores).
+__global__ void __launch_bounds__(kTopkThreads) audience_final_kernel(const AudienceArgs a, const AudienceWs w,
+                                                                      const int32_t* __restrict__ items,
+                                                                      int32_t num_items, int32_t* __restrict__ top_users,
+                                                                      float* __restrict__ top_scores,
+                                                                      int32_t* __restrict__ pos) {
+  const int lane = threadIdx.x & 31;
+  const int64_t j = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (j >= a.M) return;  // warp-uniform
+  const int k = a.k, S = w.S;
+  const bool bad = items != nullptr && (unsigned)__ldg(items + j) >= (unsigned)num_items;
+  const int t = a.targets != nullptr ? __ldg(a.targets + j) : -1;
+  const size_t mine = ((size_t)j * S + lane) * k;
+  int cur = 0, hit = k;
+  unsigned long long head = lane < S ? w.keys[mine] : kNoKey;
+  for (int i = 0; i < k; ++i) {
+    unsigned long long m = head;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long x = __shfl_xor_sync(0xffffffffu, m, o);
+      m = x < m ? x : m;
+    }
+    const bool win = m != kNoKey && head == m;  // distinct keys: one winner at most
+    float sc = win ? w.scores[mine + cur] : 0.f;
+    const uint32_t wm = __ballot_sync(0xffffffffu, win);
+    sc = __shfl_sync(0xffffffffu, sc, wm ? __ffs(wm) - 1 : 0);
+    if (win) {
+      ++cur;
+      head = cur < k ? w.keys[mine + cur] : kNoKey;
+    }
+    const int user = (m == kNoKey || bad) ? -1 : (int)(uint32_t)m;
+    if (lane == (i & 31)) {
+      if (top_users != nullptr) top_users[j * k + i] = user;
+      if (top_scores != nullptr) top_scores[j * k + i] = user < 0 ? nanf("") : sc;
+    }
+    if (user >= 0 && user == t && hit == k) hit = i;
+  }
+  if (pos != nullptr && lane == 0) pos[j] = hit;
+}
+
+int launch_audience_init(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st) {
+  MR_CUDA(cudaMemsetAsync(w.keys, 0xff, (size_t)a.M * w.S * a.k * sizeof(unsigned long long), st));
+  const size_t smem = (size_t)kAudCols * audience_cap(a.k) * sizeof(unsigned long long);  // <= 128 KB
+  MR_CUDA(cudaFuncSetAttribute(audience_chunk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  MR_CUDA(cudaFuncSetAttribute(audience_chunk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  return MR_OK;
+}
+
+int launch_audience_chunk(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st) {
+  if (a.U == 0 || a.M == 0) return MR_OK;
+  const int cap = audience_cap(a.k);
+  const size_t smem = (size_t)kAudCols * cap * sizeof(unsigned long long);
+  const dim3 grid((unsigned)(((int64_t)a.M + kAudCols - 1) / kAudCols), (unsigned)w.S);
+  if (a.users != nullptr) audience_chunk_kernel<true><<<grid, kAudThreads, smem, st>>>(a, w, cap);
+  else audience_chunk_kernel<false><<<grid, kAudThreads, smem, st>>>(a, w, cap);
+  MR_LAUNCH_CHECK("audience_chunk_kernel");
+  return MR_OK;
+}
+
+int launch_audience_final(const AudienceArgs& a, const AudienceWs& w, const int32_t* items, int32_t num_items,
+                          int32_t* top_users, float* top_scores, int32_t* pos, float* sums, cudaStream_t st) {
+  if (a.M == 0) {
+    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+    return MR_OK;
+  }
+  int32_t* p = pos != nullptr ? pos : (sums != nullptr ? w.pos : nullptr);
+  const int wpc = kTopkThreads / 32;
+  audience_final_kernel<<<(unsigned)(((int64_t)a.M + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, w, items, num_items,
+                                                                                             top_users, top_scores, p);
+  MR_LAUNCH_CHECK("audience_final_kernel");
+  return launch_topk_metrics(p, a.M, a.k, sums, st);
+}
+
+__global__ void iota_kernel(int32_t* __restrict__ out, int64_t n, int64_t first) {
+  for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (int64_t)gridDim.x * blockDim.x)
+    out[r] = (int32_t)(first + r);
+}
+
+int launch_iota(int32_t* out, int64_t n, int64_t first, cudaStream_t st) {
+  if (n == 0) return MR_OK;
+  int64_t grid = (n + 255) / 256;
+  const int64_t cap = (int64_t)sm_count() * 8;
+  if (grid > cap) grid = cap;
+  iota_kernel<<<(unsigned)grid, 256, 0, st>>>(out, n, first);
+  MR_LAUNCH_CHECK("iota_kernel");
+  return MR_OK;
+}
+
+__global__ void tile_list_kernel(int32_t* __restrict__ out, int64_t rows, const int32_t* __restrict__ items, int32_t M) {
+  for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x)
+    out[r] = __ldg(items + r % M);
+}
+
+int launch_tile_list(int32_t* out, int64_t rows, const int32_t* items, int32_t M, cudaStream_t st) {
+  if (rows == 0) return MR_OK;
+  int64_t grid = (rows + 255) / 256;
+  const int64_t cap = (int64_t)sm_count() * 8;
+  if (grid > cap) grid = cap;
+  tile_list_kernel<<<(unsigned)grid, 256, 0, st>>>(out, rows, items, M);
+  MR_LAUNCH_CHECK("tile_list_kernel");
+  return MR_OK;
+}
+
 }  // namespace mr

@@ -557,6 +557,51 @@ class NeuMFEngine(object):
         self.last_catalogue_bad = bad
         return top_items, top_scores, pos, sums, full
 
+    def catalogue_audience(self, items, k, users=None, exclude=None, targets=None, want_scores=False):
+        """The k best users for each of `items` (mr_catalogue_audience): descending probability, the lower user id first
+        among ties, over a pool -- every user (users None) or the given ids, sorted and de-duplicated here -- minus the
+        item's exclusion list.  exclude: None or (rowptr int64, users int32) -- per ITEM id, an ascending user list
+        (host or device), typically the item's raters.  targets (M,): one held-out user per item, never excluded.
+        Returns device tensors (users (M, k) int32, scores (M, k) float32, pos (M,) int32 or None, sums (2,) float32
+        [hit_sum, dcg_sum] or None, scores_full (U, M) float32 or None, the pool (U,) int32 or None when it is every
+        user); pos / sums need targets; pos is the target's place among the item's candidates when < k, else k.  Slots
+        beyond the number of candidates hold user -1 / score NaN.  Raises ValueError on a malformed exclusion CSR before
+        any launch.  Leaves in `self.last_catalogue_bad` a one-element device tensor, non-zero when an item, pool user
+        or target id was out of range (such an item's rows are -1 / NaN; such pool users are never candidates)."""
+        dev = self.device
+        items = as_device_i32(items, dev)
+        M = items.numel()
+        k = int(k)
+        pool = audience_pool(users)
+        U = self.num_users if pool is None else int(pool.size)
+        d_pool = None if pool is None else torch.from_numpy(pool if pool.size else np.zeros(1, np.int32)).to(dev)
+        t = as_device_i32(targets, dev) if targets is not None else None
+        if t is not None and t.numel() != M:
+            raise ValueError("targets ({}) and items ({}) differ in length".format(t.numel(), M))
+        rowptr, excl, excl_rows = _audience_exclusion(exclude, dev)
+        top_users = torch.empty((M, k), dtype=torch.int32, device=dev)
+        top_scores = torch.empty((M, k), dtype=torch.float32, device=dev)
+        pos = torch.empty(M, dtype=torch.int32, device=dev) if t is not None else None
+        sums = torch.zeros(2, dtype=torch.float32, device=dev) if t is not None else None
+        full = torch.empty((U, M), dtype=torch.float32, device=dev) if want_scores else None
+        nbytes = int(nat.lib.mr_catalogue_audience_workspace_bytes(C.byref(self._model), U, M, k))
+        if nbytes == 0:
+            raise ValueError("catalogue_audience: bad sizes U={} M={} k={}".format(U, M, k))
+        ws = self._workspace(nbytes)
+        nat.check(nat.lib.mr_catalogue_audience(C.byref(self._model), _ptr(items if M else None), M, k, _ptr(d_pool), U,
+                                                excl_rows, _ptr(rowptr), _ptr(excl), _ptr(t), _ptr(top_users),
+                                                _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(full), _ptr(ws), ws.numel(),
+                                                self._stream()), "mr_catalogue_audience")
+        bad = torch.zeros(1, dtype=torch.float32, device=dev)
+        if M:
+            bad = bad + ((items.min() < 0) | (items.max() >= self.num_items)).to(torch.float32).reshape(1)
+            if t is not None:
+                bad = bad + ((t.min() < 0) | (t.max() >= self.num_users)).to(torch.float32).reshape(1)
+        if pool is not None and pool.size and (pool[0] < 0 or pool[-1] >= self.num_users):
+            bad = bad + 1.0
+        self.last_catalogue_bad = bad
+        return top_users, top_scores, pos, sums, full, (None if pool is None else d_pool[:U])
+
     def rank_lists(self, users, lists, k, targets=None, want_probs=False):
         """Score and rank ragged candidate lists in one call (mr_rank_lists): list u pairs users[u] with
         items[rowptr[u]:rowptr[u + 1]].  lists = (rowptr int64 (U + 1,), items int32 (nnz,)), host or device; targets
@@ -949,6 +994,84 @@ def topk_scores(scores, k, exclude=None, excl_ids=None, targets=None, device=Non
                                      _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(ws), nbytes, st),
               "mr_topk_scores")
     return top_items, top_scores, pos, sums
+
+
+def audience_pool(users):
+    """The pool of an audience call: None (every user) or ids -> host int32, ascending and de-duplicated."""
+    if users is None:
+        return None
+    u = np.asarray(users.cpu() if hasattr(users, "cpu") else users).reshape(-1).astype(np.int64)
+    return np.unique(u).astype(np.int32)
+
+
+def check_exclusion_csr(rowptr, ids):
+    """(rowptr, ids) host or device -> the same as tensors (int64 rowptr, int32 ids) on their own device; ValueError
+    unless rowptr has at least one entry, starts at 0, never decreases and ends at len(ids), and every list is strictly
+    ascending.  Device input is checked on the device and read back once."""
+    as_t = lambda x, dt: (x if isinstance(x, torch.Tensor) else torch.from_numpy(np.asarray(x).astype(dt))).reshape(-1)
+    rp = as_t(rowptr, np.int64).to(torch.int64)
+    it = as_t(ids, np.int64).to(rp.device, torch.int64)
+    n = it.numel()
+    if rp.numel() < 1:
+        raise ValueError("exclusion lists: rowptr is empty")
+    bad = (rp[0] != 0) | (rp[-1] != n) | (rp[1:] < rp[:-1]).any()
+    if n > 1:
+        inner = torch.ones(n - 1, dtype=torch.bool, device=rp.device)  # pairs of neighbours inside one list
+        starts = rp[1:-1]
+        starts = starts[(starts > 0) & (starts < n)]
+        inner[starts - 1] = False
+        bad = bad | ((it[1:] <= it[:-1]) & inner).any()
+    if bool(bad.item()):
+        raise ValueError("exclusion lists: offsets must start at 0, never decrease and end at len(ids) = {}, and every "
+                         "list must be strictly ascending".format(n))
+    return rp, it.to(torch.int32)
+
+
+def _audience_exclusion(exclude, device):
+    """None | (rowptr, ids) -> (device rowptr int64 or None, device ids int32 or None, rows), checked first."""
+    if exclude is None:
+        return None, None, 0
+    rp, it = check_exclusion_csr(*exclude)
+    return _exclusion_on_device((rp, it), device)
+
+
+def audience_scores(scores, k, users=None, exclude=None, excl_ids=None, targets=None, device=None):
+    """Audiences on a (U, M) score matrix (mr_audience_scores): for each column j the k best rows, row u being user
+    users[u] (default u; strictly ascending), ordered by descending score (NaN last, the lower user id first among
+    ties), minus the users of the column's exclusion list.  exclude: None or (rowptr int64, users int32); column j uses
+    list excl_ids[j] (default j).  targets (M,): one user per column, never excluded.  Returns device tensors
+    (users (M, k) int32, scores (M, k) float32, pos (M,) int32 or None -- clipped at k --, sums (2,) or None).  Raises
+    ValueError on a malformed exclusion CSR or a pool that is not strictly ascending."""
+    require_cuda()
+    device = torch.device(device if device is not None else "cuda:{}".format(torch.cuda.current_device()))
+    s = scores if isinstance(scores, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(scores)))
+    if s.dim() != 2:
+        raise ValueError("scores must be (U, M), got shape {}".format(tuple(s.shape)))
+    U, M = int(s.shape[0]), int(s.shape[1])
+    s = s.to(device, torch.float32).contiguous()
+    k = int(k)
+    pool = None
+    if users is not None:
+        h = np.asarray(users.cpu() if hasattr(users, "cpu") else users).reshape(-1).astype(np.int64)
+        if h.size != U or np.any(h[1:] <= h[:-1]):
+            raise ValueError("users must hold {} strictly ascending ids".format(U))
+        pool = torch.from_numpy(h.astype(np.int32)).to(device)
+    ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
+    t = as_device_i32(targets, device) if targets is not None else None
+    rowptr, excl, excl_rows = _audience_exclusion(exclude, device)
+    top_users = torch.empty((M, k), dtype=torch.int32, device=device)
+    top_scores = torch.empty((M, k), dtype=torch.float32, device=device)
+    pos = torch.empty(M, dtype=torch.int32, device=device) if t is not None else None
+    sums = torch.zeros(2, dtype=torch.float32, device=device) if t is not None else None
+    nbytes = int(nat.lib.mr_audience_scores_workspace_bytes(U, M, k))
+    if nbytes == 0:
+        raise ValueError("audience_scores: bad sizes U={} M={} k={}".format(U, M, k))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
+    st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+    nat.check(nat.lib.mr_audience_scores(_ptr(s), U, M, k, _ptr(pool), _ptr(ids), excl_rows, _ptr(rowptr), _ptr(excl),
+                                         _ptr(t), _ptr(top_users), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(ws),
+                                         nbytes, st), "mr_audience_scores")
+    return top_users, top_scores, pos, sums
 
 
 def _check_lists(lists, U, device):

@@ -107,6 +107,12 @@ SIGNATURES = {
     "mr_catalogue_targets_workspace_bytes": (_sz, [_PM, _i64, _i64]),
     "mr_catalogue_targets": (C.c_int, [_PM, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _sz,
                                        _vp]),
+    "mr_audience_scores_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "mr_audience_scores": (C.c_int, [_vp, _i64, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                     _vp]),
+    "mr_catalogue_audience_workspace_bytes": (_sz, [_PM, _i64, _i32, _i32]),
+    "mr_catalogue_audience": (C.c_int, [_PM, _vp, _i32, _i32, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                        _sz, _vp]),
     "mr_topk_lists_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "mr_topk_lists": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_rank_lists_workspace_bytes": (_sz, [_PM, _i64, _i64, _i32]),

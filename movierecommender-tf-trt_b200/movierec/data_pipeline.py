@@ -84,6 +84,20 @@ class MovieLensDataGenerator(object):
         return int(np.floor(len(self.indexes) / self.batch_size))
 
     # ---- device state ------------------------------------------------------------------------------
+    def _all_pairs(self):
+        """(users, items) int64 of data ∪ extra_data, with their id bounds (max + 1, at least 1)."""
+        users = np.asarray(self.data[COL_USER_ID].values, dtype=np.int64)
+        items = np.asarray(self.data[COL_ITEM_ID].values, dtype=np.int64)
+        all_u, all_i = users, items
+        if self.extra_data is not None:
+            all_u = np.concatenate([users, np.asarray(self.extra_data[COL_USER_ID].values, dtype=np.int64)])
+            all_i = np.concatenate([items, np.asarray(self.extra_data[COL_ITEM_ID].values, dtype=np.int64)])
+        if len(all_u) and (all_u.min() < 0 or all_i.min() < 0):
+            raise ValueError("negative user / item ids")
+        n_u = int(all_u.max()) + 1 if len(all_u) else 1
+        n_i = int(all_i.max()) + 1 if len(all_i) else 1
+        return all_u, all_i, n_u, n_i
+
     def _upload(self):
         import torch
         from . import _engine
@@ -91,16 +105,9 @@ class MovieLensDataGenerator(object):
         dev = torch.device("cuda:{}".format(torch.cuda.current_device()))
         users = np.asarray(self.data[COL_USER_ID].values, dtype=np.int64)
         items = np.asarray(self.data[COL_ITEM_ID].values, dtype=np.int64)
-        all_u, all_i = users, items
-        if self.extra_data is not None:
-            all_u = np.concatenate([users, np.asarray(self.extra_data[COL_USER_ID].values, dtype=np.int64)])
-            all_i = np.concatenate([items, np.asarray(self.extra_data[COL_ITEM_ID].values, dtype=np.int64)])
         # per-user sorted item lists built on the device (mr_build_user_csr: two stable radix sorts + compaction);
         # build_user_csr below is the same table in NumPy, kept for host-side use and as the tests' cross-check
-        if len(all_u) and (all_u.min() < 0 or all_i.min() < 0):
-            raise ValueError("negative user / item ids")
-        n_u = int(all_u.max()) + 1 if len(all_u) else 1
-        n_i = int(all_i.max()) + 1 if len(all_i) else 1
+        all_u, all_i, n_u, n_i = self._all_pairs()
         rowptr, csr = _engine.build_user_csr(all_u.astype(np.int32), all_i.astype(np.int32), n_u, n_i)
         self._device = {
             "dev": dev,
@@ -130,6 +137,20 @@ class MovieLensDataGenerator(object):
         if self._device is None:
             self._upload()
         return self._device["rowptr"], self._device["csr"]
+
+    def item_user_lists(self):
+        """(rowptr int64, users int32) device tensors: per item, the ascending distinct users of data ∪ extra_data --
+        user_item_lists transposed (the same device build with the roles swapped), the exclusion lists of an
+        audience: who has already rated the item."""
+        if self._device is None:
+            self._upload()
+        d = self._device
+        if "item_rowptr" not in d:
+            from . import _engine
+            all_u, all_i, n_u, n_i = self._all_pairs()
+            d["item_rowptr"], d["item_csr"] = _engine.build_user_csr(all_i.astype(np.int32), all_u.astype(np.int32), n_i,
+                                                                     n_u)
+        return d["item_rowptr"], d["item_csr"]
 
     def device_batch(self, idx):
         """Batch `idx` as device tensors ([x_user int32, x_item int32], y float32), layout of the

@@ -189,6 +189,18 @@ class NeuMFModel(object):
         self._raise_on_bad_ids(float(eng.last_catalogue_bad.item()))
         return items.cpu().numpy(), scores.cpu().numpy()
 
+    def audience_for_items(self, items, top_k=10, users=None, exclude=None):
+        """The top_k users most likely to want each of `items` (who to show or notify about it), over the whole user
+        base or over the pool `users` (any order, duplicates ignored), leaving out each item's exclusion list.  Order:
+        descending score, the lower user id first among ties.  exclude: None, a MovieLensDataGenerator (each item's
+        raters in data ∪ extra_data) or a (rowptr, users) pair of ascending per-item lists.  Returns NumPy
+        (users (M, top_k) int32, scores (M, top_k) float32); slots beyond the number of candidates hold -1 / NaN.  One
+        device call for all items.  Raises IndexError on an out-of-range item or pool user."""
+        eng = self.engine
+        top, scores, _, _, _, _ = eng.catalogue_audience(items, top_k, users=users, exclude=_audience_lists(exclude))
+        self._raise_on_bad_ids(float(eng.last_catalogue_bad.item()))
+        return top.cpu().numpy(), scores.cpu().numpy()
+
     def recommend_batch(self, users, candidate_lists, top_k=10):
         """recommend() for many requests at once: user users[u] against its own candidate list, of any length.
         candidate_lists: a list (or other sequence) of 1-D item arrays, one per user, or a tuple (rowptr, items) of
@@ -636,10 +648,11 @@ class MovierecModel(object):
         last-step loss.  Raises IndexError on an out-of-range user and ValueError on a malformed CSR or a rater list
         that covers every user."""
         eng = self.model.engine
+        raters = _engine_module().fold_in_histories(raters, eng.num_users, side="items")
         mlp, gmf, loss = eng.fold_in_items(raters, FOLD_IN_STEPS if steps is None else steps,
                                            FOLD_IN_LR if lr is None else lr,
                                            self._num_negs_per_pos if negs is None else negs, seed=seed)
-        return ItemFoldedModel(self, mlp, gmf, loss)
+        return ItemFoldedModel(self, mlp, gmf, loss, raters)
 
     def evaluate(self, users, items, k=None):
         """Full-sweep ranking evaluation (BASELINE config 4): one user id per group and
@@ -670,6 +683,25 @@ class MovierecModel(object):
         s = torch.cat([sums.reshape(-1), eng.last_catalogue_bad.to(sums.dtype)]).cpu().numpy().astype(np.float64)
         self.model._raise_on_bad_ids(s[2])
         G = max(int(pos.numel()), 1)
+        return s[0] / G, s[1] / G
+
+    def evaluate_item_audiences(self, items, users, exclude=None, k=None):
+        """Item-side leave-one-out evaluation: for item items[g], its held-out rater users[g] is ranked among every user
+        not on the item's exclusion list (the held-out user itself always counts).  exclude: as
+        NeuMFModel.audience_for_items -- typically the training generator, whose lists hold every user who already
+        rated the item.  Returns (hr, ndcg) at k (default: the model's k), means over the items.  Raises IndexError on
+        an out-of-range item or user."""
+        k = self._k if k is None else k
+        import torch
+        eng = self.model.engine
+        items = np.asarray(items, dtype=np.int32).reshape(-1)
+        users = np.asarray(users, dtype=np.int32).reshape(-1)
+        if users.size != items.size:
+            raise ValueError("users ({}) and items ({}) differ in length".format(users.size, items.size))
+        _, _, pos, sums, _, _ = eng.catalogue_audience(items, k, exclude=_audience_lists(exclude), targets=users)
+        s = torch.cat([sums.reshape(-1), eng.last_catalogue_bad.to(sums.dtype)]).cpu().numpy().astype(np.float64)
+        self.model._raise_on_bad_ids(s[2])
+        G = max(int(items.size), 1)
         return s[0] / G, s[1] / G
 
     def evaluate_candidate_lists(self, users, candidate_lists, targets, k=None):
@@ -778,7 +810,7 @@ class ItemFoldedModel(MovierecModel):
     the new items (a copy of the item tables with the new rows appended).  Scoring, evaluation and user fold-in work as
     on the model; training and saving raise."""
 
-    def __init__(self, base, item_mlp, item_gmf, loss):
+    def __init__(self, base, item_mlp, item_gmf, loss, raters=None):
         self.__dict__.update(base.__dict__)
         view = base.model.engine.item_view(item_mlp, item_gmf)
         self.new_item_ids = np.arange(self._num_items, view.num_items, dtype=np.int32)
@@ -786,6 +818,15 @@ class ItemFoldedModel(MovierecModel):
         self.model = _FoldedNeuMF(self, view)
         self.loss = loss.cpu().numpy()
         self._new_rows = (item_mlp, item_gmf)
+        self._raters = raters  # host (rowptr, users) of the new items, as folded
+
+    def audience_for_new_items(self, top_k=10, users=None):
+        """The cold-start flow in one call: NeuMFModel.audience_for_items for every new item (rows in new_item_ids
+        order), leaving out the raters each item was folded in from.  users: the pool, as audience_for_items."""
+        rowptr, raters = self._raters
+        first = int(self.new_item_ids[0]) if self.new_item_ids.size else self._num_items
+        by_item = np.concatenate([np.zeros(first, np.int64), np.asarray(rowptr, np.int64)])  # earlier items: no list
+        return self.model.audience_for_items(self.new_item_ids, top_k, users=users, exclude=(by_item, raters))
 
     def item_weights(self):
         """The new items' rows as NumPy: (item_mlp (M, L[0] - L[0]/2), item_gmf (M, mf_dim) or None)."""
@@ -848,6 +889,16 @@ def _exclusion_lists(exclude):
         return exclude.user_item_lists()
     rowptr, items = exclude
     return rowptr, items
+
+
+def _audience_lists(exclude):
+    """None | MovieLensDataGenerator | (rowptr, users) -> None | (rowptr, users), lists by item id."""
+    if exclude is None:
+        return None
+    if hasattr(exclude, "item_user_lists"):
+        return exclude.item_user_lists()
+    rowptr, users = exclude
+    return rowptr, users
 
 
 class RankLayer(object):
