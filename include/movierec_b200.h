@@ -29,11 +29,11 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 105     /* major*100 + minor */
+#define MR_VERSION 106     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
-#define MR_MAX_TOPK 256    /* k of the catalogue top-k calls */
+#define MR_MAX_TOPK 4096   /* k of the top-k, list and audience calls: one output list sorts in one CTA (48 KB) */
 #define MR_MAX_CUTOFFS 8   /* cutoffs of one mr_targets_scores / mr_catalogue_targets call */
 
 typedef enum MrStatus {
@@ -219,7 +219,10 @@ int mr_rank_scores(const float* scores, int64_t G, int32_t group, int32_t k, con
  * for a target outside [0, N)); sums = {hit_sum, dcg_sum} over the U targets (hit = pos < k, dcg = ln2/ln(pos+2)*hit).
  * pos and sums need targets.  top_items / top_scores (U x k, each may be NULL): the k best candidates in order;
  * slots beyond the number of candidates hold item -1 and score NaN.  1 <= k <= MR_MAX_TOPK.  Deterministic (the
- * selection compares distinct integer keys).  The workspace does not grow with U beyond one chunk of users. */
+ * selection compares distinct integer keys).  The workspace does not grow with U beyond one chunk of users: for
+ * k <= 256 about 8 k bytes per (row, slice of the items); for k > 256 (one CTA per row, radix select) 8 bytes per
+ * (row, item) of a chunk of about 2^22 rows, 32 MB, whatever k is.  Which of the two selections runs depends on k
+ * alone, so a row's result never depends on the other rows of a call. */
 size_t mr_topk_scores_workspace_bytes(int64_t U, int32_t N, int32_t k);
 int mr_topk_scores(const float* scores, int64_t U, int32_t N, int32_t k, const int32_t* excl_ids, int32_t excl_rows,
                    const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
@@ -290,9 +293,12 @@ int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, 
  * the target's rows; HR@k and NDCG@k do not need it.  sums = {hit_sum, dcg_sum} over the M columns
  * (hit = pos < k, dcg = ln2/ln(pos+2)*hit).  pos and sums need targets.  1 <= k <= MR_MAX_TOPK, U <= INT32_MAX.
  * Columns are selected in chunks of the users of one mr_catalogue_topk chunk of M items (C = min(U, about 2^22 / M,
- * 16384) rows); per item a running top-k is carried across chunks as S <= 32 lists (S > 1 only for narrow calls:
- * S = min(32, max(1, 1024 / ceil(M / 32)), ceil(C / 32))).  Workspace: 12 k S bytes per item (keys and raw scores)
- * + 4 bytes per item, plus alignment: 3.2 MB at M = 26,744, k = 10 (S = 1); 82 MB at k = 256.  Deterministic; no
+ * 16384) rows).  k <= 256: per item a running top-k is carried across chunks as S <= 32 lists (S > 1 only for narrow
+ * calls: S = min(32, max(1, 1024 / ceil(M / 32)), ceil(C / 32))).  Workspace: 12 k S bytes per item (keys and raw
+ * scores) + 4 bytes per item, plus alignment: 3.2 MB at M = 26,744, k = 10 (S = 1); 82 MB at k = 256.
+ * k > 256: per item a sorted list of k keys and raw scores plus an append buffer of k + C entries, compacted whenever
+ * the next chunk could overflow it.  Workspace: 12 (2 k + C) + 8 bytes per item, plus alignment: 0.69 GB at
+ * M = 26,744, k = 1000 (C = 156); 2.7 GB at k = 4096; 22 MB for M = 100, k = 1000 (C = 16,384).  Deterministic; no
  * host synchronisation, no read-back. */
 size_t mr_audience_scores_workspace_bytes(int64_t U, int32_t M, int32_t k);
 int mr_audience_scores(const float* scores, int64_t U, int32_t M, int32_t k, const int32_t* users,
@@ -325,8 +331,9 @@ int mr_catalogue_audience(const MrModel* model, const int32_t* items, int32_t M,
  * sums = {hit_sum, dcg_sum} over the U lists (hit = pos < k, dcg = ln2/ln(pos+2)*hit).  pos and sums need targets.
  * 1 <= k <= MR_MAX_TOPK.  Deterministic (distinct integer keys).  Every list is clamped to [0, nnz), so a malformed
  * rowptr never makes a kernel read or write outside the arrays; its lists' results are unspecified.
- * Workspace: 8 bytes per list + 4 per list + about 8 k + 4 bytes per 512 rows (staged partial results of the lists
- * longer than 1024, which are cut into <= 32 slices), plus alignment.  No host synchronisation, no read-back. */
+ * Workspace for k <= 256: 8 bytes per list + 4 per list + about 8 k + 4 bytes per 512 rows (staged partial results
+ * of the lists longer than 1024, which are cut into <= 32 slices), plus alignment; for k > 256 (one CTA per list,
+ * radix select on keys recomputed from the scores): 4 bytes per list.  No host synchronisation, no read-back. */
 size_t mr_topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k);
 int mr_topk_lists(const float* scores, int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
                   int32_t* top_pos, float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream);

@@ -2022,7 +2022,7 @@ int mr_audience_scores(const float* scores, int64_t U, int32_t M, int32_t k, con
   }
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t C = clamp_users(U, catalogue_chunk_users(M));
-  const AudienceWs w = carve_audience(ws, C, M, k);
+  const AudienceState w = carve_audience(ws, C, M, k);
   AudienceArgs a{};
   a.M = M;
   a.k = k;
@@ -2075,7 +2075,7 @@ int mr_catalogue_audience(const MrModel* model, const int32_t* items, int32_t M,
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t C = clamp_users(U, catalogue_chunk_users(M));
   Carver cv(ws);
-  const AudienceWs w = carve_audience(cv.take<char>(audience_select_bytes(C, M, k)), C, M, k);
+  const AudienceState w = carve_audience(cv.take<char>(audience_select_bytes(C, M, k)), C, M, k);
   AudienceArgs a{};
   a.M = M;
   a.k = k;

@@ -99,6 +99,9 @@ int launch_rank_scores(const float* scores, int64_t G, int group, int k, const i
                        int32_t* pos, float* sums, float* partials, cudaStream_t st, const float* labels = nullptr);
 
 // ---- topk.cu: top-k selection over rows of scores with per-row exclusion lists ------------------------------
+// k <= kTopkSmallK: per-warp buffers and warp merges (topk.cu); larger k: one CTA per segment by radix select
+// (topk_large.cu).  The choice depends on k alone, so a row's result never depends on the other rows of a call.
+constexpr int kTopkSmallK = 256;
 struct TopkArgs {
   const float* scores;  // the chunk's rows: U x N, row 0 = global row u0
   int64_t U, u0;
@@ -169,14 +172,40 @@ struct AudienceWs {
   int S;                     // lists per item (row splits of a chunk)
   size_t total;
 };
+// k > kTopkSmallK: per item a sorted list of k keys and raw scores (its k-th key is the item's threshold) and an append
+// buffer of cap = k + C entries filled by the chunks, cnt[j] entries used; compaction merges list and buffer into the
+// list whenever the next chunk could overflow the buffer.
+struct AudienceLargeWs {
+  unsigned long long* keys;   // M x k
+  float* scores;
+  unsigned long long* bkeys;  // M x cap
+  float* bscores;
+  int32_t* cnt;               // M
+  int32_t* pos;               // M: positions when the caller wants sums only
+  int64_t cap;
+};
+struct AudienceState {
+  AudienceWs w;  // k <= kTopkSmallK
+  AudienceLargeWs lg;  // k > kTopkSmallK
+  size_t total;
+};
 // The running state of a call whose chunks have at most C users (ws = NULL: sizes only).
-AudienceWs carve_audience(void* ws, int64_t C, int32_t M, int32_t k);
-int launch_audience_init(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st);
-int launch_audience_chunk(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st);
+AudienceState carve_audience(void* ws, int64_t C, int32_t M, int32_t k);
+int launch_audience_init(const AudienceArgs& a, const AudienceState& w, cudaStream_t st);
+int launch_audience_chunk(const AudienceArgs& a, const AudienceState& w, cudaStream_t st);
 // top_users / top_scores (M x k), pos (M; the target's slot, k when absent); items (may be NULL): a column whose
 // items[j] lies outside [0, num_items) gets -1 / NaN and pos = k.  sums (needs targets) = {hit_sum, dcg_sum} at k.
-int launch_audience_final(const AudienceArgs& a, const AudienceWs& w, const int32_t* items, int32_t num_items,
+int launch_audience_final(const AudienceArgs& a, const AudienceState& w, const int32_t* items, int32_t num_items,
                           int32_t* top_users, float* top_scores, int32_t* pos, float* sums, cudaStream_t st);
+// ---- topk_large.cu: the k > kTopkSmallK counterparts, with the same arguments and results ---------------------------
+size_t topk_large_workspace_bytes(int64_t U, int32_t N);  // per chunk of U rows: the staged keys
+int launch_topk_large(const TopkArgs& a, void* ws, cudaStream_t st);
+int launch_topk_lists_large(const TopkListsArgs& a, int32_t* pos, cudaStream_t st);
+AudienceLargeWs carve_audience_large(void* ws, int64_t C, int32_t M, int32_t k, size_t& total);
+int launch_audience_large_init(const AudienceArgs& a, const AudienceLargeWs& w, cudaStream_t st);
+int launch_audience_large_chunk(const AudienceArgs& a, const AudienceLargeWs& w, cudaStream_t st);
+int launch_audience_large_final(const AudienceArgs& a, const AudienceLargeWs& w, const int32_t* items,
+                                int32_t num_items, int32_t* top_users, float* top_scores, int32_t* pos, cudaStream_t st);
 // Positions of many targets per row: row u's targets are tgt_items[tgt_rowptr[u] .. tgt_rowptr[u+1]) (segments clamped
 // to [0, nnz_t)); candidates, order and exclusion lists as TopkArgs, a target never excluded.
 struct TargetsArgs {

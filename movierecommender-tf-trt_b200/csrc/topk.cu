@@ -13,16 +13,13 @@
 // Pass 2: one warp per row merges the <= 32 sorted slice lists (lane = slice, k rounds of a warp minimum), writes the
 //         k items / scores with -1 / NaN padding and adds the slice counts into pos.
 // Algorithmic bytes per row: 4 N (scores) + 4 x (exclusion list) read; 8 k x slices written and read back.
-#include <limits.h>
-
-#include "launchers.h"
+#include "topk_common.cuh"
 
 namespace mr {
 
 constexpr int kTopkThreads = 128;  // four warps per CTA, each with its own buffer
 constexpr int kTopkMinSlice = 1024;
 constexpr int kTopkMaxSlices = 32;  // one merge lane per slice
-constexpr unsigned long long kNoKey = ~0ull;
 
 __host__ __device__ static int topk_slice_len(int32_t N) {
   int64_t s = ((int64_t)N + kTopkMaxSlices - 1) / kTopkMaxSlices;
@@ -39,14 +36,9 @@ static int topk_cap(int k) {  // buffer entries: a power of two >= k + 32 (room 
 }
 
 size_t topk_workspace_bytes(int64_t U, int32_t N, int32_t k) {
+  if (k > kTopkSmallK) return topk_large_workspace_bytes(U, N);
   const size_t rows = (size_t)(U < 1 ? 1 : U) * topk_slices(N);
   return align_up(rows * k * sizeof(unsigned long long), 256) + align_up(rows * sizeof(int32_t), 256);
-}
-
-__device__ __forceinline__ unsigned long long topk_key(float p, int item) {
-  uint32_t b = __float_as_uint(rank_key(p) + 0.0f);
-  b = (b & 0x80000000u) ? ~b : (b | 0x80000000u);  // ascending with the float value
-  return ((unsigned long long)(~b) << 32) | (uint32_t)item;
 }
 
 // Sorts buf[0, cap) ascending after padding [n, cap) with kNoKey; returns the number of entries kept (<= k).
@@ -105,47 +97,6 @@ __device__ __forceinline__ void topk_merge_warp(const unsigned long long* lists,
     }
     if (lane == (i & 31)) emit(i, m);
   }
-}
-
-// The first index of the ascending list items[b, e) whose entry is >= v (e when none).
-__device__ __forceinline__ int64_t list_lower_bound(const int32_t* __restrict__ items, int64_t b, int64_t e, int v) {
-  while (b < e) {
-    const int64_t mid = (b + e) >> 1;
-    if (__ldg(items + mid) < v) b = mid + 1;
-    else e = mid;
-  }
-  return b;
-}
-
-// A warp's cursor [ep, ee) into the exclusion list of global row gu, from the first entry >= lo (empty when the row
-// has no list).
-__device__ __forceinline__ void excl_cursor(const int32_t* __restrict__ excl_ids, int32_t excl_rows,
-                                            const int64_t* __restrict__ excl_rowptr, const int32_t* __restrict__ excl_items,
-                                            int64_t gu, int lo, int64_t& ep, int64_t& ee) {
-  ep = ee = 0;
-  if (excl_rowptr == nullptr) return;
-  const int64_t r = excl_ids != nullptr ? (int64_t)__ldg(excl_ids + gu) : gu;
-  if (r >= 0 && r < excl_rows) {
-    ee = excl_rowptr[r + 1];
-    ep = list_lower_bound(excl_items, excl_rowptr[r], ee, lo);
-  }
-}
-
-// Bit i = items[ep, ee) holds c + i, for a warp walking its items 32 at a time in ascending c; advances ep past the
-// entries below c + 32.  Warp-uniform: lists are sorted, so the entries below c + 32 are a prefix of the lanes.
-__device__ __forceinline__ uint32_t list_mask(const int32_t* __restrict__ items, int64_t& ep, int64_t ee, int c,
-                                              int lane) {
-  uint32_t mask = 0;
-  for (;;) {
-    const int64_t i = ep + lane;
-    const int e = i < ee ? __ldg(items + i) : INT_MAX;
-    const bool in = e < c + 32;
-    const int nin = __popc(__ballot_sync(0xffffffffu, in));
-    mask |= __reduce_or_sync(0xffffffffu, (in && e >= c) ? 1u << (e - c) : 0u);
-    ep += nin;
-    if (nin < 32) break;
-  }
-  return mask;
 }
 
 __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs a, int S, int slice, int cap,
@@ -208,6 +159,7 @@ __global__ void __launch_bounds__(kTopkThreads) topk_merge_kernel(const TopkArgs
 
 int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st) {
   if (a.U == 0) return MR_OK;
+  if (a.k > kTopkSmallK) return launch_topk_large(a, ws, st);
   const int S = topk_slices(a.N), slice = topk_slice_len(a.N), cap = topk_cap(a.k);
   Carver cv(ws);
   unsigned long long* lists = cv.take<unsigned long long>((size_t)a.U * S * a.k);
@@ -230,14 +182,6 @@ int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st) {
 // bound U + ceil(nnz / 1024) covers them (a long list has fewer than len / 1024 slices beyond its first).
 // Only long lists stage: fewer than 2 nnz / 1024 slices of 8 k bytes, i.e. < nnz k / 64 bytes.
 // Segments are clamped to [0, nnz), so a malformed rowptr cannot make any kernel leave its arrays.
-
-__device__ __forceinline__ void list_bounds(const int64_t* __restrict__ rowptr, int64_t u, int64_t nnz, int64_t& b,
-                                            int64_t& e) {
-  b = __ldg(rowptr + u);
-  e = __ldg(rowptr + u + 1);
-  b = b < 0 ? 0 : (b > nnz ? nnz : b);
-  e = e < b ? b : (e > nnz ? nnz : e);
-}
 
 // off[u] (u = 0 .. U): low 32 bits = staged slices of the long lists before u, high 32 bits = long lists before u; the
 // slices 1.. of long list u are then work items U + (low - high) ..  One CTA, 4096 lists per round.
@@ -290,16 +234,6 @@ __global__ void __launch_bounds__(1024) topk_lists_scan_kernel(const int64_t* __
 }
 
 __device__ __forceinline__ int64_t lists_extra(unsigned long long o) { return (int64_t)(uint32_t)o - (int64_t)(o >> 32); }
-
-// Final outputs of slot i of list u (list start b, length len) from key m.
-__device__ __forceinline__ void lists_emit(const TopkListsArgs& a, int64_t u, int64_t b, int i, unsigned long long m,
-                                           bool bad_u) {
-  const int p = (m == kNoKey || bad_u) ? -1 : (int)(uint32_t)m;
-  const size_t o = (size_t)u * a.k + i;
-  if (a.top_pos != nullptr) a.top_pos[o] = p;
-  if (a.top_items != nullptr) a.top_items[o] = p < 0 ? -1 : __ldg(a.items + b + p);
-  if (a.top_scores != nullptr) a.top_scores[o] = p < 0 ? nanf("") : __ldg(a.scores + b + p);
-}
 
 __global__ void __launch_bounds__(kTopkThreads) topk_lists_slice_kernel(const TopkListsArgs a, int cap,
                                                                         const unsigned long long* __restrict__ off,
@@ -385,12 +319,18 @@ __global__ void __launch_bounds__(kTopkThreads) topk_lists_merge_kernel(const To
 static int64_t lists_stage_slots(int64_t nnz) { return (nnz + 511) / 512; }  // > the staged slices of any rowptr
 
 size_t topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k) {
+  if (k > kTopkSmallK) return align_up((size_t)U * sizeof(int32_t), 256);  // positions when the caller wants sums only
   const size_t slots = (size_t)lists_stage_slots(nnz);
   return align_up((size_t)(U + 1) * sizeof(unsigned long long), 256) + align_up((size_t)U * sizeof(int32_t), 256) +
          align_up(slots * k * sizeof(unsigned long long), 256) + align_up(slots * sizeof(int32_t), 256);
 }
 
 int launch_topk_lists(const TopkListsArgs& a, float* sums, void* ws, cudaStream_t st) {
+  if (a.k > kTopkSmallK) {
+    int32_t* pos = a.pos != nullptr ? a.pos : (sums != nullptr ? static_cast<int32_t*>(ws) : nullptr);
+    const int rc = launch_topk_lists_large(a, pos, st);
+    return rc != MR_OK ? rc : launch_topk_metrics(pos, a.U, a.k, sums, st);
+  }
   Carver cv(ws);
   unsigned long long* off = cv.take<unsigned long long>((size_t)a.U + 1);
   int32_t* pos_buf = cv.take<int32_t>((size_t)a.U);
@@ -861,43 +801,21 @@ static int audience_splits(int64_t C, int32_t M) {
   return (int)(s < 1 ? 1 : s);
 }
 
-AudienceWs carve_audience(void* ws, int64_t C, int32_t M, int32_t k) {
-  AudienceWs w{};
+AudienceState carve_audience(void* ws, int64_t C, int32_t M, int32_t k) {
+  AudienceState st{};
+  if (k > kTopkSmallK) {
+    st.lg = carve_audience_large(ws, C, M, k, st.total);
+    return st;
+  }
+  AudienceWs& w = st.w;
   Carver cv(ws);
   w.S = audience_splits(C, M);
   const size_t entries = (size_t)(M < 1 ? 1 : M) * w.S * k;
   w.keys = cv.take<unsigned long long>(entries);
   w.scores = cv.take<float>(entries);
   w.pos = cv.take<int32_t>((size_t)(M < 1 ? 1 : M));
-  w.total = cv.off;
-  return w;
-}
-
-// Bit i = the ascending list items[ep, ee) holds ids[i], for ids ascending over i (INT_MAX past the chunk's end);
-// advances ep past the entries <= ids[31].  The pool's counterpart of list_mask: each list entry finds its place among
-// the 32 ids by a binary search in shared memory.
-__device__ __forceinline__ uint32_t ids_mask(const int32_t* __restrict__ items, int64_t& ep, int64_t ee,
-                                             const int* ids, int lane) {
-  const int last = ids[31];
-  uint32_t mask = 0;
-  for (;;) {
-    const int64_t i = ep + lane;
-    const int e = i < ee ? __ldg(items + i) : 0;
-    const bool in = i < ee && e <= last;
-    const int nin = __popc(__ballot_sync(0xffffffffu, in));
-    uint32_t bit = 0;
-    if (in) {
-      int p = 0;  // ids below e (< 32: e <= last)
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1)
-        if (ids[p + step - 1] < e) p += step;
-      bit = ids[p] == e ? 1u << p : 0u;
-    }
-    mask |= __reduce_or_sync(0xffffffffu, bit);
-    ep += nin;
-    if (nin < 32) break;
-  }
-  return mask;
+  w.total = st.total = cv.off;
+  return st;
 }
 
 // Merges the n survivors in buf into list s of column j (k keys + k scores in the workspace).
@@ -912,9 +830,9 @@ __device__ void audience_merge(const AudienceArgs& a, const AudienceWs& w, int j
   for (int i = lane; i < k; i += 32) buf[n + i] = lk[i];
   __syncwarp();
   topk_flush(buf, n + k, cap, k, lane);
-  float sc[MR_MAX_TOPK / 32];
+  float sc[kTopkSmallK / 32];
 #pragma unroll
-  for (int q = 0; q < MR_MAX_TOPK / 32; ++q) {
+  for (int q = 0; q < kTopkSmallK / 32; ++q) {
     const int i = lane + 32 * q;
     sc[q] = 0.f;
     if (i >= k) continue;
@@ -936,7 +854,7 @@ __device__ void audience_merge(const AudienceArgs& a, const AudienceWs& w, int j
   }
   __syncwarp();  // every lane has read the old list
 #pragma unroll
-  for (int q = 0; q < MR_MAX_TOPK / 32; ++q) {
+  for (int q = 0; q < kTopkSmallK / 32; ++q) {
     const int i = lane + 32 * q;
     if (i < k) {
       lk[i] = buf[i];
@@ -1044,7 +962,9 @@ __global__ void __launch_bounds__(kTopkThreads) audience_final_kernel(const Audi
   if (pos != nullptr && lane == 0) pos[j] = hit;
 }
 
-int launch_audience_init(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st) {
+int launch_audience_init(const AudienceArgs& a, const AudienceState& state, cudaStream_t st) {
+  if (a.k > kTopkSmallK) return launch_audience_large_init(a, state.lg, st);
+  const AudienceWs& w = state.w;
   MR_CUDA(cudaMemsetAsync(w.keys, 0xff, (size_t)a.M * w.S * a.k * sizeof(unsigned long long), st));
   const size_t smem = (size_t)kAudCols * audience_cap(a.k) * sizeof(unsigned long long);  // <= 128 KB
   MR_CUDA(cudaFuncSetAttribute(audience_chunk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1052,8 +972,10 @@ int launch_audience_init(const AudienceArgs& a, const AudienceWs& w, cudaStream_
   return MR_OK;
 }
 
-int launch_audience_chunk(const AudienceArgs& a, const AudienceWs& w, cudaStream_t st) {
+int launch_audience_chunk(const AudienceArgs& a, const AudienceState& state, cudaStream_t st) {
   if (a.U == 0 || a.M == 0) return MR_OK;
+  if (a.k > kTopkSmallK) return launch_audience_large_chunk(a, state.lg, st);
+  const AudienceWs& w = state.w;
   const int cap = audience_cap(a.k);
   const size_t smem = (size_t)kAudCols * cap * sizeof(unsigned long long);
   const dim3 grid((unsigned)(((int64_t)a.M + kAudCols - 1) / kAudCols), (unsigned)w.S);
@@ -1063,12 +985,18 @@ int launch_audience_chunk(const AudienceArgs& a, const AudienceWs& w, cudaStream
   return MR_OK;
 }
 
-int launch_audience_final(const AudienceArgs& a, const AudienceWs& w, const int32_t* items, int32_t num_items,
+int launch_audience_final(const AudienceArgs& a, const AudienceState& state, const int32_t* items, int32_t num_items,
                           int32_t* top_users, float* top_scores, int32_t* pos, float* sums, cudaStream_t st) {
   if (a.M == 0) {
     if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
     return MR_OK;
   }
+  if (a.k > kTopkSmallK) {
+    int32_t* p = pos != nullptr ? pos : (sums != nullptr ? state.lg.pos : nullptr);
+    const int rc = launch_audience_large_final(a, state.lg, items, num_items, top_users, top_scores, p, st);
+    return rc != MR_OK ? rc : launch_topk_metrics(p, a.M, a.k, sums, st);
+  }
+  const AudienceWs& w = state.w;
   int32_t* p = pos != nullptr ? pos : (sums != nullptr ? w.pos : nullptr);
   const int wpc = kTopkThreads / 32;
   audience_final_kernel<<<(unsigned)(((int64_t)a.M + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, w, items, num_items,

@@ -12,7 +12,7 @@ import os
 MR_MAX_LAYERS = 8
 MR_MAX_WIDTH = 1024
 MR_MAX_NEGS = 1023
-MR_MAX_TOPK = 256
+MR_MAX_TOPK = 4096
 MR_MAX_CUTOFFS = 8
 # sums of mr_targets_scores / mr_catalogue_targets: [users, mrr] then TGT_PER_CUTOFF metrics per cutoff
 TGT_USERS, TGT_MRR, TGT_CUTOFF0, TGT_PER_CUTOFF = 0, 1, 2, 5
