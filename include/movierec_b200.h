@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MR_VERSION 106     /* major*100 + minor */
+#define MR_VERSION 107     /* major*100 + minor */
 #define MR_MAX_LAYERS 8    /* len(layers_sizes) <= 8 (model.py:75) */
 #define MR_MAX_WIDTH 1024  /* layers_sizes[i] <= 1024, mf_dim <= 1024 */
 #define MR_MAX_NEGS 1023   /* negatives per positive handled by the sampler / rank kernels */
@@ -320,6 +320,39 @@ int mr_catalogue_audience(const MrModel* model, const int32_t* items, int32_t M,
                           int64_t U, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
                           const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
                           float* scores, void* ws, size_t ws_bytes, void* stream);
+
+/* Similar items and similar users: the k nearest rows of one side (MR_SIDE_ITEMS: items, N = num_items; MR_SIDE_USERS:
+ * users, N = num_users) to each query row ids[j], exactly, in the model's scoring space (item to item "more like this",
+ * user to user look-alikes).  For a row x of the side s:
+ *   p_x = E_s[x] . W1_s  (W1_s = the side's row block of W[1]: user rows 0 .. L0/2-1, item rows L0/2 .. L0-1; linear,
+ *                         no bias: what the first hidden layer sees of x; only when n_layers >= 2)
+ *   g_x = w_out[0:mf_dim] * G_s[x]  (elementwise: what the GMF head sees of x; only when mf_dim > 0)
+ *   r_x = concat(p_x / |p_x|, g_x / |g_x|) / sqrt(n_parts)  (a part with zero norm stays zero; n_parts = the parts the
+ *                         MODEL has, 1 or 2)
+ *   sim(a, b) = r_a . r_b: the mean of the per-part cosines, in [-1, 1].
+ * A model with one layer and mf_dim == 0 has no vector to compare: MR_ERR_INVALID.  Candidates of query j: every id of
+ * [0, N) except the query itself and the exclusion list of row r = excl_ids ? excl_ids[j] : j, i.e.
+ * excl_list[excl_rowptr[r] .. excl_rowptr[r+1]) (ascending; rows outside [0, excl_rows) and excl_rowptr == NULL exclude
+ * nothing) -- mr_topk_scores' convention.  Order: descending similarity, NaN as -inf, -0 == +0, the lower id first among
+ * ties.  top_ids / top_scores (M x k, each may be NULL): -1 / NaN beyond the number of candidates and in every slot of
+ * an out-of-range query; duplicated queries are allowed.  scores (M x N, may be NULL): every similarity computed,
+ * including the query's own entry (left out of the selection only).  1 <= k <= MR_MAX_TOPK, M <= INT32_MAX; M == 0 is
+ * a no-op.  The representation is formed once per call (the first-layer part on tensor cores when the model takes
+ * them, has three layers or more and the side's MLP width equals L[1], 128 or 256; else on CUDA cores), then queries run in chunks of C = min(M, max(1, min(2^22 / N, 16384))) rows: a tcgen05 3xTF32 GEMM writes the
+ * chunk's C x N scores (<= 16 MB, L2-resident) and the top-k selection reads them.  A query's results do not depend on
+ * the other queries of a call or on chunking; deterministic; no host synchronisation, no read-back.
+ * Workspace, with L1 = L[1] (0 when n_layers == 1), f = mf_dim, D = round_up(L1 + f, 32), d = the side's MLP width:
+ *   4 N L1 (projection) + [8 d L1 when the projection takes the tensor cores] + 8 D round_up(N, 256) (the side's
+ *   operand image, TF32 hi + lo) + 8 D round_up(C, 128) (the chunk's queries) + 4 C N (the score chunk)
+ *   + mr_topk_scores' selection workspace for C rows, each term rounded up to 256 bytes.
+ * ML-20M, tower 256-128-64 + GMF 64 (D = 192): items (N = 26,744, C = 156) 72.5 MB at k = 10, 106 MB at k = 1000;
+ * users (N = 138,493, C = 30) 301 MB at k = 10, 334 MB at k = 1000. */
+enum { MR_SIDE_ITEMS = 0, MR_SIDE_USERS = 1 };
+size_t mr_similar_workspace_bytes(const MrModel* model, int32_t side, int64_t M, int32_t k);
+int mr_similar(const MrModel* model, int32_t side, const int32_t* ids, int64_t M, int32_t k, const int32_t* excl_ids,
+               int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_list,
+               int32_t* top_ids /* M x k, may be NULL */, float* top_scores /* M x k, may be NULL */,
+               float* scores /* M x N, may be NULL */, void* ws, size_t ws_bytes, void* stream);
 
 /* Top-k of ragged lists of caller-supplied scores: list u is scores[rowptr[u] .. rowptr[u+1]) (device rowptr, U + 1
  * int64, rowptr[0] = 0, non-decreasing, rowptr[U] = nnz; U and nnz <= INT32_MAX, no rows when U = 0).  Order: the

@@ -2234,6 +2234,16 @@ static bool fold_in_tc_proj(const MrModel& m, const FoldSide& sd) {
   return use_tc(m) && m.n_layers >= 3 && sd.d_o % 128 == 0 && sd.d_o <= 256 && m.L[1] == sd.d_o;
 }
 
+// Po = E_other . W1[other rows] over the other side's whole table, no bias (needs a hidden layer; pack: room for the
+// packed row block when fold_in_tc_proj).
+static int project_other_side(const MrModel& m, const FoldSide& sd, float* pack, float* Po, cudaStream_t st) {
+  if (fold_in_tc_proj(m, sd)) {
+    const int rc = launch_pack_weights(sd.W1o, sd.d_o, m.L[1], 0, pack, st);
+    return rc != MR_OK ? rc : tc_project_table(m, sd.other_mlp, sd.num_other, sd.d_o, pack, Po, st);
+  }
+  return launch_fold_in_project(sd.other_mlp, sd.num_other, sd.d_o, sd.W1o, m.L[1], Po, st);
+}
+
 struct FoldWs {
   int32_t *flags, *keys, *sorted_keys, *order;
   void* sort_ws;
@@ -2328,14 +2338,7 @@ static int fold_in_call(const MrModel* model, bool items, const int64_t* rowptr,
   rc = launch_sort_pairs(w.keys, U, bits_for((int64_t)sd.num_other + 1), w.sorted_keys, w.order, w.sort_ws,
                          w.sort_ws_bytes, st);
   if (rc == MR_OK) rc = launch_transpose_kernels(m, w.wt, st);
-  if (rc == MR_OK && m.n_layers > 1) {
-    if (fold_in_tc_proj(m, sd)) {
-      rc = launch_pack_weights(sd.W1o, sd.d_o, m.L[1], 0, w.pack_fo, st);
-      if (rc == MR_OK) rc = tc_project_table(m, sd.other_mlp, sd.num_other, sd.d_o, w.pack_fo, w.Po, st);
-    } else {
-      rc = launch_fold_in_project(sd.other_mlp, sd.num_other, sd.d_o, sd.W1o, m.L[1], w.Po, st);
-    }
-  }
+  if (rc == MR_OK && m.n_layers > 1) rc = project_other_side(m, sd, w.pack_fo, w.Po, st);
   if (rc != MR_OK) return rc;
   FoldInArgs a{};
   a.model = model;
@@ -2366,6 +2369,120 @@ int mr_fold_in_items(const MrModel* model, const int64_t* rowptr, const int32_t*
                      float* out_loss, void* ws, size_t ws_bytes, void* stream) {
   return fold_in_call(model, true, rowptr, users, M, nnz, init_items, cfg, out_item_mlp, out_item_gmf, out_loss, ws,
                       ws_bytes, stream);
+}
+
+// ---- similar items / users: the side's representation once per call (its first-layer part as fold-in projects the
+// other side, then normalised and packed as a tensor-core operand), then per chunk of queries the representation of the
+// queries, the score GEMM and the row selection without the query itself ----------------------------------------------
+struct SimilarShape {
+  FoldSide sd;       // its OTHER side is the side searched
+  int L1, f, n_parts, Dpad;
+  int64_t C, C_pad, N_pad;  // queries per chunk and the row counts of the two operand images
+};
+
+static SimilarShape similar_shape(const MrModel& m, int32_t side, int64_t M) {
+  SimilarShape s{};
+  s.sd = fold_side(m, side == MR_SIDE_USERS);
+  s.L1 = m.n_layers >= 2 ? m.L[1] : 0;
+  s.f = m.mf_dim;
+  s.n_parts = (s.L1 > 0 ? 1 : 0) + (s.f > 0 ? 1 : 0);
+  s.Dpad = (int)align_up((size_t)(s.L1 + s.f), 32);
+  const int32_t N = s.sd.num_other;
+  s.C = clamp_users(M, catalogue_chunk_users(N));
+  s.C_pad = (int64_t)align_up((size_t)s.C, kSimTileQ);
+  s.N_pad = (int64_t)align_up((size_t)N, kSimTileC);
+  return s;
+}
+
+struct SimilarWs {
+  float *P, *pack, *R, *A, *S;
+  void* topk;
+  size_t total;
+};
+
+static SimilarWs carve_similar(const MrModel& m, const SimilarShape& s, int32_t k, void* ws) {
+  SimilarWs w{};
+  Carver cv(ws);
+  const int32_t N = s.sd.num_other;
+  if (s.L1 > 0) w.P = cv.take<float>((size_t)N * s.L1);
+  if (s.L1 > 0 && fold_in_tc_proj(m, s.sd)) w.pack = cv.take<float>((size_t)2 * s.sd.d_o * s.L1);
+  w.R = cv.take<float>((size_t)2 * s.Dpad * s.N_pad);
+  w.A = cv.take<float>((size_t)2 * s.Dpad * s.C_pad);
+  w.S = cv.take<float>((size_t)s.C * N);
+  w.topk = cv.take<char>(topk_workspace_bytes(s.C, N, k));
+  w.total = cv.off;
+  return w;
+}
+
+static int similar_check(const MrModel* model, int32_t side, int64_t M, int32_t k, int32_t excl_rows,
+                         const int64_t* excl_rowptr, const int32_t* excl_list) {
+  int rc = check_model(model);
+  if (rc != MR_OK) return rc;
+  MR_REQUIRE(side == MR_SIDE_ITEMS || side == MR_SIDE_USERS, "similar: side=%d is neither MR_SIDE_ITEMS nor "
+             "MR_SIDE_USERS", side);
+  MR_REQUIRE(k >= 1 && k <= MR_MAX_TOPK, "similar: k=%d out of [1,%d]", k, MR_MAX_TOPK);
+  MR_REQUIRE(M >= 0 && M <= INT32_MAX, "similar: bad M=%lld", (long long)M);
+  MR_REQUIRE(model->n_layers >= 2 || model->mf_dim > 0, "similar: a model with one layer and mf_dim == 0 has no "
+             "vector to compare");
+  MR_REQUIRE(excl_rows >= 0 && (excl_rowptr == nullptr || excl_list != nullptr), "similar: bad exclusion lists");
+  return MR_OK;
+}
+
+size_t mr_similar_workspace_bytes(const MrModel* model, int32_t side, int64_t M, int32_t k) {
+  if (similar_check(model, side, M, k, 0, nullptr, nullptr) != MR_OK) return 0;
+  return carve_similar(*model, similar_shape(*model, side, M), k, nullptr).total;
+}
+
+int mr_similar(const MrModel* model, int32_t side, const int32_t* ids, int64_t M, int32_t k, const int32_t* excl_ids,
+               int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_list, int32_t* top_ids,
+               float* top_scores, float* scores, void* ws, size_t ws_bytes, void* stream) {
+  int rc = similar_check(model, side, M, k, excl_rows, excl_rowptr, excl_list);
+  if (rc != MR_OK) return rc;
+  if (M == 0) return MR_OK;
+  MR_REQUIRE(ids != nullptr && ws != nullptr, "similar: ids / ws is NULL");
+  const MrModel& m = *model;
+  const SimilarShape s = similar_shape(m, side, M);
+  const SimilarWs w = carve_similar(m, s, k, ws);
+  if (ws_bytes < w.total) {
+    set_error("similar workspace too small: %zu < %zu", ws_bytes, w.total);
+    return MR_ERR_WORKSPACE;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const FoldSide& sd = s.sd;
+  const int32_t N = sd.num_other;
+  prof_mark(MR_PHASE_MISC, st);
+  if (s.L1 > 0) rc = project_other_side(m, sd, w.pack, w.P, st);
+  if (rc == MR_OK)
+    rc = launch_similar_pack(w.P, s.L1, sd.other_gmf, m.w_out, s.f, N, nullptr, N, s.N_pad, s.Dpad, s.n_parts, w.R, st);
+  TopkArgs a{};
+  a.N = N;
+  a.k = k;
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_list;
+  a.users = ids;  // an out-of-range query gets -1 / NaN; the query's own id is left out of its selection
+  a.num_users = N;
+  a.top_items = top_ids;
+  a.top_scores = top_scores;
+  for (int64_t q0 = 0; q0 < M && rc == MR_OK; q0 += s.C) {
+    const int64_t c = M - q0 < s.C ? M - q0 : s.C;
+    float* out = scores != nullptr ? scores + q0 * N : w.S;
+    prof_mark(MR_PHASE_MISC, st);
+    rc = launch_similar_pack(w.P, s.L1, sd.other_gmf, m.w_out, s.f, N, ids + q0, c, s.C_pad, s.Dpad, s.n_parts, w.A,
+                             st);
+    if (rc != MR_OK) break;
+    prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+    rc = launch_similar_gemm(w.A, s.C_pad, w.R, s.N_pad, s.Dpad, c, N, out, st);
+    if (rc != MR_OK || (top_ids == nullptr && top_scores == nullptr)) continue;
+    prof_mark(MR_PHASE_RANK, st);
+    a.u0 = q0;
+    a.U = c;
+    a.scores = out;
+    rc = launch_topk(a, w.topk, st, true);
+  }
+  prof_mark(-1, st);
+  return rc;
 }
 
 int mr_users_grouped(const int32_t* users, int64_t n, int32_t group, int32_t* flag, void* stream) {

@@ -119,7 +119,8 @@ struct TopkArgs {
   int32_t* pos;
 };
 size_t topk_workspace_bytes(int64_t U, int32_t N, int32_t k);  // per chunk of U rows
-int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st);
+// skip_self (needs a.users): row u's own id a.users[u0 + u] is never a candidate (similar items / users)
+int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st, bool skip_self = false);
 // sums = {hit_sum, dcg_sum} of pos[0, U) in a fixed order, no workspace
 int launch_topk_metrics(const int32_t* pos, int64_t U, int k, float* sums, cudaStream_t st);
 // Ragged lists: list u is scores[rowptr[u] .. rowptr[u+1]) (segments clamped to [0, nnz)); keys carry the position
@@ -199,7 +200,7 @@ int launch_audience_final(const AudienceArgs& a, const AudienceState& w, const i
                           int32_t* top_users, float* top_scores, int32_t* pos, float* sums, cudaStream_t st);
 // ---- topk_large.cu: the k > kTopkSmallK counterparts, with the same arguments and results ---------------------------
 size_t topk_large_workspace_bytes(int64_t U, int32_t N);  // per chunk of U rows: the staged keys
-int launch_topk_large(const TopkArgs& a, void* ws, cudaStream_t st);
+int launch_topk_large(const TopkArgs& a, void* ws, cudaStream_t st, bool skip_self = false);
 int launch_topk_lists_large(const TopkListsArgs& a, int32_t* pos, cudaStream_t st);
 AudienceLargeWs carve_audience_large(void* ws, int64_t C, int32_t M, int32_t k, size_t& total);
 int launch_audience_large_init(const AudienceArgs& a, const AudienceLargeWs& w, cudaStream_t st);
@@ -244,6 +245,21 @@ int launch_targets_chunk(const TargetsArgs& a, const TargetsWs& w, cudaStream_t 
 // sums (MR_TGT_* layout, may be NULL) from the positions of all U rows, in a fixed order
 int launch_targets_metrics(const int64_t* tgt_rowptr, int64_t U, int64_t nnz_t, const int32_t* spos,
                            const TargetCutoffs& ks, float* sums, double* partials, cudaStream_t st);
+
+// ---- similar.cu: k nearest neighbours of rows of one side in the model's scoring space -----------------------------
+// Operand images hold rows in tiles of kSimTileQ (queries) or kSimTileC (candidates) rows, Dpad (a multiple of 32)
+// columns: [Dpad / 32 chunks][hi, lo][rows x 32] floats in core-matrix order, as launch_pack_weights lays out weights.
+constexpr int kSimTileQ = 128, kSimTileC = 256;
+// Rows [0, rows_pad) of an image: row n is the representation of table row ids[n] (ids NULL: n) for n < count and an
+// id in [0, num_rows); zeros otherwise.  P: (num_rows x L1) first-layer part (L1 = 0: none); G (num_rows x f) and
+// w_gmf (f): the GMF part; n_parts = the parts the model has (1 or 2).
+int launch_similar_pack(const float* P, int L1, const float* G, const float* w_gmf, int f, int32_t num_rows,
+                        const int32_t* ids, int64_t count, int64_t rows_pad, int Dpad, int n_parts, float* img,
+                        cudaStream_t st);
+// out (C x N row-major) = A . B^T over the first C rows of the query image (a_rows rows) and the first N rows of the
+// candidate image (b_rows rows)
+int launch_similar_gemm(const float* a_img, int64_t a_rows, const float* b_img, int64_t b_rows, int Dpad, int64_t C,
+                        int32_t N, float* out, cudaStream_t st);
 
 // ---- sampler.cu ------------------------------------------------------------------------------
 int launch_sample_negatives(const int64_t* rowptr, const int32_t* csr_items, int32_t num_items,

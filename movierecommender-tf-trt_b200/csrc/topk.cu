@@ -99,6 +99,8 @@ __device__ __forceinline__ void topk_merge_warp(const unsigned long long* lists,
   }
 }
 
+// SKIP_SELF: the row's own id a.users[gu] is never a candidate (similar items / users).
+template <bool SKIP_SELF>
 __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs a, int S, int slice, int cap,
                                                                   unsigned long long* __restrict__ lists,
                                                                   int32_t* __restrict__ counts) {
@@ -118,12 +120,14 @@ __global__ void __launch_bounds__(kTopkThreads) topk_slice_kernel(const TopkArgs
   const int t = a.targets != nullptr ? __ldg(a.targets + gu) : -1;
   const bool has_t = (unsigned)t < (unsigned)N;
   const unsigned long long key_t = has_t ? topk_key(__ldg(row + t), t) : 0ull;
+  const int self = SKIP_SELF ? __ldg(a.users + gu) : -1;
   int below = 0, n = 0;
   unsigned long long thr = kNoKey;
   for (int c = lo; c < hi; c += 32) {
     const uint32_t xmask = list_mask(a.excl_items, ep, ee, c, lane);  // excluded items of [c, c + 32)
     const int item = c + lane;
-    const bool cand = item < hi && (!((xmask >> lane) & 1u) || item == t);  // the target is never excluded
+    const bool cand = item < hi && (!((xmask >> lane) & 1u) || item == t) &&  // the target is never excluded
+                      (!SKIP_SELF || item != self);
     const unsigned long long key = cand ? topk_key(__ldg(row + item), item) : kNoKey;
     below += (has_t && key < key_t) ? 1 : 0;
     topk_push(buf, n, thr, key, cap, k, lane);
@@ -157,16 +161,19 @@ __global__ void __launch_bounds__(kTopkThreads) topk_merge_kernel(const TopkArgs
   }
 }
 
-int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st) {
+int launch_topk(const TopkArgs& a, void* ws, cudaStream_t st, bool skip_self) {
   if (a.U == 0) return MR_OK;
-  if (a.k > kTopkSmallK) return launch_topk_large(a, ws, st);
+  if (skip_self && a.users == nullptr) return MR_ERR_INVALID;
+  if (a.k > kTopkSmallK) return launch_topk_large(a, ws, st, skip_self);
   const int S = topk_slices(a.N), slice = topk_slice_len(a.N), cap = topk_cap(a.k);
   Carver cv(ws);
   unsigned long long* lists = cv.take<unsigned long long>((size_t)a.U * S * a.k);
   int32_t* counts = cv.take<int32_t>((size_t)a.U * S);
   const int wpc = kTopkThreads / 32;
   const size_t smem = (size_t)wpc * cap * sizeof(unsigned long long);  // <= 16 KB (cap <= 512)
-  topk_slice_kernel<<<(unsigned)((a.U * S + wpc - 1) / wpc), kTopkThreads, smem, st>>>(a, S, slice, cap, lists, counts);
+  const unsigned grid = (unsigned)((a.U * S + wpc - 1) / wpc);
+  if (skip_self) topk_slice_kernel<true><<<grid, kTopkThreads, smem, st>>>(a, S, slice, cap, lists, counts);
+  else topk_slice_kernel<false><<<grid, kTopkThreads, smem, st>>>(a, S, slice, cap, lists, counts);
   MR_LAUNCH_CHECK("topk_slice_kernel");
   topk_merge_kernel<<<(unsigned)((a.U + wpc - 1) / wpc), kTopkThreads, 0, st>>>(a, S, lists, counts);
   MR_LAUNCH_CHECK("topk_merge_kernel");

@@ -184,6 +184,9 @@ __device__ void lg_sort(unsigned long long* keys, int* vals, int m, int cap) {
 }
 
 // ---- rows --------------------------------------------------------------------------------------------------------
+// SKIP_SELF: the row's own id a.users[gu] is never a candidate (similar items / users).  Launched with kLgThreads or
+// kLgWideThreads threads.
+template <bool SKIP_SELF>
 __global__ void __launch_bounds__(kLgWideThreads) topk_large_rows_kernel(const TopkArgs a, int cap,
                                                                      unsigned long long* __restrict__ stage) {
   extern __shared__ unsigned long long lg_keys[];
@@ -205,11 +208,13 @@ __global__ void __launch_bounds__(kLgWideThreads) topk_large_rows_kernel(const T
     const int lo = (int)min((int64_t)warp * slice, (int64_t)N), hi = (int)min((int64_t)lo + slice, (int64_t)N);
     int64_t ep, ee;
     excl_cursor(a.excl_ids, a.excl_rows, a.excl_rowptr, a.excl_items, gu, lo, ep, ee);
+    const int self = SKIP_SELF ? __ldg(a.users + gu) : -1;
     int below = 0;
     for (int c = lo; c < hi; c += 32) {
       const uint32_t xmask = list_mask(a.excl_items, ep, ee, c, lane);
       const int item = c + lane;
-      const bool cand = item < hi && (!((xmask >> lane) & 1u) || item == t);  // the target is never excluded
+      const bool cand = item < hi && (!((xmask >> lane) & 1u) || item == t) &&  // the target is never excluded
+                        (!SKIP_SELF || item != self);
       const unsigned long long key = cand ? topk_key(__ldg(row + item), item) : kNoKey;
       if (item < hi) keys[item] = key;
       below += (has_t && key < key_t) ? 1 : 0;
@@ -235,11 +240,13 @@ size_t topk_large_workspace_bytes(int64_t U, int32_t N) {
   return align_up((size_t)(U < 1 ? 1 : U) * N * sizeof(unsigned long long), 256);
 }
 
-int launch_topk_large(const TopkArgs& a, void* ws, cudaStream_t st) {
+int launch_topk_large(const TopkArgs& a, void* ws, cudaStream_t st, bool skip_self) {
   const int cap = lg_cap(a.k);
   const int threads = a.N >= kLgWideRow ? kLgWideThreads : kLgThreads;
-  topk_large_rows_kernel<<<(unsigned)a.U, threads, (size_t)cap * sizeof(unsigned long long), st>>>(
-      a, cap, static_cast<unsigned long long*>(ws));
+  const size_t smem = (size_t)cap * sizeof(unsigned long long);
+  unsigned long long* stage = static_cast<unsigned long long*>(ws);
+  if (skip_self) topk_large_rows_kernel<true><<<(unsigned)a.U, threads, smem, st>>>(a, cap, stage);
+  else topk_large_rows_kernel<false><<<(unsigned)a.U, threads, smem, st>>>(a, cap, stage);
   MR_LAUNCH_CHECK("topk_large_rows_kernel");
   return MR_OK;
 }

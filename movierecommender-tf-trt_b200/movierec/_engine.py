@@ -602,6 +602,38 @@ class NeuMFEngine(object):
         self.last_catalogue_bad = bad
         return top_users, top_scores, pos, sums, full, (None if pool is None else d_pool[:U])
 
+    def similar(self, ids, k, side="items", exclude=None, excl_ids=None, want_scores=False):
+        """The k nearest items (side "items") or users (side "users") to each of `ids` (mr_similar): similarity is the
+        mean of two cosines -- of the rows' first-hidden-layer parts E[x] . W1[side rows] and of their GMF parts
+        w_out[:mf_dim] * G[x] -- ordered by descending similarity, the lower id first among ties, leaving out the query
+        itself and its exclusion list.  exclude: None or (rowptr int64, ids int32) of ascending lists (host or device);
+        query j uses list excl_ids[j] (default j).  Returns device tensors (ids (M, k) int32, similarities (M, k)
+        float32, scores_full (M, N) float32 or None); slots beyond the number of candidates, and every slot of an
+        out-of-range query, hold -1 / NaN.  Raises ValueError on a malformed exclusion CSR or a model without a hidden
+        layer and without GMF, before any launch."""
+        if side not in ("items", "users"):
+            raise ValueError("side must be 'items' or 'users', found {!r}".format(side))
+        dev = self.device
+        ids = as_device_i32(ids, dev)
+        M = ids.numel()
+        k = int(k)
+        code, N = (nat.SIDE_ITEMS, self.num_items) if side == "items" else (nat.SIDE_USERS, self.num_users)
+        rowptr, excl, excl_rows = _audience_exclusion(exclude, dev)
+        e_ids = as_device_i32(excl_ids, dev) if excl_ids is not None else None
+        if e_ids is not None and e_ids.numel() != M:
+            raise ValueError("excl_ids ({}) and ids ({}) differ in length".format(e_ids.numel(), M))
+        nbytes = int(nat.lib.mr_similar_workspace_bytes(C.byref(self._model), code, M, k))
+        if nbytes == 0:
+            raise ValueError("similar: M={} k={} side={}: {}".format(M, k, side, nat.last_error()))
+        top_ids = torch.empty((M, k), dtype=torch.int32, device=dev)
+        top_scores = torch.empty((M, k), dtype=torch.float32, device=dev)
+        full = torch.empty((M, N), dtype=torch.float32, device=dev) if want_scores else None
+        ws = self._workspace(nbytes)
+        nat.check(nat.lib.mr_similar(C.byref(self._model), code, _ptr(ids if M else None), M, k, _ptr(e_ids), excl_rows,
+                                     _ptr(rowptr), _ptr(excl), _ptr(top_ids), _ptr(top_scores), _ptr(full), _ptr(ws),
+                                     ws.numel(), self._stream()), "mr_similar")
+        return top_ids, top_scores, full
+
     def rank_lists(self, users, lists, k, targets=None, want_probs=False):
         """Score and rank ragged candidate lists in one call (mr_rank_lists): list u pairs users[u] with
         items[rowptr[u]:rowptr[u + 1]].  lists = (rowptr int64 (U + 1,), items int32 (nnz,)), host or device; targets

@@ -14,6 +14,7 @@ MR_MAX_WIDTH = 1024
 MR_MAX_NEGS = 1023
 MR_MAX_TOPK = 4096
 MR_MAX_CUTOFFS = 8
+SIDE_ITEMS, SIDE_USERS = 0, 1  # MR_SIDE_ITEMS / MR_SIDE_USERS of mr_similar
 # sums of mr_targets_scores / mr_catalogue_targets: [users, mrr] then TGT_PER_CUTOFF metrics per cutoff
 TGT_USERS, TGT_MRR, TGT_CUTOFF0, TGT_PER_CUTOFF = 0, 1, 2, 5
 TGT_METRICS = ("hr", "precision", "recall", "ndcg", "map")  # MR_TGT_HIT .. MR_TGT_MAP
@@ -113,6 +114,8 @@ SIGNATURES = {
     "mr_catalogue_audience_workspace_bytes": (_sz, [_PM, _i64, _i32, _i32]),
     "mr_catalogue_audience": (C.c_int, [_PM, _vp, _i32, _i32, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                         _sz, _vp]),
+    "mr_similar_workspace_bytes": (_sz, [_PM, _i32, _i64, _i32]),
+    "mr_similar": (C.c_int, [_PM, _i32, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_topk_lists_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "mr_topk_lists": (C.c_int, [_vp, _i64, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mr_rank_lists_workspace_bytes": (_sz, [_PM, _i64, _i64, _i32]),

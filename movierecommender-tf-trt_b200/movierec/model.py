@@ -201,6 +201,26 @@ class NeuMFModel(object):
         self._raise_on_bad_ids(float(eng.last_catalogue_bad.item()))
         return top.cpu().numpy(), scores.cpu().numpy()
 
+    def similar_items(self, items, top_k=10, exclude=None):
+        """The top_k items most like each of `items` ("more like this"): descending similarity -- the mean of the cosines
+        of the two items' first-hidden-layer parts and of their GMF parts, in [-1, 1] --, the lower item id first among
+        ties, never the query item itself.  exclude: None or a (rowptr, items) pair of ascending lists, list j for
+        query j.  Returns NumPy (items (M, top_k) int32, similarities (M, top_k) float32); slots beyond the number of
+        candidates hold -1 / NaN.  One device call for all queries.  Raises IndexError on an out-of-range item."""
+        return self._similar(items, top_k, exclude, "items")
+
+    def similar_users(self, users, top_k=10, exclude=None):
+        """similar_items for users ("people like you"): the top_k users most like each of `users`, by the same
+        similarity of their first-hidden-layer and GMF parts.  Raises IndexError on an out-of-range user."""
+        return self._similar(users, top_k, exclude, "users")
+
+    def _similar(self, ids, top_k, exclude, side):
+        ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+        eng = self.engine
+        self._raise_on_bad_ids(_ids_outside(ids, eng.num_items if side == "items" else eng.num_users))
+        top, sims, _ = eng.similar(ids.astype(np.int32), top_k, side=side, exclude=exclude)
+        return top.cpu().numpy(), sims.cpu().numpy()
+
     def recommend_batch(self, users, candidate_lists, top_k=10):
         """recommend() for many requests at once: user users[u] against its own candidate list, of any length.
         candidate_lists: a list (or other sequence) of 1-D item arrays, one per user, or a tuple (rowptr, items) of
