@@ -1407,17 +1407,24 @@ static int topk_check(int64_t U, int32_t N, int32_t k, int32_t excl_rows, const 
   return MR_OK;
 }
 
-// The chunk loop of the catalogue calls: per chunk of C users, the probabilities of every (user, item) pair through the
-// plan's tower, then select(u0, users in the chunk, probabilities) under MR_PHASE_RANK.  The items are the catalogue,
-// or with `items` the list items[0, M) (chunk row r pairs user r / M with items[r % M]; the item half of the first
-// layer is still projected once over the whole table).  users == NULL: user u is id u.  The probabilities go to
-// scores + u0 * N (N = the items per user) when scores is given, else to the sweep's buffer (C x N).
-// ws: catalogue_sweep_bytes(m, C, N, users == NULL) bytes.  mr_catalogue_topk, mr_catalogue_targets and
-// mr_catalogue_audience all score through here, so a pair's probability is the same in all of them by construction.
+// The chunk loop of every serving query over users: per chunk of C users, select(u0, users in the chunk, the chunk's
+// scores).  model == NULL: the scores are the caller's U x N matrix, read at scores + u0 * N under MR_PHASE_RANK.
+// Otherwise they are the model's probabilities of every (user, item) pair through the plan's tower, each chunk's
+// selection under MR_PHASE_RANK.  The items are the catalogue (N = num_items), or with `items` the list items[0, N)
+// (chunk row r pairs user r / N with items[r % N]; the item half of the first layer is still projected once over the
+// whole table).  users == NULL: user u is id u.  The probabilities go to scores + u0 * N when scores is given, else to
+// the sweep's buffer (C x N).  ws: catalogue_sweep_bytes(m, C, N, users == NULL) bytes.  Every model query scores
+// through here, so a pair's probability is the same in all of them by construction.
 template <class Select>
-static int catalogue_sweep(const MrModel& m, const int32_t* users, int64_t U, int64_t C, float* scores, void* ws,
-                           cudaStream_t st, Select select, const int32_t* items = nullptr, int32_t M = 0) {
-  const int32_t N = items != nullptr ? M : m.num_items;
+static int catalogue_sweep(const MrModel* model, const int32_t* users, int64_t U, int64_t C, int32_t N, float* scores,
+                           void* ws, cudaStream_t st, Select select, const int32_t* items = nullptr) {
+  int rc = MR_OK;
+  if (model == nullptr) {
+    prof_mark(MR_PHASE_RANK, st);
+    for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) rc = select(u0, U - u0 < C ? U - u0 : C, scores + u0 * N);
+    return rc;
+  }
+  const MrModel& m = *model;
   const EvalPlan p = catalogue_plan(m, C, N);
   Carver cv(ws);
   int32_t* iota = cv.take<int32_t>((size_t)C * N);
@@ -1425,7 +1432,7 @@ static int catalogue_sweep(const MrModel& m, const int32_t* users, int64_t U, in
   int32_t* own_users = users == nullptr ? cv.take<int32_t>((size_t)C) : nullptr;
   const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
   prof_mark(MR_PHASE_MISC, st);
-  int rc = items != nullptr ? launch_tile_list(iota, C * N, items, N, st) : launch_tile_iota(iota, C * N, N, st);
+  rc = items != nullptr ? launch_tile_list(iota, C * N, items, N, st) : launch_tile_iota(iota, C * N, N, st);
   if (rc == MR_OK) rc = eval_prepare(m, p, w, users, st);
   for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
     const int64_t c = U - u0 < C ? U - u0 : C;
@@ -1474,6 +1481,15 @@ static int targets_check(int64_t U, int32_t N, int32_t excl_rows, const int64_t*
   return MR_OK;
 }
 
+static int audience_check(int64_t U, int32_t M, int32_t k, int32_t excl_rows, const int64_t* excl_rowptr,
+                          const int32_t* excl_users, const int32_t* targets, const int32_t* pos, const float* sums) {
+  MR_REQUIRE(U >= 0 && U <= INT32_MAX && M >= 0, "audience: bad U=%lld M=%d", (long long)U, M);
+  MR_REQUIRE(k >= 1 && k <= MR_MAX_TOPK, "audience: k=%d out of [1,%d]", k, MR_MAX_TOPK);
+  MR_REQUIRE(excl_rows >= 0 && (excl_rowptr == nullptr || excl_users != nullptr), "audience: bad exclusion lists");
+  MR_REQUIRE(targets != nullptr || (pos == nullptr && sums == nullptr), "audience: pos / sums need targets");
+  return MR_OK;
+}
+
 // ---- ragged candidate lists: list u pairs users[u] with items[rowptr[u] .. rowptr[u+1]) ------------------------------
 static int lists_check(int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
                        const int32_t* pos, const float* sums) {
@@ -1484,6 +1500,272 @@ static int lists_check(int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k,
   MR_REQUIRE(targets != nullptr || (pos == nullptr && sums == nullptr), "lists: pos / sums need targets");
   MR_REQUIRE(U == 0 || rowptr != nullptr, "lists: rowptr is NULL");
   return MR_OK;
+}
+
+
+// ---- serving queries: one body per query --------------------------------------------------------------------------
+// Each query runs on the caller's scores (model == NULL: mr_topk_scores, mr_targets_scores, mr_audience_scores,
+// mr_topk_lists) or on the model's probabilities (mr_catalogue_topk, mr_catalogue_targets, mr_catalogue_audience,
+// mr_rank_lists); catalogue_sweep is the one chunk loop of both.  `fn` names the call in error messages.  A model
+// call's workspace adds the scoring's and 512 bytes of carving slack to the selection's; a matrix call's adds 256.
+
+static int workspace_check(const char* fn, size_t ws_bytes, size_t need) {
+  if (ws_bytes >= need) return MR_OK;
+  set_error("%s workspace too small: %zu < %zu", fn, ws_bytes, need);
+  return MR_ERR_WORKSPACE;
+}
+
+// What a model's workspace query needs of it (0 bytes otherwise); lists and targets also need a first layer to split.
+static bool serving_model_ok(const MrModel* model, bool split_first_layer) {
+  return model != nullptr && model->n_layers >= 1 && model->n_layers <= MR_MAX_LAYERS && model->num_items >= 1 &&
+         model->num_users >= 1 && (!split_first_layer || model->L[0] >= 2);
+}
+
+static size_t topk_bytes(const MrModel* model, int64_t U, int32_t N, int32_t k) {
+  if (U < 0 || N < 1 || k < 1 || k > MR_MAX_TOPK) return 0;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
+  if (model == nullptr) return topk_workspace_bytes(C, N, k) + 256;
+  return align_up(topk_workspace_bytes(C, N, k), 256) + catalogue_sweep_bytes(*model, C, N) + 512;
+}
+
+// Top-k per row: row u is users[u] against the catalogue (model) or row u of the matrix; exclusion list excl_ids[u].
+static int topk_query(const char* fn, const MrModel* model, float* scores, int32_t N, const int32_t* users,
+                      int32_t num_users, int64_t U, int32_t k, const int32_t* excl_ids, int32_t excl_rows,
+                      const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
+                      float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, cudaStream_t st) {
+  int rc = topk_check(U, N, k, excl_rows, excl_rowptr, excl_items, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  if (U == 0) {
+    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
+    return MR_OK;
+  }
+  MR_REQUIRE((model != nullptr ? users != nullptr : scores != nullptr) && ws != nullptr, "%s: %s / ws is NULL", fn,
+             model != nullptr ? "users" : "scores");
+  rc = workspace_check(fn, ws_bytes, topk_bytes(model, U, N, k));
+  if (rc != MR_OK) return rc;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
+  Carver cv(ws);
+  void* sel_ws = cv.take<char>(topk_workspace_bytes(C, N, k));
+  TopkArgs a{};
+  a.N = N;
+  a.k = k;
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_items;
+  a.targets = targets;
+  a.users = users;
+  a.num_users = num_users;
+  a.top_items = top_items;
+  a.top_scores = top_scores;
+  a.pos = pos;
+  rc = catalogue_sweep(model, users, U, C, N, scores, static_cast<char*>(ws) + cv.off, st,
+                       [&](int64_t u0, int64_t c, const float* out) {
+                         a.u0 = u0;
+                         a.U = c;
+                         a.scores = out;
+                         return launch_topk(a, sel_ws, st);
+                       });
+  if (rc == MR_OK) {
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_topk_metrics(pos, U, k, sums, st);
+  }
+  prof_mark(-1, st);
+  return rc;
+}
+
+static size_t targets_bytes(const MrModel* model, int64_t U, int32_t N, int64_t nnz_t) {
+  if (U < 0 || U > INT32_MAX || N < 1 || nnz_t < 0 || nnz_t > INT32_MAX) return 0;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
+  const size_t sel = targets_workspace_bytes(C, nnz_t) + 256;
+  return model == nullptr ? sel : align_up(sel, 256) + catalogue_sweep_bytes(*model, C, N) + 512;
+}
+
+// Places of many targets per row; rows and exclusion lists as topk_query.
+static int targets_query(const char* fn, const MrModel* model, float* scores, int32_t N, const int32_t* users,
+                         int32_t num_users, int64_t U, const int32_t* excl_ids, int32_t excl_rows,
+                         const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
+                         const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks, int32_t n_ks, int32_t* tpos,
+                         float* sums, void* ws, size_t ws_bytes, cudaStream_t st) {
+  TargetCutoffs cut{};
+  int rc = targets_check(U, N, excl_rows, excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums,
+                         cut);
+  if (rc != MR_OK) return rc;
+  // A model call without users needs no users or workspace; a matrix call without rows still wants its workspace and
+  // zeroes the sums in launch_targets_metrics.
+  if (model != nullptr && U == 0) {
+    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, (MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * n_ks) * sizeof(float), st));
+    return MR_OK;
+  }
+  MR_REQUIRE(U == 0 || (model != nullptr ? users != nullptr : scores != nullptr), "%s: %s is NULL", fn,
+             model != nullptr ? "users" : "scores");
+  MR_REQUIRE(ws != nullptr, "%s: workspace is NULL", fn);
+  rc = workspace_check(fn, ws_bytes, targets_bytes(model, U, N, nnz_t));
+  if (rc != MR_OK) return rc;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
+  Carver cv(ws);
+  const TargetsWs w = carve_targets(cv.take<char>(targets_bytes(nullptr, U, N, nnz_t)), C, nnz_t);
+  TargetsArgs a{};
+  a.N = N;
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_items = excl_items;
+  a.tgt_rowptr = tgt_rowptr;
+  a.tgt_items = tgt_items;
+  a.nnz_t = nnz_t;
+  a.users = users;
+  a.num_users = num_users;
+  a.tpos = tpos;
+  rc = catalogue_sweep(model, users, U, C, N, scores, static_cast<char*>(ws) + cv.off, st,
+                       [&](int64_t u0, int64_t c, const float* out) {
+                         a.u0 = u0;
+                         a.U = c;
+                         a.scores = out;
+                         return launch_targets_chunk(a, w, st);
+                       });
+  if (rc == MR_OK) {
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
+  }
+  prof_mark(-1, st);
+  return rc;
+}
+
+static size_t audience_bytes(const MrModel* model, int64_t U, int32_t M, int32_t k) {
+  if (U < 0 || U > INT32_MAX || M < 0 || k < 1 || k > MR_MAX_TOPK) return 0;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
+  const size_t sel = carve_audience(nullptr, C, M, k).total;  // the running lists of every item
+  if (model == nullptr) return sel + 256;
+  return align_up(sel, 256) + catalogue_sweep_bytes(*model, C, M < 1 ? 1 : M, true) + 512;
+}
+
+// Audiences: the k best of U pool users (users, NULL = ids 0 .. U-1) for each of M columns: the matrix's columns, or
+// the model's items[0, M) (which also index the exclusion lists).
+static int audience_query(const char* fn, const MrModel* model, float* scores, const int32_t* items, int32_t M,
+                          int32_t k, const int32_t* users, int32_t num_users, int64_t U, const int32_t* excl_ids,
+                          int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
+                          const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
+                          void* ws, size_t ws_bytes, cudaStream_t st) {
+  int rc = audience_check(U, M, k, excl_rows, excl_rowptr, excl_users, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  if (model != nullptr) {
+    MR_REQUIRE(users != nullptr || U == model->num_users, "%s: without a pool U must be num_users (%d), got %lld", fn,
+               model->num_users, (long long)U);
+    MR_REQUIRE((M == 0 || items != nullptr) && ws != nullptr, "%s: items / ws is NULL", fn);
+  } else {
+    MR_REQUIRE((U == 0 || M == 0 || scores != nullptr) && ws != nullptr, "%s: scores / ws is NULL", fn);
+  }
+  rc = workspace_check(fn, ws_bytes, audience_bytes(model, U, M, k));
+  if (rc != MR_OK) return rc;
+  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
+  Carver cv(ws);
+  const AudienceState w = carve_audience(cv.take<char>(carve_audience(nullptr, C, M, k).total), C, M, k);
+  AudienceArgs a{};
+  a.M = M;
+  a.k = k;
+  a.users = users;
+  a.num_users = num_users;
+  a.excl_ids = excl_ids;
+  a.excl_rows = excl_rows;
+  a.excl_rowptr = excl_rowptr;
+  a.excl_users = excl_users;
+  a.targets = targets;
+  if (M > 0) {
+    rc = launch_audience_init(a, w, st);
+    if (rc == MR_OK)
+      rc = catalogue_sweep(model, users, U, C, M, scores, static_cast<char*>(ws) + cv.off, st,
+                           [&](int64_t u0, int64_t c, const float* out) {
+                             a.u0 = u0;
+                             a.U = c;
+                             a.scores = out;
+                             return launch_audience_chunk(a, w, st);
+                           },
+                           items);
+  }
+  if (rc == MR_OK) {
+    prof_mark(MR_PHASE_RANK, st);
+    rc = launch_audience_final(a, w, items, model != nullptr ? model->num_items : 0, top_users, top_scores, pos, sums,
+                               st);
+  }
+  prof_mark(-1, st);
+  return rc;
+}
+
+static size_t lists_bytes(const MrModel* model, int64_t U, int64_t nnz, int32_t k) {
+  if (U < 0 || U > INT32_MAX || nnz < 0 || nnz > INT32_MAX || k < 1 || k > MR_MAX_TOPK) return 0;
+  const size_t sel = topk_lists_workspace_bytes(U, nnz, k) + 256;
+  if (model == nullptr) return sel;
+  return sel + align_up((size_t)nnz * sizeof(int32_t), 256) + align_up((size_t)nnz * sizeof(float), 256) +
+         eval_carve(*model, eval_plan(*model, SCORE_LISTS, U, 0, nnz), nullptr).total + 256;
+}
+
+// Top-k of ragged lists: list u is rows rowptr[u] .. rowptr[u+1] of the caller's scores (model == NULL), or pairs
+// users[u] with items[rowptr[u] .. rowptr[u+1]) and is scored first (into scores when given).
+static int lists_query(const char* fn, const MrModel* model, float* scores, const int32_t* users, int64_t U,
+                       const int64_t* rowptr, const int32_t* items, int64_t nnz, int32_t k, const int32_t* targets,
+                       int32_t* top_pos, int32_t* top_items, float* top_scores, int32_t* pos, float* sums, void* ws,
+                       size_t ws_bytes, cudaStream_t st) {
+  int rc = lists_check(U, rowptr, nnz, k, targets, pos, sums);
+  if (rc != MR_OK) return rc;
+  if (model != nullptr) MR_REQUIRE(U == 0 || users != nullptr, "%s: users is NULL", fn);
+  MR_REQUIRE(nnz == 0 || (model != nullptr ? items != nullptr : scores != nullptr), "%s: %s is NULL", fn,
+             model != nullptr ? "items" : "scores");
+  MR_REQUIRE(ws != nullptr, "%s: workspace is NULL", fn);
+  rc = workspace_check(fn, ws_bytes, lists_bytes(model, U, nnz, k));
+  if (rc != MR_OK) return rc;
+  Carver cv(ws);
+  void* sel_ws = cv.take<char>(topk_lists_workspace_bytes(U, nnz, k));
+  if (model != nullptr) {
+    const MrModel& m = *model;
+    int32_t* seg = cv.take<int32_t>((size_t)nnz);
+    float* probs_buf = cv.take<float>((size_t)nnz);
+    if (scores == nullptr) scores = probs_buf;
+    const EvalPlan p = eval_plan(m, SCORE_LISTS, U, 0, nnz);
+    const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
+    if (nnz > 0) {
+      prof_mark(MR_PHASE_MISC, st);
+      // seg: the list of each row, or the user of each row (plain forward)
+      rc = launch_list_rows(rowptr, U, nnz, p.tower == EVAL_FORWARD ? users : nullptr, seg, st);
+      if (rc == MR_OK) rc = eval_prepare(m, p, w, users, st);
+      if (rc == MR_OK && p.tower == EVAL_SMALL) prof_mark(MR_PHASE_FUSED_TILE, st);
+      for (int64_t r0 = 0; r0 < nnz && rc == MR_OK; r0 += p.sb) {
+        const int64_t r1 = r0 + p.sb < nnz ? r0 + p.sb : nnz;
+        if (p.tower == EVAL_TC) {  // the second layer's producers compute relu(Pi[items[row]] + Zu[seg[row]])
+          prof_mark(MR_PHASE_TC_DENSE_FWD, st);
+          rc = tc_forward_rows(m, w.t, users, items, 1, r0, r1, st, 0, false, p.head_dot, seg, (int32_t)U);
+          if (rc != MR_OK) break;
+          prof_mark(MR_PHASE_HEAD, st);
+          rc = launch_catalogue_head(m, w.t.H[m.n_layers - 1], users, r1 - r0, 1, scores, st, seg, items, r0, U);
+        } else if (p.tower == EVAL_SMALL) {
+          rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, users, items + r0, r1 - r0, 1, scores + r0, st, seg + r0,
+                                          U);
+        } else {
+          rc = mr_neumf_forward(model, seg + r0, items + r0, r1 - r0, 1, nullptr, scores + r0, nullptr, nullptr, w.fwd,
+                                w.fwd_bytes, st);
+        }
+      }
+      if (rc != MR_OK) return rc;
+    }
+  }
+  TopkListsArgs a{};
+  a.scores = scores;
+  a.rowptr = rowptr;
+  a.U = U;
+  a.nnz = nnz;
+  a.k = k;
+  a.targets = targets;
+  a.users = users;
+  a.num_users = model != nullptr ? model->num_users : 0;
+  a.items = items;
+  a.top_pos = top_pos;
+  a.top_items = top_items;
+  a.top_scores = top_scores;
+  a.pos = pos;
+  prof_mark(MR_PHASE_RANK, st);
+  rc = launch_topk_lists(a, sums, sel_ws, st);
+  prof_mark(-1, st);
+  return rc;
 }
 
 }  // namespace mr
@@ -1780,438 +2062,107 @@ int mr_rank_scores(const float* scores, int64_t G, int32_t group, int32_t k, con
                             labels);
 }
 
-size_t mr_topk_scores_workspace_bytes(int64_t U, int32_t N, int32_t k) {
-  if (U < 0 || N < 1 || k < 1 || k > MR_MAX_TOPK) return 0;
-  return topk_workspace_bytes(clamp_users(U, catalogue_chunk_users(N)), N, k) + 256;
-}
+// The matrix calls only read `scores`; the bodies take it writable for the model calls' optional full-score output.
+size_t mr_topk_scores_workspace_bytes(int64_t U, int32_t N, int32_t k) { return topk_bytes(nullptr, U, N, k); }
 
 int mr_topk_scores(const float* scores, int64_t U, int32_t N, int32_t k, const int32_t* excl_ids, int32_t excl_rows,
                    const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
                    float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream) {
-  int rc = topk_check(U, N, k, excl_rows, excl_rowptr, excl_items, targets, pos, sums);
-  if (rc != MR_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (U == 0) {
-    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
-    return MR_OK;
-  }
-  MR_REQUIRE(scores != nullptr && ws != nullptr, "topk_scores: scores / ws is NULL");
-  if (ws_bytes < mr_topk_scores_workspace_bytes(U, N, k)) {
-    set_error("topk_scores workspace too small: %zu < %zu", ws_bytes, mr_topk_scores_workspace_bytes(U, N, k));
-    return MR_ERR_WORKSPACE;
-  }
-  const int64_t C = catalogue_chunk_users(N);
-  TopkArgs a{};
-  a.N = N;
-  a.k = k;
-  a.excl_ids = excl_ids;
-  a.excl_rows = excl_rows;
-  a.excl_rowptr = excl_rowptr;
-  a.excl_items = excl_items;
-  a.targets = targets;
-  a.top_items = top_items;
-  a.top_scores = top_scores;
-  a.pos = pos;
-  prof_mark(MR_PHASE_RANK, st);
-  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
-    a.u0 = u0;
-    a.U = U - u0 < C ? U - u0 : C;
-    a.scores = scores + u0 * N;
-    rc = launch_topk(a, ws, st);
-  }
-  if (rc == MR_OK) rc = launch_topk_metrics(pos, U, k, sums, st);
-  prof_mark(-1, st);
-  return rc;
+  return topk_query("topk_scores", nullptr, const_cast<float*>(scores), N, nullptr, 0, U, k, excl_ids, excl_rows,
+                    excl_rowptr, excl_items, targets, top_items, top_scores, pos, sums, ws, ws_bytes,
+                    (cudaStream_t)stream);
 }
 
 size_t mr_catalogue_topk_workspace_bytes(const MrModel* model, int64_t U, int32_t k) {
-  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
-      model->num_users < 1 || U < 0 || k < 1 || k > MR_MAX_TOPK)
-    return 0;
-  const MrModel& m = *model;
-  const int64_t C = clamp_users(U, catalogue_chunk_users(m.num_items));
-  return align_up(topk_workspace_bytes(C, m.num_items, k), 256) + catalogue_sweep_bytes(m, C, m.num_items) + 512;
+  return serving_model_ok(model, false) ? topk_bytes(model, U, model->num_items, k) : 0;
 }
 
 int mr_catalogue_topk(const MrModel* model, const int32_t* users, int64_t U, int32_t k, int32_t excl_rows,
                       const int64_t* excl_rowptr, const int32_t* excl_items, const int32_t* targets, int32_t* top_items,
                       float* top_scores, int32_t* pos, float* sums, float* scores, void* ws, size_t ws_bytes,
                       void* stream) {
-  int rc = check_model(model);
+  const int rc = check_model(model);
   if (rc != MR_OK) return rc;
-  const MrModel& m = *model;
-  const int32_t N = m.num_items;
-  rc = topk_check(U, N, k, excl_rows, excl_rowptr, excl_items, targets, pos, sums);
-  if (rc != MR_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (U == 0) {
-    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
-    return MR_OK;
-  }
-  MR_REQUIRE(users != nullptr && ws != nullptr, "catalogue_topk: users / ws is NULL");
-  if (ws_bytes < mr_catalogue_topk_workspace_bytes(model, U, k)) {
-    set_error("catalogue_topk workspace too small: %zu < %zu", ws_bytes, mr_catalogue_topk_workspace_bytes(model, U, k));
-    return MR_ERR_WORKSPACE;
-  }
-  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
-  Carver cv(ws);
-  void* topk_ws = cv.take<char>(topk_workspace_bytes(C, N, k));
-  TopkArgs a{};
-  a.N = N;
-  a.k = k;
-  a.excl_ids = users;  // exclusion lists are indexed by user id
-  a.excl_rows = excl_rows;
-  a.excl_rowptr = excl_rowptr;
-  a.excl_items = excl_items;
-  a.targets = targets;
-  a.users = users;
-  a.num_users = m.num_users;
-  a.top_items = top_items;
-  a.top_scores = top_scores;
-  a.pos = pos;
-  rc = catalogue_sweep(m, users, U, C, scores, static_cast<char*>(ws) + cv.off, st,
-                       [&](int64_t u0, int64_t c, const float* out) {
-                         a.u0 = u0;
-                         a.U = c;
-                         a.scores = out;
-                         return launch_topk(a, topk_ws, st);
-                       });
-  if (rc == MR_OK) {
-    prof_mark(MR_PHASE_RANK, st);
-    rc = launch_topk_metrics(pos, U, k, sums, st);
-  }
-  prof_mark(-1, st);
-  return rc;
+  // exclusion lists are indexed by user id
+  return topk_query("catalogue_topk", model, scores, model->num_items, users, model->num_users, U, k, users, excl_rows,
+                    excl_rowptr, excl_items, targets, top_items, top_scores, pos, sums, ws, ws_bytes,
+                    (cudaStream_t)stream);
 }
 
-size_t mr_targets_scores_workspace_bytes(int64_t U, int32_t N, int64_t nnz_t) {
-  if (U < 0 || U > INT32_MAX || N < 1 || nnz_t < 0 || nnz_t > INT32_MAX) return 0;
-  return targets_workspace_bytes(clamp_users(U, catalogue_chunk_users(N)), nnz_t) + 256;
-}
+size_t mr_targets_scores_workspace_bytes(int64_t U, int32_t N, int64_t nnz_t) { return targets_bytes(nullptr, U, N, nnz_t); }
 
 int mr_targets_scores(const float* scores, int64_t U, int32_t N, const int32_t* excl_ids, int32_t excl_rows,
                       const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
                       const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks, int32_t n_ks, int32_t* tpos,
                       float* sums, void* ws, size_t ws_bytes, void* stream) {
-  TargetCutoffs cut{};
-  int rc = targets_check(U, N, excl_rows, excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums,
-                         cut);
-  if (rc != MR_OK) return rc;
-  MR_REQUIRE(U == 0 || scores != nullptr, "targets_scores: scores is NULL");
-  MR_REQUIRE(ws != nullptr, "targets_scores: workspace is NULL");
-  if (ws_bytes < mr_targets_scores_workspace_bytes(U, N, nnz_t)) {
-    set_error("targets_scores workspace too small: %zu < %zu", ws_bytes, mr_targets_scores_workspace_bytes(U, N, nnz_t));
-    return MR_ERR_WORKSPACE;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  const int64_t C = catalogue_chunk_users(N);
-  const TargetsWs w = carve_targets(ws, clamp_users(U, C), nnz_t);
-  TargetsArgs a{};
-  a.N = N;
-  a.excl_ids = excl_ids;
-  a.excl_rows = excl_rows;
-  a.excl_rowptr = excl_rowptr;
-  a.excl_items = excl_items;
-  a.tgt_rowptr = tgt_rowptr;
-  a.tgt_items = tgt_items;
-  a.nnz_t = nnz_t;
-  a.tpos = tpos;
-  prof_mark(MR_PHASE_RANK, st);
-  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
-    a.u0 = u0;
-    a.U = U - u0 < C ? U - u0 : C;
-    a.scores = scores + u0 * N;
-    rc = launch_targets_chunk(a, w, st);
-  }
-  if (rc == MR_OK) rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
-  prof_mark(-1, st);
-  return rc;
+  return targets_query("targets_scores", nullptr, const_cast<float*>(scores), N, nullptr, 0, U, excl_ids, excl_rows,
+                       excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums, ws, ws_bytes,
+                       (cudaStream_t)stream);
 }
 
 size_t mr_catalogue_targets_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz_t) {
-  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
-      model->num_users < 1 || model->L[0] < 2)
-    return 0;
-  const MrModel& m = *model;
-  const size_t sel = mr_targets_scores_workspace_bytes(U, m.num_items, nnz_t);
-  if (sel == 0) return 0;
-  return align_up(sel, 256) + catalogue_sweep_bytes(m, clamp_users(U, catalogue_chunk_users(m.num_items)), m.num_items) +
-         512;
+  return serving_model_ok(model, true) ? targets_bytes(model, U, model->num_items, nnz_t) : 0;
 }
 
 int mr_catalogue_targets(const MrModel* model, const int32_t* users, int64_t U, int32_t excl_rows,
                          const int64_t* excl_rowptr, const int32_t* excl_items, const int64_t* tgt_rowptr,
                          const int32_t* tgt_items, int64_t nnz_t, const int32_t* ks, int32_t n_ks, int32_t* tpos,
                          float* sums, void* ws, size_t ws_bytes, void* stream) {
-  int rc = check_model(model);
+  const int rc = check_model(model);
   if (rc != MR_OK) return rc;
-  const MrModel& m = *model;
-  const int32_t N = m.num_items;
-  TargetCutoffs cut{};
-  rc = targets_check(U, N, excl_rows, excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums, cut);
-  if (rc != MR_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (U == 0) {
-    if (sums != nullptr) MR_CUDA(cudaMemsetAsync(sums, 0, (MR_TGT_CUTOFF0 + MR_TGT_PER_CUTOFF * n_ks) * sizeof(float), st));
-    return MR_OK;
-  }
-  MR_REQUIRE(users != nullptr, "catalogue_targets: users is NULL");
-  MR_REQUIRE(ws != nullptr, "catalogue_targets: workspace is NULL");
-  if (ws_bytes < mr_catalogue_targets_workspace_bytes(model, U, nnz_t)) {
-    set_error("catalogue_targets workspace too small: %zu < %zu", ws_bytes,
-              mr_catalogue_targets_workspace_bytes(model, U, nnz_t));
-    return MR_ERR_WORKSPACE;
-  }
-  const int64_t C = clamp_users(U, catalogue_chunk_users(N));
-  Carver cv(ws);
-  const TargetsWs w = carve_targets(cv.take<char>(mr_targets_scores_workspace_bytes(U, N, nnz_t)), C, nnz_t);
-  TargetsArgs a{};
-  a.N = N;
-  a.excl_ids = users;  // exclusion lists are indexed by user id
-  a.excl_rows = excl_rows;
-  a.excl_rowptr = excl_rowptr;
-  a.excl_items = excl_items;
-  a.tgt_rowptr = tgt_rowptr;
-  a.tgt_items = tgt_items;
-  a.nnz_t = nnz_t;
-  a.users = users;
-  a.num_users = m.num_users;
-  a.tpos = tpos;
-  rc = catalogue_sweep(m, users, U, C, nullptr, static_cast<char*>(ws) + cv.off, st,
-                       [&](int64_t u0, int64_t c, const float* out) {
-                         a.u0 = u0;
-                         a.U = c;
-                         a.scores = out;
-                         return launch_targets_chunk(a, w, st);
-                       });
-  if (rc == MR_OK) {
-    prof_mark(MR_PHASE_RANK, st);
-    rc = launch_targets_metrics(tgt_rowptr, U, nnz_t, w.spos, cut, sums, w.partials, st);
-  }
-  prof_mark(-1, st);
-  return rc;
+  // exclusion lists are indexed by user id
+  return targets_query("catalogue_targets", model, nullptr, model->num_items, users, model->num_users, U, users,
+                       excl_rows, excl_rowptr, excl_items, tgt_rowptr, tgt_items, nnz_t, ks, n_ks, tpos, sums, ws,
+                       ws_bytes, (cudaStream_t)stream);
 }
 
-static int audience_check(int64_t U, int32_t M, int32_t k, int32_t excl_rows, const int64_t* excl_rowptr,
-                          const int32_t* excl_users, const int32_t* targets, const int32_t* pos, const float* sums) {
-  MR_REQUIRE(U >= 0 && U <= INT32_MAX && M >= 0, "audience: bad U=%lld M=%d", (long long)U, M);
-  MR_REQUIRE(k >= 1 && k <= MR_MAX_TOPK, "audience: k=%d out of [1,%d]", k, MR_MAX_TOPK);
-  MR_REQUIRE(excl_rows >= 0 && (excl_rowptr == nullptr || excl_users != nullptr), "audience: bad exclusion lists");
-  MR_REQUIRE(targets != nullptr || (pos == nullptr && sums == nullptr), "audience: pos / sums need targets");
-  return MR_OK;
-}
-
-// The selection's workspace for chunks of C users: the running lists of every item.
-static size_t audience_select_bytes(int64_t C, int32_t M, int32_t k) { return carve_audience(nullptr, C, M, k).total; }
-
-size_t mr_audience_scores_workspace_bytes(int64_t U, int32_t M, int32_t k) {
-  if (U < 0 || U > INT32_MAX || M < 0 || k < 1 || k > MR_MAX_TOPK) return 0;
-  return audience_select_bytes(clamp_users(U, catalogue_chunk_users(M)), M, k) + 256;
-}
+size_t mr_audience_scores_workspace_bytes(int64_t U, int32_t M, int32_t k) { return audience_bytes(nullptr, U, M, k); }
 
 int mr_audience_scores(const float* scores, int64_t U, int32_t M, int32_t k, const int32_t* users,
                        const int32_t* excl_ids, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
                        const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
                        void* ws, size_t ws_bytes, void* stream) {
-  int rc = audience_check(U, M, k, excl_rows, excl_rowptr, excl_users, targets, pos, sums);
-  if (rc != MR_OK) return rc;
-  MR_REQUIRE((U == 0 || M == 0 || scores != nullptr) && ws != nullptr, "audience_scores: scores / ws is NULL");
-  if (ws_bytes < mr_audience_scores_workspace_bytes(U, M, k)) {
-    set_error("audience_scores workspace too small: %zu < %zu", ws_bytes, mr_audience_scores_workspace_bytes(U, M, k));
-    return MR_ERR_WORKSPACE;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
-  const AudienceState w = carve_audience(ws, C, M, k);
-  AudienceArgs a{};
-  a.M = M;
-  a.k = k;
-  a.users = users;
-  a.num_users = INT32_MAX;  // no model: every id >= 0 is a user
-  a.excl_ids = excl_ids;
-  a.excl_rows = excl_rows;
-  a.excl_rowptr = excl_rowptr;
-  a.excl_users = excl_users;
-  a.targets = targets;
-  prof_mark(MR_PHASE_RANK, st);
-  if (M > 0) rc = launch_audience_init(a, w, st);
-  for (int64_t u0 = 0; u0 < U && rc == MR_OK; u0 += C) {
-    a.u0 = u0;
-    a.U = U - u0 < C ? U - u0 : C;
-    a.scores = scores + u0 * M;
-    rc = launch_audience_chunk(a, w, st);
-  }
-  if (rc == MR_OK) rc = launch_audience_final(a, w, nullptr, 0, top_users, top_scores, pos, sums, st);
-  prof_mark(-1, st);
-  return rc;
+  // no model: every id >= 0 is a user
+  return audience_query("audience_scores", nullptr, const_cast<float*>(scores), nullptr, M, k, users, INT32_MAX, U,
+                        excl_ids, excl_rows, excl_rowptr, excl_users, targets, top_users, top_scores, pos, sums, ws,
+                        ws_bytes, (cudaStream_t)stream);
 }
 
 size_t mr_catalogue_audience_workspace_bytes(const MrModel* model, int64_t U, int32_t M, int32_t k) {
-  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
-      model->num_users < 1 || U < 0 || U > INT32_MAX || M < 0 || k < 1 || k > MR_MAX_TOPK)
-    return 0;
-  const MrModel& m = *model;
-  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
-  return align_up(audience_select_bytes(C, M, k), 256) + catalogue_sweep_bytes(m, C, M < 1 ? 1 : M, true) + 512;
+  return serving_model_ok(model, false) ? audience_bytes(model, U, M, k) : 0;
 }
 
 int mr_catalogue_audience(const MrModel* model, const int32_t* items, int32_t M, int32_t k, const int32_t* users,
                           int64_t U, int32_t excl_rows, const int64_t* excl_rowptr, const int32_t* excl_users,
                           const int32_t* targets, int32_t* top_users, float* top_scores, int32_t* pos, float* sums,
                           float* scores, void* ws, size_t ws_bytes, void* stream) {
-  int rc = check_model(model);
+  const int rc = check_model(model);
   if (rc != MR_OK) return rc;
-  const MrModel& m = *model;
-  rc = audience_check(U, M, k, excl_rows, excl_rowptr, excl_users, targets, pos, sums);
-  if (rc != MR_OK) return rc;
-  MR_REQUIRE(users != nullptr || U == m.num_users, "catalogue_audience: without a pool U must be num_users (%d), got %lld",
-             m.num_users, (long long)U);
-  MR_REQUIRE((M == 0 || items != nullptr) && ws != nullptr, "catalogue_audience: items / ws is NULL");
-  if (ws_bytes < mr_catalogue_audience_workspace_bytes(model, U, M, k)) {
-    set_error("catalogue_audience workspace too small: %zu < %zu", ws_bytes,
-              mr_catalogue_audience_workspace_bytes(model, U, M, k));
-    return MR_ERR_WORKSPACE;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  const int64_t C = clamp_users(U, catalogue_chunk_users(M));
-  Carver cv(ws);
-  const AudienceState w = carve_audience(cv.take<char>(audience_select_bytes(C, M, k)), C, M, k);
-  AudienceArgs a{};
-  a.M = M;
-  a.k = k;
-  a.users = users;
-  a.num_users = m.num_users;
-  a.excl_ids = items;  // exclusion lists are indexed by item id
-  a.excl_rows = excl_rows;
-  a.excl_rowptr = excl_rowptr;
-  a.excl_users = excl_users;
-  a.targets = targets;
-  if (M > 0) {
-    rc = launch_audience_init(a, w, st);
-    if (rc == MR_OK)
-      rc = catalogue_sweep(m, users, U, C, scores, static_cast<char*>(ws) + cv.off, st,
-                           [&](int64_t u0, int64_t c, const float* out) {
-                             a.u0 = u0;
-                             a.U = c;
-                             a.scores = out;
-                             return launch_audience_chunk(a, w, st);
-                           },
-                           items, M);
-  }
-  if (rc == MR_OK) {
-    prof_mark(MR_PHASE_RANK, st);
-    rc = launch_audience_final(a, w, items, m.num_items, top_users, top_scores, pos, sums, st);
-  }
-  prof_mark(-1, st);
-  return rc;
+  // exclusion lists are indexed by item id
+  return audience_query("catalogue_audience", model, scores, items, M, k, users, model->num_users, U, items, excl_rows,
+                        excl_rowptr, excl_users, targets, top_users, top_scores, pos, sums, ws, ws_bytes,
+                        (cudaStream_t)stream);
 }
 
-size_t mr_topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k) {
-  if (U < 0 || U > INT32_MAX || nnz < 0 || nnz > INT32_MAX || k < 1 || k > MR_MAX_TOPK) return 0;
-  return topk_lists_workspace_bytes(U, nnz, k) + 256;
-}
+size_t mr_topk_lists_workspace_bytes(int64_t U, int64_t nnz, int32_t k) { return lists_bytes(nullptr, U, nnz, k); }
 
 int mr_topk_lists(const float* scores, int64_t U, const int64_t* rowptr, int64_t nnz, int32_t k, const int32_t* targets,
                   int32_t* top_pos, float* top_scores, int32_t* pos, float* sums, void* ws, size_t ws_bytes, void* stream) {
-  int rc = lists_check(U, rowptr, nnz, k, targets, pos, sums);
-  if (rc != MR_OK) return rc;
-  MR_REQUIRE(nnz == 0 || scores != nullptr, "topk_lists: scores is NULL");
-  MR_REQUIRE(ws != nullptr, "topk_lists: workspace is NULL");
-  if (ws_bytes < mr_topk_lists_workspace_bytes(U, nnz, k)) {
-    set_error("topk_lists workspace too small: %zu < %zu", ws_bytes, mr_topk_lists_workspace_bytes(U, nnz, k));
-    return MR_ERR_WORKSPACE;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  TopkListsArgs a{};
-  a.scores = scores;
-  a.rowptr = rowptr;
-  a.U = U;
-  a.nnz = nnz;
-  a.k = k;
-  a.targets = targets;
-  a.top_pos = top_pos;
-  a.top_scores = top_scores;
-  a.pos = pos;
-  prof_mark(MR_PHASE_RANK, st);
-  rc = launch_topk_lists(a, sums, ws, st);
-  prof_mark(-1, st);
-  return rc;
+  return lists_query("topk_lists", nullptr, const_cast<float*>(scores), nullptr, U, rowptr, nullptr, nnz, k, targets,
+                     top_pos, nullptr, top_scores, pos, sums, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 size_t mr_rank_lists_workspace_bytes(const MrModel* model, int64_t U, int64_t nnz, int32_t k) {
-  if (model == nullptr || model->n_layers < 1 || model->n_layers > MR_MAX_LAYERS || model->num_items < 1 ||
-      model->num_users < 1 || model->L[0] < 2)
-    return 0;
-  const size_t sel = mr_topk_lists_workspace_bytes(U, nnz, k);
-  if (sel == 0) return 0;
-  return sel + align_up((size_t)nnz * sizeof(int32_t), 256) + align_up((size_t)nnz * sizeof(float), 256) +
-         eval_carve(*model, eval_plan(*model, SCORE_LISTS, U, 0, nnz), nullptr).total + 256;
+  return serving_model_ok(model, true) ? lists_bytes(model, U, nnz, k) : 0;
 }
 
 int mr_rank_lists(const MrModel* model, const int32_t* users, int64_t U, const int64_t* rowptr, const int32_t* items,
                   int64_t nnz, int32_t k, const int32_t* targets, int32_t* top_pos, int32_t* top_items, float* top_scores,
                   int32_t* pos, float* sums, float* probs, void* ws, size_t ws_bytes, void* stream) {
-  int rc = check_model(model);
+  const int rc = check_model(model);
   if (rc != MR_OK) return rc;
-  rc = lists_check(U, rowptr, nnz, k, targets, pos, sums);
-  if (rc != MR_OK) return rc;
-  MR_REQUIRE(U == 0 || users != nullptr, "rank_lists: users is NULL");
-  MR_REQUIRE(nnz == 0 || items != nullptr, "rank_lists: items is NULL");
-  MR_REQUIRE(ws != nullptr, "rank_lists: workspace is NULL");
-  if (ws_bytes < mr_rank_lists_workspace_bytes(model, U, nnz, k)) {
-    set_error("rank_lists workspace too small: %zu < %zu", ws_bytes, mr_rank_lists_workspace_bytes(model, U, nnz, k));
-    return MR_ERR_WORKSPACE;
-  }
-  const MrModel& m = *model;
-  cudaStream_t st = (cudaStream_t)stream;
-  Carver cv(ws);
-  void* sel_ws = cv.take<char>(topk_lists_workspace_bytes(U, nnz, k));
-  int32_t* seg = cv.take<int32_t>((size_t)nnz);
-  float* probs_buf = cv.take<float>((size_t)nnz);
-  float* pr = probs != nullptr ? probs : probs_buf;
-  const EvalPlan p = eval_plan(m, SCORE_LISTS, U, 0, nnz);
-  const EvalWs w = eval_carve(m, p, static_cast<char*>(ws) + cv.off);
-  if (nnz > 0) {
-    prof_mark(MR_PHASE_MISC, st);
-    // seg: the list of each row, or the user of each row (plain forward)
-    rc = launch_list_rows(rowptr, U, nnz, p.tower == EVAL_FORWARD ? users : nullptr, seg, st);
-    if (rc == MR_OK) rc = eval_prepare(m, p, w, users, st);
-    if (rc == MR_OK && p.tower == EVAL_SMALL) prof_mark(MR_PHASE_FUSED_TILE, st);
-    for (int64_t r0 = 0; r0 < nnz && rc == MR_OK; r0 += p.sb) {
-      const int64_t r1 = r0 + p.sb < nnz ? r0 + p.sb : nnz;
-      if (p.tower == EVAL_TC) {  // the second layer's producers compute relu(Pi[items[row]] + Zu[seg[row]])
-        prof_mark(MR_PHASE_TC_DENSE_FWD, st);
-        rc = tc_forward_rows(m, w.t, users, items, 1, r0, r1, st, 0, false, p.head_dot, seg, (int32_t)U);
-        if (rc != MR_OK) break;
-        prof_mark(MR_PHASE_HEAD, st);
-        rc = launch_catalogue_head(m, w.t.H[m.n_layers - 1], users, r1 - r0, 1, pr, st, seg, items, r0, U);
-      } else if (p.tower == EVAL_SMALL) {
-        rc = launch_small_tower_forward(m, w.t.Pi, w.t.Pu, users, items + r0, r1 - r0, 1, pr + r0, st, seg + r0, U);
-      } else {
-        rc = mr_neumf_forward(model, seg + r0, items + r0, r1 - r0, 1, nullptr, pr + r0, nullptr, nullptr, w.fwd,
-                              w.fwd_bytes, stream);
-      }
-    }
-    if (rc != MR_OK) return rc;
-  }
-  TopkListsArgs a{};
-  a.scores = pr;
-  a.rowptr = rowptr;
-  a.U = U;
-  a.nnz = nnz;
-  a.k = k;
-  a.targets = targets;
-  a.users = users;
-  a.num_users = m.num_users;
-  a.items = items;
-  a.top_pos = top_pos;
-  a.top_items = top_items;
-  a.top_scores = top_scores;
-  a.pos = pos;
-  prof_mark(MR_PHASE_RANK, st);
-  rc = launch_topk_lists(a, sums, sel_ws, st);
-  prof_mark(-1, st);
-  return rc;
+  return lists_query("rank_lists", model, probs, users, U, rowptr, items, nnz, k, targets, top_pos, top_items,
+                     top_scores, pos, sums, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 int mr_sample_negatives(const int64_t* csr_rowptr, const int32_t* csr_items, int32_t num_items, const int32_t* pos_users,

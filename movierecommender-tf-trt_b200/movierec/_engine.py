@@ -536,24 +536,18 @@ class NeuMFEngine(object):
         users = as_device_i32(users, dev)
         U = users.numel()
         k = int(k)
-        t = as_device_i32(targets, dev) if targets is not None else None
-        if t is not None and t.numel() != U:
-            raise ValueError("targets ({}) and users ({}) differ in length".format(t.numel(), U))
-        rowptr, items, excl_rows = _exclusion_on_device(exclude, dev)
-        top_items = torch.empty((U, k), dtype=torch.int32, device=dev)
-        top_scores = torch.empty((U, k), dtype=torch.float32, device=dev)
-        pos = torch.empty(U, dtype=torch.int32, device=dev) if t is not None else None
-        sums = torch.zeros(2, dtype=torch.float32, device=dev) if t is not None else None
+        t = _targets(targets, U, "users", dev)
+        rowptr, items, excl_rows = _exclusion(exclude, dev)
+        top_items, top_scores, pos, sums = _selection_outputs(U, k, t, dev)
         full = torch.empty((U, self.num_items), dtype=torch.float32, device=dev) if want_scores else None
-        ws = self._workspace(max(int(nat.lib.mr_catalogue_topk_workspace_bytes(C.byref(self._model), U, k)), 256))
+        ws = self._workspace(_workspace_bytes(nat.lib.mr_catalogue_topk_workspace_bytes(C.byref(self._model), U, k),
+                                              "catalogue_topk", U=U, k=k))
         nat.check(nat.lib.mr_catalogue_topk(C.byref(self._model), _ptr(users), U, k, excl_rows, _ptr(rowptr), _ptr(items),
                                             _ptr(t), _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(full),
                                             _ptr(ws), ws.numel(), self._stream()), "mr_catalogue_topk")
-        bad = torch.zeros(1, dtype=torch.float32, device=dev)
-        if U:
-            bad = ((users.min() < 0) | (users.max() >= self.num_users)).to(torch.float32).reshape(1)
-            if t is not None:
-                bad = bad + ((t.min() < 0) | (t.max() >= self.num_items)).to(torch.float32).reshape(1)
+        bad = _outside(users, self.num_users)
+        if t is not None:
+            bad = bad + _outside(t, self.num_items)
         self.last_catalogue_bad = bad
         return top_items, top_scores, pos, sums, full
 
@@ -575,28 +569,19 @@ class NeuMFEngine(object):
         pool = audience_pool(users)
         U = self.num_users if pool is None else int(pool.size)
         d_pool = None if pool is None else torch.from_numpy(pool if pool.size else np.zeros(1, np.int32)).to(dev)
-        t = as_device_i32(targets, dev) if targets is not None else None
-        if t is not None and t.numel() != M:
-            raise ValueError("targets ({}) and items ({}) differ in length".format(t.numel(), M))
-        rowptr, excl, excl_rows = _audience_exclusion(exclude, dev)
-        top_users = torch.empty((M, k), dtype=torch.int32, device=dev)
-        top_scores = torch.empty((M, k), dtype=torch.float32, device=dev)
-        pos = torch.empty(M, dtype=torch.int32, device=dev) if t is not None else None
-        sums = torch.zeros(2, dtype=torch.float32, device=dev) if t is not None else None
+        t = _targets(targets, M, "items", dev)
+        rowptr, excl, excl_rows = _exclusion(exclude, dev)
+        top_users, top_scores, pos, sums = _selection_outputs(M, k, t, dev)
         full = torch.empty((U, M), dtype=torch.float32, device=dev) if want_scores else None
-        nbytes = int(nat.lib.mr_catalogue_audience_workspace_bytes(C.byref(self._model), U, M, k))
-        if nbytes == 0:
-            raise ValueError("catalogue_audience: bad sizes U={} M={} k={}".format(U, M, k))
-        ws = self._workspace(nbytes)
+        ws = self._workspace(_workspace_bytes(nat.lib.mr_catalogue_audience_workspace_bytes(C.byref(self._model), U, M, k),
+                                              "catalogue_audience", U=U, M=M, k=k))
         nat.check(nat.lib.mr_catalogue_audience(C.byref(self._model), _ptr(items if M else None), M, k, _ptr(d_pool), U,
                                                 excl_rows, _ptr(rowptr), _ptr(excl), _ptr(t), _ptr(top_users),
                                                 _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(full), _ptr(ws), ws.numel(),
                                                 self._stream()), "mr_catalogue_audience")
-        bad = torch.zeros(1, dtype=torch.float32, device=dev)
-        if M:
-            bad = bad + ((items.min() < 0) | (items.max() >= self.num_items)).to(torch.float32).reshape(1)
-            if t is not None:
-                bad = bad + ((t.min() < 0) | (t.max() >= self.num_users)).to(torch.float32).reshape(1)
+        bad = _outside(items, self.num_items)
+        if t is not None:
+            bad = bad + _outside(t, self.num_users)
         if pool is not None and pool.size and (pool[0] < 0 or pool[-1] >= self.num_users):
             bad = bad + 1.0
         self.last_catalogue_bad = bad
@@ -618,7 +603,7 @@ class NeuMFEngine(object):
         M = ids.numel()
         k = int(k)
         code, N = (nat.SIDE_ITEMS, self.num_items) if side == "items" else (nat.SIDE_USERS, self.num_users)
-        rowptr, excl, excl_rows = _audience_exclusion(exclude, dev)
+        rowptr, excl, excl_rows = _exclusion(exclude, dev)
         e_ids = as_device_i32(excl_ids, dev) if excl_ids is not None else None
         if e_ids is not None and e_ids.numel() != M:
             raise ValueError("excl_ids ({}) and ids ({}) differ in length".format(e_ids.numel(), M))
@@ -646,30 +631,19 @@ class NeuMFEngine(object):
         dev = self.device
         users = as_device_i32(users, dev)
         U = users.numel()
-        rowptr, items = _check_lists(lists, U, dev)
+        rowptr, items = check_csr(*lists, "lists", rows=U, device=dev)
         nnz = items.numel()
         k = int(k)
-        t = as_device_i32(targets, dev) if targets is not None else None
-        if t is not None and t.numel() != U:
-            raise ValueError("targets ({}) and users ({}) differ in length".format(t.numel(), U))
+        t = _targets(targets, U, "users", dev)
         top_pos = torch.empty((U, k), dtype=torch.int32, device=dev)
-        top_items = torch.empty((U, k), dtype=torch.int32, device=dev)
-        top_scores = torch.empty((U, k), dtype=torch.float32, device=dev)
-        pos = torch.empty(U, dtype=torch.int32, device=dev) if t is not None else None
-        sums = torch.zeros(2, dtype=torch.float32, device=dev) if t is not None else None
+        top_items, top_scores, pos, sums = _selection_outputs(U, k, t, dev)
         probs = torch.empty(nnz, dtype=torch.float32, device=dev) if want_probs else None
-        nbytes = int(nat.lib.mr_rank_lists_workspace_bytes(C.byref(self._model), U, nnz, k))
-        if nbytes == 0:
-            raise ValueError("rank_lists: bad sizes U={} nnz={} k={}".format(U, nnz, k))
-        ws = self._workspace(nbytes)
+        ws = self._workspace(_workspace_bytes(nat.lib.mr_rank_lists_workspace_bytes(C.byref(self._model), U, nnz, k),
+                                              "rank_lists", U=U, nnz=nnz, k=k))
         nat.check(nat.lib.mr_rank_lists(C.byref(self._model), _ptr(users), U, _ptr(rowptr), _ptr(items), nnz, k, _ptr(t),
                                         _ptr(top_pos), _ptr(top_items), _ptr(top_scores), _ptr(pos), _ptr(sums),
                                         _ptr(probs), _ptr(ws), ws.numel(), self._stream()), "mr_rank_lists")
-        bad = torch.zeros(1, dtype=torch.float32, device=dev)
-        if U:
-            bad = bad + ((users.min() < 0) | (users.max() >= self.num_users)).to(torch.float32).reshape(1)
-        if nnz:
-            bad = bad + ((items.min() < 0) | (items.max() >= self.num_items)).to(torch.float32).reshape(1)
+        bad = _outside(users, self.num_users) + _outside(items, self.num_items)
         if t is not None and U:
             lens = rowptr[1:] - rowptr[:-1]
             bad = bad + ((t < 0) | (t.to(torch.int64) >= lens)).any().to(torch.float32).reshape(1)
@@ -688,26 +662,19 @@ class NeuMFEngine(object):
         dev = self.device
         users = as_device_i32(users, dev)
         U = users.numel()
-        rowptr, items = _check_lists(targets, U, dev)
+        rowptr, items = check_csr(*targets, "lists", rows=U, device=dev)
         nnz = items.numel()
         kbuf, n_ks = _cutoffs(ks)
-        excl_rowptr, excl_items, excl_rows = _exclusion_on_device(exclude, dev)
+        excl_rowptr, excl_items, excl_rows = _exclusion(exclude, dev)
         tpos = torch.empty(nnz, dtype=torch.int32, device=dev)
         sums = torch.zeros(nat.TGT_CUTOFF0 + nat.TGT_PER_CUTOFF * n_ks, dtype=torch.float32, device=dev)
-        nbytes = int(nat.lib.mr_catalogue_targets_workspace_bytes(C.byref(self._model), U, nnz))
-        if nbytes == 0:
-            raise ValueError("catalogue_targets: bad sizes U={} nnz={}".format(U, nnz))
-        ws = self._workspace(nbytes)
+        ws = self._workspace(_workspace_bytes(nat.lib.mr_catalogue_targets_workspace_bytes(C.byref(self._model), U, nnz),
+                                              "catalogue_targets", U=U, nnz=nnz))
         nat.check(nat.lib.mr_catalogue_targets(C.byref(self._model), _ptr(users), U, excl_rows, _ptr(excl_rowptr),
                                                _ptr(excl_items), _ptr(rowptr), _ptr(items if nnz else None), nnz, kbuf,
                                                n_ks, _ptr(tpos if nnz else None), _ptr(sums), _ptr(ws), ws.numel(),
                                                self._stream()), "mr_catalogue_targets")
-        bad = torch.zeros(1, dtype=torch.float32, device=dev)
-        if U:
-            bad = bad + ((users.min() < 0) | (users.max() >= self.num_users)).to(torch.float32).reshape(1)
-        if nnz:
-            bad = bad + ((items.min() < 0) | (items.max() >= self.num_items)).to(torch.float32).reshape(1)
-        self.last_catalogue_bad = bad
+        self.last_catalogue_bad = _outside(users, self.num_users) + _outside(items, self.num_items)
         return tpos, sums
 
     def fold_in(self, histories, steps, lr, negs, seed=0, init_users=None, optimizer=None, beta_1=None, beta_2=None):
@@ -792,8 +759,7 @@ class NeuMFEngine(object):
     def _ids_out_of_range(self, users, items):
         if users.numel() == 0:
             return torch.zeros(1, dtype=torch.float32, device=self.device)
-        return ((users.min() < 0) | (users.max() >= self.num_users) | (items.min() < 0) |
-                (items.max() >= self.num_items)).to(torch.float32).reshape(1)
+        return torch.maximum(_outside(users, self.num_users), _outside(items, self.num_items))
 
 
     # A sweep over host arrays of at least this many rows is cut into chunks whose uploads run on a copy stream under
@@ -911,8 +877,8 @@ _VIEW_DESC = ("compute_path", "item_projection", "fused_train", "device", "L", "
               "optimizer", "lr", "beta_1", "beta_2", "table_mode", "iterations", "_dense_slices", "dense_count", "dense")
 
 
-_LIST_WORDS = {"users": ("histories", "item", "user's items", "a history covers every item", "items"),
-               "items": ("raters", "user", "item's users", "a rater list covers every user", "users")}
+_LIST_WORDS = {"users": ("histories", "an item", "a history covers every item"),
+               "items": ("raters", "a user", "a rater list covers every user")}
 
 
 def fold_in_histories(histories, num_other, side="users"):
@@ -921,7 +887,7 @@ def fold_in_histories(histories, num_other, side="users"):
     checked as is; a list of id arrays is sorted and de-duplicated per list.  num_other: the number of items (users)
     the ids index.  Raises IndexError on an id outside [0, num_other) and ValueError on a malformed rowptr, a list that
     is not strictly ascending or a list that covers every id."""
-    name, other, members, covers, ids_name = _LIST_WORDS[side]
+    name, id_name, covers = _LIST_WORDS[side]
     host = lambda x: np.asarray(x.cpu() if hasattr(x, "cpu") else x)
     if isinstance(histories, tuple) and len(histories) == 2:
         rowptr = host(histories[0]).astype(np.int64).reshape(-1)
@@ -931,19 +897,10 @@ def fold_in_histories(histories, num_other, side="users"):
         rowptr = np.zeros(len(parts) + 1, np.int64)
         rowptr[1:] = np.cumsum([p.size for p in parts])
         items = np.concatenate(parts) if parts else np.zeros(0, np.int64)
-    if rowptr.size < 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
-        raise ValueError("{}: offsets must start at 0, never decrease and end at len({}) = {}".format(name, ids_name, items.size))
-    if items.size and (items.min() < 0 or items.max() >= num_other):
-        raise IndexError("{}: {} {} lies outside [0, {})".format(name, "an" if other == "item" else "a", other,
-                                                                 num_other))
-    inner = np.ones(max(items.size - 1, 0), bool)  # pairs of neighbours inside one list
-    starts = rowptr[1:-1]
-    inner[starts[(starts > 0) & (starts < items.size)] - 1] = False
-    if np.any((items[1:] <= items[:-1]) & inner):
-        raise ValueError("{}: every {} must be strictly ascending".format(name, members))
+    rowptr, items = (t.numpy() for t in check_csr(rowptr, items, name, ascending=True, limit=num_other, id_name=id_name))
     if np.any(rowptr[1:] - rowptr[:-1] >= num_other):
         raise ValueError("{}: {}, so there is no negative to draw".format(name, covers))
-    return rowptr, items.astype(np.int32)
+    return rowptr, items
 
 
 # Kernel selection is part of the model description handed to the library (MrModel), not library state.  These
@@ -1013,13 +970,10 @@ def topk_scores(scores, k, exclude=None, excl_ids=None, targets=None, device=Non
     s = s.to(device, torch.float32).contiguous()
     k = int(k)
     ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
-    t = as_device_i32(targets, device) if targets is not None else None
-    rowptr, items, excl_rows = _exclusion_on_device(exclude, device)
-    top_items = torch.empty((U, k), dtype=torch.int32, device=device)
-    top_scores = torch.empty((U, k), dtype=torch.float32, device=device)
-    pos = torch.empty(U, dtype=torch.int32, device=device) if t is not None else None
-    sums = torch.zeros(2, dtype=torch.float32, device=device) if t is not None else None
-    nbytes = max(int(nat.lib.mr_topk_scores_workspace_bytes(U, N, k)), 256)
+    t = _targets(targets, U, "rows", device)
+    rowptr, items, excl_rows = _exclusion(exclude, device)
+    top_items, top_scores, pos, sums = _selection_outputs(U, k, t, device)
+    nbytes = _workspace_bytes(nat.lib.mr_topk_scores_workspace_bytes(U, N, k), "topk_scores", U=U, N=N, k=k)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
     st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
     nat.check(nat.lib.mr_topk_scores(_ptr(s), U, N, k, _ptr(ids), excl_rows, _ptr(rowptr), _ptr(items), _ptr(t),
@@ -1036,35 +990,93 @@ def audience_pool(users):
     return np.unique(u).astype(np.int32)
 
 
-def check_exclusion_csr(rowptr, ids):
-    """(rowptr, ids) host or device -> the same as tensors (int64 rowptr, int32 ids) on their own device; ValueError
-    unless rowptr has at least one entry, starts at 0, never decreases and ends at len(ids), and every list is strictly
-    ascending.  Device input is checked on the device and read back once."""
-    as_t = lambda x, dt: (x if isinstance(x, torch.Tensor) else torch.from_numpy(np.asarray(x).astype(dt))).reshape(-1)
-    rp = as_t(rowptr, np.int64).to(torch.int64)
-    it = as_t(ids, np.int64).to(rp.device, torch.int64)
+def check_csr(rowptr, ids, what, rows=None, ascending=False, limit=None, id_name="an id", device=None):
+    """(rowptr, ids) host or device -> (rowptr int64, ids int32) tensors on `device` (default: rowptr's), checked there
+    with one read-back.  ValueError unless rowptr starts at 0, never decreases and ends at len(ids) (and has rows + 1
+    entries when rows is given), or when ascending and a list is not strictly ascending; IndexError when limit is given
+    and an id lies outside [0, limit).  The kernels read lists as given, so every list argument passes through here."""
+    def as_t(x):
+        if isinstance(x, torch.Tensor):
+            return x.reshape(-1)
+        a = np.asarray(x).reshape(-1)
+        return torch.from_numpy(np.ascontiguousarray(a if a.dtype.kind in "iu" else a.astype(np.int64)))
+    rp = as_t(rowptr)
+    device = rp.device if device is None else device
+    rp = rp.to(device, torch.int64).contiguous()
+    it = as_t(ids).to(device)
     n = it.numel()
-    if rp.numel() < 1:
-        raise ValueError("exclusion lists: rowptr is empty")
-    bad = (rp[0] != 0) | (rp[-1] != n) | (rp[1:] < rp[:-1]).any()
-    if n > 1:
-        inner = torch.ones(n - 1, dtype=torch.bool, device=rp.device)  # pairs of neighbours inside one list
+    if rp.numel() < 1 or (rows is not None and rp.numel() != rows + 1):
+        raise ValueError("{}: rowptr has {} entries, expected {}".format(what, rp.numel(),
+                                                                         "at least 1" if rows is None else rows + 1))
+    flags = [(rp[0] != 0) | (rp[-1] != n) | (rp[1:] < rp[:-1]).any()]
+    no = torch.zeros((), dtype=torch.bool, device=device)
+    flags.append(((it < 0) | (it >= limit)).any() if limit is not None else no)
+    if ascending and n > 1:
+        inner = torch.ones(n - 1, dtype=torch.bool, device=device)  # pairs of neighbours inside one list
         starts = rp[1:-1]
-        starts = starts[(starts > 0) & (starts < n)]
-        inner[starts - 1] = False
-        bad = bad | ((it[1:] <= it[:-1]) & inner).any()
-    if bool(bad.item()):
-        raise ValueError("exclusion lists: offsets must start at 0, never decrease and end at len(ids) = {}, and every "
-                         "list must be strictly ascending".format(n))
-    return rp, it.to(torch.int32)
+        inner[starts[(starts > 0) & (starts < n)] - 1] = False
+        flags.append(((it[1:] <= it[:-1]) & inner).any())
+    bad_offsets, bad_ids, *unsorted = torch.stack(flags).tolist()
+    if bad_offsets:
+        raise ValueError("{}: offsets must start at 0, never decrease and end at len(ids) = {}".format(what, n))
+    if bad_ids:
+        raise IndexError("{}: {} lies outside [0, {})".format(what, id_name, limit))
+    if any(unsorted):
+        raise ValueError("{}: every list must be strictly ascending".format(what))
+    return rp, it.to(torch.int32).contiguous()
 
 
-def _audience_exclusion(exclude, device):
-    """None | (rowptr, ids) -> (device rowptr int64 or None, device ids int32 or None, rows), checked first."""
+def check_exclusion_csr(rowptr, ids):
+    """Exclusion lists (rowptr, ids), host or device -> the same as tensors (int64 rowptr, int32 ids) on their own
+    device; ValueError unless rowptr starts at 0, never decreases and ends at len(ids), and every list is strictly
+    ascending (check_csr)."""
+    return check_csr(rowptr, ids, "exclusion lists", ascending=True)
+
+
+def _exclusion(exclude, device):
+    """None | (rowptr, ids) host or device -> (device rowptr int64 or None, device ids int32 or None, rows): uploaded,
+    then checked on the device as check_exclusion_csr, so host lists cost no host pass."""
     if exclude is None:
         return None, None, 0
-    rp, it = check_exclusion_csr(*exclude)
-    return _exclusion_on_device((rp, it), device)
+    rowptr, ids = check_csr(*exclude, "exclusion lists", ascending=True, device=device)
+    if ids.numel() == 0:  # every list empty: the library still wants a pointer
+        ids = torch.zeros(1, dtype=torch.int32, device=device)
+    return rowptr, ids, rowptr.numel() - 1
+
+
+def _targets(targets, n, what, device):
+    """One target per row (or None) -> device int32 (or None); ValueError unless there are n of them."""
+    if targets is None:
+        return None
+    t = as_device_i32(targets, device)
+    if t.numel() != n:
+        raise ValueError("targets ({}) and {} ({}) differ in length".format(t.numel(), what, n))
+    return t
+
+
+def _selection_outputs(R, k, t, device):
+    """The outputs of a top-k over R rows: ids (R, k) int32, scores (R, k) float32, and with targets t pos (R,) int32
+    and sums (2,) float32 zeros (else None)."""
+    ids = torch.empty((R, k), dtype=torch.int32, device=device)
+    scores = torch.empty((R, k), dtype=torch.float32, device=device)
+    if t is None:
+        return ids, scores, None, None
+    return ids, scores, torch.empty(R, dtype=torch.int32, device=device), torch.zeros(2, dtype=torch.float32,
+                                                                                      device=device)
+
+
+def _workspace_bytes(nbytes, what, **sizes):
+    """A *_workspace_bytes result; ValueError when the library refuses the sizes (0 bytes)."""
+    if int(nbytes) == 0:
+        raise ValueError("{}: bad sizes {}".format(what, " ".join("{}={}".format(*kv) for kv in sizes.items())))
+    return int(nbytes)
+
+
+def _outside(t, n):
+    """One-element float32 device tensor: 1 when an id of t lies outside [0, n), else 0 (also when t is empty)."""
+    if t.numel() == 0:
+        return torch.zeros(1, dtype=torch.float32, device=t.device)
+    return ((t.min() < 0) | (t.max() >= n)).to(torch.float32).reshape(1)
 
 
 def audience_scores(scores, k, users=None, exclude=None, excl_ids=None, targets=None, device=None):
@@ -1089,42 +1101,16 @@ def audience_scores(scores, k, users=None, exclude=None, excl_ids=None, targets=
             raise ValueError("users must hold {} strictly ascending ids".format(U))
         pool = torch.from_numpy(h.astype(np.int32)).to(device)
     ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
-    t = as_device_i32(targets, device) if targets is not None else None
-    rowptr, excl, excl_rows = _audience_exclusion(exclude, device)
-    top_users = torch.empty((M, k), dtype=torch.int32, device=device)
-    top_scores = torch.empty((M, k), dtype=torch.float32, device=device)
-    pos = torch.empty(M, dtype=torch.int32, device=device) if t is not None else None
-    sums = torch.zeros(2, dtype=torch.float32, device=device) if t is not None else None
-    nbytes = int(nat.lib.mr_audience_scores_workspace_bytes(U, M, k))
-    if nbytes == 0:
-        raise ValueError("audience_scores: bad sizes U={} M={} k={}".format(U, M, k))
+    t = _targets(targets, M, "columns", device)
+    rowptr, excl, excl_rows = _exclusion(exclude, device)
+    top_users, top_scores, pos, sums = _selection_outputs(M, k, t, device)
+    nbytes = _workspace_bytes(nat.lib.mr_audience_scores_workspace_bytes(U, M, k), "audience_scores", U=U, M=M, k=k)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
     st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
     nat.check(nat.lib.mr_audience_scores(_ptr(s), U, M, k, _ptr(pool), _ptr(ids), excl_rows, _ptr(rowptr), _ptr(excl),
                                          _ptr(t), _ptr(top_users), _ptr(top_scores), _ptr(pos), _ptr(sums), _ptr(ws),
                                          nbytes, st), "mr_audience_scores")
     return top_users, top_scores, pos, sums
-
-
-def _check_lists(lists, U, device):
-    """(rowptr, items) host or device -> device (int64 rowptr, int32 items); ValueError unless rowptr has U + 1 entries,
-    starts at 0, never decreases and ends at len(items)."""
-    rp, it = lists
-    items = as_device_i32(it, device)
-    nnz = items.numel()
-    if isinstance(rp, torch.Tensor) and rp.is_cuda:
-        rowptr = rp.reshape(-1).to(device, torch.int64).contiguous()
-        n = rowptr.numel()
-        ok = n == U + 1 and (n == 0 or bool(((rowptr[0] == 0) & (rowptr[-1] == nnz) &
-                                             ~(rowptr[1:] < rowptr[:-1]).any()).item()))
-    else:
-        h = (rp.numpy() if isinstance(rp, torch.Tensor) else np.asarray(rp)).reshape(-1).astype(np.int64)
-        ok = h.size == U + 1 and h[0] == 0 and h[-1] == nnz and bool(np.all(h[1:] >= h[:-1]))
-        rowptr = torch.from_numpy(np.ascontiguousarray(h)).to(device)
-    if not ok:
-        raise ValueError("lists: rowptr must have U + 1 = {} entries, start at 0, never decrease and end at len(items) = "
-                         "{}".format(U + 1, nnz))
-    return rowptr, items
 
 
 def topk_lists(scores, rowptr, k, targets=None, device=None):
@@ -1137,19 +1123,12 @@ def topk_lists(scores, rowptr, k, targets=None, device=None):
     s = as_device_f32(scores, device)
     n = (rowptr.numel() if isinstance(rowptr, torch.Tensor) else np.asarray(rowptr).size)
     U = max(int(n) - 1, 0)
-    rp, _ = _check_lists((rowptr, np.zeros(s.numel(), np.int32)), U, device)
+    rp, _ = check_csr(rowptr, np.zeros(s.numel(), np.int32), "lists", rows=U, device=device)
     nnz = s.numel()
     k = int(k)
-    t = as_device_i32(targets, device) if targets is not None else None
-    if t is not None and t.numel() != U:
-        raise ValueError("targets ({}) and lists ({}) differ in length".format(t.numel(), U))
-    top_pos = torch.empty((U, k), dtype=torch.int32, device=device)
-    top_scores = torch.empty((U, k), dtype=torch.float32, device=device)
-    pos = torch.empty(U, dtype=torch.int32, device=device) if t is not None else None
-    sums = torch.zeros(2, dtype=torch.float32, device=device) if t is not None else None
-    nbytes = int(nat.lib.mr_topk_lists_workspace_bytes(U, nnz, k))
-    if nbytes == 0:
-        raise ValueError("topk_lists: bad sizes U={} nnz={} k={}".format(U, nnz, k))
+    t = _targets(targets, U, "lists", device)
+    top_pos, top_scores, pos, sums = _selection_outputs(U, k, t, device)
+    nbytes = _workspace_bytes(nat.lib.mr_topk_lists_workspace_bytes(U, nnz, k), "topk_lists", U=U, nnz=nnz, k=k)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
     st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
     nat.check(nat.lib.mr_topk_lists(_ptr(s), U, _ptr(rp), nnz, k, _ptr(t), _ptr(top_pos), _ptr(top_scores), _ptr(pos),
@@ -1165,19 +1144,6 @@ def _cutoffs(ks):
     return (C.c_int32 * len(ks))(*ks), len(ks)
 
 
-def _exclusion_on_device(exclude, device):
-    """None | (rowptr, items) host or device -> (device rowptr int64 or None, device items int32 or None, rows)."""
-    if exclude is None:
-        return None, None, 0
-    rp, it = exclude
-    rowptr = (rp if isinstance(rp, torch.Tensor) else torch.from_numpy(np.asarray(rp, dtype=np.int64)))
-    rowptr = rowptr.reshape(-1).to(device, torch.int64).contiguous()
-    items = as_device_i32(it, device)
-    if items.numel() == 0:  # every list empty: the library still wants a pointer
-        items = torch.zeros(1, dtype=torch.int32, device=device)
-    return rowptr, items, max(rowptr.numel() - 1, 0)
-
-
 def targets_scores(scores, targets, ks, exclude=None, excl_ids=None, device=None):
     """Positions of many targets per row of a (U, N) score matrix (mr_targets_scores): row u's ascending targets are
     items[rowptr[u]:rowptr[u + 1]] of targets = (rowptr, items); candidates are the items not on the row's exclusion
@@ -1191,16 +1157,14 @@ def targets_scores(scores, targets, ks, exclude=None, excl_ids=None, device=None
         raise ValueError("scores must be (U, N), got shape {}".format(tuple(s.shape)))
     U, N = int(s.shape[0]), int(s.shape[1])
     s = s.to(device, torch.float32).contiguous()
-    rowptr, items = _check_lists(targets, U, device)
+    rowptr, items = check_csr(*targets, "lists", rows=U, device=device)
     nnz = items.numel()
     kbuf, n_ks = _cutoffs(ks)
     ids = as_device_i32(excl_ids, device) if excl_ids is not None else None
-    excl_rowptr, excl_items, excl_rows = _exclusion_on_device(exclude, device)
+    excl_rowptr, excl_items, excl_rows = _exclusion(exclude, device)
     tpos = torch.empty(nnz, dtype=torch.int32, device=device)
     sums = torch.zeros(nat.TGT_CUTOFF0 + nat.TGT_PER_CUTOFF * n_ks, dtype=torch.float32, device=device)
-    nbytes = int(nat.lib.mr_targets_scores_workspace_bytes(U, N, nnz))
-    if nbytes == 0:
-        raise ValueError("targets_scores: bad sizes U={} N={} nnz={}".format(U, N, nnz))
+    nbytes = _workspace_bytes(nat.lib.mr_targets_scores_workspace_bytes(U, N, nnz), "targets_scores", U=U, N=N, nnz=nnz)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=device)
     st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
     nat.check(nat.lib.mr_targets_scores(_ptr(s), U, N, _ptr(ids), excl_rows, _ptr(excl_rowptr), _ptr(excl_items),

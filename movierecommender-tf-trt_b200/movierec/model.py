@@ -774,14 +774,8 @@ class MovierecModel(object):
             rp, it = test
             rowptr = np.asarray(rp.cpu() if hasattr(rp, "cpu") else rp, dtype=np.int64).reshape(-1)
             items = np.asarray(it.cpu() if hasattr(it, "cpu") else it, dtype=np.int64).reshape(-1)
-            if rowptr.size < 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
-                raise ValueError("test lists: offsets must start at 0, never decrease and end at {}".format(items.size))
+            rowptr, items = (t.numpy() for t in _engine_module().check_csr(rowptr, items, "test lists", ascending=True))
             self.model._raise_on_bad_ids(_ids_outside(items, ni) or bool(np.any(rowptr[nu + 1:] > rowptr[nu])))
-            inner = np.ones(max(items.size - 1, 0), bool)
-            inner[rowptr[1:-1][(rowptr[1:-1] > 0) & (rowptr[1:-1] < items.size)] - 1] = False
-            if np.any((items[1:] <= items[:-1]) & inner):
-                raise ValueError("test lists: every user's items must be strictly ascending")
-            items = items.astype(np.int32)
         users = np.flatnonzero(rowptr[1:] > rowptr[:-1]).astype(np.int32)
         total = np.zeros(2 + 5 * len(ks), np.float64)  # [users, mrr] + 5 per cutoff: MR_TGT_* of movierec_b200.h
         if users.size:
@@ -878,10 +872,8 @@ def _candidate_csr(candidate_lists, U):
         rowptr = np.zeros(len(parts) + 1, np.int64)
         rowptr[1:] = np.cumsum([p.size for p in parts])
         items = np.concatenate(parts) if parts else np.zeros(0, np.int32)
-    if rowptr.size != U + 1 or rowptr[0] != 0 or rowptr[-1] != items.size or np.any(rowptr[1:] < rowptr[:-1]):
-        raise ValueError("candidate lists: expected {} lists with offsets starting at 0, never decreasing and ending at "
-                         "{}".format(U, items.size))
-    return rowptr, items
+    rowptr, items = _engine_module().check_csr(rowptr, items, "candidate lists", rows=U)
+    return rowptr.numpy(), items.numpy()
 
 
 def _ids_outside(ids, limit):
@@ -901,24 +893,20 @@ def _list_chunks(rowptr, max_rows=None):
     return out or [(0, 0)]
 
 
-def _exclusion_lists(exclude):
-    """None | MovieLensDataGenerator | (rowptr, items) -> None | (rowptr, items)."""
+def _exclusion_lists(exclude, lists="user_item_lists"):
+    """None | MovieLensDataGenerator | (rowptr, ids) -> None | (rowptr, ids).  A generator gives its method `lists`:
+    user_item_lists (items by user id) or item_user_lists (users by item id)."""
     if exclude is None:
         return None
-    if hasattr(exclude, "user_item_lists"):
-        return exclude.user_item_lists()
-    rowptr, items = exclude
-    return rowptr, items
+    if hasattr(exclude, lists):
+        return getattr(exclude, lists)()
+    rowptr, ids = exclude
+    return rowptr, ids
 
 
 def _audience_lists(exclude):
-    """None | MovieLensDataGenerator | (rowptr, users) -> None | (rowptr, users), lists by item id."""
-    if exclude is None:
-        return None
-    if hasattr(exclude, "item_user_lists"):
-        return exclude.item_user_lists()
-    rowptr, users = exclude
-    return rowptr, users
+    """_exclusion_lists for audiences: lists by item id."""
+    return _exclusion_lists(exclude, "item_user_lists")
 
 
 class RankLayer(object):

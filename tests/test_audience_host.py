@@ -132,3 +132,30 @@ def test_pool_and_exclusion_handling():
                         ([0, 3], [1, 3, 2]), ([0, 2], [4, 4])):
         with pytest.raises(ValueError):
             _engine.check_exclusion_csr(np.int64(rowptr), np.int32(ids))
+
+
+def test_check_csr_refuses_each_malformed_case():
+    ok = (np.int64([0, 2, 2, 5]), np.int32([1, 4, 0, 3, 9]))
+    rp, it = _engine.check_csr(*ok, "lists", rows=3, ascending=True, limit=10)
+    assert rp.tolist() == [0, 2, 2, 5] and it.tolist() == [1, 4, 0, 3, 9] and str(it.dtype) == "torch.int32"
+    cases = [  # (rowptr, ids, flags, error): the rule each case breaks, under the flag that asks for it
+        ([], [], {}, ValueError),  # no offsets at all
+        ([1, 2], [3, 4], {}, ValueError),  # does not start at 0
+        ([0, 2, 1, 3], [1, 2, 3], {}, ValueError),  # decreases
+        ([0, 1], [1, 2], {}, ValueError),  # ends before len(ids)
+        ([0, 3], [1, 2], {}, ValueError),  # ends past len(ids): a kernel would read past the ids
+        ([0, 2, 5], [1, 4, 0, 3, 9], dict(rows=3), ValueError),  # wrong row count
+        ([0, 2, 5], [1, 4, 0, 3, 9], dict(rows=1), ValueError),
+        ([0, 3], [1, 3, 2], dict(ascending=True), ValueError),  # not ascending
+        ([0, 2], [4, 4], dict(ascending=True), ValueError),  # not strictly ascending
+        ([0, 2], [1, 10], dict(limit=10), IndexError),  # id >= limit
+        ([0, 2], [-1, 3], dict(limit=10), IndexError),  # id < 0
+    ]
+    for rowptr, ids, flags, error in cases:
+        with pytest.raises(error):
+            _engine.check_csr(np.int64(rowptr), np.int32(ids), "lists", **flags)
+    # without their flags, the last four cases pass: lists need not be sorted or in range unless asked
+    for rowptr, ids, flags, _ in cases[-4:]:
+        _engine.check_csr(np.int64(rowptr), np.int32(ids), "lists")
+    # a list may end where the next starts with a smaller id
+    _engine.check_csr(np.int64([0, 2, 4]), np.int32([3, 7, 1, 2]), "lists", ascending=True)

@@ -240,3 +240,19 @@ def test_out_of_range_ids_raise(eng_mod, tmp_path):
     items, scores, pos, _, _ = m.model.engine.catalogue_topk([nu, 1], 5, targets=[2, -1])
     assert (items.cpu().numpy()[0] == -1).all() and np.isnan(scores.cpu().numpy()[0]).all()
     assert pos.cpu().numpy().tolist() == [ni, ni]
+
+
+def test_malformed_exclusion_lists_raise_before_any_launch(eng_mod):
+    eng = _engine(eng_mod, [64, 32, 16, 8], 8, 6, 40)
+    scores = torch.rand((6, 40), device="cuda")
+    users = np.arange(6, dtype=np.int32)
+    targets = (np.int64([0, 1, 1, 1, 2, 2, 2]), np.int32([3, 5]))
+    # an unsorted list, and rowptr[-1] < len(items): neither can make a kernel leave its arrays
+    for bad in ((np.int64([0, 2, 2, 2, 2, 2, 2]), np.int32([7, 3])),
+                (np.int64([0, 1, 1, 1, 1, 1, 1]), np.int32([3, 7]))):
+        for call in (lambda: eng.catalogue_topk(users, 5, exclude=bad),
+                     lambda: eng_mod.topk_scores(scores, 5, exclude=bad),
+                     lambda: eng.catalogue_targets(users, targets, [5], exclude=bad),
+                     lambda: eng_mod.targets_scores(scores, targets, [5], exclude=bad)):
+            with pytest.raises(ValueError, match="exclusion lists"):
+                call()
